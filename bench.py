@@ -3,6 +3,7 @@
 "perturbed shader fwd+bwd pixel·face·samples/sec; % HBM roofline; 1/2/4/8 GPU").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--fragments rasterised|realistic|dense] [--impl reference]
+                    [--dump-outputs DIR]
 
 A step is one fused forward + one fused backward of the shader over one batch of fragments at BASELINE config 2 per GPU
 (8 views, 256x256, K=50, nb_samples=64; weak scaling: every rank shades its own 8 views, the only collective on the path
@@ -26,6 +27,8 @@ import types
 
 import torch
 
+# the benchmark writes nothing into the source tree (which may be read-only), bytecode caches included
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -34,7 +37,7 @@ METRIC = "perturbed shader fwd+bwd pixel·face·samples/sec"
 UNIT = "pixel·face·samples/s"
 SIGMA, GAMMA, ALPHA, EPS = 1e-3, 1e-2, 1.0, 1e-10  # experiments/eval.py:69 defaults (SURVEY.md §8d)
 BACKGROUND = (1.0, 1.0, 1.0)
-REPEATS = 5  # the headline is the median of this many repeats of the requested steps
+DUMP_BYTES = 60_000_000  # --dump-outputs writes at most this much (under 64 MB with the .npy headers)
 
 # BASELINE.json configs (per-GPU shapes; SURVEY.md §8 table).  Config 3 is 64 poses sharded by batch over 8 GPUs: 8 per GPU.
 CONFIGS = {
@@ -84,7 +87,13 @@ def parse_args():
     ap.add_argument("--no-renderer-legs", action="store_true", help="skip the Phong / renderer legs of `also`")
     ap.add_argument("--no-config-legs", action="store_true", help="skip BASELINE configs 1, 3, 4, 5 in `also`")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32; a fixed sample of pixels "
+                         "when the whole would exceed 60 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -342,18 +351,36 @@ def workload_config(args, world):
         "views_per_gpu": args.views, "global_views": args.views * world,
         "image_size": args.image_size, "faces_per_pixel": args.faces_per_pixel, "nb_samples": args.nb_samples,
         "sigma": SIGMA, "gamma": GAMMA, "alpha": ALPHA, "flags": 0, "parallelism": f"batch-shard x{world}",
-        "timing": f"median of {REPEATS} repeats of the requested steps, each repeat bracketed by barrier + synchronize, "
-                  "max over ranks per repeat",
+        "timing": "one device-timed window of the requested steps, bracketed by barrier + synchronize, max over ranks",
         "l2": f"inputs ({inputs_gb:.2f} GB per step) exceed the 126 MB L2; no explicit flush",
     }
+
+
+def dump_outputs(dirname, outputs):
+    """Writes what one step hands its caller, (image, grad_dists, grad_zbuf, grad_colors, grad_scalars), as
+    <dirname>/<name>.npy in float32, so that two builds run with the same arguments can be compared entry by entry.  The
+    per-pixel arrays are flattened to (pixels, ...); when together they exceed DUMP_BYTES, every one of them keeps the same
+    fixed sample of pixels (seed 0, ascending pixel order)."""
+    import numpy as np
+    image = outputs[0]
+    P = image.shape[0] * image.shape[1] * image.shape[2]
+    per_pixel = {name: t.reshape((P,) + t.shape[3:])
+                 for name, t in zip(("image", "grad_dists", "grad_zbuf", "grad_colors"), outputs[:4])}
+    n = min(P, DUMP_BYTES // sum(4 * t[0].numel() for t in per_pixel.values()))
+    pix = torch.randperm(P, generator=torch.Generator().manual_seed(0))[:n].sort().values.to(image.device)
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in per_pixel.items():
+        np.save(os.path.join(dirname, name + ".npy"), t[pix].float().cpu().numpy())
+    np.save(os.path.join(dirname, "grad_scalars.npy"), outputs[4].float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
 # B200 arm
 # ------------------------------------------------------------------------------------------------
-def device_timed(cfg, kind, dev, steps, warmup, world, rank, sampler=None, flags=0, face=False, soft=False, repeats=1,
-                 fragments=None):
-    """Inputs resident in HBM; `repeats` x K steps of pert_shade_fwd + pert_shade_bwd through the C ABI."""
+def device_timed(cfg, kind, dev, steps, warmup, world, rank, sampler=None, flags=0, face=False, soft=False,
+                 fragments=None, dump_dir=None):
+    """Inputs resident in HBM; K timed steps of pert_shade_fwd + pert_shade_bwd through the C ABI.  With `dump_dir`,
+    rank 0 writes what the last timed step returned there (dump_outputs)."""
     import torch.distributed as dist
     from pertrenderer_b200 import ops
     N, HW, K, S = cfg["N"], cfg["HW"], cfg["K"], cfg["S"]
@@ -377,7 +404,7 @@ def device_timed(cfg, kind, dev, steps, warmup, world, rank, sampler=None, flags
                                 S_rast=S, S_agg=S, seed_rast=ops.draw_seed(), seed_agg=ops.draw_seed(),
                                 pixel_offset=rank * P, flags=flags)
 
-    ev = [[[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(steps)] for _ in range(repeats)]
+    ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(steps)]
     comm = torch.cuda.Stream(device=dev) if world > 1 else None
 
     def step(e=None):
@@ -404,7 +431,7 @@ def device_timed(cfg, kind, dev, steps, warmup, world, rank, sampler=None, flags
             with torch.cuda.stream(comm):
                 scal.record_stream(comm)
                 dist.all_reduce(scal)
-        return image, scal
+        return image, gd, gz, gc, scal
 
     for _ in range(warmup):
         step()
@@ -413,34 +440,34 @@ def device_timed(cfg, kind, dev, steps, warmup, world, rank, sampler=None, flags
     mem_base = torch.cuda.memory_allocated(dev)
     if sampler is not None:
         sampler.start()
-    totals = []
-    for r in range(repeats):
-        if world > 1:
-            dist.barrier()
-        torch.cuda.synchronize(dev)
-        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        t0.record()
-        for i in range(steps):
-            step(ev[r][i])
-        if world > 1:
-            torch.cuda.current_stream(dev).wait_stream(comm)
-        t1.record()
-        torch.cuda.synchronize(dev)
-        if world > 1:
-            dist.barrier()
-        torch.cuda.synchronize(dev)
-        ms = t0.elapsed_time(t1)
-        if world > 1:
-            t = torch.tensor([ms], device=dev)
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            ms = t.item()
-        totals.append(ms)
+    if world > 1:
+        dist.barrier()
+    torch.cuda.synchronize(dev)
+    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    t0.record()
+    for i in range(steps):
+        if i == steps - 1:
+            outputs = step(ev[i])
+        else:
+            step(ev[i])
+    if world > 1:
+        torch.cuda.current_stream(dev).wait_stream(comm)
+    t1.record()
+    torch.cuda.synchronize(dev)
+    if world > 1:
+        dist.barrier()
+    torch.cuda.synchronize(dev)
+    total_ms = t0.elapsed_time(t1)
+    if world > 1:
+        t = torch.tensor([total_ms], device=dev)
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        total_ms = t.item()
     peak_mem = int(torch.cuda.max_memory_allocated(dev) - mem_base)
-    order = sorted(range(repeats), key=lambda r: totals[r])
-    rmed = order[repeats // 2]
-    total_ms = totals[rmed]
-    fwd_ms = sum(e[0].elapsed_time(e[1]) for e in ev[rmed]) / steps
-    bwd_ms = sum(e[1].elapsed_time(e[2]) for e in ev[rmed]) / steps
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, outputs)
+    del outputs
+    fwd_ms = sum(e[0].elapsed_time(e[1]) for e in ev) / steps
+    bwd_ms = sum(e[1].elapsed_time(e[2]) for e in ev) / steps
     units = P * K * S
     fb, bb = alg_bytes(P, K)
     fmin, bmin = min_bytes(P, K, V)
@@ -462,7 +489,7 @@ def device_timed(cfg, kind, dev, steps, warmup, world, rank, sampler=None, flags
             "min_bytes": {"fwd": fmin, "bwd": bmin, "fwd_bwd_frac": (fmin + bmin) / (fwd_ms + bwd_ms) / 1e6 / peak,
                           "valid_entries": V, "valid_fraction": V / (P * K)}}
     return {"value": units * world * steps / (total_ms * 1e-3), "ms_per_step": total_ms / steps, "roofline": roof,
-            "repeat_ms_per_step": [t / steps for t in totals], "peak_memory_bytes": peak_mem,
+            "peak_memory_bytes": peak_mem,
             # kernels of libpertshade.so per step: forward main + fallback pass (two launches: coverage samples,
             # aggregation + blend), backward main + fallback pass, scalar-gradient finalize
             "launches": 6 * steps}
@@ -913,7 +940,7 @@ def run_b200_arm(args):
         dist.init_process_group("nccl", device_id=dev)
     cfg = dict(N=args.views, HW=args.image_size, K=args.faces_per_pixel, S=args.nb_samples)
     sampler = ClockSampler(local) if rank == 0 else None
-    main = device_timed(cfg, args.fragments, dev, args.steps, args.warmup, world, rank, sampler, repeats=REPEATS)
+    main = device_timed(cfg, args.fragments, dev, args.steps, args.warmup, world, rank, sampler, dump_dir=args.dump_outputs)
     clocks = sampler.finish() if sampler is not None else None
     also = None
     if not args.no_also:
@@ -992,8 +1019,7 @@ def run_b200_arm(args):
         "warmup": args.warmup, "ms_per_step": main["ms_per_step"], "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": workload_config(args, world),
         "clocks": clocks, "e2e": e2e, "gpu_launches": main["launches"], "roofline": main["roofline"],
-        "cpu_baseline": cpu, "repeat_ms_per_step": main["repeat_ms_per_step"],
-        "peak_memory_bytes": main["peak_memory_bytes"], "also": also,
+        "cpu_baseline": cpu, "peak_memory_bytes": main["peak_memory_bytes"], "also": also,
     }
     emit(line)
 
