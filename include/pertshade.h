@@ -55,7 +55,7 @@
 extern "C" {
 #endif
 
-#define PERT_ABI_VERSION 14
+#define PERT_ABI_VERSION 15
 
 /* error codes */
 #define PERT_OK 0
@@ -82,8 +82,13 @@ extern "C" {
  *     for the squared term): same expectation, lower variance. */
 #define PERT_F_SKIP_DEAD_NOISE 2u
 #define PERT_F_PER_SAMPLE_NOISE 4u
-/* stand-alone operators only: standard Cauchy noise instead of Gaussian (ArctanRast smoothrast.py:162-173,
- * CauchyAgg smoothagg.py:230-250): noise tan(pi(u-1/2)) clamped to +-1e7, score 2n/(1+n^2) in backward */
+/* standard Cauchy noise instead of Gaussian (ArctanRast smoothrast.py:162-173, CauchyAgg smoothagg.py:230-250): noise
+ * tan(pi(u-1/2)) clamped to +-1e7, score 2n/(1+n^2) in backward.  Stand-alone operators, and pert_shade_fwd /
+ * pert_shade_bwd with in-kernel or explicit noise, in one call or phase-split: there every valid entry draws all its
+ * coverage samples, every finite logit takes part in the argmax and backward regenerates every V_sj of every logit
+ * (the pert_noise_fill tensor of stage | 2 is the in-kernel stream).  The fused entry points return
+ * PERT_E_UNSUPPORTED for PERT_F_CAUCHY with PERT_F_PHILOX7, PERT_F_NO_VR, PERT_F_SKIP_DEAD_NOISE, PERT_F_UNIFORM or
+ * PERT_F_GUMBEL. */
 #define PERT_F_CAUCHY 8u
 /* stand-alone operators only, Gaussian noise: the estimators WITHOUT the control variates, the paper's ablation
  * (randomHeaviside_wovr smoothrast.py:61-108: sum_s h_s U_s instead of sum_s (h_s - h0) U_s;

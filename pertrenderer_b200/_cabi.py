@@ -15,7 +15,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpertshade.so")
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 # flags (include/pertshade.h)
 F_NO_SKIP = 1

@@ -125,6 +125,7 @@ struct PhiloxCauchy {
             n[t] = fminf(fmaxf(__fdividef(mufu_sin(a), mufu_cos(a)), -1e7f), 1e7f);
         }
     }
+    __device__ __forceinline__ void mix(uint64_t v) { base.mix(v); }
     static constexpr bool kBounded = false;
 };
 
@@ -160,6 +161,8 @@ struct PhiloxGumbel {
 
 // score of the noise density used by the gradient estimators: -d/dn log p(n)
 //   Gaussian: n   (smoothrast.py:46, smoothagg.py:51-53)     Cauchy: 2n / (1 + n^2)   (smoothrast.py:49, smoothagg.py:58-59)
+// SCORE = 0 / 1 is a compile-time parameter of the kernels, separate from the noise source: explicit noise works with
+// either law
 template <int SCORE>
 __device__ __forceinline__ float noise_score(float n) {
     return SCORE == 0 ? n : __fdividef(2.0f * n, 1.0f + n * n);

@@ -53,7 +53,9 @@ void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes,
 // and every array holds a.L.cap valid entries; tiles with more go to the fallback pass.
 // BLOB = true (only with COMPACT): the compact valid list and the per-pixel logit summary come from the tile
 // blob forward saved (common.cuh) instead of a re-scan of pix_to_face and a recomputation of the logits.
-template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB>
+// SCORE = the score psi of the aggregation noise (philox.cuh noise_score): acc_j = sum_s c_s psi(V_sj) and
+// t2_j = sum_s c_s V_sj psi(V_sj); 0 Gaussian (psi(n) = n), 1 Cauchy.
+template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0>
 __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& noise_a, const int64_t tile,
                                                const int64_t prow /* row of the scalar partials */,
                                                unsigned char* smem_raw, const int lane) {
@@ -65,8 +67,9 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
     const bool do_sample = !PHASED || (flags & PERT_PH_BWD_SAMPLE), do_finish = !PHASED || (flags & PERT_PH_BWD_FINISH);
     const int32_t* const ghist = PHASED ? a.hist : nullptr;
     const bool no_skip = flags & PERT_F_NO_SKIP;
-    // how the noise of logits that can never win (zero-mean, independent of everything) is handled
-    const bool per_sample = !NoiseA::kBounded || no_skip || (flags & PERT_F_PER_SAMPLE_NOISE);
+    // how the noise of logits that can never win (zero-mean, independent of everything) is handled; the one-draw
+    // shortcut rests on sum_s c_s V_sj being normal, which holds for the Gaussian score only
+    const bool per_sample = SCORE != 0 || !NoiseA::kBounded || no_skip || (flags & PERT_F_PER_SAMPLE_NOISE);
     const bool drop_dead = !per_sample && (flags & PERT_F_SKIP_DEAD_NOISE);
     float p_sigma = 0.f, p_gamma = 0.f, p_q = 0.f;
 
@@ -422,7 +425,8 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                             if (!no_skip && c4.x == 0.f && c4.y == 0.f && c4.z == 0.f && c4.w == 0.f) continue;
                             float nz[4];
                             noise_a.get4(qb + (c0 >> 2) + ql, j, pix0 + pp, nz);
-                            const float cv0 = c4.x * nz[0], cv1 = c4.y * nz[1], cv2 = c4.z * nz[2], cv3 = c4.w * nz[3];
+                            const float cv0 = c4.x * noise_score<SCORE>(nz[0]), cv1 = c4.y * noise_score<SCORE>(nz[1]),
+                                        cv2 = c4.z * noise_score<SCORE>(nz[2]), cv3 = c4.w * noise_score<SCORE>(nz[3]);
                             acc += (cv0 + cv1) + (cv2 + cv3);
                             t2 += (cv0 * nz[0] + cv1 * nz[1]) + (cv2 * nz[2] + cv3 * nz[3]);
                         }
@@ -608,12 +612,12 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
 #ifndef BWD_MAIN_CTAS
 #define BWD_MAIN_CTAS 28
 #endif
-template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB>
+template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0>
 __global__ void __launch_bounds__(FNT, BWD_MAIN_CTAS) shade_bwd_kernel(const BwdArgs a, const NoiseA noise_a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     NoiseA na = noise_a;
     if (a.pb.seed_device) na.mix(__ldg(a.pb.seed_device + 1));  // device-side seed, see shade_fwd.cu
-    shade_bwd_tile<NoiseA, GT, PHASED, FACE, COMPACT, BLOB>(a, na, blockIdx.x, blockIdx.x, smem_raw, threadIdx.x);
+    shade_bwd_tile<NoiseA, GT, PHASED, FACE, COMPACT, BLOB, SCORE>(a, na, blockIdx.x, blockIdx.x, smem_raw, threadIdx.x);
 }
 
 // Fallback pass of the sparse-first mode (see shade_fwd.cu): work-list tiles as half-size tiles with dense
@@ -702,17 +706,17 @@ static int set_smem(K kern, size_t smem) {
     return 0;
 }
 
-template <class NA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB = false>
+template <class NA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB = false, int SCORE = 0>
 static int launch_bwd_f(const BwdArgs& a, const NA& na, cudaStream_t st) {
     const size_t smem = (size_t)a.L.warp_smem;
-    if (int rc = set_smem(shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB>, smem)) return rc;
-    shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, na);
+    if (int rc = set_smem(shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE>, smem)) return rc;
+    shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, na);
     return (int)cudaGetLastError();
 }
-template <class NA, int GT, bool PHASED>
+template <class NA, int GT, bool PHASED, int SCORE = 0>
 static int launch_bwd_t(const BwdArgs& a, const NA& na, cudaStream_t st) {
-    return a.pb.face_colors ? launch_bwd_f<NA, GT, PHASED, true, false>(a, na, st)
-                            : launch_bwd_f<NA, GT, PHASED, false, false>(a, na, st);
+    return a.pb.face_colors ? launch_bwd_f<NA, GT, PHASED, true, false, false, SCORE>(a, na, st)
+                            : launch_bwd_f<NA, GT, PHASED, false, false, false, SCORE>(a, na, st);
 }
 // sparse-first main pass (compact per-logit arrays); PN = the Philox variant
 template <class PN, int GT>
@@ -770,7 +774,14 @@ int launch_shade_bwd(const BwdArgs& a, const BwdArgs* fb, float* grad_scalars, c
     int rc;
     const uint32_t both = PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH;
     const bool phased = (a.pb.flags & both) != both || a.hist != nullptr;
-    if (a.pb.noise_agg) {
+    if (a.pb.flags & PERT_F_CAUCHY) {  // Cauchy pair: the dense phase-capable instantiation, as forward (shade_fwd.cu)
+        if (a.pb.noise_agg) {
+            ExplicitNoise xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
+            rc = launch_bwd_t<ExplicitNoise, 0, true, 1>(a, xa, st);
+        } else {
+            rc = launch_bwd_t<PhiloxCauchy, 0, true, 1>(a, PhiloxCauchy(a.pb.seed_agg, 1, a.pb.pixel_offset), st);
+        }
+    } else if (a.pb.noise_agg) {
         ExplicitNoise xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
         rc = launch_bwd_t<ExplicitNoise, 0, true>(a, xa, st);
     } else if (phased) {  // sample-sharded job: compile-time lanes per pixel for the benchmark geometries

@@ -133,10 +133,10 @@ __device__ __forceinline__ void pixel_ranges(const uint16_t* vlist, int nv, int 
 // ------------------------------------------------------------------------------------------------
 // stage 1: coverage samples of the listed entries
 //   randomras/smoothrast.py:32-36: h = 1[x + sigma*U >= 0] (rounded multiply, rounded add), mean over s
-//   saved for backward: cnt = sum_s h, rs = sum_s (h - h0) U   (smoothrast.py:46)
+//   saved for backward: cnt = sum_s h, rs = sum_s (h - h0) psi(U)   (smoothrast.py:46,49; psi = noise_score<SCORE>)
 // rlist holds compact indices n; xs/cnt/rs are compact arrays.
 // ------------------------------------------------------------------------------------------------
-template <class NoiseT>
+template <class NoiseT, int SCORE = 0>
 __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint16_t* rlist, int nlist,
                                                  const uint16_t* vlist, const float* xs, uint16_t* cnt, float* rs,
                                                  int K, float invK, int64_t pix0, float sigma, float inv_sigma,
@@ -204,7 +204,7 @@ __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint
                         const bool h = __fadd_rn(x, __fmul_rn(sigma, nz[t])) >= 0.0f;
                         if (s >= s_begin && s < s_end) {
                             c += h ? 1 : 0;
-                            if (h != h0) r += h ? nz[t] : -nz[t];
+                            if (h != h0) r += h ? noise_score<SCORE>(nz[t]) : -noise_score<SCORE>(nz[t]);
                         }
                     }
                 }

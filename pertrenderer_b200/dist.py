@@ -216,13 +216,13 @@ def smooth_rgb_blend_sample_sharded(colors, fragments, smoothrast, smoothagg, bl
     gradients).  ``sync_seeds=True`` makes rank 0's torch generator drive the noise of every rank, which
     reproduces the single-GPU sample path exactly (one broadcast + host read per call); by default each
     rank seeds its own disjoint sample shard from its own generator."""
-    from .random_rasterizer import _background_tuple
-    from .smoothagg import GaussianAgg
-    from .smoothrast import GaussianRast
-    if not (isinstance(smoothrast, GaussianRast) and isinstance(smoothagg, GaussianAgg)):
-        raise ValueError("sample sharding is implemented for the (GaussianRast, GaussianAgg) pair")
+    from .random_rasterizer import _background_tuple, _perturbed_pair_flags
+    flags = _perturbed_pair_flags(smoothrast, smoothagg)
+    if flags is None:
+        raise ValueError("sample sharding is implemented for the (GaussianRast, GaussianAgg) and (ArctanRast, CauchyAgg) pairs")
     cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps, S_rast=smoothrast.nb_samples,
-               S_agg=smoothagg.nb_samples, fixed_noise=bool(smoothagg.fixed_noise), group=group, sync_seeds=sync_seeds)
+               S_agg=smoothagg.nb_samples, fixed_noise=bool(smoothagg.fixed_noise), group=group, sync_seeds=sync_seeds,
+               flags=flags)
     return _SampleShardedShade.apply(colors, fragments.dists, fragments.zbuf, smoothrast.sigma, smoothagg.gamma,
                                      smoothagg.alpha, fragments.pix_to_face, znear, zfar, cfg)
 

@@ -85,7 +85,8 @@ def refuse_device_seeds(op: str):
     replay the same noise for ever.  Fail loudly instead."""
     if current_seed_device() is not None:
         raise RuntimeError(f"{op}: device-side seeds (ops.device_seeds) are implemented for the fused operator pairs "
-                           "(GaussianRast + GaussianAgg, SoftRast + SoftAgg) only; run this pair outside the block")
+                           "(GaussianRast + GaussianAgg, ArctanRast + CauchyAgg, SoftRast + SoftAgg) only; run this pair "
+                           "outside the block")
 
 
 def _f32c(t):
@@ -265,11 +266,11 @@ def shade_forward(pr: ShadeProblem, want_hist: bool = False, phases: int = 0, sa
         if saved is None:
             # phase-split (sample-sharded) jobs all-reduce counts / rsum as whole tensors: define every entry
             alloc = torch.zeros if phases else torch.empty
-            # the tile blobs are written by the production path only (in-kernel noise, all phases in one call, no global
-            # histogram, default noise flags: csrc/cabi.cu sparse_first_ok); the buffer only exists then, so that a
+            # the tile blobs are written by the production path only (in-kernel Gaussian noise, all phases in one call, no
+            # global histogram, default noise flags: csrc/cabi.cu sparse_first_ok); the buffer only exists then, so that a
             # backward with other flags can never read what forward did not write
             prod = not phases and not want_hist and pr.noise_rast is None and pr.noise_agg is None and \
-                not (pr.flags & (F_NO_SKIP | F_PER_SAMPLE_NOISE))
+                not (pr.flags & (F_NO_SKIP | F_PER_SAMPLE_NOISE | F_CAUCHY))
             saved = ShadeSaved(
                 counts=alloc((N, H, W, K), dtype=torch.int16, device=dev),
                 rsum=alloc((N, H, W, K), dtype=torch.float32, device=dev),

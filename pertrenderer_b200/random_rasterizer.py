@@ -2,11 +2,11 @@
 
 ``smooth_rgb_blend`` (random_rasterizer.py:34-56) and ``RandomSimpleShader`` (:132-191) keep the
 reference's signatures, so ``MeshRenderer(rasterizer=..., shader=RandomSimpleShader(...))`` works
-unchanged.  With the (GaussianRast, GaussianAgg) pair the whole chain — coverage sampling, mask,
-alpha, logits, perturbed argmax, blend, and the score-function backward — is ONE forward and ONE
-backward sm_100a kernel (``pert_shade_fwd`` / ``pert_shade_bwd``).  Any other operator pair falls
-through to the operator-by-operator composition of the reference, where the Gaussian operators
-still run on their own CUDA kernels.
+unchanged.  With the (GaussianRast, GaussianAgg) pair and the Cauchy pair (ArctanRast, CauchyAgg) the
+whole chain — coverage sampling, mask, alpha, logits, perturbed argmax, blend, and the score-function
+backward — is ONE forward and ONE backward sm_100a kernel (``pert_shade_fwd`` / ``pert_shade_bwd``).
+Any other operator pair falls through to the operator-by-operator composition of the reference, where
+the perturbed operators still run on their own CUDA kernels.
 """
 
 from __future__ import annotations
@@ -16,8 +16,8 @@ import torch.nn as nn
 from torch.autograd import Function
 
 from . import ops
-from .smoothagg import GaussianAgg, SoftAgg  # noqa: F401
-from .smoothrast import GaussianRast, SoftRast
+from .smoothagg import CauchyAgg, GaussianAgg, SoftAgg  # noqa: F401
+from .smoothrast import ArctanRast, GaussianRast, SoftRast
 from .structures import BlendParams, FaceTexels, UVTexels, VertexTexels
 
 
@@ -32,7 +32,7 @@ def _background_tuple(blend_params):
 
 
 class _PerturbedShade(Function):
-    """Fused GaussianRast -> mask/alpha -> GaussianAgg -> blend.
+    """Fused GaussianRast -> mask/alpha -> GaussianAgg -> blend (``cfg["flags"]`` = F_CAUCHY: ArctanRast / CauchyAgg).
 
     Differentiable inputs: colors, dists, zbuf and the three 0-dim scalars sigma, gamma, alpha
     (CPU leaves in the reference: smoothrast.py:116, smoothagg.py:153-154).  Saved for backward:
@@ -111,6 +111,22 @@ class _SoftShade(Function):
                 out_scal[0], out_scal[1], out_scal[2], None, None, None, None)
 
 
+def _perturbed_pair_flags(smoothrast, smoothagg):
+    """PERT_F_* noise flags of the fused perturbed kernels for this operator pair: 0 for (GaussianRast, GaussianAgg),
+    F_CAUCHY for (ArctanRast, CauchyAgg); None for a pair without them."""
+    if isinstance(smoothrast, GaussianRast) and isinstance(smoothagg, GaussianAgg):
+        return 0
+    if isinstance(smoothrast, ArctanRast) and isinstance(smoothagg, CauchyAgg):
+        return ops.F_CAUCHY
+    return None
+
+
+def _fused_pair(smoothrast, smoothagg) -> bool:
+    """The pair runs on fused kernels, which read the colours of valid entries only."""
+    return _perturbed_pair_flags(smoothrast, smoothagg) is not None or \
+        (type(smoothrast) is SoftRast and type(smoothagg) is SoftAgg)
+
+
 def smooth_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, znear: float = 1.0,
                      zfar: float = 100) -> torch.Tensor:
     """random_rasterizer.py:34-56.  Returns the (N,H,W,4) RGBA image.
@@ -121,15 +137,14 @@ def smooth_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, zne
         # TexturesVertex / TexturesUV: interpolate the vertex colours with the texture-only mode of the Phong kernel; the fused
         # pairs read colours of valid entries only, so the padded ones need not be written
         from .shading import sample_lazy_textures
-        fused = (isinstance(smoothrast, GaussianRast) and isinstance(smoothagg, GaussianAgg)) or \
-            (type(smoothrast) is SoftRast and type(smoothagg) is SoftAgg)
-        colors = sample_lazy_textures(colors, fragments, sparse=fused)
+        colors = sample_lazy_textures(colors, fragments, sparse=_fused_pair(smoothrast, smoothagg))
     face = isinstance(colors, FaceTexels)
     ops.require_cuda(colors.face_colors if face else colors, fragments.pix_to_face, fragments.zbuf, fragments.dists)
-    if isinstance(smoothrast, GaussianRast) and isinstance(smoothagg, GaussianAgg):
+    flags = _perturbed_pair_flags(smoothrast, smoothagg)
+    if flags is not None:
         cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps,
                    S_rast=smoothrast.nb_samples, S_agg=smoothagg.nb_samples,
-                   fixed_noise=bool(smoothagg.fixed_noise), face_colors=face)
+                   fixed_noise=bool(smoothagg.fixed_noise), face_colors=face, flags=flags)
         return _PerturbedShade.apply(colors.face_colors if face else colors, fragments.dists, fragments.zbuf, smoothrast.sigma,
                                      smoothagg.gamma, smoothagg.alpha, fragments.pix_to_face, znear, zfar, cfg)
 
@@ -137,9 +152,14 @@ def smooth_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, zne
         cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps)
         return _SoftShade.apply(colors, fragments.dists, fragments.zbuf, smoothrast.sigma, smoothagg.gamma,
                                 smoothagg.alpha, fragments.pix_to_face, znear, zfar, cfg)
+    return _composed_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, znear, zfar)
 
-    # operator-by-operator composition for every other pair (e.g. GaussianRast + SoftAgg)
-    if face:
+
+def _composed_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, znear=1.0, zfar=100) -> torch.Tensor:
+    """random_rasterizer.py:44-56 operator by operator: every pair without fused kernels runs here (e.g. GaussianRast +
+    SoftAgg), and for a fused pair it draws the same seeds in the same order, hence the same noise, as the fused path.
+    ``colors`` is a (N,H,W,K,3) tensor or a ``FaceTexels``."""
+    if isinstance(colors, FaceTexels):
         colors = colors.materialize(fragments.pix_to_face)
     device = fragments.pix_to_face.device
     background = blend_params.background_color
@@ -294,10 +314,8 @@ class RandomPhongShader(RandomSimpleShader):
         materials = kwargs.get("materials", self.materials)
         blend_params = kwargs.get("blend_params", self.blend_params)
         # every consumer below reads colours of valid entries only when the blend is one of the fused pairs
-        fused = (isinstance(self.smoothrast, GaussianRast) and isinstance(self.smoothagg, GaussianAgg)) or \
-            (type(self.smoothrast) is SoftRast and type(self.smoothagg) is SoftAgg)
         colors = phong_shading(meshes=meshes, fragments=fragments, texels=texels, lights=lights, cameras=cameras,
-                               materials=materials, sparse=fused)
+                               materials=materials, sparse=_fused_pair(self.smoothrast, self.smoothagg))
         znear = kwargs.get("znear", getattr(cameras, "znear", 1.0))
         zfar = kwargs.get("zfar", getattr(cameras, "zfar", 100.0))
         if torch.is_tensor(znear):

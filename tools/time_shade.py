@@ -1,5 +1,8 @@
 """Device-timed fused forward / backward at BASELINE config 2 (or --cfg N,HW,K,S) on the named fragment sets.
-    python tools/time_shade.py [realistic dense rasterised] [--flags F] [--steps n] [--cfg 8,256,50,64]"""
+    python tools/time_shade.py [realistic dense rasterised] [--flags F] [--steps n] [--cfg 8,256,50,64]
+    python tools/time_shade.py [kinds] --noise cauchy     the Cauchy pair (ArctanRast + CauchyAgg) through the public
+        autograd interface, fused kernels against the operator-by-operator composition: forward ms, backward ms and
+        peak memory (torch.cuda.max_memory_allocated) of each"""
 import argparse
 import os
 import sys
@@ -19,6 +22,7 @@ ap.add_argument("--steps", type=int, default=10)
 ap.add_argument("--cfg", default="8,256,50,64")
 ap.add_argument("--tag", default="")
 ap.add_argument("--lib", default=None, help="alternate libpertshade.so (A/B runs of two builds in one GPU call)")
+ap.add_argument("--noise", default="gaussian", choices=["gaussian", "cauchy"])
 a = ap.parse_args()
 if a.lib:
     from pertrenderer_b200 import _cabi
@@ -26,12 +30,48 @@ if a.lib:
 N, HW, K, S = (int(v) for v in a.cfg.split(","))
 dev = torch.device("cuda:0")
 peak = bench.peaks()[0]
+
+
+def time_cauchy_pair(kind, fr, col, G):
+    """Fused (smooth_rgb_blend) and composition arm of the Cauchy pair, same inputs, median of a.steps steps each."""
+    import pertrenderer_b200 as pb
+    from pertrenderer_b200.random_rasterizer import _composed_rgb_blend
+    for name, fn in (("fused", pb.smooth_rgb_blend), ("composition", _composed_rgb_blend)):
+        rast, agg = pb.ArctanRast(nb_samples=S, sigma=1e-3), pb.CauchyAgg(nb_samples=S, gamma=1e-2, alpha=1.0)
+        d, z, c = fr.dists.clone().requires_grad_(True), fr.zbuf.clone().requires_grad_(True), col.clone().requires_grad_(True)
+        frag = pb.Fragments(fr.pix_to_face, z, None, d)
+        ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(a.steps)]
+        torch.cuda.synchronize()
+        torch.cuda.reset_peak_memory_stats()
+        base = torch.cuda.memory_allocated()
+        for i in range(-3, a.steps):
+            if i >= 0:
+                ev[i][0].record()
+            img = fn(c, frag, rast, agg, pb.BlendParams())
+            if i >= 0:
+                ev[i][1].record()
+            (img * G).sum().backward()
+            if i >= 0:
+                ev[i][2].record()
+            d.grad = z.grad = c.grad = None
+            del img
+        torch.cuda.synchronize()
+        f = sorted(e[0].elapsed_time(e[1]) for e in ev)[len(ev) // 2]
+        b = sorted(e[1].elapsed_time(e[2]) for e in ev)[len(ev) // 2]
+        mem = (torch.cuda.max_memory_allocated() - base) / 2 ** 20
+        print(f"{a.tag} cauchy {kind:10s} {name:11s} fwd {f:.4f} ms  bwd {b:.4f} ms  fwd+bwd {f + b:.4f} ms  "
+              f"peak +{mem:.0f} MiB over the inputs", flush=True)
+
+
 for kind in a.kinds:
     if kind == "rasterised":
         fr, col = bench.rasterised_fragments(types.SimpleNamespace(views=N, image_size=HW, faces_per_pixel=K, nb_samples=S), dev)
     else:
         fr, col = synthetic_fragments(N, HW, HW, K, kind=kind, sigma=1e-3, seed=0, device=dev)
     G = torch.randn((N, HW, HW, 4), device=dev, generator=torch.Generator(device=dev).manual_seed(1))
+    if a.noise == "cauchy":
+        time_cauchy_pair(kind, fr, col, G)
+        continue
     ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(a.steps)]
     for i in range(-3, a.steps):
         pr = ops.ShadeProblem(pix_to_face=fr.pix_to_face, zbuf=fr.zbuf, dists=fr.dists, colors=col, znear=1.0, zfar=100.0,
