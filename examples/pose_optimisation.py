@@ -226,7 +226,7 @@ def main():
             renderer = make_renderer(noise, cameras, lights, args.sigma, args.gamma, args.nb_samples, args.imsize, dev)
             torch.cuda.synchronize()
             t0 = time.perf_counter()
-            if args.graph and not args.adapt and noise in ("gaussian", "cauchy", "softras"):  # the fused pairs (device-side seeds)
+            if args.graph and not args.adapt and noise in ("gaussian", "gaussian_wovr", "cauchy", "softras"):  # the fused pairs (device-side seeds)
                 w = optimize_pose_graphed(mesh, verts, renderer, target, w0, args.niter, args.lr)
             else:
                 w = optimize_pose(mesh, verts, renderer, target, w0, args.niter, args.lr, args.adapt)

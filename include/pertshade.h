@@ -90,9 +90,18 @@ extern "C" {
  * PERT_E_UNSUPPORTED for PERT_F_CAUCHY with PERT_F_PHILOX7, PERT_F_NO_VR, PERT_F_SKIP_DEAD_NOISE, PERT_F_UNIFORM or
  * PERT_F_GUMBEL. */
 #define PERT_F_CAUCHY 8u
-/* stand-alone operators only, Gaussian noise: the estimators WITHOUT the control variates, the paper's ablation
+/* Gaussian noise: the estimators WITHOUT the control variates, the paper's ablation
  * (randomHeaviside_wovr smoothrast.py:61-108: sum_s h_s U_s instead of sum_s (h_s - h0) U_s;
- *  randomArgmax_wovr smoothagg.py:75-141: c_s = <g, onehot(a_s)> instead of <g, onehot(a_s) - onehot(a_0)>) */
+ *  randomArgmax_wovr smoothagg.py:75-141: c_s = <g, onehot(a_s)> instead of <g, onehot(a_s) - onehot(a_0)>).
+ * Stand-alone operators, and pert_shade_fwd / pert_shade_bwd with in-kernel or explicit noise, in one call or
+ * phase-split, with or without seed_device (GaussianRast_wovr + GaussianAgg_wovr).  Forward draws every coverage sample
+ * of each valid entry with x >= -sigma*Umax (the others have h = 0 always) and has the per-sample path of
+ * PERT_F_PER_SAMPLE_NOISE: counts, winners, image and alpha are those of the Gaussian pair with that flag, only rsum
+ * differs.  Backward works on every valid pixel, including those whose samples all picked a_0 and those without any
+ * valid entry (the background always wins; gamma term only), and regenerates every V_sj of every logit.  The fused
+ * entry points return PERT_E_UNSUPPORTED for PERT_F_NO_VR with PERT_F_PHILOX7, PERT_F_SKIP_DEAD_NOISE, PERT_F_UNIFORM,
+ * PERT_F_GUMBEL or PERT_F_CAUCHY.  Libraries older than pert_shade_fused_flags() ignore the flag in the fused entry
+ * points: check that function before relying on it. */
 #define PERT_F_NO_VR 0x400u
 /* pert_argmax_fwd only: uniform noise on [-1/2, 1/2) (UniformAgg, smoothagg.py:252-272) or standard Gumbel noise
  * (randomArgmax "gumbel", smoothagg.py:22-24).  Forward only, as in the reference (no backward: smoothagg.py:64-67);
@@ -151,6 +160,10 @@ typedef struct pert_problem {
 } pert_problem;
 
 int pert_version(void);
+/* PERT_F_* estimator / noise flags that pert_shade_fwd / pert_shade_bwd implement (PERT_F_CAUCHY, PERT_F_NO_VR, ...).
+ * A flag that is not in this set is rejected or ignored by the fused entry points of this library; callers check a
+ * flag here before its first fused call, so that an older library is detected rather than silently ignoring it. */
+uint32_t pert_shade_fused_flags(void);
 const char* pert_strerror(int code);
 /* last cudaError_t name seen by this thread's most recent failing call (diagnostic only) */
 const char* pert_last_cuda_error(void);

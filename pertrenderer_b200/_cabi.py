@@ -30,7 +30,7 @@ PH_RAST, PH_AGG, PH_BLEND = 0x10, 0x20, 0x40
 PH_BWD_SAMPLE, PH_BWD_FINISH = 0x100, 0x200
 
 EXPORTS = [
-    "pert_version", "pert_strerror", "pert_last_cuda_error", "pert_num_tiles", "pert_winner_bytes", "pert_blob_bytes",
+    "pert_version", "pert_shade_fused_flags", "pert_strerror", "pert_last_cuda_error", "pert_num_tiles", "pert_winner_bytes", "pert_blob_bytes",
     "pert_shade_fwd", "pert_shade_bwd", "pert_soft_shade_fwd", "pert_soft_shade_bwd", "pert_rast_fwd", "pert_rast_bwd", "pert_argmax_fwd",
     "pert_argmax_bwd", "pert_noise_fill", "pert_seed_advance", "pert_phong_fwd", "pert_phong_bwd", "pert_rasterize_fwd", "pert_rasterize_bwd", "pert_rasterize_num_bins", "pert_rasterize_bin",
 ]
@@ -164,6 +164,30 @@ def load():
             raise PertLibraryError(f"libpertshade.so ABI {lib.pert_version()} != expected {ABI_VERSION}: rebuild")
         _lib = lib
     return _lib
+
+
+_fused_flags = None  # (library, pert_shade_fused_flags()) of the library that answered
+
+
+def require_fused_flags(flags: int):
+    """Raise PertLibraryError unless the loaded library's pert_shade_fwd / pert_shade_bwd implement F_NO_VR when
+    ``flags`` asks for it.  Libraries built before it ignore the flag there and would return the variance-reduced
+    gradients; they also lack ``pert_shade_fused_flags``, which is therefore bound lazily here rather than in
+    :func:`load`, so that such a library keeps serving every other call."""
+    global _fused_flags
+    if not flags & F_NO_VR:
+        return
+    lib = load()
+    if _fused_flags is None or _fused_flags[0] is not lib:
+        fn = getattr(lib, "pert_shade_fused_flags", None)
+        if fn is not None:
+            fn.restype = C.c_uint32
+            fn.argtypes = []
+        _fused_flags = (lib, int(fn()) if fn is not None else 0)
+    if not _fused_flags[1] & F_NO_VR:
+        raise PertLibraryError(
+            f"{LIB_PATH} predates the fused GaussianRast_wovr + GaussianAgg_wovr pair (PERT_F_NO_VR in pert_shade_fwd / "
+            "pert_shade_bwd): rebuild it with `python -m pertrenderer_b200.build --force`")
 
 
 def check(rc: int, what: str):

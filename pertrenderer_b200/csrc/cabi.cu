@@ -17,6 +17,10 @@ static int cuda_rc(int e) { return e == 0 ? PERT_OK : cuda_fail(e); }
 
 extern "C" int pert_version(void) { return PERT_ABI_VERSION; }
 
+extern "C" uint32_t pert_shade_fused_flags(void) {
+    return PERT_F_NO_SKIP | PERT_F_SKIP_DEAD_NOISE | PERT_F_PER_SAMPLE_NOISE | PERT_F_CAUCHY | PERT_F_NO_VR | PERT_F_PHILOX7;
+}
+
 extern "C" const char* pert_last_cuda_error(void) { return g_last_cuda; }
 
 extern "C" const char* pert_strerror(int code) {
@@ -205,7 +209,7 @@ constexpr int kNabFallback = 8;
 
 static bool sparse_first_ok(const pert_problem* pb, const void* worklist, bool all_phases) {
     if (!worklist || !all_phases || pb->noise_rast || pb->noise_agg) return false;
-    if (pb->flags & (PERT_F_NO_SKIP | PERT_F_PER_SAMPLE_NOISE | PERT_F_CAUCHY)) return false;  // need logits dense in j
+    if (pb->flags & (PERT_F_NO_SKIP | PERT_F_PER_SAMPLE_NOISE | PERT_F_CAUCHY | PERT_F_NO_VR)) return false;  // need logits dense in j
     return true;
 }
 
@@ -214,6 +218,12 @@ static bool sparse_first_ok(const pert_problem* pb, const void* worklist, bool a
 static bool cauchy_flags_bad(uint32_t f) {
     return (f & PERT_F_CAUCHY) &&
            (f & (PERT_F_PHILOX7 | PERT_F_NO_VR | PERT_F_SKIP_DEAD_NOISE | PERT_F_UNIFORM | PERT_F_GUMBEL));
+}
+
+// flags the fused entry points cannot combine with PERT_F_NO_VR: its kernels draw the Philox4x32-10 stream of every
+// sample (the shortcut for never-winning logits is a variance-reduced estimator's), and the forward-only noises
+static bool no_vr_flags_bad(uint32_t f) {
+    return (f & PERT_F_NO_VR) && (f & (PERT_F_PHILOX7 | PERT_F_SKIP_DEAD_NOISE | PERT_F_UNIFORM | PERT_F_GUMBEL));
 }
 
 // Bulk-copy scan of the forward (tile.cuh scan_valid_staged; TMA 1-D copy + mbarrier, UBLKCP in SASS): bytes of the staging
@@ -270,7 +280,7 @@ extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t*
     if ((uintptr_t)worklist & 15) return PERT_E_ALIGN;
     const uint32_t all = PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
     if ((f & PERT_F_PHILOX7) && ((f & all) != all || hist || a.pb.noise_rast || a.pb.noise_agg)) return PERT_E_UNSUPPORTED;
-    if (cauchy_flags_bad(f)) return PERT_E_UNSUPPORTED;
+    if (cauchy_flags_bad(f) || no_vr_flags_bad(f)) return PERT_E_UNSUPPORTED;
     bool sparse = sparse_first_ok(&a.pb, worklist, (f & all) == all && !hist);
     if (sparse) {  // the fallback pass runs FBT/32 warps per CTA: its tiles must fit that many times
         SmemLayout t;
@@ -332,7 +342,7 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
         return PERT_E_ALIGN;
     if ((uintptr_t)worklist & 15) return PERT_E_ALIGN;
     if ((f & PERT_F_PHILOX7) && (!(smp && fin) || hist || a.pb.noise_agg)) return PERT_E_UNSUPPORTED;
-    if (cauchy_flags_bad(f)) return PERT_E_UNSUPPORTED;
+    if (cauchy_flags_bad(f) || no_vr_flags_bad(f)) return PERT_E_UNSUPPORTED;
     bool sparse = sparse_first_ok(&a.pb, worklist, smp && fin && !hist);
     if (sparse) {  // the fallback pass runs FBT/32 warps per CTA: its tiles must fit that many times
         const int tp2 = sparse_tp(a.pb.K, a.pb.N * a.pb.H * a.pb.W) / 2;

@@ -55,7 +55,12 @@ void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes,
 // blob forward saved (common.cuh) instead of a re-scan of pix_to_face and a recomputation of the logits.
 // SCORE = the score psi of the aggregation noise (philox.cuh noise_score): acc_j = sum_s c_s psi(V_sj) and
 // t2_j = sum_s c_s V_sj psi(V_sj); 0 Gaussian (psi(n) = n), 1 Cauchy.
-template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0>
+// WOVR = true (PERT_F_NO_VR, randomArgmax_wovr smoothagg.py:75-141): c_s = g[a_s] without the control variate g[a_0].
+// Samples that picked a0 contribute, so every valid pixel is worked on, including those whose samples all picked a0
+// (forward wrote no winners row for them when a0 was their only live logit: a_s = a0 is known) and the pixels
+// without any valid entry (the background wins every sample; their only output is the gamma term, whose norm runs
+// over all K + 1 logits).  Every V_sj of every logit is regenerated (per-sample noise, dense per-logit arrays).
+template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0, bool WOVR = false>
 __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& noise_a, const int64_t tile,
                                                const int64_t prow /* row of the scalar partials */,
                                                unsigned char* smem_raw, const int lane) {
@@ -69,7 +74,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
     const bool no_skip = flags & PERT_F_NO_SKIP;
     // how the noise of logits that can never win (zero-mean, independent of everything) is handled; the one-draw
     // shortcut rests on sum_s c_s V_sj being normal, which holds for the Gaussian score only
-    const bool per_sample = SCORE != 0 || !NoiseA::kBounded || no_skip || (flags & PERT_F_PER_SAMPLE_NOISE);
+    const bool per_sample = WOVR || SCORE != 0 || !NoiseA::kBounded || no_skip || (flags & PERT_F_PER_SAMPLE_NOISE);
     const bool drop_dead = !per_sample && (flags & PERT_F_SKIP_DEAD_NOISE);
     float p_sigma = 0.f, p_gamma = 0.f, p_q = 0.f;
 
@@ -154,7 +159,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
     if (overflow) {
         // more valid entries than the compact arrays hold: the fallback pass redoes this tile
         if (lane == 0) a.worklist[4 + atomicAdd(a.worklist, 1)] = (int32_t)tile;
-    } else if (nv > 0) {
+    } else if (nv > 0 || WOVR) {
         const float gal = a.L.gal;
         PixPrep pi;
         if constexpr (BLOB) {
@@ -228,8 +233,8 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
         const int nvp = ve - vs;
         const int a0 = pi.a0;
         // a pixel whose samples all picked a0 has c_s = 0 for every s: every score sum is exactly 0
-        // (and forward wrote no winners row for it)
-        const bool act = pvalid && do_sample && (pstate & 0x8000);
+        // (and forward wrote no winners row for it); without the control variate c_s = g[a0] there
+        const bool act = pvalid && do_sample && (WOVR || (pstate & 0x8000));
         const int sb = COMPACT ? vs + 2 * p : p * K1;                  // this pixel's slots
         const int slot_pad = COMPACT ? sb + nvp + 1 : sb + pi.kpad;     // where the masked logits' joint draw goes
         const bool prefix = pi.kpad == nvp;                             // valid entries are k = 0..nvp-1
@@ -258,7 +263,8 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
             // g_j of every logit that can win (the saved winners are among them) and cleared sums
             if (act && lig == 0) {
                 apx[my_ai] = (uint8_t)p;
-                pa0[p] = a0;
+                // WOVR: bit 16 = every sample picked a0, the saved winners row is not read
+                pa0[p] = (WOVR && !(pstate & 0x8000)) ? a0 | 0x10000 : a0;
                 if (COMPACT) {
                     psb[p] = sb;
                     pnv[p] = nvp | (prefix ? 0 : 0x10000);
@@ -357,11 +363,24 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                     for (int s = lane; s < cn4; s += 32) {
                         float c = 0.f;
                         if (s < cn) {
-                            const int w = early_w ? load_winner(wst, wb, pp * sa_loc + s) : load_winner(a.winners, wb, wbase + s);
-                            if (w != ppa0) {  // a0 (the most frequent by far) is counted as the remainder
-                                const int ws = slot_of(pp, w);
-                                atomicAdd(&hj[ws], 1);
-                                c = gsel[ws] - g0v;
+                            if constexpr (WOVR) {
+                                const int pa = ppa0 & 0xffff;
+                                const int w = (ppa0 & 0x10000) ? pa
+                                              : early_w ? load_winner(wst, wb, pp * sa_loc + s) : load_winner(a.winners, wb, wbase + s);
+                                if (w != pa) {
+                                    const int ws = slot_of(pp, w);
+                                    atomicAdd(&hj[ws], 1);
+                                    c = gsel[ws];
+                                } else {
+                                    c = g0v;
+                                }
+                            } else {
+                                const int w = early_w ? load_winner(wst, wb, pp * sa_loc + s) : load_winner(a.winners, wb, wbase + s);
+                                if (w != ppa0) {  // a0 (the most frequent by far) is counted as the remainder
+                                    const int ws = slot_of(pp, w);
+                                    atomicAdd(&hj[ws], 1);
+                                    c = gsel[ws] - g0v;
+                                }
                             }
                         }
                         cs[ai * sc + s] = c;
@@ -383,7 +402,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                             const int h = hj[sl];
                             if (h > 0 && j != a0) {
                                 others += h;
-                                const float d = gsel[sl] - g0v;
+                                const float d = WOVR ? gsel[sl] : gsel[sl] - g0v;
                                 c1 += (float)h * d;
                                 c2 += (float)h * d * d;
                             }
@@ -393,7 +412,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                     c1 = group_sum(c1, G);
                     c2 = group_sum(c2, G);
                     if (mine) {
-                        csum = c1;
+                        csum = WOVR ? c1 + (float)(sa_loc - others) * pg0[p] : c1;  // the samples won by a0
                         C2 = c2;
                         if (lig == 0) hj[slot_of(p, a0)] = sa_loc - others;
                     }
@@ -612,12 +631,12 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
 #ifndef BWD_MAIN_CTAS
 #define BWD_MAIN_CTAS 28
 #endif
-template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0>
+template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0, bool WOVR = false>
 __global__ void __launch_bounds__(FNT, BWD_MAIN_CTAS) shade_bwd_kernel(const BwdArgs a, const NoiseA noise_a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     NoiseA na = noise_a;
     if (a.pb.seed_device) na.mix(__ldg(a.pb.seed_device + 1));  // device-side seed, see shade_fwd.cu
-    shade_bwd_tile<NoiseA, GT, PHASED, FACE, COMPACT, BLOB, SCORE>(a, na, blockIdx.x, blockIdx.x, smem_raw, threadIdx.x);
+    shade_bwd_tile<NoiseA, GT, PHASED, FACE, COMPACT, BLOB, SCORE, WOVR>(a, na, blockIdx.x, blockIdx.x, smem_raw, threadIdx.x);
 }
 
 // Fallback pass of the sparse-first mode (see shade_fwd.cu): work-list tiles as half-size tiles with dense
@@ -706,17 +725,17 @@ static int set_smem(K kern, size_t smem) {
     return 0;
 }
 
-template <class NA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB = false, int SCORE = 0>
+template <class NA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB = false, int SCORE = 0, bool WOVR = false>
 static int launch_bwd_f(const BwdArgs& a, const NA& na, cudaStream_t st) {
     const size_t smem = (size_t)a.L.warp_smem;
-    if (int rc = set_smem(shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE>, smem)) return rc;
-    shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, na);
+    if (int rc = set_smem(shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE, WOVR>, smem)) return rc;
+    shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE, WOVR><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, na);
     return (int)cudaGetLastError();
 }
-template <class NA, int GT, bool PHASED, int SCORE = 0>
+template <class NA, int GT, bool PHASED, int SCORE = 0, bool WOVR = false>
 static int launch_bwd_t(const BwdArgs& a, const NA& na, cudaStream_t st) {
-    return a.pb.face_colors ? launch_bwd_f<NA, GT, PHASED, true, false, false, SCORE>(a, na, st)
-                            : launch_bwd_f<NA, GT, PHASED, false, false, false, SCORE>(a, na, st);
+    return a.pb.face_colors ? launch_bwd_f<NA, GT, PHASED, true, false, false, SCORE, WOVR>(a, na, st)
+                            : launch_bwd_f<NA, GT, PHASED, false, false, false, SCORE, WOVR>(a, na, st);
 }
 // sparse-first main pass (compact per-logit arrays); PN = the Philox variant
 template <class PN, int GT>
@@ -780,6 +799,13 @@ int launch_shade_bwd(const BwdArgs& a, const BwdArgs* fb, float* grad_scalars, c
             rc = launch_bwd_t<ExplicitNoise, 0, true, 1>(a, xa, st);
         } else {
             rc = launch_bwd_t<PhiloxCauchy, 0, true, 1>(a, PhiloxCauchy(a.pb.seed_agg, 1, a.pb.pixel_offset), st);
+        }
+    } else if (a.pb.flags & PERT_F_NO_VR) {  // no control variates: the same dense instantiation, Gaussian noise
+        if (a.pb.noise_agg) {
+            ExplicitNoise xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
+            rc = launch_bwd_t<ExplicitNoise, 0, true, 0, true>(a, xa, st);
+        } else {
+            rc = launch_bwd_t<PhiloxNoise, 0, true, 0, true>(a, PhiloxNoise(a.pb.seed_agg, 1, a.pb.pixel_offset), st);
         }
     } else if (a.pb.noise_agg) {
         ExplicitNoise xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};

@@ -56,7 +56,11 @@ __device__ __forceinline__ void fwd_init_barrier(const FwdArgs& a, unsigned char
 // wants them anyway) and then aggregation + blend (CPH = AGG | BLEND: reads the counts back), because one kernel with
 // both exceeds the 32 KB instruction cache of an SM and every warp walks the whole body once per tile.
 // SCORE = the score of the coverage noise in rsum (philox.cuh noise_score): 0 Gaussian, 1 Cauchy.
-template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int CPH = 0x70, int SCORE = 0>
+// WOVR = true: the estimator without control variates (PERT_F_NO_VR): rsum = sum_s h psi(U), so an entry that is
+// covered by every sample still draws them all; only the side x < -sigma*Umax (h = 0 always) is skipped, and the
+// compound sampler (which produces sum_s (h - h0) U only) is compiled out.  Counts, winners and image are unchanged.
+template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int CPH = 0x70, int SCORE = 0,
+          bool WOVR = false>
 __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& noise_r, const NoiseA& noise_a,
                                                const int64_t tile, unsigned char* smem_raw, const int lane) {
     const pert_problem& pb = a.pb;
@@ -140,7 +144,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
     const int sr_loc = pb.s_rast_end - pb.s_rast_begin;
     const float thr = (NoiseR::kBounded && !no_skip) ? pb.sigma * kNoiseAbsMax * 1.0001f : CUDART_INF_F;
     // compound sampler (tile.cuh) for the entries with |x| >= x_cmp: the default with in-kernel noise
-    const bool compound = NoiseR::kBounded && !no_skip && !(flags & PERT_F_PER_SAMPLE_NOISE);
+    const bool compound = !WOVR && NoiseR::kBounded && !no_skip && !(flags & PERT_F_PER_SAMPLE_NOISE);
     const float x_cmp = compound ? a.L.t_compound * pb.sigma : CUDART_INF_F;
     uint16_t* const blist = rlist + cap - 1;  // stored downwards: the two lists share one array of cap entries
     int nlist = 0, nblist = 0;
@@ -158,7 +162,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
                 const float x = -__ldg(dists_t + e);
                 xs[n] = x;
                 // |x| beyond the largest possible sigma*|U| cannot flip: exact, not an approximation
-                need = fabsf(x) <= thr;
+                need = WOVR ? x >= -thr : fabsf(x) <= thr;
                 cmp = need && fabsf(x) >= x_cmp;
                 if (!need) {
                     cnt[n] = (x >= 0.0f) ? (uint16_t)sr_loc : (uint16_t)0;
@@ -204,14 +208,14 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
             nblist = 0;
             __syncwarp();
         }
-        if constexpr (NoiseR::kBounded && !DEFER) {
+        if constexpr (NoiseR::kBounded && !DEFER && !WOVR) {
             if (nblist > 0) {
                 const CompoundCtx<NoiseR> cc{noise_r, vlist, xs, cnt, rs, K, a.L.invK, pix0, a.L.inv_sigma, sr_loc,
                                              0x40000000u + 2u * (uint32_t)(pb.s_rast_begin >> 2)};
                 rast_compound_list(cc, blist, nblist, a.L.t_bucket[0] * pb.sigma, a.L.t_bucket[1] * pb.sigma, ring);
             }
         }
-        rast_sample_list<NoiseR, SCORE>(noise_r, rlist, nlist, vlist, xs, cnt, rs, K, a.L.invK, pix0, pb.sigma, a.L.inv_sigma, pb.s_rast_begin,
+        rast_sample_list<NoiseR, SCORE, WOVR>(noise_r, rlist, nlist, vlist, xs, cnt, rs, K, a.L.invK, pix0, pb.sigma, a.L.inv_sigma, pb.s_rast_begin,
                          pb.s_rast_end, !no_skip, a.L.lpe_r);
         __syncwarp();
 #pragma unroll 1
@@ -448,10 +452,10 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
     if (pvalid && lig == 0) reinterpret_cast<float4*>(a.image)[gp] = make_float4(r, g, bl, px_alpha);
 }
 
-// CTAs (= warps) per SM: 32 (64 registers); the Cauchy instantiations (SCORE = 1) get 24 (80 registers): at 64 the
-// in-kernel Cauchy stream spills
-template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int SCORE = 0>
-__global__ void __launch_bounds__(FNT, SCORE ? 24 : 32) shade_fwd_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
+// CTAs (= warps) per SM: 32 (64 registers); the Cauchy instantiations (SCORE = 1) and those without control variates
+// (WOVR) get 24 (80 registers): at 64 the in-kernel Cauchy stream and the ungated coverage samples of WOVR spill
+template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int SCORE = 0, bool WOVR = false>
+__global__ void __launch_bounds__(FNT, (SCORE || WOVR) ? 24 : 32) shade_fwd_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     NoiseR nr = noise_r;
     NoiseA na = noise_a;
@@ -462,7 +466,7 @@ __global__ void __launch_bounds__(FNT, SCORE ? 24 : 32) shade_fwd_kernel(const F
 #ifdef PERT_EXPERIMENTS
     if (a.L.stage_bytes) fwd_init_barrier(a, smem_raw);
 #endif
-    shade_fwd_tile<NoiseR, NoiseA, GT, PHASED, DEFER, 0x70, SCORE>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x);
+    shade_fwd_tile<NoiseR, NoiseA, GT, PHASED, DEFER, 0x70, SCORE, WOVR>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x);
 }
 
 // Fallback pass of the sparse-first mode: the tiles whose valid entries did not fit the compact arrays,
@@ -501,15 +505,15 @@ __global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(co
     }
 }
 
-template <class NR, class NA, int GT, bool PHASED, bool DEFER = false, int SCORE = 0>
+template <class NR, class NA, int GT, bool PHASED, bool DEFER = false, int SCORE = 0, bool WOVR = false>
 static int launch_fwd_t(const FwdArgs& a, const NR& nr, const NA& na, cudaStream_t st) {
     const size_t smem = (size_t)a.L.warp_smem;
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE>,
+        cudaError_t e = cudaFuncSetAttribute(shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
-    shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na);
+    shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na);
     return (int)cudaGetLastError();
 }
 
@@ -561,21 +565,25 @@ static int launch_fwd_production(const FwdArgs& a, const FwdArgs* fb, cudaStream
     }
 }
 
-// Cauchy pair (PERT_F_CAUCHY): the dense instantiation with runtime lanes per pixel and the phase-split code, for single
-// and phase-split calls alike.  Unbounded noise turns off every skip of the Gaussian path (kBounded): each valid entry
-// draws all its coverage samples and every finite logit takes part in the argmax.
-static int launch_fwd_cauchy(const FwdArgs& a, cudaStream_t st) {
+// Cauchy pair (PERT_F_CAUCHY: PN = PhiloxCauchy, SCORE = 1) and the pair without control variates (PERT_F_NO_VR:
+// PN = PhiloxNoise, WOVR): the dense instantiation with runtime lanes per pixel and the phase-split code, for single
+// and phase-split calls alike.  Unbounded Cauchy noise turns off every skip of the Gaussian path (kBounded): each valid
+// entry draws all its coverage samples and every finite logit takes part in the argmax.  The pair without control
+// variates keeps the two skips that stay exact for it, entries with x < -sigma*Umax and logits that cannot win.
+template <class PN, int SCORE, bool WOVR>
+static int launch_fwd_dense(const FwdArgs& a, cudaStream_t st) {
     const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
-    PhiloxCauchy pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
+    PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
     ExplicitNoise xr{a.pb.noise_rast, a.L.P, a.pb.K, a.pb.S_rast}, xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
-    if (er && ea) return launch_fwd_t<ExplicitNoise, ExplicitNoise, 0, true, false, 1>(a, xr, xa, st);
-    if (er) return launch_fwd_t<ExplicitNoise, PhiloxCauchy, 0, true, false, 1>(a, xr, pa, st);
-    if (ea) return launch_fwd_t<PhiloxCauchy, ExplicitNoise, 0, true, false, 1>(a, pr, xa, st);
-    return launch_fwd_t<PhiloxCauchy, PhiloxCauchy, 0, true, false, 1>(a, pr, pa, st);
+    if (er && ea) return launch_fwd_t<ExplicitNoise, ExplicitNoise, 0, true, false, SCORE, WOVR>(a, xr, xa, st);
+    if (er) return launch_fwd_t<ExplicitNoise, PN, 0, true, false, SCORE, WOVR>(a, xr, pa, st);
+    if (ea) return launch_fwd_t<PN, ExplicitNoise, 0, true, false, SCORE, WOVR>(a, pr, xa, st);
+    return launch_fwd_t<PN, PN, 0, true, false, SCORE, WOVR>(a, pr, pa, st);
 }
 
 int launch_shade_fwd(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    if (a.pb.flags & PERT_F_CAUCHY) return launch_fwd_cauchy(a, st);
+    if (a.pb.flags & PERT_F_CAUCHY) return launch_fwd_dense<PhiloxCauchy, 1, false>(a, st);
+    if (a.pb.flags & PERT_F_NO_VR) return launch_fwd_dense<PhiloxNoise, 0, true>(a, st);
     const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
     const uint32_t all = PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
     const bool phased = (a.pb.flags & all) != all || a.hist != nullptr;

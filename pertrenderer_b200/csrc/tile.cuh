@@ -134,9 +134,11 @@ __device__ __forceinline__ void pixel_ranges(const uint16_t* vlist, int nv, int 
 // stage 1: coverage samples of the listed entries
 //   randomras/smoothrast.py:32-36: h = 1[x + sigma*U >= 0] (rounded multiply, rounded add), mean over s
 //   saved for backward: cnt = sum_s h, rs = sum_s (h - h0) psi(U)   (smoothrast.py:46,49; psi = noise_score<SCORE>)
+//   WOVR = true, without the control variate (randomHeaviside_wovr, smoothrast.py:61-108): rs = sum_s h psi(U); the
+//   radius gate then only applies to x < 0 (h0 = 0), where a sample that cannot flip adds nothing
 // rlist holds compact indices n; xs/cnt/rs are compact arrays.
 // ------------------------------------------------------------------------------------------------
-template <class NoiseT, int SCORE = 0>
+template <class NoiseT, int SCORE = 0, bool WOVR = false>
 __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint16_t* rlist, int nlist,
                                                  const uint16_t* vlist, const float* xs, uint16_t* cnt, float* rs,
                                                  int K, float invK, int64_t pix0, float sigma, float inv_sigma,
@@ -166,7 +168,7 @@ __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint
             if constexpr (NoiseT::kBounded) {
                 // a pair of samples can only flip when its Box-Muller radius reaches |x|/sigma: decide that
                 // on the raw word and skip the transcendental work otherwise (exact, see radius_gate)
-                const uint32_t gate = gate_ok ? radius_gate(fabsf(x) * inv_sigma * 0.99999f) : 0u;
+                const uint32_t gate = (gate_ok && !(WOVR && h0)) ? radius_gate(fabsf(x) * inv_sigma * 0.99999f) : 0u;
 #pragma unroll 1
                 for (int q = qb + lig; q < qe; q += lpe) {
                     uint32_t w[4];
@@ -182,13 +184,24 @@ __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint
                             box_muller(w[hp * 2], w[hp * 2 + 1], n0, n1);
                             const bool ha = __fadd_rn(x, __fmul_rn(sigma, n0)) >= 0.0f;
                             const bool hb = __fadd_rn(x, __fmul_rn(sigma, n1)) >= 0.0f;
-                            if (in0) {
-                                c += ha ? 1 : 0;
-                                if (ha != h0) r += ha ? n0 : -n0;
-                            }
-                            if (in1) {
-                                c += hb ? 1 : 0;
-                                if (hb != h0) r += hb ? n1 : -n1;
+                            if constexpr (WOVR) {
+                                if (in0) {
+                                    c += ha ? 1 : 0;
+                                    if (ha) r += n0;
+                                }
+                                if (in1) {
+                                    c += hb ? 1 : 0;
+                                    if (hb) r += n1;
+                                }
+                            } else {
+                                if (in0) {
+                                    c += ha ? 1 : 0;
+                                    if (ha != h0) r += ha ? n0 : -n0;
+                                }
+                                if (in1) {
+                                    c += hb ? 1 : 0;
+                                    if (hb != h0) r += hb ? n1 : -n1;
+                                }
                             }
                         }
                     }
@@ -204,7 +217,11 @@ __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint
                         const bool h = __fadd_rn(x, __fmul_rn(sigma, nz[t])) >= 0.0f;
                         if (s >= s_begin && s < s_end) {
                             c += h ? 1 : 0;
-                            if (h != h0) r += h ? noise_score<SCORE>(nz[t]) : -noise_score<SCORE>(nz[t]);
+                            if constexpr (WOVR) {
+                                if (h) r += noise_score<SCORE>(nz[t]);
+                            } else if (h != h0) {
+                                r += h ? noise_score<SCORE>(nz[t]) : -noise_score<SCORE>(nz[t]);
+                            }
                         }
                     }
                 }

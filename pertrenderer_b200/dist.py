@@ -219,7 +219,8 @@ def smooth_rgb_blend_sample_sharded(colors, fragments, smoothrast, smoothagg, bl
     from .random_rasterizer import _background_tuple, _perturbed_pair_flags
     flags = _perturbed_pair_flags(smoothrast, smoothagg)
     if flags is None:
-        raise ValueError("sample sharding is implemented for the (GaussianRast, GaussianAgg) and (ArctanRast, CauchyAgg) pairs")
+        raise ValueError("sample sharding is implemented for the (GaussianRast, GaussianAgg), (ArctanRast, CauchyAgg) and "
+                         "(GaussianRast_wovr, GaussianAgg_wovr) pairs")
     cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps, S_rast=smoothrast.nb_samples,
                S_agg=smoothagg.nb_samples, fixed_noise=bool(smoothagg.fixed_noise), group=group, sync_seeds=sync_seeds,
                flags=flags)

@@ -85,8 +85,8 @@ def refuse_device_seeds(op: str):
     replay the same noise for ever.  Fail loudly instead."""
     if current_seed_device() is not None:
         raise RuntimeError(f"{op}: device-side seeds (ops.device_seeds) are implemented for the fused operator pairs "
-                           "(GaussianRast + GaussianAgg, ArctanRast + CauchyAgg, SoftRast + SoftAgg) only; run this pair "
-                           "outside the block")
+                           "(GaussianRast + GaussianAgg, ArctanRast + CauchyAgg, GaussianRast_wovr + GaussianAgg_wovr, "
+                           "SoftRast + SoftAgg) only; run this pair outside the block")
 
 
 def _f32c(t):
@@ -259,6 +259,7 @@ class ShadeSaved:
 def shade_forward(pr: ShadeProblem, want_hist: bool = False, phases: int = 0, saved: Optional[ShadeSaved] = None):
     """Launch pert_shade_fwd.  Returns (image (N,H,W,4), ShadeSaved)."""
     lib = _cabi.load()
+    _cabi.require_fused_flags(pr.flags)
     N, H, W, K = pr.shape
     dev = pr.device
     with torch.cuda.device(dev):
@@ -267,10 +268,10 @@ def shade_forward(pr: ShadeProblem, want_hist: bool = False, phases: int = 0, sa
             # phase-split (sample-sharded) jobs all-reduce counts / rsum as whole tensors: define every entry
             alloc = torch.zeros if phases else torch.empty
             # the tile blobs are written by the production path only (in-kernel Gaussian noise, all phases in one call, no
-            # global histogram, default noise flags: csrc/cabi.cu sparse_first_ok); the buffer only exists then, so that a
-            # backward with other flags can never read what forward did not write
+            # global histogram, default noise flags and estimator: csrc/cabi.cu sparse_first_ok); the buffer only exists
+            # then, so that a backward with other flags can never read what forward did not write
             prod = not phases and not want_hist and pr.noise_rast is None and pr.noise_agg is None and \
-                not (pr.flags & (F_NO_SKIP | F_PER_SAMPLE_NOISE | F_CAUCHY))
+                not (pr.flags & (F_NO_SKIP | F_PER_SAMPLE_NOISE | F_CAUCHY | F_NO_VR))
             saved = ShadeSaved(
                 counts=alloc((N, H, W, K), dtype=torch.int16, device=dev),
                 rsum=alloc((N, H, W, K), dtype=torch.float32, device=dev),
@@ -292,6 +293,7 @@ def shade_backward(pr: ShadeProblem, saved: ShadeSaved, grad_image: torch.Tensor
                    phases: int = 0, acc=None, pixstat=None, use_hist: bool = False):
     """Launch pert_shade_bwd.  Returns (grad_dists, grad_zbuf, grad_colors | None, grad_scalars(3))."""
     lib = _cabi.load()
+    _cabi.require_fused_flags(pr.flags)
     N, H, W, K = pr.shape
     dev = pr.device
     require_cuda(grad_image)

@@ -2,8 +2,8 @@
 
 ``smooth_rgb_blend`` (random_rasterizer.py:34-56) and ``RandomSimpleShader`` (:132-191) keep the
 reference's signatures, so ``MeshRenderer(rasterizer=..., shader=RandomSimpleShader(...))`` works
-unchanged.  With the (GaussianRast, GaussianAgg) pair and the Cauchy pair (ArctanRast, CauchyAgg) the
-whole chain — coverage sampling, mask, alpha, logits, perturbed argmax, blend, and the score-function
+unchanged.  With the (GaussianRast, GaussianAgg) pair, the Cauchy pair (ArctanRast, CauchyAgg) and the pair
+without control variates (GaussianRast_wovr, GaussianAgg_wovr) the whole chain — coverage sampling, mask, alpha, logits, perturbed argmax, blend, and the score-function
 backward — is ONE forward and ONE backward sm_100a kernel (``pert_shade_fwd`` / ``pert_shade_bwd``).
 Any other operator pair falls through to the operator-by-operator composition of the reference, where
 the perturbed operators still run on their own CUDA kernels.
@@ -16,8 +16,8 @@ import torch.nn as nn
 from torch.autograd import Function
 
 from . import ops
-from .smoothagg import CauchyAgg, GaussianAgg, SoftAgg  # noqa: F401
-from .smoothrast import ArctanRast, GaussianRast, SoftRast
+from .smoothagg import CauchyAgg, GaussianAgg, GaussianAgg_wovr, SoftAgg  # noqa: F401
+from .smoothrast import ArctanRast, GaussianRast, GaussianRast_wovr, SoftRast
 from .structures import BlendParams, FaceTexels, UVTexels, VertexTexels
 
 
@@ -32,7 +32,8 @@ def _background_tuple(blend_params):
 
 
 class _PerturbedShade(Function):
-    """Fused GaussianRast -> mask/alpha -> GaussianAgg -> blend (``cfg["flags"]`` = F_CAUCHY: ArctanRast / CauchyAgg).
+    """Fused GaussianRast -> mask/alpha -> GaussianAgg -> blend (``cfg["flags"]`` = F_CAUCHY: ArctanRast / CauchyAgg;
+    F_NO_VR: GaussianRast_wovr / GaussianAgg_wovr).
 
     Differentiable inputs: colors, dists, zbuf and the three 0-dim scalars sigma, gamma, alpha
     (CPU leaves in the reference: smoothrast.py:116, smoothagg.py:153-154).  Saved for backward:
@@ -113,11 +114,14 @@ class _SoftShade(Function):
 
 def _perturbed_pair_flags(smoothrast, smoothagg):
     """PERT_F_* noise flags of the fused perturbed kernels for this operator pair: 0 for (GaussianRast, GaussianAgg),
-    F_CAUCHY for (ArctanRast, CauchyAgg); None for a pair without them."""
+    F_CAUCHY for (ArctanRast, CauchyAgg), F_NO_VR for (GaussianRast_wovr, GaussianAgg_wovr); None for a pair without
+    them (mixed pairs such as GaussianRast + GaussianAgg_wovr run op by op)."""
     if isinstance(smoothrast, GaussianRast) and isinstance(smoothagg, GaussianAgg):
         return 0
     if isinstance(smoothrast, ArctanRast) and isinstance(smoothagg, CauchyAgg):
         return ops.F_CAUCHY
+    if isinstance(smoothrast, GaussianRast_wovr) and isinstance(smoothagg, GaussianAgg_wovr):
+        return ops.F_NO_VR
     return None
 
 

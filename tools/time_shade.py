@@ -2,7 +2,9 @@
     python tools/time_shade.py [realistic dense rasterised] [--flags F] [--steps n] [--cfg 8,256,50,64]
     python tools/time_shade.py [kinds] --noise cauchy     the Cauchy pair (ArctanRast + CauchyAgg) through the public
         autograd interface, fused kernels against the operator-by-operator composition: forward ms, backward ms and
-        peak memory (torch.cuda.max_memory_allocated) of each"""
+        peak memory (torch.cuda.max_memory_allocated) of each
+    python tools/time_shade.py [kinds] --noise wovr       the same for the pair without control variates
+        (GaussianRast_wovr + GaussianAgg_wovr)"""
 import argparse
 import os
 import sys
@@ -22,7 +24,7 @@ ap.add_argument("--steps", type=int, default=10)
 ap.add_argument("--cfg", default="8,256,50,64")
 ap.add_argument("--tag", default="")
 ap.add_argument("--lib", default=None, help="alternate libpertshade.so (A/B runs of two builds in one GPU call)")
-ap.add_argument("--noise", default="gaussian", choices=["gaussian", "cauchy"])
+ap.add_argument("--noise", default="gaussian", choices=["gaussian", "cauchy", "wovr"])
 a = ap.parse_args()
 if a.lib:
     from pertrenderer_b200 import _cabi
@@ -32,12 +34,13 @@ dev = torch.device("cuda:0")
 peak = bench.peaks()[0]
 
 
-def time_cauchy_pair(kind, fr, col, G):
-    """Fused (smooth_rgb_blend) and composition arm of the Cauchy pair, same inputs, median of a.steps steps each."""
+def time_pair(kind, fr, col, G):
+    """Fused (smooth_rgb_blend) and composition arm of the --noise pair, same inputs, median of a.steps steps each."""
     import pertrenderer_b200 as pb
     from pertrenderer_b200.random_rasterizer import _composed_rgb_blend
+    rast_cls, agg_cls = (pb.ArctanRast, pb.CauchyAgg) if a.noise == "cauchy" else (pb.GaussianRast_wovr, pb.GaussianAgg_wovr)
     for name, fn in (("fused", pb.smooth_rgb_blend), ("composition", _composed_rgb_blend)):
-        rast, agg = pb.ArctanRast(nb_samples=S, sigma=1e-3), pb.CauchyAgg(nb_samples=S, gamma=1e-2, alpha=1.0)
+        rast, agg = rast_cls(nb_samples=S, sigma=1e-3), agg_cls(nb_samples=S, gamma=1e-2, alpha=1.0)
         d, z, c = fr.dists.clone().requires_grad_(True), fr.zbuf.clone().requires_grad_(True), col.clone().requires_grad_(True)
         frag = pb.Fragments(fr.pix_to_face, z, None, d)
         ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(a.steps)]
@@ -59,7 +62,7 @@ def time_cauchy_pair(kind, fr, col, G):
         f = sorted(e[0].elapsed_time(e[1]) for e in ev)[len(ev) // 2]
         b = sorted(e[1].elapsed_time(e[2]) for e in ev)[len(ev) // 2]
         mem = (torch.cuda.max_memory_allocated() - base) / 2 ** 20
-        print(f"{a.tag} cauchy {kind:10s} {name:11s} fwd {f:.4f} ms  bwd {b:.4f} ms  fwd+bwd {f + b:.4f} ms  "
+        print(f"{a.tag} {a.noise} {kind:10s} {name:11s} fwd {f:.4f} ms  bwd {b:.4f} ms  fwd+bwd {f + b:.4f} ms  "
               f"peak +{mem:.0f} MiB over the inputs", flush=True)
 
 
@@ -69,8 +72,8 @@ for kind in a.kinds:
     else:
         fr, col = synthetic_fragments(N, HW, HW, K, kind=kind, sigma=1e-3, seed=0, device=dev)
     G = torch.randn((N, HW, HW, 4), device=dev, generator=torch.Generator(device=dev).manual_seed(1))
-    if a.noise == "cauchy":
-        time_cauchy_pair(kind, fr, col, G)
+    if a.noise != "gaussian":
+        time_pair(kind, fr, col, G)
         continue
     ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(a.steps)]
     for i in range(-3, a.steps):
