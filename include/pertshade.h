@@ -195,6 +195,22 @@ int pert_shade_fwd(const pert_problem* pb, float* image, uint16_t* counts, float
                    uint16_t* pixstate, int32_t* hist, int32_t* worklist, void* tile_blob, void* stream);
 
 /*
+ * Forward-only render: the image of pert_shade_fwd for a call that needs no gradient (evaluation renders, high sample
+ * counts).  Nothing is stored for backward: no counts, rsum, winners, pixstate or tile blob.  Coverage computes hit
+ * counts only (the compound sampler draws the number of flips and no tail normals, the per-sample path keeps its h
+ * tests and drops the score sums), from the same counters as pert_shade_fwd, and the winner histogram stays in shared
+ * memory.  For the same problem (seeds, flags, noise) the image equals pert_shade_fwd's bit for bit, and no buffer
+ * depends on S_rast or S_agg.  Same flags and flag rules as pert_shade_fwd (PERT_F_CAUCHY, PERT_F_NO_VR, PERT_F_PHILOX7,
+ * explicit noise, face_colors, pixel_offset, seed_device); single calls only: any PERT_PH_* bit, or a sample shard
+ * other than [0, S), returns PERT_E_UNSUPPORTED.  Workspaces (caller-allocated):
+ *   worklist   int32 4 + pert_num_tiles, 16-byte aligned, optional (NULL: sparse-first mode off), as in pert_shade_fwd
+ *   counts_ws  uint16 (P,K), required when the sparse-first mode can run (worklist set, in-kernel Gaussian noise without
+ *              PERT_F_NO_SKIP / PER_SAMPLE_NOISE / CAUCHY / NO_VR): its fallback pass runs as two launches and keeps the
+ *              counts of its tiles here between them.  Unused (may be NULL) otherwise
+ */
+int pert_shade_render(const pert_problem* pb, float* image, uint16_t* counts_ws, int32_t* worklist, void* stream);
+
+/*
  * Backward.  grad_image (P,4).  Outputs grad_dists, grad_zbuf (P,K), grad_colors (P,K,3; may be
  * NULL), grad_scalars float[3] = d/d(sigma, gamma, alpha).  With pb->face_colors set, grad_colors is
  * instead float (num_faces,3), ZEROED BY THE CALLER, and receives w_k * dL/drgb by atomic adds (the

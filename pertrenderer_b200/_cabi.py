@@ -31,7 +31,7 @@ PH_BWD_SAMPLE, PH_BWD_FINISH = 0x100, 0x200
 
 EXPORTS = [
     "pert_version", "pert_shade_fused_flags", "pert_strerror", "pert_last_cuda_error", "pert_num_tiles", "pert_winner_bytes", "pert_blob_bytes",
-    "pert_shade_fwd", "pert_shade_bwd", "pert_soft_shade_fwd", "pert_soft_shade_bwd", "pert_rast_fwd", "pert_rast_bwd", "pert_argmax_fwd",
+    "pert_shade_fwd", "pert_shade_render", "pert_shade_bwd", "pert_soft_shade_fwd", "pert_soft_shade_bwd", "pert_rast_fwd", "pert_rast_bwd", "pert_argmax_fwd",
     "pert_argmax_bwd", "pert_noise_fill", "pert_seed_advance", "pert_phong_fwd", "pert_phong_bwd", "pert_rasterize_fwd", "pert_rasterize_bwd", "pert_rasterize_num_bins", "pert_rasterize_bin",
 ]
 
@@ -188,6 +188,27 @@ def require_fused_flags(flags: int):
         raise PertLibraryError(
             f"{LIB_PATH} predates the fused GaussianRast_wovr + GaussianAgg_wovr pair (PERT_F_NO_VR in pert_shade_fwd / "
             "pert_shade_bwd): rebuild it with `python -m pertrenderer_b200.build --force`")
+
+
+_render = None  # (library, its bound pert_shade_render)
+
+
+def shade_render_fn():
+    """``pert_shade_render`` of the loaded library, bound on first use rather than in :func:`load`, so that a library
+    built before the forward-only render keeps serving every other call; with such a library this raises
+    PertLibraryError asking for a rebuild."""
+    global _render
+    lib = load()
+    if _render is None or _render[0] is not lib:
+        fn = getattr(lib, "pert_shade_render", None)
+        if fn is None:
+            raise PertLibraryError(
+                f"{LIB_PATH} predates the forward-only render (pert_shade_render): rebuild it with "
+                "`python -m pertrenderer_b200.build --force`")
+        fn.restype = C.c_int
+        fn.argtypes = [C.POINTER(PertProblem)] + [C.c_void_p] * 4
+        _render = (lib, fn)
+    return _render[1]
 
 
 def check(rc: int, what: str):

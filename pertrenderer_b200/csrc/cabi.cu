@@ -261,6 +261,35 @@ extern "C" int64_t pert_blob_bytes(const pert_problem* pb) {
 
 static bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
 
+// Launch records of a single forward call: `a` (pointers set) gets the main pass's tile geometry and, in sparse-first mode,
+// `fb` the fallback pass's (half-size tiles, full capacity).  Returns 1 in sparse-first mode, 0 without it, or a PERT_E_*.
+static int fwd_launch_records(FwdArgs& a, FwdArgs& fb, bool sparse) {
+    const int64_t P = a.pb.N * a.pb.H * a.pb.W;
+    if (sparse) {  // the fallback pass runs FBT/32 warps per CTA: its tiles must fit that many times
+        SmemLayout t;
+        const int tp2 = sparse_tp(a.pb.K, P) / 2;
+        fwd_smem_layout(tp2, tp2 * a.pb.K, 0, t);
+        if ((size_t)t.bytes * (FBT / 32) > 200 * 1024) sparse = false;
+    }
+    a.L = make_launch(&a.pb, sparse ? sparse_tp(a.pb.K, P) : dense_tp(a.pb.K, P));
+    a.L.vec_ok = a.L.vec_ok && aligned16(a.pb.pix_to_face);
+    if (sparse) a.L.cap = sparse_cap(a.pb.K, a.L.tp);
+    a.L.stage_bytes = stage_bytes_for(a.L.tp, a.pb.K, false);
+    fwd_smem_layout(a.L.tp, a.L.cap, a.L.stage_bytes, a.L.sm);
+    a.L.warp_smem = a.L.sm.bytes;
+    if ((size_t)a.L.warp_smem > 200 * 1024) return PERT_E_UNSUPPORTED;
+    if (a.L.ntiles > 0x7fffffff) return PERT_E_UNSUPPORTED;
+    if (!sparse) return 0;
+    fb = a;
+    fb.blob = nullptr;
+    fb.L = make_launch(&a.pb, a.L.tp / 2);
+    fb.L.vec_ok = fb.L.vec_ok && aligned16(a.pb.pix_to_face);
+    fb.L.stage_bytes = stage_bytes_for(fb.L.tp, a.pb.K, true);
+    fb.L.warp_smem_rast = fwd_smem_layout(fb.L.tp, fb.L.cap, fb.L.stage_bytes, fb.L.sm);
+    fb.L.warp_smem = fb.L.sm.bytes;
+    return 1;
+}
+
 extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t* counts, float* rsum, void* winners,
                               uint16_t* pixstate, int32_t* hist, int32_t* worklist, void* tile_blob, void* stream) {
     int rc = check_problem(pb_in);
@@ -281,21 +310,6 @@ extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t*
     const uint32_t all = PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
     if ((f & PERT_F_PHILOX7) && ((f & all) != all || hist || a.pb.noise_rast || a.pb.noise_agg)) return PERT_E_UNSUPPORTED;
     if (cauchy_flags_bad(f) || no_vr_flags_bad(f)) return PERT_E_UNSUPPORTED;
-    bool sparse = sparse_first_ok(&a.pb, worklist, (f & all) == all && !hist);
-    if (sparse) {  // the fallback pass runs FBT/32 warps per CTA: its tiles must fit that many times
-        SmemLayout t;
-        const int tp2 = sparse_tp(a.pb.K, a.pb.N * a.pb.H * a.pb.W) / 2;
-        fwd_smem_layout(tp2, tp2 * a.pb.K, 0, t);
-        if ((size_t)t.bytes * (FBT / 32) > 200 * 1024) sparse = false;
-    }
-    a.L = make_launch(&a.pb, sparse ? sparse_tp(a.pb.K, a.pb.N * a.pb.H * a.pb.W) : dense_tp(a.pb.K, a.pb.N * a.pb.H * a.pb.W));
-    a.L.vec_ok = a.L.vec_ok && aligned16(a.pb.pix_to_face);
-    if (sparse) a.L.cap = sparse_cap(a.pb.K, a.L.tp);
-    a.L.stage_bytes = stage_bytes_for(a.L.tp, a.pb.K, false);
-    fwd_smem_layout(a.L.tp, a.L.cap, a.L.stage_bytes, a.L.sm);
-    a.L.warp_smem = a.L.sm.bytes;
-    if ((size_t)a.L.warp_smem > 200 * 1024) return PERT_E_UNSUPPORTED;
-    if (a.L.ntiles > 0x7fffffff) return PERT_E_UNSUPPORTED;
     a.image = image;
     a.counts = counts;
     a.rsum = rsum;
@@ -303,20 +317,53 @@ extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t*
     a.pixstate = pixstate;
     a.hist = hist;
     a.worklist = worklist;
+    a.blob = nullptr;
+    FwdArgs fb;
+    rc = fwd_launch_records(a, fb, sparse_first_ok(&a.pb, worklist, (f & all) == all && !hist));
+    if (rc < 0) return rc;
+    const bool sparse = rc == 1;
     if ((uintptr_t)tile_blob & 15) return PERT_E_ALIGN;
     a.blob = sparse ? (int32_t*)tile_blob : nullptr;
     cudaStream_t st = (cudaStream_t)stream;
     if (!sparse) return cuda_rc(launch_shade_fwd(a, nullptr, st));
-    FwdArgs fb = a;  // fallback pass: half-size tiles, full capacity
-    fb.blob = nullptr;
-    fb.L = make_launch(&a.pb, a.L.tp / 2);
-    fb.L.vec_ok = fb.L.vec_ok && aligned16(a.pb.pix_to_face);
-    fb.L.stage_bytes = stage_bytes_for(fb.L.tp, a.pb.K, true);
-    fb.L.warp_smem_rast = fwd_smem_layout(fb.L.tp, fb.L.cap, fb.L.stage_bytes, fb.L.sm);
-    fb.L.warp_smem = fb.L.sm.bytes;
     cudaError_t e = cudaMemsetAsync(worklist, 0, 16, st);
     if (e != cudaSuccess) return cuda_fail((int)e);
     return cuda_rc(launch_shade_fwd(a, &fb, st));
+}
+
+extern "C" int pert_shade_render(const pert_problem* pb_in, float* image, uint16_t* counts_ws, int32_t* worklist,
+                                 void* stream) {
+    int rc = check_problem(pb_in);
+    if (rc) return rc;
+    FwdArgs a = {};
+    a.pb = *pb_in;
+    const uint32_t f = a.pb.flags;
+    // one call renders every sample: the phase-split (sample-sharded) forward has no forward-only form
+    if (f & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND | PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH)) return PERT_E_UNSUPPORTED;
+    if (a.pb.s_rast_begin != 0 || a.pb.s_rast_end != a.pb.S_rast || a.pb.s_agg_begin != 0 || a.pb.s_agg_end != a.pb.S_agg)
+        return PERT_E_UNSUPPORTED;
+    if (!image || (!a.pb.colors && !a.pb.face_colors)) return PERT_E_NULL;
+    if (((uintptr_t)image & 15) || ((uintptr_t)counts_ws & 1) || ((uintptr_t)a.pb.colors & 3) || ((uintptr_t)worklist & 15))
+        return PERT_E_ALIGN;
+    if ((f & PERT_F_PHILOX7) && (a.pb.noise_rast || a.pb.noise_agg)) return PERT_E_UNSUPPORTED;
+    if (cauchy_flags_bad(f) || no_vr_flags_bad(f)) return PERT_E_UNSUPPORTED;
+    // the pair without control variates differs from the Gaussian pair in rsum only, which a render does not produce: its
+    // counts, histogram and image are those of the Gaussian per-sample path (no compound sampler), on the same tiles
+    if (f & PERT_F_NO_VR) a.pb.flags |= PERT_F_PER_SAMPLE_NOISE;
+    // the fallback pass of the sparse-first mode keeps its counts in counts_ws; no other mode touches it
+    const bool sparse_ok = sparse_first_ok(&a.pb, worklist, true);
+    if (sparse_ok && !counts_ws) return PERT_E_NULL;
+    a.image = image;
+    a.counts = counts_ws;
+    a.worklist = worklist;
+    FwdArgs fb;
+    rc = fwd_launch_records(a, fb, sparse_ok);
+    if (rc < 0) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (rc == 0) return cuda_rc(launch_shade_render(a, nullptr, st));
+    cudaError_t e = cudaMemsetAsync(worklist, 0, 16, st);
+    if (e != cudaSuccess) return cuda_fail((int)e);
+    return cuda_rc(launch_shade_render(a, &fb, st));
 }
 
 extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image, const uint16_t* counts,

@@ -59,8 +59,12 @@ __device__ __forceinline__ void fwd_init_barrier(const FwdArgs& a, unsigned char
 // WOVR = true: the estimator without control variates (PERT_F_NO_VR): rsum = sum_s h psi(U), so an entry that is
 // covered by every sample still draws them all; only the side x < -sigma*Umax (h = 0 always) is skipped, and the
 // compound sampler (which produces sum_s (h - h0) U only) is compiled out.  Counts, winners and image are unchanged.
+// RENDER = true: the forward-only render (pert_shade_render): nothing is stored for backward (no rsum, winners, pixstate
+// or tile blob); coverage computes counts only, from the same counters, so counts, histogram and image are those of the
+// training forward.  Counts go to global memory only in the coverage-sample launch of a split fallback pass (a.counts is
+// then the caller's S-independent workspace), which the aggregation launch reads back.
 template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int CPH = 0x70, int SCORE = 0,
-          bool WOVR = false>
+          bool WOVR = false, bool RENDER = false>
 __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& noise_r, const NoiseA& noise_a,
                                                const int64_t tile, unsigned char* smem_raw, const int lane) {
     const pert_problem& pb = a.pb;
@@ -130,8 +134,8 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
 #pragma unroll 1
             for (int i = lane; i < npx * K1; i += 32) ghist[pix0 * K1 + i] = ((i % K1) == K) ? sa_loc : 0;
         }
-        if (do_agg && lane < npx) a.pixstate[pix0 + lane] = (uint16_t)K;
-        if (!PHASED && a.blob && lane == 0) a.blob[tile * (int64_t)blob_words(tp, a.L.cap)] = 0;
+        if (!RENDER && do_agg && lane < npx) a.pixstate[pix0 + lane] = (uint16_t)K;
+        if (!PHASED && !RENDER && a.blob && lane == 0) a.blob[tile * (int64_t)blob_words(tp, a.L.cap)] = 0;
         if (do_blend && lane < npx)
             reinterpret_cast<float4*>(a.image)[pix0 + lane] =
                 make_float4(pb.background[0], pb.background[1], pb.background[2], 0.0f);
@@ -166,7 +170,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
                 cmp = need && fabsf(x) >= x_cmp;
                 if (!need) {
                     cnt[n] = (x >= 0.0f) ? (uint16_t)sr_loc : (uint16_t)0;
-                    rs[n] = 0.0f;
+                    if constexpr (!RENDER) rs[n] = 0.0f;
                 }
             } else {
                 cnt[n] = counts_t[e];
@@ -212,17 +216,22 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
             if (nblist > 0) {
                 const CompoundCtx<NoiseR> cc{noise_r, vlist, xs, cnt, rs, K, a.L.invK, pix0, a.L.inv_sigma, sr_loc,
                                              0x40000000u + 2u * (uint32_t)(pb.s_rast_begin >> 2)};
-                rast_compound_list(cc, blist, nblist, a.L.t_bucket[0] * pb.sigma, a.L.t_bucket[1] * pb.sigma, ring);
+                if constexpr (RENDER)
+                    rast_compound_count_list(cc, blist, nblist, a.L.t_bucket[0] * pb.sigma, a.L.t_bucket[1] * pb.sigma, ring);
+                else
+                    rast_compound_list(cc, blist, nblist, a.L.t_bucket[0] * pb.sigma, a.L.t_bucket[1] * pb.sigma, ring);
             }
         }
-        rast_sample_list<NoiseR, SCORE, WOVR>(noise_r, rlist, nlist, vlist, xs, cnt, rs, K, a.L.invK, pix0, pb.sigma, a.L.inv_sigma, pb.s_rast_begin,
+        rast_sample_list<NoiseR, SCORE, WOVR, RENDER>(noise_r, rlist, nlist, vlist, xs, cnt, rs, K, a.L.invK, pix0, pb.sigma, a.L.inv_sigma, pb.s_rast_begin,
                          pb.s_rast_end, !no_skip, a.L.lpe_r);
         __syncwarp();
+        if (!RENDER || !do_agg) {
 #pragma unroll 1
-        for (int n = lane; n < nv; n += 32) {
-            const int e = vlist[n];
-            counts_t[e] = cnt[n];
-            rsum_t[e] = rs[n];
+            for (int n = lane; n < nv; n += 32) {
+                const int e = vlist[n];
+                counts_t[e] = cnt[n];
+                if constexpr (!RENDER) rsum_t[e] = rs[n];
+            }
         }
     }
     if (!do_agg && !do_blend) return;
@@ -338,6 +347,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
                         const int s = q * 4 + t;
                         if (s >= pb.s_agg_begin && s < pb.s_agg_end && bi[t] != pa0) atomicAdd(&hl[plb + bi[t]], 1);
                     }
+                    if constexpr (RENDER) continue;  // the histogram stays on chip; no winners
                     const int s0 = q * 4 - pb.s_agg_begin;
                     if (pack && q * 4 + 3 < pb.s_agg_end) {
                         reinterpret_cast<uint32_t*>(a.winners)[(pgp * sa_loc + s0) >> 2] =
@@ -360,9 +370,9 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
         active = others > 0;
         if (pvalid && lig == 0) {
             hl[lb + a0l] = sa_loc - others;
-            a.pixstate[gp] = (uint16_t)(pi.a0 | (active ? 0x8000 : 0));
+            if constexpr (!RENDER) a.pixstate[gp] = (uint16_t)(pi.a0 | (active ? 0x8000 : 0));
         }
-        if (!PHASED && a.blob) {
+        if (!PHASED && !RENDER && a.blob) {
             // what backward would recompute from pix_to_face / zbuf / counts (layout: common.cuh)
             int32_t* const bl = a.blob + tile * (int64_t)blob_words(tp, cap);
             if (lane == 0) bl[0] = nv;
@@ -476,9 +486,9 @@ __global__ void __launch_bounds__(FNT, (SCORE || WOVR) ? 24 : 32) shade_fwd_kern
 // the coverage-sample launch makes room for them -- were measured at -1 % / 0 %: the passes are bound by the FMA and ALU
 // pipes, not by latency; profiles/r2_notes.md)
 constexpr int FB_MIN_CTAS = 12;
-template <class NoiseR, class NoiseA, int GT, int CPH>
-__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
-    extern __shared__ __align__(16) unsigned char smem_all[];
+template <class NoiseR, class NoiseA, int GT, int CPH, bool RENDER>
+__device__ __forceinline__ void fwd_fallback_loop(const FwdArgs& a, const NoiseR& noise_r, const NoiseA& noise_a,
+                                                  unsigned char* smem_all) {
     // FBT/32 independent warps per CTA; the coverage-sample launch of a split pass carries the front of the layout only
     unsigned char* smem_raw = smem_all + (threadIdx.x >> 5) * (CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem);
     const int n = 2 * a.worklist[0];
@@ -500,9 +510,15 @@ __global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(co
         if (i >= n) break;
         const int64_t tile = (int64_t)a.worklist[4 + (i >> 1)] * 2 + (i & 1);
         if (tile < a.L.ntiles)
-            shade_fwd_tile<NoiseR, NoiseA, GT, false, false, CPH>(a, nr, na, tile, smem_raw, threadIdx.x & 31);
+            shade_fwd_tile<NoiseR, NoiseA, GT, false, false, CPH, 0, false, RENDER>(a, nr, na, tile, smem_raw, threadIdx.x & 31);
         __syncwarp();
     }
+}
+
+template <class NoiseR, class NoiseA, int GT, int CPH>
+__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
+    extern __shared__ __align__(16) unsigned char smem_all[];
+    fwd_fallback_loop<NoiseR, NoiseA, GT, CPH, false>(a, noise_r, noise_a, smem_all);
 }
 
 template <class NR, class NA, int GT, bool PHASED, bool DEFER = false, int SCORE = 0, bool WOVR = false>
@@ -603,6 +619,112 @@ int launch_shade_fwd(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
     if (er && ea) return launch_fwd_t<ExplicitNoise, ExplicitNoise, 0, true>(a, xr, xa, st);
     if (er) return launch_fwd_t<ExplicitNoise, PhiloxNoise, 0, true>(a, xr, pa, st);
     return launch_fwd_t<PhiloxNoise, ExplicitNoise, 0, true>(a, pr, xa, st);
+}
+
+// ---- forward-only render (pert_shade_render) ----------------------------------------------------------------------
+// The forward above with RENDER = true (shade_fwd_tile): single calls only, nothing saved for backward.  Separate kernel
+// templates, so that the training kernels keep their code.  The Gaussian production path (sparse-first main pass, its
+// split fallback pass, Philox-10 or -7) and the dense instantiation (explicit noise, Cauchy) have render twins; the pair
+// without control variates renders on the Gaussian per-sample path, whose counts, histogram and image it shares.
+// CTAs per SM: 28 (72 registers; at 64 the Philox-10 and explicit-noise renders spill), 24 for Cauchy as in training.
+template <class NoiseR, class NoiseA, int GT, bool DEFER = false, int SCORE = 0>
+__global__ void __launch_bounds__(FNT, SCORE ? 24 : 28) shade_render_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    NoiseR nr = noise_r;
+    NoiseA na = noise_a;
+    if (a.pb.seed_device) {
+        nr.mix(__ldg(a.pb.seed_device));
+        na.mix(__ldg(a.pb.seed_device + 1));
+    }
+#ifdef PERT_EXPERIMENTS
+    if (a.L.stage_bytes) fwd_init_barrier(a, smem_raw);
+#endif
+    shade_fwd_tile<NoiseR, NoiseA, GT, false, DEFER, 0x70, SCORE, false, true>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x);
+}
+
+// split fallback pass of the render: CPH = PERT_PH_RAST writes the counts to the workspace, CPH = AGG | BLEND reads them
+template <class PN, int GT, int CPH>
+__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_render_fallback_kernel(const FwdArgs a, const PN noise_r, const PN noise_a) {
+    extern __shared__ __align__(16) unsigned char smem_all[];
+    fwd_fallback_loop<PN, PN, GT, CPH, true>(a, noise_r, noise_a, smem_all);
+}
+
+template <class NR, class NA, int GT, bool DEFER = false, int SCORE = 0>
+static int launch_render_t(const FwdArgs& a, const NR& nr, const NA& na, cudaStream_t st) {
+    const size_t smem = (size_t)a.L.warp_smem;
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(shade_render_kernel<NR, NA, GT, DEFER, SCORE>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+    }
+    shade_render_kernel<NR, NA, GT, DEFER, SCORE><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na);
+    return (int)cudaGetLastError();
+}
+
+template <class PN, int GT, int CPH>
+static int launch_render_fallback_ph(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
+    const size_t smem = (size_t)(CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem) * (FBT / 32);
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(shade_render_fallback_kernel<PN, GT, CPH>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+    }
+    shade_render_fallback_kernel<PN, GT, CPH><<<resident_grid(shade_render_fallback_kernel<PN, GT, CPH>, FBT, smem), FBT, smem, st>>>(a, nr, na);
+    return (int)cudaGetLastError();
+}
+
+template <class PN, int GT>
+static int launch_render_fallback(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
+    const int rc = launch_render_fallback_ph<PN, GT, PERT_PH_RAST>(a, nr, na, st);
+    return rc ? rc : launch_render_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND>(a, nr, na, st);
+}
+
+template <class PN>
+static int launch_render_production(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
+    const PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
+    int rc;
+    if (fb) {
+        switch (a.L.G) {
+            case 1: rc = launch_render_t<PN, PN, 1, true>(a, pr, pa, st); break;
+            case 2: rc = launch_render_t<PN, PN, 2, true>(a, pr, pa, st); break;
+            case 4: rc = launch_render_t<PN, PN, 4, true>(a, pr, pa, st); break;
+            default: rc = launch_render_t<PN, PN, 8, true>(a, pr, pa, st); break;
+        }
+    } else {
+        switch (a.L.G) {
+            case 1: rc = launch_render_t<PN, PN, 1>(a, pr, pa, st); break;
+            case 2: rc = launch_render_t<PN, PN, 2>(a, pr, pa, st); break;
+            case 4: rc = launch_render_t<PN, PN, 4>(a, pr, pa, st); break;
+            default: rc = launch_render_t<PN, PN, 8>(a, pr, pa, st); break;
+        }
+    }
+    if (rc || !fb) return rc;
+    switch (fb->L.G) {
+        case 2: return launch_render_fallback<PN, 2>(*fb, pr, pa, st);
+        case 4: return launch_render_fallback<PN, 4>(*fb, pr, pa, st);
+        case 8: return launch_render_fallback<PN, 8>(*fb, pr, pa, st);
+        default: return launch_render_fallback<PN, 16>(*fb, pr, pa, st);
+    }
+}
+
+// runtime lanes per pixel: explicit noise in either stage (PN = the in-kernel stream of the other), or the Cauchy pair
+template <class PN, int SCORE>
+static int launch_render_dense(const FwdArgs& a, cudaStream_t st) {
+    const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
+    PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
+    ExplicitNoise xr{a.pb.noise_rast, a.L.P, a.pb.K, a.pb.S_rast}, xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
+    if (er && ea) return launch_render_t<ExplicitNoise, ExplicitNoise, 0, false, SCORE>(a, xr, xa, st);
+    if (er) return launch_render_t<ExplicitNoise, PN, 0, false, SCORE>(a, xr, pa, st);
+    if (ea) return launch_render_t<PN, ExplicitNoise, 0, false, SCORE>(a, pr, xa, st);
+    if constexpr (SCORE != 0) return launch_render_t<PN, PN, 0, false, SCORE>(a, pr, pa, st);
+    return (int)cudaErrorInvalidValue;  // not reached: in-kernel Gaussian noise renders on the production kernels
+}
+
+int launch_shade_render(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
+    if (a.pb.flags & PERT_F_CAUCHY) return launch_render_dense<PhiloxCauchy, 1>(a, st);
+    if (a.pb.noise_rast || a.pb.noise_agg) return launch_render_dense<PhiloxNoise, 0>(a, st);
+    return (a.pb.flags & PERT_F_PHILOX7) ? launch_render_production<PhiloxNoise7>(a, fb, st)
+                                         : launch_render_production<PhiloxNoise>(a, fb, st);
 }
 
 }  // namespace pert

@@ -136,9 +136,10 @@ __device__ __forceinline__ void pixel_ranges(const uint16_t* vlist, int nv, int 
 //   saved for backward: cnt = sum_s h, rs = sum_s (h - h0) psi(U)   (smoothrast.py:46,49; psi = noise_score<SCORE>)
 //   WOVR = true, without the control variate (randomHeaviside_wovr, smoothrast.py:61-108): rs = sum_s h psi(U); the
 //   radius gate then only applies to x < 0 (h0 = 0), where a sample that cannot flip adds nothing
+//   RENDER = true (forward-only render): counts only, rs is neither accumulated nor written; the same draws and h tests
 // rlist holds compact indices n; xs/cnt/rs are compact arrays.
 // ------------------------------------------------------------------------------------------------
-template <class NoiseT, int SCORE = 0, bool WOVR = false>
+template <class NoiseT, int SCORE = 0, bool WOVR = false, bool RENDER = false>
 __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint16_t* rlist, int nlist,
                                                  const uint16_t* vlist, const float* xs, uint16_t* cnt, float* rs,
                                                  int K, float invK, int64_t pix0, float sigma, float inv_sigma,
@@ -184,7 +185,9 @@ __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint
                             box_muller(w[hp * 2], w[hp * 2 + 1], n0, n1);
                             const bool ha = __fadd_rn(x, __fmul_rn(sigma, n0)) >= 0.0f;
                             const bool hb = __fadd_rn(x, __fmul_rn(sigma, n1)) >= 0.0f;
-                            if constexpr (WOVR) {
+                            if constexpr (RENDER) {
+                                c += (in0 && ha ? 1 : 0) + (in1 && hb ? 1 : 0);
+                            } else if constexpr (WOVR) {
                                 if (in0) {
                                     c += ha ? 1 : 0;
                                     if (ha) r += n0;
@@ -217,7 +220,8 @@ __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint
                         const bool h = __fadd_rn(x, __fmul_rn(sigma, nz[t])) >= 0.0f;
                         if (s >= s_begin && s < s_end) {
                             c += h ? 1 : 0;
-                            if constexpr (WOVR) {
+                            if constexpr (RENDER) {
+                            } else if constexpr (WOVR) {
                                 if (h) r += noise_score<SCORE>(nz[t]);
                             } else if (h != h0) {
                                 r += h ? noise_score<SCORE>(nz[t]) : -noise_score<SCORE>(nz[t]);
@@ -230,11 +234,11 @@ __device__ __forceinline__ void rast_sample_list(const NoiseT& noise, const uint
 #pragma unroll 1
         for (int o = lpe >> 1; o > 0; o >>= 1) {
             c += __shfl_xor_sync(FULL, c, o);
-            r += __shfl_xor_sync(FULL, r, o);
+            if constexpr (!RENDER) r += __shfl_xor_sync(FULL, r, o);
         }
         if (active && lig == 0) {
             cnt[n] = (uint16_t)c;
-            rs[n] = r;
+            if constexpr (!RENDER) rs[n] = r;
         }
     }
 }
@@ -268,23 +272,19 @@ struct CompoundCtx {
     uint32_t c0;  // first counter
 };
 
-// one entry (compact index n) per calling lane; out of line: the body is bulky (erfc, log1p, expm1, erfcinv) and the
-// fused kernels are instruction-fetch sensitive
+// The number of flips F of entry n (compound_entry): one uniform, the first word of counter c0.  Also returns what the
+// tail draws need: the word quad of c0, p = Phi(-t) and t.
 template <class NoiseT>
-static __device__ __noinline__ void compound_entry(const CompoundCtx<NoiseT>& c, int n) {
-    const int e = c.vlist[n];
-    const int pix = entry_pixel(e, c.invK), k = e - pix * c.K;
-    const float x = c.xs[n];
-    const float t = fabsf(x) * c.inv_sigma;
-    const float p = 0.5f * erfcf(t * 0.70710678118654752f);
+__device__ __forceinline__ int compound_flips(const CompoundCtx<NoiseT>& c, int k, int pix, float x, uint32_t (&w)[4],
+                                              float& p, float& t) {
+    t = fabsf(x) * c.inv_sigma;
+    p = 0.5f * erfcf(t * 0.70710678118654752f);
     const float fn = (float)c.n_loc;
     const float nl = fn * log1pf(-p);
     const float sf1 = -expm1f(nl);  // P(F >= 1)
-    uint32_t w[4];
     c.noise.words(c.c0, (uint32_t)k, c.pix0 + pix, w);
     const float u = ((float)w[0] + 1.0f) * 2.3283064365386963e-10f;  // (0, 1], 2^-32 resolution near 0
     int F = 0;
-    float r = 0.0f;
     if (u <= sf1) {
         float pmf = __expf(nl), sf = sf1;
         const float ratio = __fdividef(p, 1.0f - p);
@@ -295,6 +295,22 @@ static __device__ __noinline__ void compound_entry(const CompoundCtx<NoiseT>& c,
             pmf *= ratio * __fdividef((float)(c.n_loc - F + 1), (float)F);
             sf -= pmf;
         } while (u <= sf && F < c.n_loc && (pmf > 1e-10f || (float)F < fn * p));
+    }
+    return F;
+}
+
+// one entry (compact index n) per calling lane; out of line: the body is bulky (erfc, log1p, expm1, erfcinv) and the
+// fused kernels are instruction-fetch sensitive
+template <class NoiseT>
+static __device__ __noinline__ void compound_entry(const CompoundCtx<NoiseT>& c, int n) {
+    const int e = c.vlist[n];
+    const int pix = entry_pixel(e, c.invK), k = e - pix * c.K;
+    const float x = c.xs[n];
+    uint32_t w[4];
+    float p, t;
+    const int F = compound_flips(c, k, pix, x, w, p, t);
+    float r = 0.0f;
+    if (F > 0) {
         uint32_t q = c.c0;
         int idx = 1;
 #pragma unroll 1
@@ -315,17 +331,31 @@ static __device__ __noinline__ void compound_entry(const CompoundCtx<NoiseT>& c,
     c.rs[n] = r;
 }
 
+// forward-only render: the count of entry n alone.  F is drawn from the same counter word as in compound_entry, so the
+// count is the training forward's; the tail normals, which only feed rs, are not drawn
+template <class NoiseT>
+static __device__ __noinline__ void compound_count_entry(const CompoundCtx<NoiseT>& c, int n) {
+    const int e = c.vlist[n];
+    const int pix = entry_pixel(e, c.invK), k = e - pix * c.K;
+    const float x = c.xs[n];
+    uint32_t w[4];
+    float p, t;
+    const int F = compound_flips(c, k, pix, x, w, p, t);
+    c.cnt[n] = (uint16_t)((x >= 0.0f) ? c.n_loc - F : F);
+}
+
 // The listed entries (blist[0], blist[-1], ..., blist[-(nb-1)]: compact indices, stored downwards) in warp passes of
 // entries with a similar expected number of flips, so that the lanes of a pass loop about equally long: three sweeps
 // over the list (|x| < x_b2: many flips, < x_b3: some, rest: rarely any), each compacting its entries through a
 // 64-slot ring in shared memory and running a pass whenever 32 are pending.
-template <class NoiseT>
-static __device__ __noinline__ void rast_compound_list(const CompoundCtx<NoiseT>& c, const uint16_t* blist, int nb, float x_b2,
-                                                       float x_b3, uint16_t* ring) {
+// ENTRY: compound_entry, or compound_count_entry for the forward-only render.
+template <class NoiseT, void (*ENTRY)(const CompoundCtx<NoiseT>&, int)>
+__device__ __forceinline__ void compound_sweep(const CompoundCtx<NoiseT>& c, const uint16_t* blist, int nb, float x_b2,
+                                               float x_b3, uint16_t* ring) {
     const int lane = threadIdx.x & 31;
     const unsigned lt = (1u << lane) - 1u;
     if (nb <= 32) {
-        if (lane < nb) compound_entry(c, blist[-lane]);
+        if (lane < nb) ENTRY(c, blist[-lane]);
         return;
     }
 #pragma unroll 1
@@ -342,14 +372,26 @@ static __device__ __noinline__ void rast_compound_list(const CompoundCtx<NoiseT>
             have += __popc(m);
             __syncwarp();
             if (have - done >= 32) {
-                compound_entry(c, ring[(done + lane) & 63]);
+                ENTRY(c, ring[(done + lane) & 63]);
                 done += 32;
                 __syncwarp();
             }
         }
-        if (lane < have - done) compound_entry(c, ring[(done + lane) & 63]);
+        if (lane < have - done) ENTRY(c, ring[(done + lane) & 63]);
         __syncwarp();
     }
+}
+
+template <class NoiseT>
+static __device__ __noinline__ void rast_compound_list(const CompoundCtx<NoiseT>& c, const uint16_t* blist, int nb, float x_b2,
+                                                       float x_b3, uint16_t* ring) {
+    compound_sweep<NoiseT, compound_entry<NoiseT>>(c, blist, nb, x_b2, x_b3, ring);
+}
+
+template <class NoiseT>
+static __device__ __noinline__ void rast_compound_count_list(const CompoundCtx<NoiseT>& c, const uint16_t* blist, int nb,
+                                                             float x_b2, float x_b3, uint16_t* ring) {
+    compound_sweep<NoiseT, compound_count_entry<NoiseT>>(c, blist, nb, x_b2, x_b3, ring);
 }
 
 // ------------------------------------------------------------------------------------------------

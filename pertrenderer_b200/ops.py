@@ -256,6 +256,12 @@ class ShadeSaved:
         return torch.where(active[..., None], w, a0)
 
 
+def _sparse_first(pr: ShadeProblem) -> bool:
+    """The noise and flags of the sparse-first mode of a single forward call (csrc/cabi.cu sparse_first_ok)."""
+    return pr.noise_rast is None and pr.noise_agg is None and \
+        not (pr.flags & (F_NO_SKIP | F_PER_SAMPLE_NOISE | F_CAUCHY | F_NO_VR))
+
+
 def shade_forward(pr: ShadeProblem, want_hist: bool = False, phases: int = 0, saved: Optional[ShadeSaved] = None):
     """Launch pert_shade_fwd.  Returns (image (N,H,W,4), ShadeSaved)."""
     lib = _cabi.load()
@@ -270,8 +276,7 @@ def shade_forward(pr: ShadeProblem, want_hist: bool = False, phases: int = 0, sa
             # the tile blobs are written by the production path only (in-kernel Gaussian noise, all phases in one call, no
             # global histogram, default noise flags and estimator: csrc/cabi.cu sparse_first_ok); the buffer only exists
             # then, so that a backward with other flags can never read what forward did not write
-            prod = not phases and not want_hist and pr.noise_rast is None and pr.noise_agg is None and \
-                not (pr.flags & (F_NO_SKIP | F_PER_SAMPLE_NOISE | F_CAUCHY | F_NO_VR))
+            prod = not phases and not want_hist and _sparse_first(pr)
             saved = ShadeSaved(
                 counts=alloc((N, H, W, K), dtype=torch.int16, device=dev),
                 rsum=alloc((N, H, W, K), dtype=torch.float32, device=dev),
@@ -287,6 +292,28 @@ def shade_forward(pr: ShadeProblem, want_hist: bool = False, phases: int = 0, sa
                                 ptr(saved.pixstate), ptr(saved.hist), ptr(saved.worklist), ptr(saved.blob), stream_ptr(dev))
     check(rc, "pert_shade_fwd")
     return image, saved
+
+
+def shade_render(pr: ShadeProblem, return_worklist: bool = False):
+    """Launch pert_shade_render: the image (N,H,W,4) of :func:`shade_forward` for the same problem, bit for bit, without
+    the state backward would need.  Nothing it allocates depends on the sample counts: the sparse-first work list and
+    the uint16 (N,H,W,K) counts workspace of its fallback pass (only where that mode runs), and the image.
+    ``return_worklist``: return ``(image, worklist)``; word 0 of the work list is the number of tiles the fallback pass
+    redid (None where the sparse-first mode does not run)."""
+    fn = _cabi.shade_render_fn()
+    _cabi.require_fused_flags(pr.flags)
+    if pr.s_rast != (0, pr.S_rast) or pr.s_agg != (0, pr.S_agg):
+        raise ValueError("shade_render renders all samples in one call: the sample-sharded forward needs shade_forward")
+    N, H, W, K = pr.shape
+    dev = pr.device
+    with torch.cuda.device(dev):
+        sparse = _sparse_first(pr)
+        worklist = torch.empty((4 + pr.num_tiles(),), dtype=torch.int32, device=dev) if sparse else None
+        counts_ws = torch.empty((N, H, W, K), dtype=torch.int16, device=dev) if sparse else None
+        image = torch.empty((N, H, W, 4), dtype=torch.float32, device=dev)
+        rc = fn(pr.c_struct(), ptr(image), ptr(counts_ws), ptr(worklist), stream_ptr(dev))
+    check(rc, "pert_shade_render")
+    return (image, worklist) if return_worklist else image
 
 
 def shade_backward(pr: ShadeProblem, saved: ShadeSaved, grad_image: torch.Tensor, need_colors: bool = True,

@@ -4,7 +4,9 @@
 reference's signatures, so ``MeshRenderer(rasterizer=..., shader=RandomSimpleShader(...))`` works
 unchanged.  With the (GaussianRast, GaussianAgg) pair, the Cauchy pair (ArctanRast, CauchyAgg) and the pair
 without control variates (GaussianRast_wovr, GaussianAgg_wovr) the whole chain — coverage sampling, mask, alpha, logits, perturbed argmax, blend, and the score-function
-backward — is ONE forward and ONE backward sm_100a kernel (``pert_shade_fwd`` / ``pert_shade_bwd``).
+backward — is ONE forward and ONE backward sm_100a kernel (``pert_shade_fwd`` / ``pert_shade_bwd``).  A call made
+without gradients (``torch.no_grad`` / ``torch.inference_mode``) renders with ``pert_shade_render`` instead: the same
+image, nothing saved for backward, no buffer that grows with the sample counts.
 Any other operator pair falls through to the operator-by-operator composition of the reference, where
 the perturbed operators still run on their own CUDA kernels.
 """
@@ -31,6 +33,27 @@ def _background_tuple(blend_params):
     return bg
 
 
+def _perturbed_problem(colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg) -> ops.ShadeProblem:
+    """The fused kernels' problem for one call of a perturbed pair, with its noise seeds drawn from torch's generator in
+    the reference's order: coverage draw first (smoothrast.py:21), then the optional global reseed (smoothagg.py:18-19),
+    then the aggregation draw (smoothagg.py:21).  The training forward and the forward-only render both build it here,
+    so that the same ``torch.manual_seed`` gives both the same noise."""
+    noise_r, noise_a = ops.current_explicit_noise()
+    seed_r = 0 if noise_r is not None else ops.draw_seed()
+    if cfg["fixed_noise"]:
+        torch.manual_seed(1)
+    seed_a = 0 if noise_a is not None else ops.draw_seed()
+    face = bool(cfg.get("face_colors", False))  # `colors` is then the (F,3) per-face table
+    return ops.ShadeProblem(
+        pix_to_face=pix_to_face, zbuf=zbuf, dists=dists, colors=None if face else colors,
+        face_colors=colors if face else None, znear=znear, zfar=zfar,
+        background=cfg["background"], sigma=float(sigma), gamma=float(gamma), alpha=float(alpha),
+        eps=float(cfg["eps"]), S_rast=int(cfg["S_rast"]), S_agg=int(cfg["S_agg"]),
+        seed_rast=seed_r, seed_agg=seed_a, pixel_offset=int(cfg.get("pixel_offset", 0)),
+        flags=ops.current_flags() | int(cfg.get("flags", 0)), noise_rast=noise_r, noise_agg=noise_a,
+        seed_device=None if (noise_r is not None or noise_a is not None) else ops.current_seed_device())
+
+
 class _PerturbedShade(Function):
     """Fused GaussianRast -> mask/alpha -> GaussianAgg -> blend (``cfg["flags"]`` = F_CAUCHY: ArctanRast / CauchyAgg;
     F_NO_VR: GaussianRast_wovr / GaussianAgg_wovr).
@@ -42,22 +65,7 @@ class _PerturbedShade(Function):
 
     @staticmethod
     def forward(ctx, colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg):
-        noise_r, noise_a = ops.current_explicit_noise()
-        # noise order of the reference: coverage draw first (smoothrast.py:21), then the optional
-        # global reseed (smoothagg.py:18-19), then the aggregation draw (smoothagg.py:21)
-        seed_r = 0 if noise_r is not None else ops.draw_seed()
-        if cfg["fixed_noise"]:
-            torch.manual_seed(1)
-        seed_a = 0 if noise_a is not None else ops.draw_seed()
-        face = bool(cfg.get("face_colors", False))  # `colors` is then the (F,3) per-face table
-        pr = ops.ShadeProblem(
-            pix_to_face=pix_to_face, zbuf=zbuf, dists=dists, colors=None if face else colors,
-            face_colors=colors if face else None, znear=znear, zfar=zfar,
-            background=cfg["background"], sigma=float(sigma), gamma=float(gamma), alpha=float(alpha),
-            eps=float(cfg["eps"]), S_rast=int(cfg["S_rast"]), S_agg=int(cfg["S_agg"]),
-            seed_rast=seed_r, seed_agg=seed_a, pixel_offset=int(cfg.get("pixel_offset", 0)),
-            flags=ops.current_flags() | int(cfg.get("flags", 0)), noise_rast=noise_r, noise_agg=noise_a,
-            seed_device=None if (noise_r is not None or noise_a is not None) else ops.current_seed_device())
+        pr = _perturbed_problem(colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg)
         image, saved = ops.shade_forward(pr)
         ctx.pr, ctx.saved = pr, saved
         ctx.scalars = (sigma, gamma, alpha)
@@ -149,8 +157,13 @@ def smooth_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, zne
         cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps,
                    S_rast=smoothrast.nb_samples, S_agg=smoothagg.nb_samples,
                    fixed_noise=bool(smoothagg.fixed_noise), face_colors=face, flags=flags)
-        return _PerturbedShade.apply(colors.face_colors if face else colors, fragments.dists, fragments.zbuf, smoothrast.sigma,
-                                     smoothagg.gamma, smoothagg.alpha, fragments.pix_to_face, znear, zfar, cfg)
+        args = (colors.face_colors if face else colors, fragments.dists, fragments.zbuf, smoothrast.sigma, smoothagg.gamma,
+                smoothagg.alpha, fragments.pix_to_face, znear, zfar, cfg)
+        # no gradient wanted (torch.no_grad / inference_mode): the forward-only kernels, which store nothing for backward.
+        # Decided here: inside Function.forward grad mode is always off
+        if not torch.is_grad_enabled():
+            return ops.shade_render(_perturbed_problem(*args))
+        return _PerturbedShade.apply(*args)
 
     if type(smoothrast) is SoftRast and type(smoothagg) is SoftAgg and not face:
         cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps)
