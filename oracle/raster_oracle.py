@@ -21,7 +21,7 @@ Restated from the published algorithm of that release:
 Semantics kept: pixel (0,0) is the top-left corner and NDC has +X left, +Y up; a face is a candidate for a pixel
 when the pixel centre lies inside it, or within sqrt(blur_radius) of its bounding box AND at squared distance
 < blur_radius of the triangle; zero-area faces, faces entirely behind the camera and points with interpolated
-depth < 0 are skipped; the K candidates of smallest depth are kept, ascending, ties in face order; barycentric
+depth < 0 are skipped, and with ``cull_backfaces`` so are faces with edge(v0, v1, v2) < 0; the K candidates of smallest depth are kept, ascending, ties in face order; barycentric
 coordinates are not clipped, not perspective-corrected; ``dists`` is the signed squared distance (negative
 inside); padding is -1 everywhere.  Known divergence: when MORE than K faces qualify, pytorch3d's replace-the-
 farthest rule may keep a different face among equal depths.
@@ -87,9 +87,45 @@ def point_triangle_distance(p, v0, v1, v2):
     return torch.minimum(torch.minimum(e01, e02), e12)
 
 
-def rasterize(face_verts, face_start, H, W, K, blur_radius):
+def _rasterize_pixels(pxy, v, f0, K, blur_radius, cull_backfaces):
+    """The K-deep fragments of the pixel centres pxy (P,1,2) against the faces v (Fn,3,3), Fn >= 1."""
+    Fn = v.shape[0]
+    v0, v1, v2 = (v[None, :, i, :2] for i in range(3))
+    z = v[None, :, :, 2]
+    area = edge_function(v0, v1, v2)
+    zero_area = (area <= K_EPS) & (area >= -K_EPS)
+    back = (area < 0) if cull_backfaces else torch.zeros_like(zero_area)
+    r = math.sqrt(blur_radius)
+    xs, ys = v[None, :, :, 0], v[None, :, :, 1]
+    outside = (pxy[..., 0] > xs.max(-1).values + r) | (pxy[..., 0] < xs.min(-1).values - r) | \
+              (pxy[..., 1] > ys.max(-1).values + r) | (pxy[..., 1] < ys.min(-1).values - r)
+    bary = barycentric(pxy, v0, v1, v2)  # (P,Fn,3)
+    pz = (bary * z).sum(-1)
+    dist = point_triangle_distance(pxy, v0, v1, v2)
+    inside = (bary > 0).all(-1)
+    ok = ~(z.max(-1).values < 0) & ~outside & ~zero_area & ~back & ~(pz < 0) & (inside | (dist < blur_radius))
+    key = torch.where(ok, pz, torch.full_like(pz, float("inf")))
+    order = torch.sort(key, dim=1, stable=True).indices[:, :K]  # ties keep face order
+    if Fn < K:
+        order = torch.cat((order, order.new_zeros(order.shape[0], K - Fn)), dim=1)
+    sel_ok = torch.gather(ok, 1, order)
+    if Fn < K:
+        sel_ok[:, Fn:] = False
+    g = lambda t: torch.gather(t, 1, order)  # noqa: E731
+    p2f = torch.where(sel_ok, order + f0, torch.full_like(order, -1))
+    zb = torch.where(sel_ok, g(pz), torch.full_like(g(pz), -1.0))
+    sd = torch.where(inside, -dist, dist)
+    ds = torch.where(sel_ok, g(sd), torch.full_like(zb, -1.0))
+    bc = torch.gather(bary, 1, order[..., None].expand(-1, -1, 3))
+    bc = torch.where(sel_ok[..., None], bc, torch.full_like(bc, -1.0))
+    return p2f, zb, bc, ds
+
+
+def rasterize(face_verts, face_start, H, W, K, blur_radius, cull_backfaces=False, chunk_pairs=1 << 21):
     """rasterize_meshes (naive).  face_verts (F,3,3): NDC x, y and view depth z of the packed faces;
-    face_start (N+1,): faces [face_start[n], face_start[n+1]) belong to image n.
+    face_start (N+1,): faces [face_start[n], face_start[n+1]) belong to image n (an empty range gives an image of
+    padding).  ``cull_backfaces`` drops the faces with edge(v0, v1, v2) < 0.  Pixels are evaluated in chunks of about
+    ``chunk_pairs`` (pixel, face) pairs, which bounds the memory and leaves the result unchanged.
     Returns pix_to_face (N,H,W,K) int64, zbuf, bary (N,H,W,K,3), dists (N,H,W,K), padding -1."""
     fv = face_verts
     N = len(face_start) - 1
@@ -98,34 +134,13 @@ def rasterize(face_verts, face_start, H, W, K, blur_radius):
     for n in range(N):
         f0, f1 = int(face_start[n]), int(face_start[n + 1])
         v = fv[f0:f1]  # (Fn,3,3)
-        Fn = v.shape[0]
-        v0, v1, v2 = (v[None, :, i, :2] for i in range(3))
-        z = v[None, :, :, 2]
-        area = edge_function(v0, v1, v2)
-        zero_area = (area <= K_EPS) & (area >= -K_EPS)
-        r = math.sqrt(blur_radius)
-        xs, ys = v[None, :, :, 0], v[None, :, :, 1]
-        outside = (pxy[..., 0] > xs.max(-1).values + r) | (pxy[..., 0] < xs.min(-1).values - r) | \
-                  (pxy[..., 1] > ys.max(-1).values + r) | (pxy[..., 1] < ys.min(-1).values - r)
-        bary = barycentric(pxy, v0, v1, v2)  # (HW,Fn,3)
-        pz = (bary * z).sum(-1)
-        dist = point_triangle_distance(pxy, v0, v1, v2)
-        inside = (bary > 0).all(-1)
-        ok = ~(z.max(-1).values < 0) & ~outside & ~zero_area & ~(pz < 0) & (inside | (dist < blur_radius))
-        key = torch.where(ok, pz, torch.full_like(pz, float("inf")))
-        order = torch.sort(key, dim=1, stable=True).indices[:, :K]  # ties keep face order
-        if Fn < K:
-            order = torch.cat((order, order.new_zeros(order.shape[0], K - Fn)), dim=1)
-        sel_ok = torch.gather(ok, 1, order)
-        if Fn < K:
-            sel_ok[:, Fn:] = False
-        g = lambda t: torch.gather(t, 1, order)  # noqa: E731
-        p2f = torch.where(sel_ok, order + f0, torch.full_like(order, -1))
-        zb = torch.where(sel_ok, g(pz), torch.full_like(g(pz), -1.0))
-        sd = torch.where(inside, -dist, dist)
-        ds = torch.where(sel_ok, g(sd), torch.full_like(zb, -1.0))
-        bc = torch.gather(bary, 1, order[..., None].expand(-1, -1, 3))
-        bc = torch.where(sel_ok[..., None], bc, torch.full_like(bc, -1.0))
+        if v.shape[0] == 0:
+            out.append((torch.full((H, W, K), -1, dtype=torch.int64), torch.full((H, W, K), -1.0, dtype=fv.dtype),
+                        torch.full((H, W, K, 3), -1.0, dtype=fv.dtype), torch.full((H, W, K), -1.0, dtype=fv.dtype)))
+            continue
+        step = max(1, chunk_pairs // v.shape[0])
+        parts = [_rasterize_pixels(pxy[i:i + step], v, f0, K, blur_radius, cull_backfaces) for i in range(0, H * W, step)]
+        p2f, zb, bc, ds = (torch.cat([p[i] for p in parts]) for i in range(4))
         out.append((p2f.reshape(H, W, K), zb.reshape(H, W, K), bc.reshape(H, W, K, 3), ds.reshape(H, W, K)))
     return tuple(torch.stack([o[i] for o in out]) for i in range(4))
 

@@ -410,10 +410,16 @@ __global__ void __launch_bounds__(256) rasterize_bin_kernel(const pert_raster rs
     const float area = edge(P2{v[0], v[1]}, P2{v[3], v[4]}, P2{v[6], v[7]});
     if (zmax < 0.0f || (area <= kEps && area >= -kEps) || ((rs.flags & PERT_RAST_CULL_BACKFACES) && area < 0.0f)) return;
     const int H = rs.H, W = rs.W;
-    // pixel index i (from the -X / -Y side) whose centre is x: x = -range + (2 i + 1) range / S
+    // pixel index i (from the -X / -Y side) whose centre is x: x = -range + (2 i + 1) range / S.  The float indices
+    // are clamped to [-2, S+1] before the conversion: a box reaching |x| ~ 2^32 / S or inf would otherwise saturate
+    // the conversion at INT_MAX and overflow the +-1 below.  Every test that follows gives the same answer on the
+    // clamped index.  A NaN bound clamps to the far end (fmaxf / fminf return the other operand), so it covers the
+    // whole axis, as in the unbinned kernels, whose tile test never culls on a NaN.
     const float rx = W > H ? (float)W / (float)H : 1.0f, ry = H > W ? (float)H / (float)W : 1.0f;
-    const int ix0 = (int)floorf(((xmin + rx) * (float)W / rx - 1.0f) * 0.5f) - 1, ix1 = (int)ceilf(((xmax + rx) * (float)W / rx - 1.0f) * 0.5f) + 1;
-    const int iy0 = (int)floorf(((ymin + ry) * (float)H / ry - 1.0f) * 0.5f) - 1, iy1 = (int)ceilf(((ymax + ry) * (float)H / ry - 1.0f) * 0.5f) + 1;
+    const float fx0 = floorf(((xmin + rx) * (float)W / rx - 1.0f) * 0.5f), fx1 = ceilf(((xmax + rx) * (float)W / rx - 1.0f) * 0.5f);
+    const float fy0 = floorf(((ymin + ry) * (float)H / ry - 1.0f) * 0.5f), fy1 = ceilf(((ymax + ry) * (float)H / ry - 1.0f) * 0.5f);
+    const int ix0 = (int)fminf(fmaxf(fx0, -2.0f), (float)(W + 1)) - 1, ix1 = (int)fmaxf(fminf(fx1, (float)(W + 1)), -2.0f) + 1;
+    const int iy0 = (int)fminf(fmaxf(fy0, -2.0f), (float)(H + 1)) - 1, iy1 = (int)fmaxf(fminf(fy1, (float)(H + 1)), -2.0f) + 1;
     if (ix1 < 0 || iy1 < 0 || ix0 > W - 1 || iy0 > H - 1) return;
     // image column = W-1-i, row = H-1-i
     const int cx0 = W - 1 - min(ix1, W - 1), cx1 = W - 1 - max(ix0, 0), cy0 = H - 1 - min(iy1, H - 1), cy1 = H - 1 - max(iy0, 0);

@@ -70,7 +70,7 @@ class _Rasterize(Function):
             rs = _raster_struct(fv, fs, N, H, W, K, blur_radius, cull_backfaces)
             keep = []
             if K <= 64 and fv.shape[0] >= BIN_MIN_FACES * N:
-                # large meshes: coarse bins, one candidate list per 32x8 pixel tile (two kernel passes around a prefix
+                # large meshes: coarse bins, one candidate list per 32x4 pixel tile (two kernel passes around a prefix
                 # sum; the total length of the lists is read back to size the buffer: the one host sync of this path)
                 nb = int(lib.pert_rasterize_num_bins(rs))
                 count = torch.zeros((nb,), dtype=torch.int32, device=dev)

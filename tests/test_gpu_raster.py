@@ -9,6 +9,7 @@ import torch
 
 from conftest import rel_err
 from oracle import raster_oracle as RO
+from raster_util import check_fragments
 
 pytestmark = pytest.mark.gpu
 
@@ -33,23 +34,6 @@ def _faces_ndc(n_faces, n_views, seed=0, elev=20.0):
     return fv, [i * F_ for i in range(n_views + 1)]
 
 
-def _same_fragments(got, ref, fv, blur):
-    """Exact equality except where a decision sits on a float boundary (the kernels contract a*b+c into FMAs, torch
-    does not): such pixels must be few and differ only by faces whose test was marginal."""
-    p2f_g, z_g, b_g, d_g = (t.cpu() for t in got)
-    p2f_r, z_r, b_r, d_r = ref
-    same = (p2f_g == p2f_r).all(-1)
-    assert same.float().mean() > 0.995, same.float().mean()
-    # sliver faces (projected area ~ 1e-6, e.g. next to the poles of the test sphere) have ill-conditioned barycentric
-    # coordinates (e_i / area): values are compared on well-conditioned faces only
-    sel = fv[p2f_r.clamp(min=0)]
-    area = RO.edge_function(sel[..., 0, :2], sel[..., 1, :2], sel[..., 2, :2]).abs()
-    m = same[..., None] & (p2f_r >= 0) & (area > 1e-3)
-    assert m.float().sum() > 0.5 * (p2f_r >= 0).float().sum()
-    pad = same[..., None] & (p2f_r < 0)
-    assert (z_g[pad] == -1).all() and (d_g[pad] == -1).all() and (b_g[pad] == -1).all()
-
-
 @pytest.mark.parametrize("cfg", [
     dict(n_faces=80, views=2, H=24, W=24, K=8, blur=1e-3),
     dict(n_faces=320, views=1, H=40, W=33, K=6, blur=5e-3),      # non-square, partial tiles
@@ -60,11 +44,10 @@ def _same_fragments(got, ref, fv, blur):
 def test_rasterize_forward_matches_oracle(cfg):
     import pertrenderer_b200 as pb
     fv, start = _faces_ndc(cfg["n_faces"], cfg["views"], seed=cfg["K"])
-    ref = RO.rasterize(fv, start, cfg["H"], cfg["W"], cfg["K"], cfg["blur"])
     got = pb.rasterize_meshes(fv.to(DEV), torch.tensor(start, device=DEV), (cfg["H"], cfg["W"]), cfg["blur"], cfg["K"])
     torch.cuda.synchronize()
+    ref = check_fragments(got, fv, start, cfg["H"], cfg["W"], cfg["K"], cfg["blur"])
     assert (ref[0] >= 0).float().mean() > 0.02
-    _same_fragments(got, ref, fv, cfg["blur"])
     z = got[1].cpu()
     valid = got[0].cpu() >= 0
     # ascending depth, padding last
@@ -87,7 +70,7 @@ def test_coarse_bins_give_the_same_fragments(monkeypatch):
     plain = pb.rasterize_meshes(fv.to(DEV), fs, (H, W), blur, K)
     for a, b in zip(binned, plain):
         assert torch.equal(a, b)
-    _same_fragments(binned, RO.rasterize(fv, start, H, W, K, blur), fv, blur)
+    check_fragments(binned, fv, start, H, W, K, blur)
     # gradients flow through the binned forward as well
     fvg = fv.to(DEV).requires_grad_(True)
     monkeypatch.setattr(rasterizer, "BIN_MIN_FACES", 1024)

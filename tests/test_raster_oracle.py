@@ -72,6 +72,45 @@ def test_depth_order_ties_and_k_truncation():
     assert p2f4[0, 2, 1].tolist() == [0, -1] and p2f4[1, 2, 1].tolist() == [1, 2]
 
 
+def test_cull_backfaces_drops_negative_winding_only():
+    tri = _tri()  # edge(v0, v1, v2) = -1.56: a back face
+    assert RO.edge_function(tri[0, 0, :2], tri[0, 1, :2], tri[0, 2, :2]) < 0
+    flipped = tri[:, [0, 2, 1]]
+    for fv, culled in ((tri, True), (flipped, False)):
+        plain = RO.rasterize(fv, [0, 1], 4, 4, 1, 0.0)
+        cull = RO.rasterize(fv, [0, 1], 4, 4, 1, 0.0, cull_backfaces=True)
+        assert plain[0][0, 2, 1, 0] == 0
+        if culled:
+            assert (cull[0] == -1).all() and (cull[1] == -1).all() and (cull[2] == -1).all() and (cull[3] == -1).all()
+        else:
+            for a, b in zip(plain, cull):
+                assert torch.equal(a, b)
+
+
+def test_empty_image_in_a_batch_is_padding():
+    fv = torch.cat((_tri(z=(1.0, 1.0, 1.0)), _tri(z=(2.0, 2.0, 2.0))))
+    p2f, zbuf, bary, dists = RO.rasterize(fv, [0, 1, 1, 2], 4, 4, 3, 1e-3)
+    assert p2f.shape == (3, 4, 4, 3) and bary.shape == (3, 4, 4, 3, 3)
+    for t in (p2f, zbuf, bary, dists):
+        assert (t[1] == -1).all()
+    assert p2f[0, 2, 1].tolist() == [0, -1, -1] and p2f[2, 2, 1].tolist() == [1, -1, -1]
+    assert abs(zbuf[2, 2, 1, 0].item() - 2.0) < 1e-6
+    empty = RO.rasterize(fv[:0], [0, 0], 4, 4, 2, 0.0)
+    assert all((t == -1).all() for t in empty)
+
+
+def test_pixel_chunks_do_not_change_the_result():
+    torch.manual_seed(3)
+    c = torch.rand(60, 1, 2) * 1.6 - 0.8
+    fv = torch.cat((c + 0.3 * torch.rand(60, 3, 2) - 0.15, 1.0 + torch.rand(60, 3, 1)), dim=-1).double()
+    full = RO.rasterize(fv, [0, 25, 60], 9, 13, 5, 4e-3, chunk_pairs=1 << 30)
+    for pairs in (1, 37, 60 * 50):
+        part = RO.rasterize(fv, [0, 25, 60], 9, 13, 5, 4e-3, chunk_pairs=pairs)
+        for a, b in zip(full, part):
+            assert torch.equal(a, b)
+    assert (full[0] >= 0).sum() > 50 and full[1].dtype == torch.float64
+
+
 def test_selected_fragment_gradients_match_finite_differences():
     torch.manual_seed(1)
     fv = (_tri(z=(1.0, 2.0, 3.0)) + 0.05 * torch.randn(1, 3, 3)).double()
