@@ -6,8 +6,7 @@
  * library never allocates, frees or retains device memory, never synchronises the device and launches on
  * the stream it is given.  The only state it keeps is diagnostic or immutable: the name of the calling thread's
  * last CUDA error (pert_last_cuda_error) and each device's SM count, cached at first use; it reads no environment
- * variable (tuning builds compiled with -DPERT_EXPERIMENTS do, the product never is).  Every function returns
- * PERT_OK (0) or a negative PERT_E_* code; nothing throws across the ABI.
+ * variable.  Every function returns PERT_OK (0) or a negative PERT_E_* code; nothing throws across the ABI.
  *
  * What each entry point replaces in the reference (paths relative to quentinll/pertrenderer):
  *

@@ -43,20 +43,15 @@ def is_stale() -> bool:
     return any(os.path.getmtime(p) > t for p in SOURCES + HEADERS)
 
 
-def build_library(force: bool = False, verbose: bool = False, experiments: bool = False, defines=(), out: str | None = None) -> str:
-    """Compile every translation unit (in parallel) and link libpertshade.so in-tree.  ``experiments`` defines
-    PERT_EXPERIMENTS: tuning knobs read from the environment (PERT_TP, PERT_CAP, ...); never set for the product.
-    ``defines`` / ``out``: A/B builds of compile-time choices (``--define FB_MINB_RAST=16 --out build/alt/x.so``)."""
-    if not force and not experiments and not defines and not out and not is_stale():
+def build_library(force: bool = False, verbose: bool = False) -> str:
+    """Compile every translation unit (in parallel) and link libpertshade.so in-tree."""
+    if not force and not is_stale():
         return LIB_PATH
     import concurrent.futures
     nvcc = find_nvcc()
-    lib_path = os.path.abspath(out) if out else LIB_PATH
-    obj_dir = os.path.join(os.path.dirname(HERE), "build", os.path.basename(lib_path)[:-3] if out else "")
+    obj_dir = os.path.join(os.path.dirname(HERE), "build")
     os.makedirs(obj_dir, exist_ok=True)
-    os.makedirs(os.path.dirname(lib_path), exist_ok=True)
-    compile_flags = [f for f in NVCC_FLAGS if f != "-shared"] + (["-DPERT_EXPERIMENTS"] if experiments else []) + \
-        ["-D" + d for d in defines]
+    compile_flags = [f for f in NVCC_FLAGS if f != "-shared"]
 
     def compile_one(src):
         obj = os.path.join(obj_dir, os.path.basename(src)[:-3] + ".o")
@@ -71,16 +66,13 @@ def build_library(force: bool = False, verbose: bool = False, experiments: bool 
     if verbose:
         for _, err in results:
             print(err)
-    cmd = [nvcc, "-shared", "-Xcompiler", "-fPIC", "-gencode", "arch=compute_100a,code=sm_100a", "-o", lib_path] + \
+    cmd = [nvcc, "-shared", "-Xcompiler", "-fPIC", "-gencode", "arch=compute_100a,code=sm_100a", "-o", LIB_PATH] + \
         [o for o, _ in results]
     proc = subprocess.run(cmd, capture_output=True, text=True)
     if proc.returncode != 0:
         raise RuntimeError("link failed:\n" + " ".join(cmd) + "\n" + proc.stdout + proc.stderr)
-    return lib_path
+    return LIB_PATH
 
 
 if __name__ == "__main__":
-    argv = sys.argv[1:]
-    defs = [argv[i + 1] for i, v in enumerate(argv) if v == "--define"]
-    outp = next((argv[i + 1] for i, v in enumerate(argv) if v == "--out"), None)
-    print(build_library(force="--force" in argv, verbose="-v" in argv, experiments="--experiments" in argv, defines=defs, out=outp))
+    print(build_library(force="--force" in sys.argv, verbose="-v" in sys.argv))

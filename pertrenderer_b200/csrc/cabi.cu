@@ -1,7 +1,6 @@
 // C ABI of libpertshade.so (include/pertshade.h): argument validation and launch geometry.  Nothing
 // here allocates, frees, retains or synchronises; every launch goes to the caller's stream.
 #include <math.h>
-#include <stdlib.h>
 
 #include "kernels.h"
 
@@ -39,12 +38,6 @@ extern "C" const char* pert_strerror(int code) {
 
 // pixels per warp tile: a power of two in [4, 32] with about 512 fragment entries per tile
 static int pick_tp(int K) {
-#ifdef PERT_EXPERIMENTS  // tuning builds only (python -m pertrenderer_b200.build --experiments): the product reads no environment
-    if (const char* e = getenv("PERT_TP")) {
-        const int v = atoi(e);
-        if (v == 4 || v == 8 || v == 16 || v == 32) return v;
-    }
-#endif
     if (K <= 16) return 32;
     if (K <= 32) return 16;
     if (K <= 64) return 8;
@@ -64,9 +57,6 @@ static double tail_quantile(double p) {  // t with Phi(-t) = p, 0 < p <= 0.5
 }
 static float compound_threshold(int n) {
     double pmax = 0.2;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_PCMP")) pmax = atof(e);
-#endif
     if (n > 0) {
         pmax = fmin(pmax, 1.0 - exp(-80.0 / n));
         pmax = fmin(pmax, 48.0 / n);
@@ -75,11 +65,7 @@ static float compound_threshold(int n) {
 }
 // bucket edges of the compound sampler: expected flips n p = 3 and 0.25
 static void compound_buckets(int n, float t_compound, float* out) {
-    double f0 = 3.0, f1 = 0.25;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_FB0")) f0 = atof(e);
-    if (const char* e = getenv("PERT_FB1")) f1 = atof(e);
-#endif
+    const double f0 = 3.0, f1 = 0.25;
     for (int i = 0; i < 2; ++i) {
         const double p = (i == 0 ? f0 : f1) / (n > 0 ? n : 1);
         float t = p >= 0.5 ? 0.0f : (float)tail_quantile(p);
@@ -147,24 +133,9 @@ static Launch make_launch(const pert_problem* pb, int tp) {
     L.inv_sr = 1.0f / ((float)pb->S_rast * pb->sigma);
     L.invS = 1.0f / (float)pb->S_agg;
     L.inv_gamma = 1.0f / pb->gamma;
-    L.stage_bytes = 0;
     L.t_compound = compound_threshold(pb->s_rast_end - pb->s_rast_begin);
     compound_buckets(pb->s_rast_end - pb->s_rast_begin, L.t_compound, L.t_bucket);
-    L.cmp_min = 12;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_CMP_MIN")) L.cmp_min = atoi(e);
-#endif
-    if (L.cmp_min > 32) L.cmp_min = 32;
-    L.defer_min = 48;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_DEFER_MIN")) L.defer_min = atoi(e);
-#endif
-    L.nab = 8;
-    L.lean = 0;
-    L.fb_split = 1;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_FB_SPLIT")) L.fb_split = atoi(e);
-#endif
+    L.lean = false;
     return L;
 }
 
@@ -194,18 +165,11 @@ static int dense_tp(int K, int64_t P) {
 }
 static int sparse_cap(int K, int tp) {
     int cap = tp * K / 5;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_CAP")) cap = atoi(e);
-#endif
     cap = (cap + 7) & ~7;  // u16 arrays are copied as 32-bit words
     if (cap < 32) cap = 32;
     if (cap > tp * K) cap = (tp * K + 1) & ~1;
     return cap;
 }
-
-// Active pixels staged at a time by the fallback pass of backward = the pixels of its tiles: one batch (4 rows of c_s
-// would buy a thirteenth CTA per SM and lose more to the second batch: profiles/r2_notes.md)
-constexpr int kNabFallback = 8;
 
 static bool sparse_first_ok(const pert_problem* pb, const void* worklist, bool all_phases) {
     if (!worklist || !all_phases || pb->noise_rast || pb->noise_agg) return false;
@@ -224,22 +188,6 @@ static bool cauchy_flags_bad(uint32_t f) {
 // sample (the shortcut for never-winning logits is a variance-reduced estimator's), and the forward-only noises
 static bool no_vr_flags_bad(uint32_t f) {
     return (f & PERT_F_NO_VR) && (f & (PERT_F_PHILOX7 | PERT_F_SKIP_DEAD_NOISE | PERT_F_UNIFORM | PERT_F_GUMBEL));
-}
-
-// Bulk-copy scan of the forward (tile.cuh scan_valid_staged; TMA 1-D copy + mbarrier, UBLKCP in SASS): bytes of the staging
-// buffer, 0 = register scan.  Measured and REJECTED as a default (round 2, config 2): in the main pass the 6.4 KB stage takes
-// the resident warps from 32 to 23 per SM and the sparse-set forward from 0.281 to 0.297 ms; in the fallback pass (3.2 KB
-// stage, no occupancy cost) the rasterised set gains 0.6 % and the dense set loses 0.8 %: the scan is 1.5 % of that pass's
-// instructions.  Kept behind the tuning build's PERT_BULK_SCAN / PERT_BULK_SCAN_FB for re-measurement on other shapes.
-static int stage_bytes_for(int tp, int K, bool fallback) {
-    int on = 0;
-    (void)fallback;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv(fallback ? "PERT_BULK_SCAN_FB" : "PERT_BULK_SCAN")) on = atoi(e);
-#endif
-    if (!on) return 0;
-    const int bytes = tp * K * 8;
-    return (bytes % 16 == 0 && bytes <= 16 * 1024) ? bytes : 0;
 }
 
 extern "C" int64_t pert_num_tiles(const pert_problem* pb) {
@@ -268,14 +216,13 @@ static int fwd_launch_records(FwdArgs& a, FwdArgs& fb, bool sparse) {
     if (sparse) {  // the fallback pass runs FBT/32 warps per CTA: its tiles must fit that many times
         SmemLayout t;
         const int tp2 = sparse_tp(a.pb.K, P) / 2;
-        fwd_smem_layout(tp2, tp2 * a.pb.K, 0, t);
+        fwd_smem_layout(tp2, tp2 * a.pb.K, t);
         if ((size_t)t.bytes * (FBT / 32) > 200 * 1024) sparse = false;
     }
     a.L = make_launch(&a.pb, sparse ? sparse_tp(a.pb.K, P) : dense_tp(a.pb.K, P));
     a.L.vec_ok = a.L.vec_ok && aligned16(a.pb.pix_to_face);
     if (sparse) a.L.cap = sparse_cap(a.pb.K, a.L.tp);
-    a.L.stage_bytes = stage_bytes_for(a.L.tp, a.pb.K, false);
-    fwd_smem_layout(a.L.tp, a.L.cap, a.L.stage_bytes, a.L.sm);
+    fwd_smem_layout(a.L.tp, a.L.cap, a.L.sm);
     a.L.warp_smem = a.L.sm.bytes;
     if ((size_t)a.L.warp_smem > 200 * 1024) return PERT_E_UNSUPPORTED;
     if (a.L.ntiles > 0x7fffffff) return PERT_E_UNSUPPORTED;
@@ -284,8 +231,7 @@ static int fwd_launch_records(FwdArgs& a, FwdArgs& fb, bool sparse) {
     fb.blob = nullptr;
     fb.L = make_launch(&a.pb, a.L.tp / 2);
     fb.L.vec_ok = fb.L.vec_ok && aligned16(a.pb.pix_to_face);
-    fb.L.stage_bytes = stage_bytes_for(fb.L.tp, a.pb.K, true);
-    fb.L.warp_smem_rast = fwd_smem_layout(fb.L.tp, fb.L.cap, fb.L.stage_bytes, fb.L.sm);
+    fb.L.warp_smem_rast = fwd_smem_layout(fb.L.tp, fb.L.cap, fb.L.sm);
     fb.L.warp_smem = fb.L.sm.bytes;
     return 1;
 }
@@ -395,7 +341,7 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
         const int tp2 = sparse_tp(a.pb.K, a.pb.N * a.pb.H * a.pb.W) / 2;
         const Launch t = make_launch(&a.pb, tp2);
         SmemLayout sl;
-        bwd_smem_layout(tp2, a.pb.K, t.cap, t.sc, t.nchunks, t.win_bytes, false, kNabFallback, 1, sl);
+        bwd_smem_layout(tp2, a.pb.K, t.cap, t.sc, t.nchunks, t.win_bytes, false, true, sl);
         if ((size_t)sl.bytes * (FBT / 32) > 200 * 1024) sparse = false;
     }
     const bool ptr_ok = aligned16(a.pb.pix_to_face) && aligned16(grad_dists) && aligned16(grad_zbuf) &&
@@ -404,10 +350,7 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
     a.L.vec_ok = a.L.vec_ok && ptr_ok;
     if (sparse) a.L.cap = sparse_cap(a.pb.K, a.L.tp);
     if (a.L.win_bytes == 2 && ((uintptr_t)winners & 1)) return PERT_E_ALIGN;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_LEAN_MAIN")) a.L.lean = atoi(e);
-#endif
-    bwd_smem_layout(a.L.tp, a.pb.K, a.L.cap, a.L.sc, a.L.nchunks, a.L.win_bytes, sparse, a.L.nab, a.L.lean, a.L.sm);
+    bwd_smem_layout(a.L.tp, a.pb.K, a.L.cap, a.L.sc, a.L.nchunks, a.L.win_bytes, sparse, a.L.lean, a.L.sm);
     a.L.warp_smem = a.L.sm.bytes;
     if ((size_t)a.L.warp_smem > 200 * 1024) return PERT_E_UNSUPPORTED;
     if (a.L.ntiles > 0x7fffffff) return PERT_E_UNSUPPORTED;
@@ -432,15 +375,8 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
     fb.blob = nullptr;
     fb.L = make_launch(&a.pb, a.L.tp / 2);
     fb.L.vec_ok = fb.L.vec_ok && ptr_ok;
-    fb.L.nab = kNabFallback;
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_NAB_FB")) fb.L.nab = atoi(e);
-#endif
-    fb.L.lean = 1;  // pair list in the counts array; the winners ARE staged (+3 %), the layout still fits 12 CTAs per SM
-#ifdef PERT_EXPERIMENTS
-    if (const char* e = getenv("PERT_LEAN_FB")) fb.L.lean = atoi(e);
-#endif
-    bwd_smem_layout(fb.L.tp, a.pb.K, fb.L.cap, fb.L.sc, fb.L.nchunks, fb.L.win_bytes, false, fb.L.nab, fb.L.lean, fb.L.sm);
+    fb.L.lean = true;  // pair list in the counts array; the winners ARE staged (+3 %), the layout still fits 12 CTAs per SM
+    bwd_smem_layout(fb.L.tp, a.pb.K, fb.L.cap, fb.L.sc, fb.L.nchunks, fb.L.win_bytes, false, fb.L.lean, fb.L.sm);
     fb.L.warp_smem = fb.L.sm.bytes;
     cudaError_t e = cudaMemsetAsync(worklist, 0, 16, st);
     if (e != cudaSuccess) return cuda_fail((int)e);

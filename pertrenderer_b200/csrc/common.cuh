@@ -198,13 +198,8 @@ struct Launch {
     float inv_sigma, invSg, inv_sr, invS;  // 1/sigma, 1/(S_agg gamma), 1/(S_rast sigma), 1/S_agg
     float inv_gamma;  // 1/gamma (SoftAgg, smoothagg.py:181)
     float t_compound; // coverage entries with |x|/sigma >= this are drawn by the compound sampler (tile.cuh)
-    int stage_bytes;   // forward: bytes of the pix_to_face staging buffer of the bulk-copy scan (0: register scan)
-    int cmp_min;       // fewer compound entries than this in a tile are drawn by the per-sample loop instead
-    int nab;           // backward: active pixels whose per-sample c_s are staged at a time (<= 8; shared memory = occupancy)
-    int lean;          // backward: lean shared-memory layout (shade_bwd.cu bwd_smem_layout)
-    int fb_split;      // fallback pass of the forward as two launches (coverage samples | aggregation + blend)
-    int defer_min;     // main pass of the sparse-first mode: tiles with at least this many go to the fallback pass
     float t_bucket[2]; // ... and bucketed by expected flips: [t_compound, t_bucket[0]) many, [.., t_bucket[1]) some, rest rare
+    bool lean;         // backward: the pair list takes over the counts array (shade_bwd.cu bwd_smem_layout)
 };
 
 // 16-byte asynchronous global -> shared copy (LDGSTS) and its completion wait

@@ -36,8 +36,8 @@ struct BwdArgs {
     const int32_t* blob;  // tile blobs of forward, or NULL: backward then rescans and recomputes
 };
 
-int fwd_smem_layout(int tp, int cap, int stage_bytes, SmemLayout& L);  // returns the bytes the coverage-sample phase needs
-void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes, bool compact, int nab, int lean, SmemLayout& L);
+int fwd_smem_layout(int tp, int cap, SmemLayout& L);  // returns the bytes the coverage-sample phase needs
+void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes, bool compact, bool lean, SmemLayout& L);
 
 // return a cudaError_t as int (0 = success)
 // `fb` (optional): launch record of the fallback pass of the sparse-first mode (half-size tiles)

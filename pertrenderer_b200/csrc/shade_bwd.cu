@@ -16,32 +16,36 @@
 //      regenerated from the Philox counters
 //   4  chain rule per valid entry -> scattered stores over the zero-filled rows; scalar partials
 #include <climits>
-#include <cstdlib>
 #include "kernels.h"
 #include "tile.cuh"
 
 namespace pert {
 
-// lean (the passes' time follows the warps an SM holds, i.e. the bytes of this layout): bit 0 = the pair list takes over
-// the counts array (phase 4 reads the counts from global memory instead), bit 1 = the saved winners are not staged
-void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes, bool compact, int nab, int lean, SmemLayout& L) {
+// Active pixels whose per-sample c_s are staged at a time (<= 8: the pair codes hold the rank in 3 bits; shared memory =
+// occupancy).  In the fallback pass that is the pixels of its tiles: one batch (4 rows of c_s would buy a thirteenth CTA per
+// SM and lose more to the second batch: profiles/r2_notes.md)
+constexpr int kNab = 8;
+
+// lean (the passes' time follows the warps an SM holds, i.e. the bytes of this layout): the pair list takes over the counts
+// array (phase 4 reads the counts from global memory instead)
+void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes, bool compact, bool lean, SmemLayout& L) {
     const size_t ns = compact ? (size_t)cap + 2 * tp : (size_t)tp * (K + 1);
     Carver cv(L);
     cv.take(cap, 2);  // vlist
     cv.take(ns > (size_t)cap ? ns : (size_t)cap, 4);  // zs, then accs (the logits are dead once the live ones are marked)
-    cv.take((lean & 1) && ns > (size_t)cap ? ns : (size_t)cap, 2);  // cnt (lean & 1: then the pair list)
+    cv.take(lean && ns > (size_t)cap ? ns : (size_t)cap, 2);  // cnt (lean: then the pair list)
     cv.take(ns, 4);   // hj
     cv.take(ns, 4);   // gsel (| t2s when there is one sample chunk)
     cv.take(nchunks > 1 ? ns : 0, 4);  // t2s
-    cv.take((lean & 1) ? 0 : ns, 2);   // pairs
-    cv.take((size_t)(tp < nab ? tp : nab) * sc, 4);  // cs
+    cv.take(lean ? 0 : ns, 2);   // pairs
+    cv.take((size_t)(tp < kNab ? tp : kNab) * sc, 4);  // cs
     cv.take(tp + 1, 4);           // vstart
     cv.take(tp, 4);               // pa0
     cv.take(tp, 4);               // pg0
     cv.take(compact ? tp : 0, 4);  // psb (dense per-logit arrays: the slot base is p * (K + 1))
     cv.take(compact ? tp : 0, 4);  // pnv
     cv.take(tp, 1);               // apx
-    cv.take(nchunks == 1 && !(lean & 2) ? (size_t)tp * sc * win_bytes : 0, 1);  // wst
+    cv.take(nchunks == 1 ? (size_t)tp * sc * win_bytes : 0, 1);  // wst
 }
 
 // GT = lanes per pixel as a compile-time constant (1, 2, 4, 8), or 0 to read it from the launch record.
@@ -105,9 +109,9 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
     float* t2s_own = cv.take<float>();
     float* t2s = a.L.nchunks > 1 ? t2s_own : gsel;
     // (pixel, logit) pairs that need per-sample noise: logit j (or, COMPACT, its position among the pixel's valid
-    // entries) in bits 0-9 (K <= 1023), the pixel's rank among the staged active pixels in bits 10-12 (nab <= 8)
+    // entries) in bits 0-9 (K <= 1023), the pixel's rank among the staged active pixels in bits 10-12 (kNab <= 8)
     uint16_t* pairs_own = cv.take<uint16_t>();
-    const bool lean = a.L.lean & 1;
+    const bool lean = a.L.lean;
     uint16_t* pairs = lean ? cnt : pairs_own;
     float* cs = cv.take<float>();  // c_s of the current sample chunk, per active pixel
     int* vstart = cv.take<int>();
@@ -118,7 +122,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
     uint8_t* apx = cv.take<uint8_t>();
     // single-chunk jobs: the tile's saved winners (tp rows of sa_loc entries, contiguous) are copied to
     // shared memory asynchronously at the very start, off the critical path
-    const bool early_w = !(a.L.lean & 2) && a.L.nchunks == 1 && ((sa_loc * wb) & 15) == 0 && do_sample && (((uintptr_t)a.winners) & 15) == 0;
+    const bool early_w = a.L.nchunks == 1 && ((sa_loc * wb) & 15) == 0 && do_sample && (((uintptr_t)a.winners) & 15) == 0;
     unsigned char* wst = cv.take<unsigned char>();
     if (early_w) {
         const unsigned char* src = reinterpret_cast<const unsigned char*>(a.winners) + pix0 * sa_loc * wb;
@@ -312,12 +316,11 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                 __syncwarp();
             }
             float C2 = 0.f;
-            // active pixels are processed nab at a time: the c_s staging buffer holds nab rows
-            const int nab = a.L.nab;
+            // active pixels are processed kNab at a time: the c_s staging buffer holds kNab rows
 #pragma unroll 1
-            for (int b0 = 0; b0 < na; b0 += nab) {
-            const int nb = min(nab, na - b0);
-            const bool mine = act && my_ai >= b0 && my_ai < b0 + nab;
+            for (int b0 = 0; b0 < na; b0 += kNab) {
+            const int nb = min(kNab, na - b0);
+            const bool mine = act && my_ai >= b0 && my_ai < b0 + kNab;
             // the (pixel, logit) pairs of this batch that need per-sample noise
             int np2 = 0;
             {
@@ -628,9 +631,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
 
 // CTAs (= warps) per SM the main pass is compiled for: 64 registers, no spills; the shared-memory layout allows 30
 // (25 / 28 / 32 measured on the sparse set: 0.326 / 0.311 / 0.323 ms)
-#ifndef BWD_MAIN_CTAS
-#define BWD_MAIN_CTAS 28
-#endif
+constexpr int BWD_MAIN_CTAS = 28;
 template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0, bool WOVR = false>
 __global__ void __launch_bounds__(FNT, BWD_MAIN_CTAS) shade_bwd_kernel(const BwdArgs a, const NoiseA noise_a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -751,10 +752,7 @@ static int launch_bwd_c(const BwdArgs& a, const PN& na, cudaStream_t st) {
 }
 template <class PN, int GT, bool FACE>
 static int launch_bwd_fb(const BwdArgs& a, const PN& na, int64_t prow0, cudaStream_t st) {
-    size_t smem = (size_t)a.L.warp_smem * (FBT / 32);
-#ifdef PERT_EXPERIMENTS  // occupancy sensitivity: pad the CTA's shared memory
-    if (const char* e = getenv("PERT_BWD_PAD")) smem += (size_t)atoi(e);
-#endif
+    const size_t smem = (size_t)a.L.warp_smem * (FBT / 32);
     if (int rc = set_smem(shade_bwd_fallback_kernel<PN, GT, FACE>, smem)) return rc;
     shade_bwd_fallback_kernel<PN, GT, FACE><<<resident_grid(shade_bwd_fallback_kernel<PN, GT, FACE>, FBT, smem), FBT, smem, st>>>(a, na, prow0);
     return (int)cudaGetLastError();

@@ -15,7 +15,7 @@
 
 namespace pert {
 
-int fwd_smem_layout(int tp, int cap, int stage_bytes, SmemLayout& L) {
+int fwd_smem_layout(int tp, int cap, SmemLayout& L) {
     Carver cv(L);
     cv.take(cap, 2);       // vlist
     cv.take(cap + tp, 4);  // xs | lz
@@ -23,8 +23,6 @@ int fwd_smem_layout(int tp, int cap, int stage_bytes, SmemLayout& L) {
     cv.take(cap + tp, 4);  // rs | hl
     cv.take(cap + tp, 2);  // rlist | lj
     cv.take(64, 2);        // ring (compound sampler)
-    cv.take(stage_bytes ? 16 : 0, 1);  // mbarrier + phase parity of the bulk-copy scan
-    cv.take(stage_bytes, 1);           // stage: the tile's pix_to_face rows
     const int rast_bytes = L.bytes;
     cv.take(cap, 4);       // zs: from here on, arrays the coverage-sample launch of a split pass never touches
     cv.take(tp + 1, 4);    // vstart
@@ -33,20 +31,15 @@ int fwd_smem_layout(int tp, int cap, int stage_bytes, SmemLayout& L) {
     return rast_bytes;
 }
 
+// Main pass of the sparse-first mode: a tile with at least this many entries for the compound sampler goes to the fallback
+// pass.  Elsewhere, fewer compound entries than kCmpMin in a tile are drawn by the per-sample loop instead.
+constexpr int kDeferMin = 48;
+constexpr int kCmpMin = 12;
+
 // GT = lanes per pixel as a compile-time constant (1, 2, 4, 8), or 0 to read it from the launch record.
 // PHASED = false is the production instantiation: all three phases in one launch, no global histogram
 // (the phase-split code of the sample-sharded job is compiled out, which keeps the hot code small: the
 // kernel is instruction-fetch sensitive, every warp walks the whole body once per tile).
-// this warp's mbarrier (one arrival: the elected lane's expect_tx) and its phase parity; layout: fwd_smem_layout
-__device__ __forceinline__ void fwd_init_barrier(const FwdArgs& a, unsigned char* smem_raw) {
-    uint64_t* const bar = reinterpret_cast<uint64_t*>(smem_raw + a.L.sm.off[6]);
-    if ((threadIdx.x & 31) == 0) {
-        mbar_init(bar, 1);
-        *reinterpret_cast<unsigned*>(bar + 1) = 0u;
-    }
-    __syncwarp();
-}
-
 // DEFER = true (main pass of the sparse-first mode): a tile with enough entries for the compound coverage sampler is
 // handed to the fallback pass like a tile that overflows the compact arrays, so that this instantiation carries no
 // compound-sampler code at all (the kernel is instruction-fetch bound on sparse fragments: every instruction of a
@@ -97,8 +90,6 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
     float* rs = cv.take<float>();          // sum_s (h-h0) U (compact); later hl: histogram of the live list
     uint16_t* rlist = cv.take<uint16_t>();  // entries that need coverage samples; later lj: live logit ids
     uint16_t* ring = cv.take<uint16_t>();
-    uint64_t* bar = cv.take<uint64_t>();
-    long long* stage = cv.take<long long>();
     float* zs = cv.take<float>();          // zbuf -> zi -> zeta (compact)
     int* vstart = cv.take<int>();
     int* pinfo = cv.take<int>();  // nlive | a0l << 16 of every pixel
@@ -109,15 +100,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
     uint16_t* lj = rlist;
 
     // ---- phase 0 -----------------------------------------------------------------------------------
-#ifdef PERT_EXPERIMENTS  // bulk-copy (TMA 1-D) scan: measured and rejected as a default (cabi.cu stage_bytes_for); tuning builds only
-    const int nv = (a.L.stage_bytes && a.L.vec_ok && ((E & 1) == 0))
-                       ? scan_valid_staged(pb.pix_to_face + g0, E, stage, bar, vlist, cap)
-                       : scan_valid(pb.pix_to_face + g0, E, a.L.vec_ok, vlist, cap);
-#else
-    (void)bar;
-    (void)stage;
     const int nv = scan_valid(pb.pix_to_face + g0, E, a.L.vec_ok, vlist, cap);
-#endif
     const int sa_loc = a.L.sa_loc;
     if (nv > cap) {
         // sparse-first mode: this tile has more valid entries than the compact arrays hold: hand it to the
@@ -194,7 +177,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
     __syncwarp();
     if (do_rast) {
         if constexpr (DEFER) {
-            if (nblist >= a.L.defer_min) {
+            if (nblist >= kDeferMin) {
                 if (lane == 0) {
                     a.worklist[4 + atomicAdd(a.worklist, 1)] = (int32_t)tile;
                     if (a.blob) a.blob[tile * (int64_t)blob_words(tp, cap)] = -1;
@@ -202,7 +185,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
                 return;
             }
         }
-        if (!DEFER && nblist > 0 && nblist < a.L.cmp_min) {
+        if (!DEFER && nblist > 0 && nblist < kCmpMin) {
             // a handful of entries: the per-sample loop spreads each entry's samples over the idle lanes, which beats
             // one lane per entry (the lists share one array: the moved entries are read before they can be overwritten)
             const int moved = lane < nblist ? blist[-lane] : 0;
@@ -462,10 +445,14 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
     if (pvalid && lig == 0) reinterpret_cast<float4*>(a.image)[gp] = make_float4(r, g, bl, px_alpha);
 }
 
-// CTAs (= warps) per SM: 32 (64 registers); the Cauchy instantiations (SCORE = 1) and those without control variates
-// (WOVR) get 24 (80 registers): at 64 the in-kernel Cauchy stream and the ungated coverage samples of WOVR spill
-template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int SCORE = 0, bool WOVR = false>
-__global__ void __launch_bounds__(FNT, (SCORE || WOVR) ? 24 : 32) shade_fwd_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
+// CTAs (= warps) per SM of the main kernel.  Training: 32 (64 registers); the Cauchy instantiations (SCORE = 1) and those
+// without control variates (WOVR) get 24 (80 registers): at 64 the in-kernel Cauchy stream and the ungated coverage samples
+// of WOVR spill.  Render: 28 (72 registers; at 64 the Philox-10 and explicit-noise renders spill), 24 for Cauchy.
+constexpr int fwd_min_ctas(int score, bool wovr, bool render) { return (score || wovr) ? 24 : render ? 28 : 32; }
+
+template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER, int SCORE, bool WOVR, bool RENDER>
+__global__ void __launch_bounds__(FNT, fwd_min_ctas(SCORE, WOVR, RENDER))
+    shade_fwd_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     NoiseR nr = noise_r;
     NoiseA na = noise_a;
@@ -473,258 +460,147 @@ __global__ void __launch_bounds__(FNT, (SCORE || WOVR) ? 24 : 32) shade_fwd_kern
         nr.mix(__ldg(a.pb.seed_device));
         na.mix(__ldg(a.pb.seed_device + 1));
     }
-#ifdef PERT_EXPERIMENTS
-    if (a.L.stage_bytes) fwd_init_barrier(a, smem_raw);
-#endif
-    shade_fwd_tile<NoiseR, NoiseA, GT, PHASED, DEFER, 0x70, SCORE, WOVR>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x);
+    shade_fwd_tile<NoiseR, NoiseA, GT, PHASED, DEFER, 0x70, SCORE, WOVR, RENDER>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x);
 }
 
 // Fallback pass of the sparse-first mode: the tiles whose valid entries did not fit the compact arrays,
 // as half-size tiles (GT lanes per pixel = twice the main pass's) with full capacity.  Few persistent CTAs
-// walk the work list; it is empty for sparse (real) fragments.
+// walk the work list; it is empty for sparse (real) fragments.  Two launches, CPH = RAST and CPH = AGG | BLEND (see
+// shade_fwd_tile).
 // CTAs per SM of the fallback launches: 80 registers.  (14 and 16 CTAs per SM -- 72 / 64 registers, the shorter layout of
 // the coverage-sample launch makes room for them -- were measured at -1 % / 0 %: the passes are bound by the FMA and ALU
 // pipes, not by latency; profiles/r2_notes.md)
 constexpr int FB_MIN_CTAS = 12;
-template <class NoiseR, class NoiseA, int GT, int CPH, bool RENDER>
-__device__ __forceinline__ void fwd_fallback_loop(const FwdArgs& a, const NoiseR& noise_r, const NoiseA& noise_a,
-                                                  unsigned char* smem_all) {
-    // FBT/32 independent warps per CTA; the coverage-sample launch of a split pass carries the front of the layout only
+template <class PN, int GT, int CPH, bool RENDER>
+__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(const FwdArgs a, const PN noise_r, const PN noise_a) {
+    extern __shared__ __align__(16) unsigned char smem_all[];
+    // FBT/32 independent warps per CTA; the coverage-sample launch carries the front of the layout only
     unsigned char* smem_raw = smem_all + (threadIdx.x >> 5) * (CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem);
     const int n = 2 * a.worklist[0];
-    NoiseR nr = noise_r;
-    NoiseA na = noise_a;
+    PN nr = noise_r;
+    PN na = noise_a;
     if (a.pb.seed_device) {
         nr.mix(__ldg(a.pb.seed_device));
         na.mix(__ldg(a.pb.seed_device + 1));
     }
-#ifdef PERT_EXPERIMENTS
-    if (a.L.stage_bytes) fwd_init_barrier(a, smem_raw);
-#endif
 #pragma unroll 1
     for (;;) {  // persistent warps fetch half-tiles dynamically
         int i = 0;
-        // the second launch of a split pass walks the list with its own counter
+        // the aggregation launch walks the list with its own counter
         if ((threadIdx.x & 31) == 0) i = n > 0 ? atomicAdd(a.worklist + ((CPH & PERT_PH_RAST) ? 1 : 2), 1) : 0;
         i = __shfl_sync(FULL, i, 0);
         if (i >= n) break;
         const int64_t tile = (int64_t)a.worklist[4 + (i >> 1)] * 2 + (i & 1);
         if (tile < a.L.ntiles)
-            shade_fwd_tile<NoiseR, NoiseA, GT, false, false, CPH, 0, false, RENDER>(a, nr, na, tile, smem_raw, threadIdx.x & 31);
+            shade_fwd_tile<PN, PN, GT, false, false, CPH, 0, false, RENDER>(a, nr, na, tile, smem_raw, threadIdx.x & 31);
         __syncwarp();
     }
 }
 
-template <class NoiseR, class NoiseA, int GT, int CPH>
-__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
-    extern __shared__ __align__(16) unsigned char smem_all[];
-    fwd_fallback_loop<NoiseR, NoiseA, GT, CPH, false>(a, noise_r, noise_a, smem_all);
-}
-
-template <class NR, class NA, int GT, bool PHASED, bool DEFER = false, int SCORE = 0, bool WOVR = false>
-static int launch_fwd_t(const FwdArgs& a, const NR& nr, const NA& na, cudaStream_t st) {
+template <class NR, class NA, int GT, bool PHASED, bool DEFER, int SCORE, bool WOVR, bool RENDER>
+static int launch_t(const FwdArgs& a, const NR& nr, const NA& na, cudaStream_t st) {
     const size_t smem = (size_t)a.L.warp_smem;
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR>,
+        cudaError_t e = cudaFuncSetAttribute(shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR, RENDER>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
-    shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na);
+    shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR, RENDER><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na);
     return (int)cudaGetLastError();
 }
 
-template <class PN, int GT, int CPH>
-static int launch_fwd_fallback_ph(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
+template <class PN, int GT, int CPH, bool RENDER>
+static int launch_fallback_ph(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
     const size_t smem = (size_t)(CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem) * (FBT / 32);
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_fwd_fallback_kernel<PN, PN, GT, CPH>,
+        cudaError_t e = cudaFuncSetAttribute(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
-    shade_fwd_fallback_kernel<PN, PN, GT, CPH><<<resident_grid(shade_fwd_fallback_kernel<PN, PN, GT, CPH>, FBT, smem), FBT, smem, st>>>(a, nr, na);
+    shade_fwd_fallback_kernel<PN, GT, CPH, RENDER>
+        <<<resident_grid(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER>, FBT, smem), FBT, smem, st>>>(a, nr, na);
     return (int)cudaGetLastError();
 }
 
-template <class PN, int GT>
-static int launch_fwd_fallback(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
-    if (!a.L.fb_split) return launch_fwd_fallback_ph<PN, GT, 0x70>(a, nr, na, st);
-    const int rc = launch_fwd_fallback_ph<PN, GT, PERT_PH_RAST>(a, nr, na, st);
-    return rc ? rc : launch_fwd_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND>(a, nr, na, st);
+template <class PN, int GT, bool RENDER>
+static int launch_fallback(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
+    const int rc = launch_fallback_ph<PN, GT, PERT_PH_RAST, RENDER>(a, nr, na, st);
+    return rc ? rc : launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, RENDER>(a, nr, na, st);
 }
 
-// production path (in-kernel noise in both stages, all phases in one launch); PN = the Philox variant
-template <class PN>
-static int launch_fwd_production(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
+// all phases in one launch, lanes per pixel known at compile time
+template <class PN, bool DEFER, bool RENDER>
+static int launch_main(const FwdArgs& a, const PN& pr, const PN& pa, cudaStream_t st) {
+    switch (a.L.G) {
+        case 1: return launch_t<PN, PN, 1, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
+        case 2: return launch_t<PN, PN, 2, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
+        case 4: return launch_t<PN, PN, 4, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
+        default: return launch_t<PN, PN, 8, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
+    }
+}
+
+// production path (in-kernel Gaussian noise in both stages, all phases in one launch); PN = the Philox variant
+template <class PN, bool RENDER>
+static int launch_production(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
     const PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
-    int rc;
-    if (fb) {  // sparse-first main pass: defers the tiles the compound sampler is worth running on
-        switch (a.L.G) {  // lanes per pixel known at compile time
-            case 1: rc = launch_fwd_t<PN, PN, 1, false, true>(a, pr, pa, st); break;
-            case 2: rc = launch_fwd_t<PN, PN, 2, false, true>(a, pr, pa, st); break;
-            case 4: rc = launch_fwd_t<PN, PN, 4, false, true>(a, pr, pa, st); break;
-            default: rc = launch_fwd_t<PN, PN, 8, false, true>(a, pr, pa, st); break;
-        }
-    } else {
-        switch (a.L.G) {
-            case 1: rc = launch_fwd_t<PN, PN, 1, false>(a, pr, pa, st); break;
-            case 2: rc = launch_fwd_t<PN, PN, 2, false>(a, pr, pa, st); break;
-            case 4: rc = launch_fwd_t<PN, PN, 4, false>(a, pr, pa, st); break;
-            default: rc = launch_fwd_t<PN, PN, 8, false>(a, pr, pa, st); break;
-        }
-    }
-    if (rc || !fb) return rc;
+    if (!fb) return launch_main<PN, false, RENDER>(a, pr, pa, st);
+    // sparse-first main pass: defers the tiles the compound sampler is worth running on
+    const int rc = launch_main<PN, true, RENDER>(a, pr, pa, st);
+    if (rc) return rc;
     switch (fb->L.G) {  // sparse-first mode: half-size tiles for whatever did not fit
-        case 2: return launch_fwd_fallback<PN, 2>(*fb, pr, pa, st);
-        case 4: return launch_fwd_fallback<PN, 4>(*fb, pr, pa, st);
-        case 8: return launch_fwd_fallback<PN, 8>(*fb, pr, pa, st);
-        default: return launch_fwd_fallback<PN, 16>(*fb, pr, pa, st);
+        case 2: return launch_fallback<PN, 2, RENDER>(*fb, pr, pa, st);
+        case 4: return launch_fallback<PN, 4, RENDER>(*fb, pr, pa, st);
+        case 8: return launch_fallback<PN, 8, RENDER>(*fb, pr, pa, st);
+        default: return launch_fallback<PN, 16, RENDER>(*fb, pr, pa, st);
     }
 }
 
-// Cauchy pair (PERT_F_CAUCHY: PN = PhiloxCauchy, SCORE = 1) and the pair without control variates (PERT_F_NO_VR:
-// PN = PhiloxNoise, WOVR): the dense instantiation with runtime lanes per pixel and the phase-split code, for single
-// and phase-split calls alike.  Unbounded Cauchy noise turns off every skip of the Gaussian path (kBounded): each valid
-// entry draws all its coverage samples and every finite logit takes part in the argmax.  The pair without control
-// variates keeps the two skips that stay exact for it, entries with x < -sigma*Umax and logits that cannot win.
-template <class PN, int SCORE, bool WOVR>
-static int launch_fwd_dense(const FwdArgs& a, cudaStream_t st) {
+// One estimator pair: the Gaussian pair (PN = PhiloxNoise), the Cauchy pair (PERT_F_CAUCHY: PN = PhiloxCauchy, SCORE = 1)
+// or the pair without control variates (PERT_F_NO_VR: PN = PhiloxNoise, WOVR).  Explicit noise in either stage (PN = the
+// in-kernel stream of the other), the Cauchy pair and the pair without control variates run the dense instantiation with
+// runtime lanes per pixel; in training it carries the phase-split code, for single and phase-split calls alike.  Unbounded
+// Cauchy noise turns off every skip of the Gaussian path (kBounded): each valid entry draws all its coverage samples and
+// every finite logit takes part in the argmax.  The pair without control variates keeps the two skips that stay exact for
+// it, entries with x < -sigma*Umax and logits that cannot win.  In-kernel Gaussian noise runs the production kernels, or in
+// training the phase-split ones of the sample-sharded job.
+template <class PN, int SCORE, bool WOVR, bool RENDER>
+static int launch_pair(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
+    constexpr bool PHASED = !RENDER;  // the render has no phase-split form
     const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
     PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
     ExplicitNoise xr{a.pb.noise_rast, a.L.P, a.pb.K, a.pb.S_rast}, xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
-    if (er && ea) return launch_fwd_t<ExplicitNoise, ExplicitNoise, 0, true, false, SCORE, WOVR>(a, xr, xa, st);
-    if (er) return launch_fwd_t<ExplicitNoise, PN, 0, true, false, SCORE, WOVR>(a, xr, pa, st);
-    if (ea) return launch_fwd_t<PN, ExplicitNoise, 0, true, false, SCORE, WOVR>(a, pr, xa, st);
-    return launch_fwd_t<PN, PN, 0, true, false, SCORE, WOVR>(a, pr, pa, st);
+    if (er && ea) return launch_t<ExplicitNoise, ExplicitNoise, 0, PHASED, false, SCORE, WOVR, RENDER>(a, xr, xa, st);
+    if (er) return launch_t<ExplicitNoise, PN, 0, PHASED, false, SCORE, WOVR, RENDER>(a, xr, pa, st);
+    if (ea) return launch_t<PN, ExplicitNoise, 0, PHASED, false, SCORE, WOVR, RENDER>(a, pr, xa, st);
+    if constexpr (SCORE || WOVR) {
+        return launch_t<PN, PN, 0, PHASED, false, SCORE, WOVR, RENDER>(a, pr, pa, st);
+    } else {
+        if constexpr (PHASED) {
+            const uint32_t all = PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
+            if ((a.pb.flags & all) != all || a.hist != nullptr) {  // compile-time lanes per pixel for the benchmark geometries
+                switch (a.L.G) {
+                    case 4: return launch_t<PN, PN, 4, true, false, 0, false, false>(a, pr, pa, st);
+                    case 8: return launch_t<PN, PN, 8, true, false, 0, false, false>(a, pr, pa, st);
+                    default: return launch_t<PN, PN, 0, true, false, 0, false, false>(a, pr, pa, st);
+                }
+            }
+        }
+        return (a.pb.flags & PERT_F_PHILOX7) ? launch_production<PhiloxNoise7, RENDER>(a, fb, st)
+                                             : launch_production<PhiloxNoise, RENDER>(a, fb, st);
+    }
 }
 
 int launch_shade_fwd(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    if (a.pb.flags & PERT_F_CAUCHY) return launch_fwd_dense<PhiloxCauchy, 1, false>(a, st);
-    if (a.pb.flags & PERT_F_NO_VR) return launch_fwd_dense<PhiloxNoise, 0, true>(a, st);
-    const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
-    const uint32_t all = PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
-    const bool phased = (a.pb.flags & all) != all || a.hist != nullptr;
-    PhiloxNoise pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
-    ExplicitNoise xr{a.pb.noise_rast, a.L.P, a.pb.K, a.pb.S_rast}, xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
-    if (!er && !ea) {
-        if (phased) {  // sample-sharded job: compile-time lanes per pixel for the benchmark geometries
-            switch (a.L.G) {
-                case 4: return launch_fwd_t<PhiloxNoise, PhiloxNoise, 4, true>(a, pr, pa, st);
-                case 8: return launch_fwd_t<PhiloxNoise, PhiloxNoise, 8, true>(a, pr, pa, st);
-                default: return launch_fwd_t<PhiloxNoise, PhiloxNoise, 0, true>(a, pr, pa, st);
-            }
-        }
-        return (a.pb.flags & PERT_F_PHILOX7) ? launch_fwd_production<PhiloxNoise7>(a, fb, st)
-                                             : launch_fwd_production<PhiloxNoise>(a, fb, st);
-    }
-    if (er && ea) return launch_fwd_t<ExplicitNoise, ExplicitNoise, 0, true>(a, xr, xa, st);
-    if (er) return launch_fwd_t<ExplicitNoise, PhiloxNoise, 0, true>(a, xr, pa, st);
-    return launch_fwd_t<PhiloxNoise, ExplicitNoise, 0, true>(a, pr, xa, st);
+    if (a.pb.flags & PERT_F_CAUCHY) return launch_pair<PhiloxCauchy, 1, false, false>(a, fb, st);
+    if (a.pb.flags & PERT_F_NO_VR) return launch_pair<PhiloxNoise, 0, true, false>(a, fb, st);
+    return launch_pair<PhiloxNoise, 0, false, false>(a, fb, st);
 }
 
-// ---- forward-only render (pert_shade_render) ----------------------------------------------------------------------
-// The forward above with RENDER = true (shade_fwd_tile): single calls only, nothing saved for backward.  Separate kernel
-// templates, so that the training kernels keep their code.  The Gaussian production path (sparse-first main pass, its
-// split fallback pass, Philox-10 or -7) and the dense instantiation (explicit noise, Cauchy) have render twins; the pair
-// without control variates renders on the Gaussian per-sample path, whose counts, histogram and image it shares.
-// CTAs per SM: 28 (72 registers; at 64 the Philox-10 and explicit-noise renders spill), 24 for Cauchy as in training.
-template <class NoiseR, class NoiseA, int GT, bool DEFER = false, int SCORE = 0>
-__global__ void __launch_bounds__(FNT, SCORE ? 24 : 28) shade_render_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    NoiseR nr = noise_r;
-    NoiseA na = noise_a;
-    if (a.pb.seed_device) {
-        nr.mix(__ldg(a.pb.seed_device));
-        na.mix(__ldg(a.pb.seed_device + 1));
-    }
-#ifdef PERT_EXPERIMENTS
-    if (a.L.stage_bytes) fwd_init_barrier(a, smem_raw);
-#endif
-    shade_fwd_tile<NoiseR, NoiseA, GT, false, DEFER, 0x70, SCORE, false, true>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x);
-}
-
-// split fallback pass of the render: CPH = PERT_PH_RAST writes the counts to the workspace, CPH = AGG | BLEND reads them
-template <class PN, int GT, int CPH>
-__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_render_fallback_kernel(const FwdArgs a, const PN noise_r, const PN noise_a) {
-    extern __shared__ __align__(16) unsigned char smem_all[];
-    fwd_fallback_loop<PN, PN, GT, CPH, true>(a, noise_r, noise_a, smem_all);
-}
-
-template <class NR, class NA, int GT, bool DEFER = false, int SCORE = 0>
-static int launch_render_t(const FwdArgs& a, const NR& nr, const NA& na, cudaStream_t st) {
-    const size_t smem = (size_t)a.L.warp_smem;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_render_kernel<NR, NA, GT, DEFER, SCORE>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-    }
-    shade_render_kernel<NR, NA, GT, DEFER, SCORE><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na);
-    return (int)cudaGetLastError();
-}
-
-template <class PN, int GT, int CPH>
-static int launch_render_fallback_ph(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
-    const size_t smem = (size_t)(CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem) * (FBT / 32);
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_render_fallback_kernel<PN, GT, CPH>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-    }
-    shade_render_fallback_kernel<PN, GT, CPH><<<resident_grid(shade_render_fallback_kernel<PN, GT, CPH>, FBT, smem), FBT, smem, st>>>(a, nr, na);
-    return (int)cudaGetLastError();
-}
-
-template <class PN, int GT>
-static int launch_render_fallback(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
-    const int rc = launch_render_fallback_ph<PN, GT, PERT_PH_RAST>(a, nr, na, st);
-    return rc ? rc : launch_render_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND>(a, nr, na, st);
-}
-
-template <class PN>
-static int launch_render_production(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    const PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
-    int rc;
-    if (fb) {
-        switch (a.L.G) {
-            case 1: rc = launch_render_t<PN, PN, 1, true>(a, pr, pa, st); break;
-            case 2: rc = launch_render_t<PN, PN, 2, true>(a, pr, pa, st); break;
-            case 4: rc = launch_render_t<PN, PN, 4, true>(a, pr, pa, st); break;
-            default: rc = launch_render_t<PN, PN, 8, true>(a, pr, pa, st); break;
-        }
-    } else {
-        switch (a.L.G) {
-            case 1: rc = launch_render_t<PN, PN, 1>(a, pr, pa, st); break;
-            case 2: rc = launch_render_t<PN, PN, 2>(a, pr, pa, st); break;
-            case 4: rc = launch_render_t<PN, PN, 4>(a, pr, pa, st); break;
-            default: rc = launch_render_t<PN, PN, 8>(a, pr, pa, st); break;
-        }
-    }
-    if (rc || !fb) return rc;
-    switch (fb->L.G) {
-        case 2: return launch_render_fallback<PN, 2>(*fb, pr, pa, st);
-        case 4: return launch_render_fallback<PN, 4>(*fb, pr, pa, st);
-        case 8: return launch_render_fallback<PN, 8>(*fb, pr, pa, st);
-        default: return launch_render_fallback<PN, 16>(*fb, pr, pa, st);
-    }
-}
-
-// runtime lanes per pixel: explicit noise in either stage (PN = the in-kernel stream of the other), or the Cauchy pair
-template <class PN, int SCORE>
-static int launch_render_dense(const FwdArgs& a, cudaStream_t st) {
-    const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
-    PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
-    ExplicitNoise xr{a.pb.noise_rast, a.L.P, a.pb.K, a.pb.S_rast}, xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
-    if (er && ea) return launch_render_t<ExplicitNoise, ExplicitNoise, 0, false, SCORE>(a, xr, xa, st);
-    if (er) return launch_render_t<ExplicitNoise, PN, 0, false, SCORE>(a, xr, pa, st);
-    if (ea) return launch_render_t<PN, ExplicitNoise, 0, false, SCORE>(a, pr, xa, st);
-    if constexpr (SCORE != 0) return launch_render_t<PN, PN, 0, false, SCORE>(a, pr, pa, st);
-    return (int)cudaErrorInvalidValue;  // not reached: in-kernel Gaussian noise renders on the production kernels
-}
-
+// The forward with RENDER = true (shade_fwd_tile): single calls only, nothing saved for backward.  The pair without control
+// variates renders on the Gaussian per-sample path (cabi.cu), whose counts, histogram and image it shares.
 int launch_shade_render(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    if (a.pb.flags & PERT_F_CAUCHY) return launch_render_dense<PhiloxCauchy, 1>(a, st);
-    if (a.pb.noise_rast || a.pb.noise_agg) return launch_render_dense<PhiloxNoise, 0>(a, st);
-    return (a.pb.flags & PERT_F_PHILOX7) ? launch_render_production<PhiloxNoise7>(a, fb, st)
-                                         : launch_render_production<PhiloxNoise>(a, fb, st);
+    if (a.pb.flags & PERT_F_CAUCHY) return launch_pair<PhiloxCauchy, 1, false, true>(a, fb, st);
+    return launch_pair<PhiloxNoise, 0, false, true>(a, fb, st);
 }
 
 }  // namespace pert

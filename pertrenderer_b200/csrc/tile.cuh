@@ -58,69 +58,6 @@ __device__ __forceinline__ int scan_valid(const int64_t* __restrict__ p2f /* til
     return total;
 }
 
-// ---- TMA bulk copy (cp.async.bulk, UBLKCP in SASS) + mbarrier: the tile's pix_to_face rows are ONE contiguous run of
-// E * 8 bytes (6.4 KB for 16 pixels at K = 50): one elected lane asks the copy engine for the whole run, the data lands in
-// shared memory in a single DRAM round trip and the scan reads it with 128-bit shared loads, instead of walking it with
-// four register-capped vector loads in flight per lane (four dependent round trips per tile).
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gsrc, unsigned bytes, uint64_t* bar) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
-                 "l"(gsrc), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
-    unsigned ok = 0;
-#pragma unroll 1
-    while (!ok) {
-        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-                     : "=r"(ok)
-                     : "r"(smem_u32(bar)), "r"(parity)
-                     : "memory");
-    }
-}
-
-// scan_valid on a tile staged in shared memory by one bulk copy.  `bar` = this warp's mbarrier, followed by its phase
-// parity (a 32-bit word): a persistent warp reuses the barrier tile after tile.  E * 8 must be a multiple of 16 and the
-// source 16-byte aligned (the caller checks).
-__device__ __forceinline__ int scan_valid_staged(const int64_t* __restrict__ p2f, int E, long long* stage, uint64_t* bar,
-                                                 uint16_t* vlist, int cap) {
-    const int lane = threadIdx.x & 31;
-    const unsigned lt = (1u << lane) - 1u;
-    unsigned* const par = reinterpret_cast<unsigned*>(bar + 1);
-    const unsigned parity = *par;
-    __syncwarp();
-    if (lane == 0) {
-        bulk_load(stage, p2f, (unsigned)E * 8u, bar);
-        *par = parity ^ 1u;
-    }
-    mbar_wait(bar, parity);
-    int total = 0;
-#pragma unroll 1
-    for (int base = 0; base < E; base += 64) {
-        const int e0 = base + 2 * lane;
-        long long a = -1, b = -1;
-        if (e0 + 1 < E) {
-            const longlong2 v = *reinterpret_cast<const longlong2*>(stage + e0);
-            a = v.x;
-            b = v.y;
-        } else if (e0 < E) {
-            a = stage[e0];
-        }
-        const bool v0 = a >= 0, v1 = b >= 0;
-        const unsigned be = __ballot_sync(FULL, v0), bo = __ballot_sync(FULL, v1);
-        const int pos = total + __popc(be & lt) + __popc(bo & lt);
-        if (v0 && pos < cap) vlist[pos] = (uint16_t)e0;
-        if (v1 && pos + (v0 ? 1 : 0) < cap) vlist[pos + (v0 ? 1 : 0)] = (uint16_t)(e0 + 1);
-        total += __popc(be) + __popc(bo);
-    }
-    return total;
-}
-
 // vstart[p] = first compact index of pixel p (p = 0..tp), by binary search on the ascending vlist
 __device__ __forceinline__ void pixel_ranges(const uint16_t* vlist, int nv, int K, int tp, int* vstart) {
     const int lane = threadIdx.x & 31;
