@@ -180,9 +180,11 @@ int64_t pert_num_tiles(const pert_problem* pb);
 /* element size in bytes of the winners buffer for this K (1 or 2) */
 int pert_winner_bytes(int32_t K);
 /* size in bytes of the optional `tile_blob` buffer (16-byte aligned).  In sparse-first mode forward saves,
- * per warp tile, the compact list of valid entries and the per-pixel logit summary it computed; backward
- * then neither re-scans pix_to_face nor recomputes the logits.  Pass the SAME flags / geometry to both
- * calls.  NULL: backward recomputes (same results). */
+ * per warp tile, the compact list of valid entries and the per-pixel logit summary it computed, for the tiles of
+ * the main pass and for the half-tiles of the fallback pass (room for every tile to take the fallback pass: at
+ * 8 x 256^2, K = 50, 57 MB of tile blobs and 173 MB of fallback records); backward then neither re-scans
+ * pix_to_face nor recomputes the logits, and the second forward launch of the fallback pass does not re-scan.
+ * Pass the SAME flags / geometry to both calls.  NULL: both recompute (same results). */
 int64_t pert_blob_bytes(const pert_problem* pb);
 
 /*

@@ -200,11 +200,19 @@ extern "C" int64_t pert_num_tiles(const pert_problem* pb) {
 
 extern "C" int pert_winner_bytes(int32_t K) { return (K + 1 <= 256) ? 1 : 2; }
 
+// The tile_blob buffer: one tile blob per tile of the sparse-first main pass, then one fallback record per half-tile, for
+// every tile (each one may be deferred).  Offset of the records region in 32-bit words:
+static int64_t blob_records_off(int K, int64_t P) {
+    const int tp = sparse_tp(K, P);
+    return ((P + tp - 1) / tp) * (int64_t)blob_words(tp, sparse_cap(K, tp));
+}
+
 extern "C" int64_t pert_blob_bytes(const pert_problem* pb) {
     if (!pb || pb->K <= 0) return 0;
     const int64_t P = pb->N * pb->H * pb->W;
     const int tp = sparse_tp(pb->K, P);
-    return ((P + tp - 1) / tp) * (int64_t)blob_words(tp, sparse_cap(pb->K, tp)) * 4;
+    const int64_t records = 2 * ((P + tp - 1) / tp) * (int64_t)fbrec_words(tp / 2, tp / 2 * pb->K);
+    return (blob_records_off(pb->K, P) + records) * 4;
 }
 
 static bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
@@ -228,7 +236,7 @@ static int fwd_launch_records(FwdArgs& a, FwdArgs& fb, bool sparse) {
     if (a.L.ntiles > 0x7fffffff) return PERT_E_UNSUPPORTED;
     if (!sparse) return 0;
     fb = a;
-    fb.blob = nullptr;
+    fb.blob = a.blob ? a.blob + blob_records_off(a.pb.K, P) : nullptr;
     fb.L = make_launch(&a.pb, a.L.tp / 2);
     fb.L.vec_ok = fb.L.vec_ok && aligned16(a.pb.pix_to_face);
     fb.L.warp_smem_rast = fwd_smem_layout(fb.L.tp, fb.L.cap, fb.L.sm);
@@ -263,13 +271,13 @@ extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t*
     a.pixstate = pixstate;
     a.hist = hist;
     a.worklist = worklist;
-    a.blob = nullptr;
+    a.blob = (int32_t*)tile_blob;  // the fallback pass's records follow the tile blobs (fwd_launch_records)
     FwdArgs fb;
     rc = fwd_launch_records(a, fb, sparse_first_ok(&a.pb, worklist, (f & all) == all && !hist));
     if (rc < 0) return rc;
     const bool sparse = rc == 1;
     if ((uintptr_t)tile_blob & 15) return PERT_E_ALIGN;
-    a.blob = sparse ? (int32_t*)tile_blob : nullptr;
+    if (!sparse) a.blob = nullptr;
     cudaStream_t st = (cudaStream_t)stream;
     if (!sparse) return cuda_rc(launch_shade_fwd(a, nullptr, st));
     cudaError_t e = cudaMemsetAsync(worklist, 0, 16, st);
@@ -372,7 +380,7 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
     cudaStream_t st = (cudaStream_t)stream;
     if (!sparse) return cuda_rc(launch_shade_bwd(a, nullptr, grad_scalars, st));
     BwdArgs fb = a;  // fallback pass: half-size tiles, full capacity, dense per-logit arrays
-    fb.blob = nullptr;
+    fb.blob = a.blob ? a.blob + blob_records_off(a.pb.K, a.L.P) : nullptr;
     fb.L = make_launch(&a.pb, a.L.tp / 2);
     fb.L.vec_ok = fb.L.vec_ok && ptr_ok;
     fb.L.lean = true;  // pair list in the counts array; the winners ARE staged (+3 %), the layout still fits 12 CTAs per SM

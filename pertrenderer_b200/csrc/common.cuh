@@ -287,6 +287,12 @@ __host__ __device__ __forceinline__ int blob_pix_off(int tp) { return 2 + tp; }
 __host__ __device__ __forceinline__ int blob_vlist_off(int tp) { return 2 + 7 * tp; }
 __host__ __device__ __forceinline__ int blob_cnt_off(int tp, int cap) { return 2 + 7 * tp + cap / 2; }
 __host__ __device__ __forceinline__ int blob_zeta_off(int tp, int cap) { return 2 + 7 * tp + cap; }
+// Fallback record: the same for one half-tile of the fallback pass (cap = tp*K, even), addressed by the half-tile's index in
+// the records region that follows the tile blobs.  [0] nv, [1 .. tp+1] vstart, 6 words per pixel as above, then vlist
+// (u16 x cap), zeta (f32 x cap).  No counts: the fallback pass of backward holds its pair list in the counts array and
+// reads the counts from global memory.  The coverage launch of forward writes nv and vlist, its aggregation launch the rest.
+__host__ __device__ __forceinline__ int fbrec_words(int tp, int cap) { return ((2 + 7 * tp + cap / 2 + cap) + 3) & ~3; }
+__host__ __device__ __forceinline__ int fbrec_zeta_off(int tp, int cap) { return 2 + 7 * tp + cap / 2; }
 
 // entry index within a tile -> pixel of the tile.  Exact for e < 2^16, K < 2^10: (e + .5)/K is at
 // least .5/K away from an integer, far more than the fp32 rounding of the product.

@@ -55,8 +55,9 @@ void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes,
 // COMPACT = true (sparse-first mode): the per-logit arrays are indexed by the position of the logit
 // among the pixel's valid entries (plus a background and a masked-logits slot) instead of densely by j,
 // and every array holds a.L.cap valid entries; tiles with more go to the fallback pass.
-// BLOB = true (only with COMPACT): the compact valid list and the per-pixel logit summary come from the tile
-// blob forward saved (common.cuh) instead of a re-scan of pix_to_face and a recomputation of the logits.
+// BLOB = true: the compact valid list and the per-pixel logit summary come from what forward saved (common.cuh) instead of a
+// re-scan of pix_to_face and a recomputation of the logits: the tile blob (COMPACT main pass) or the half-tile's fallback
+// record (fallback pass, which takes the counts from global memory: a.L.lean).
 // SCORE = the score psi of the aggregation noise (philox.cuh noise_score): acc_j = sum_s c_s psi(V_sj) and
 // t2_j = sum_s c_s V_sj psi(V_sj); 0 Gaussian (psi(n) = n), 1 Cauchy.
 // WOVR = true (PERT_F_NO_VR, randomArgmax_wovr smoothagg.py:75-141): c_s = g[a_s] without the control variate g[a_0].
@@ -143,7 +144,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
         zf = __ldg(pb.zfar + b);
         pstate = a.pixstate[gp];
     }
-    const int32_t* const bl = BLOB ? a.blob + tile * (int64_t)blob_words(tp, cap) : nullptr;
+    const int32_t* const bl = BLOB ? a.blob + tile * (int64_t)(COMPACT ? blob_words(tp, cap) : fbrec_words(tp, cap)) : nullptr;
     const int nv = BLOB ? __ldg(bl) : scan_valid(pb.pix_to_face + g0, E, a.L.vec_ok, vlist, cap);
     const bool overflow = COMPACT && (BLOB ? nv < 0 : nv > cap);
     if (!overflow) {
@@ -178,7 +179,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
             for (int i = lane; i < nw; i += 32) {
                 const uint32_t v2 = (uint32_t)__ldg(bl + blob_vlist_off(tp) + i);
                 vl32[i] = v2;
-                cn32[i] = (uint32_t)__ldg(bl + blob_cnt_off(tp, cap) + i);
+                if constexpr (COMPACT) cn32[i] = (uint32_t)__ldg(bl + blob_cnt_off(tp, cap) + i);
                 // needed a few round trips later (g_j of the logits that can win; chain rule): start them now
                 const int e0 = v2 & 0xffff, e1 = v2 >> 16;
                 if (!FACE) prefetch_l1(colors_t + e0 * 3);
@@ -188,8 +189,9 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                     prefetch_l1(rsum_t + e1);
                 }
             }
+            const int zoff = COMPACT ? blob_zeta_off(tp, cap) : fbrec_zeta_off(tp, cap);
 #pragma unroll 1
-            for (int i = lane; i < nv; i += 32) zs[i] = __int_as_float(__ldg(bl + blob_zeta_off(tp, cap) + i));
+            for (int i = lane; i < nv; i += 32) zs[i] = __int_as_float(__ldg(bl + zoff + i));
             if (pvalid) {
                 const int32_t* const bp = bl + blob_pix_off(tp) + 6 * p;
                 pi.zmax = __int_as_float(__ldg(bp));
@@ -641,8 +643,8 @@ __global__ void __launch_bounds__(FNT, BWD_MAIN_CTAS) shade_bwd_kernel(const Bwd
 }
 
 // Fallback pass of the sparse-first mode (see shade_fwd.cu): work-list tiles as half-size tiles with dense
-// per-logit arrays; their scalar partials go to the rows after the main pass's.
-template <class NoiseA, int GT, bool FACE>
+// per-logit arrays; their scalar partials go to the rows after the main pass's.  BLOB: from forward's fallback records.
+template <class NoiseA, int GT, bool FACE, bool BLOB>
 __global__ void __launch_bounds__(FBT, 12) shade_bwd_fallback_kernel(const BwdArgs a, const NoiseA noise_a, int64_t prow0) {
     extern __shared__ __align__(16) unsigned char smem_all[];
     unsigned char* smem_raw = smem_all + (threadIdx.x >> 5) * a.L.warp_smem;  // FBT/32 independent warps per CTA
@@ -657,7 +659,7 @@ __global__ void __launch_bounds__(FBT, 12) shade_bwd_fallback_kernel(const BwdAr
         if (i >= n) break;
         const int64_t tile = (int64_t)a.worklist[4 + (i >> 1)] * 2 + (i & 1);
         if (tile < a.L.ntiles) {
-            shade_bwd_tile<NoiseA, GT, false, FACE, false, false>(a, na, tile, prow0 + i, smem_raw, threadIdx.x & 31);
+            shade_bwd_tile<NoiseA, GT, false, FACE, false, BLOB>(a, na, tile, prow0 + i, smem_raw, threadIdx.x & 31);
         } else if ((threadIdx.x & 31) == 0) {
             reinterpret_cast<float4*>(a.partials)[prow0 + i] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
@@ -750,12 +752,17 @@ static int launch_bwd_c(const BwdArgs& a, const PN& na, cudaStream_t st) {
     return a.pb.face_colors ? launch_bwd_f<PN, GT, false, true, true>(a, na, st)
                             : launch_bwd_f<PN, GT, false, false, true>(a, na, st);
 }
+template <class PN, int GT, bool FACE, bool BLOB>
+static int launch_bwd_fb_b(const BwdArgs& a, const PN& na, int64_t prow0, cudaStream_t st) {
+    const size_t smem = (size_t)a.L.warp_smem * (FBT / 32);
+    if (int rc = set_smem(shade_bwd_fallback_kernel<PN, GT, FACE, BLOB>, smem)) return rc;
+    shade_bwd_fallback_kernel<PN, GT, FACE, BLOB>
+        <<<resident_grid(shade_bwd_fallback_kernel<PN, GT, FACE, BLOB>, FBT, smem), FBT, smem, st>>>(a, na, prow0);
+    return (int)cudaGetLastError();
+}
 template <class PN, int GT, bool FACE>
 static int launch_bwd_fb(const BwdArgs& a, const PN& na, int64_t prow0, cudaStream_t st) {
-    const size_t smem = (size_t)a.L.warp_smem * (FBT / 32);
-    if (int rc = set_smem(shade_bwd_fallback_kernel<PN, GT, FACE>, smem)) return rc;
-    shade_bwd_fallback_kernel<PN, GT, FACE><<<resident_grid(shade_bwd_fallback_kernel<PN, GT, FACE>, FBT, smem), FBT, smem, st>>>(a, na, prow0);
-    return (int)cudaGetLastError();
+    return a.blob ? launch_bwd_fb_b<PN, GT, FACE, true>(a, na, prow0, st) : launch_bwd_fb_b<PN, GT, FACE, false>(a, na, prow0, st);
 }
 
 // both phases in one launch, in-kernel noise

@@ -56,8 +56,11 @@ constexpr int kCmpMin = 12;
 // or tile blob); coverage computes counts only, from the same counters, so counts, histogram and image are those of the
 // training forward.  Counts go to global memory only in the coverage-sample launch of a split fallback pass (a.counts is
 // then the caller's S-independent workspace), which the aggregation launch reads back.
+// Fallback records (common.cuh; training with a tile blob, a.blob then points at the records region): the coverage launch
+// stores the half-tile's valid list; REC = true (aggregation launch) loads it instead of re-scanning pix_to_face and stores
+// what backward would recompute, the per-pixel logit summary and zeta.
 template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int CPH = 0x70, int SCORE = 0,
-          bool WOVR = false, bool RENDER = false>
+          bool WOVR = false, bool RENDER = false, bool REC = false>
 __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& noise_r, const NoiseA& noise_a,
                                                const int64_t tile, unsigned char* smem_raw, const int lane) {
     const pert_problem& pb = a.pb;
@@ -98,16 +101,27 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
     float* lz = xs;
     int* hl = reinterpret_cast<int*>(rs);
     uint16_t* lj = rlist;
+    // this tile's blob (main pass) or record (fallback pass) in a.blob; derived where used, so that no pointer stays live
+    auto blob_of = [&]() { return a.blob + tile * (int64_t)(CPH == 0x70 ? blob_words(tp, cap) : fbrec_words(tp, cap)); };
 
     // ---- phase 0 -----------------------------------------------------------------------------------
-    const int nv = scan_valid(pb.pix_to_face + g0, E, a.L.vec_ok, vlist, cap);
+    int nv;
+    if constexpr (REC) {
+        const int32_t* const bl = blob_of();
+        nv = __ldg(bl);
+        const int32_t* const src = bl + blob_vlist_off(tp);
+#pragma unroll 1
+        for (int i = lane; i < ((nv + 1) >> 1); i += 32) reinterpret_cast<int32_t*>(vlist)[i] = __ldg(src + i);
+    } else {
+        nv = scan_valid(pb.pix_to_face + g0, E, a.L.vec_ok, vlist, cap);
+    }
     const int sa_loc = a.L.sa_loc;
     if (nv > cap) {
         // sparse-first mode: this tile has more valid entries than the compact arrays hold: hand it to the
         // fallback pass (half-size tiles, full capacity)
         if (lane == 0) {
             a.worklist[4 + atomicAdd(a.worklist, 1)] = (int32_t)tile;
-            if (a.blob) a.blob[tile * (int64_t)blob_words(tp, cap)] = -1;
+            if (a.blob) blob_of()[0] = -1;
         }
         return;
     }
@@ -118,13 +132,22 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
             for (int i = lane; i < npx * K1; i += 32) ghist[pix0 * K1 + i] = ((i % K1) == K) ? sa_loc : 0;
         }
         if (!RENDER && do_agg && lane < npx) a.pixstate[pix0 + lane] = (uint16_t)K;
-        if (!PHASED && !RENDER && a.blob && lane == 0) a.blob[tile * (int64_t)blob_words(tp, a.L.cap)] = 0;
+        if (!PHASED && !RENDER && !REC && a.blob && lane == 0) blob_of()[0] = 0;
         if (do_blend && lane < npx)
             reinterpret_cast<float4*>(a.image)[pix0 + lane] =
                 make_float4(pb.background[0], pb.background[1], pb.background[2], 0.0f);
         return;
     }
     __syncwarp();
+    if constexpr (CPH == (int)PERT_PH_RAST && !RENDER) {
+        if (a.blob) {  // the valid list, for the aggregation launch and backward
+            int32_t* const bl = blob_of();
+            if (lane == 0) bl[0] = nv;
+#pragma unroll 1
+            for (int i = lane; i < ((nv + 1) >> 1); i += 32)
+                bl[blob_vlist_off(tp) + i] = reinterpret_cast<const int32_t*>(vlist)[i];
+        }
+    }
     if (do_agg || do_blend) pixel_ranges(vlist, nv, K, tp, vstart);
 
     // ---- phase 1: stage valid entries, coverage samples ---------------------------------------------
@@ -180,7 +203,7 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
             if (nblist >= kDeferMin) {
                 if (lane == 0) {
                     a.worklist[4 + atomicAdd(a.worklist, 1)] = (int32_t)tile;
-                    if (a.blob) a.blob[tile * (int64_t)blob_words(tp, cap)] = -1;
+                    if (a.blob) blob_of()[0] = -1;
                 }
                 return;
             }
@@ -355,10 +378,11 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
             hl[lb + a0l] = sa_loc - others;
             if constexpr (!RENDER) a.pixstate[gp] = (uint16_t)(pi.a0 | (active ? 0x8000 : 0));
         }
-        if (!PHASED && !RENDER && a.blob) {
-            // what backward would recompute from pix_to_face / zbuf / counts (layout: common.cuh)
-            int32_t* const bl = a.blob + tile * (int64_t)blob_words(tp, cap);
-            if (lane == 0) bl[0] = nv;
+        if (!PHASED && !RENDER && (CPH == 0x70 || REC) && a.blob) {
+            // what backward would recompute from pix_to_face / zbuf / counts (layout: common.cuh); a fallback record already
+            // holds nv and the valid list (coverage launch) and carries no counts
+            int32_t* const bl = blob_of();
+            if (CPH == 0x70 && lane == 0) bl[0] = nv;
             for (int i = lane; i <= tp; i += 32) bl[1 + i] = i <= npx ? vstart[i] : nv;
             if (pvalid && lig == 0) {
                 int32_t* const bp = bl + blob_pix_off(tp) + 6 * p;
@@ -369,16 +393,19 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
                 bp[4] = pi.argzi | (pi.a0 << 16);
                 bp[5] = pi.nzero | (pi.kpad << 16);
             }
-            const uint32_t* const vl32 = reinterpret_cast<const uint32_t*>(vlist);
-            const uint32_t* const cn32 = reinterpret_cast<const uint32_t*>(cnt);
-            const int nw = (nv + 1) >> 1;
+            if constexpr (CPH == 0x70) {
+                const uint32_t* const vl32 = reinterpret_cast<const uint32_t*>(vlist);
+                const uint32_t* const cn32 = reinterpret_cast<const uint32_t*>(cnt);
+                const int nw = (nv + 1) >> 1;
 #pragma unroll 1
-            for (int i = lane; i < nw; i += 32) {
-                bl[blob_vlist_off(tp) + i] = (int32_t)vl32[i];
-                bl[blob_cnt_off(tp, cap) + i] = (int32_t)cn32[i];
+                for (int i = lane; i < nw; i += 32) {
+                    bl[blob_vlist_off(tp) + i] = (int32_t)vl32[i];
+                    bl[blob_cnt_off(tp, cap) + i] = (int32_t)cn32[i];
+                }
             }
+            const int zoff = CPH == 0x70 ? blob_zeta_off(tp, cap) : fbrec_zeta_off(tp, cap);
 #pragma unroll 1
-            for (int i = lane; i < nv; i += 32) bl[blob_zeta_off(tp, cap) + i] = __float_as_int(zs[i]);
+            for (int i = lane; i < nv; i += 32) bl[zoff + i] = __float_as_int(zs[i]);
         }
         __syncwarp();
         if (ghist) {
@@ -466,12 +493,12 @@ __global__ void __launch_bounds__(FNT, fwd_min_ctas(SCORE, WOVR, RENDER))
 // Fallback pass of the sparse-first mode: the tiles whose valid entries did not fit the compact arrays,
 // as half-size tiles (GT lanes per pixel = twice the main pass's) with full capacity.  Few persistent CTAs
 // walk the work list; it is empty for sparse (real) fragments.  Two launches, CPH = RAST and CPH = AGG | BLEND (see
-// shade_fwd_tile).
+// shade_fwd_tile); with a tile blob the second one reads the valid lists the first one stored (REC).
 // CTAs per SM of the fallback launches: 80 registers.  (14 and 16 CTAs per SM -- 72 / 64 registers, the shorter layout of
 // the coverage-sample launch makes room for them -- were measured at -1 % / 0 %: the passes are bound by the FMA and ALU
 // pipes, not by latency; profiles/r2_notes.md)
 constexpr int FB_MIN_CTAS = 12;
-template <class PN, int GT, int CPH, bool RENDER>
+template <class PN, int GT, int CPH, bool RENDER, bool REC>
 __global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(const FwdArgs a, const PN noise_r, const PN noise_a) {
     extern __shared__ __align__(16) unsigned char smem_all[];
     // FBT/32 independent warps per CTA; the coverage-sample launch carries the front of the layout only
@@ -492,7 +519,7 @@ __global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(co
         if (i >= n) break;
         const int64_t tile = (int64_t)a.worklist[4 + (i >> 1)] * 2 + (i & 1);
         if (tile < a.L.ntiles)
-            shade_fwd_tile<PN, PN, GT, false, false, CPH, 0, false, RENDER>(a, nr, na, tile, smem_raw, threadIdx.x & 31);
+            shade_fwd_tile<PN, PN, GT, false, false, CPH, 0, false, RENDER, REC>(a, nr, na, tile, smem_raw, threadIdx.x & 31);
         __syncwarp();
     }
 }
@@ -509,23 +536,28 @@ static int launch_t(const FwdArgs& a, const NR& nr, const NA& na, cudaStream_t s
     return (int)cudaGetLastError();
 }
 
-template <class PN, int GT, int CPH, bool RENDER>
+template <class PN, int GT, int CPH, bool RENDER, bool REC = false>
 static int launch_fallback_ph(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
     const size_t smem = (size_t)(CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem) * (FBT / 32);
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER>,
+        cudaError_t e = cudaFuncSetAttribute(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
-    shade_fwd_fallback_kernel<PN, GT, CPH, RENDER>
-        <<<resident_grid(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER>, FBT, smem), FBT, smem, st>>>(a, nr, na);
+    shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC>
+        <<<resident_grid(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC>, FBT, smem), FBT, smem, st>>>(a, nr, na);
     return (int)cudaGetLastError();
 }
 
+// with a tile blob (training) the aggregation launch takes the valid lists from the fallback records
 template <class PN, int GT, bool RENDER>
 static int launch_fallback(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
     const int rc = launch_fallback_ph<PN, GT, PERT_PH_RAST, RENDER>(a, nr, na, st);
-    return rc ? rc : launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, RENDER>(a, nr, na, st);
+    if (rc) return rc;
+    if constexpr (!RENDER) {
+        if (a.blob) return launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, false, true>(a, nr, na, st);
+    }
+    return launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, RENDER>(a, nr, na, st);
 }
 
 // all phases in one launch, lanes per pixel known at compile time
