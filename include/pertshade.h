@@ -18,6 +18,8 @@
  *                    randomras/smoothagg.py:45-73          randomArgmax.backward
  *                    randomras/smoothagg.py:303-311,325-337 log_corrected / prod_corrected backward
  *                    randomras/smoothrast.py:40-59         randomHeaviside.backward
+ *   pert_shade_render / pert_shade_render_phase   the forward of pert_shade_fwd (single call / one phase of a
+ *                    sample-sharded call) when no gradient is wanted (torch.no_grad around smooth_rgb_blend)
  *   pert_soft_shade_fwd / _bwd        the same blend with SoftRast (smoothrast.py:126-134) + SoftAgg
  *                                     (smoothagg.py:165-182), the shaders' default operators
  *   pert_rast_fwd / pert_rast_bwd     randomras/smoothrast.py:12-59   (stand-alone randomHeaviside)
@@ -210,6 +212,20 @@ int pert_shade_fwd(const pert_problem* pb, float* image, uint16_t* counts, float
  *              counts of its tiles here between them.  Unused (may be NULL) otherwise
  */
 int pert_shade_render(const pert_problem* pb, float* image, uint16_t* counts_ws, int32_t* worklist, void* stream);
+
+/*
+ * Forward-only render of one phase of the sample-sharded (phase-split) forward: pb->flags carries exactly one of
+ * PERT_PH_RAST, PERT_PH_AGG and PERT_PH_BLEND, and [s_rast_begin, s_rast_end) / [s_agg_begin, s_agg_end) are this call's
+ * sample shards.  Nothing is stored for backward and no buffer depends on S_rast or S_agg:
+ *   PERT_PH_RAST   writes the shard's hit counts to `counts` (uint16 (P,K)) at the entries with pix_to_face >= 0 only;
+ *                  padding entries are left as they are (zero the buffer before summing it over shards)
+ *   PERT_PH_AGG    reads the all-shard `counts`, writes every entry of `hist` (int32 (P,K1)): the shard's winner histogram
+ *   PERT_PH_BLEND  reads `counts` (alpha) and the all-shard `hist`, writes `image`
+ * For the same problem and phase the outputs equal those of pert_shade_fwd bit for bit.  Flag rules are pert_shade_render's
+ * (PERT_F_CAUCHY, PERT_F_NO_VR, explicit noise, face_colors, pixel_offset, seed_device), except that PERT_F_PHILOX7 is
+ * refused, as in every phase-split call.  No phase bit, several, or a PERT_PH_BWD_* bit returns PERT_E_UNSUPPORTED.
+ */
+int pert_shade_render_phase(const pert_problem* pb, float* image, uint16_t* counts, int32_t* hist, void* stream);
 
 /*
  * Backward.  grad_image (P,4).  Outputs grad_dists, grad_zbuf (P,K), grad_colors (P,K,3; may be

@@ -320,6 +320,33 @@ extern "C" int pert_shade_render(const pert_problem* pb_in, float* image, uint16
     return cuda_rc(launch_shade_render(a, &fb, st));
 }
 
+extern "C" int pert_shade_render_phase(const pert_problem* pb_in, float* image, uint16_t* counts, int32_t* hist,
+                                       void* stream) {
+    int rc = check_problem(pb_in);
+    if (rc) return rc;
+    FwdArgs a = {};
+    a.pb = *pb_in;
+    const uint32_t f = a.pb.flags;
+    const uint32_t ph = f & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND);
+    // one forward phase per call (the collectives sit between them); backward phases have no forward-only form
+    if (ph == 0 || (ph & (ph - 1)) || (f & (PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH))) return PERT_E_UNSUPPORTED;
+    if (!counts) return PERT_E_NULL;
+    if (ph != PERT_PH_RAST && !hist) return PERT_E_NULL;
+    if (ph == PERT_PH_BLEND && (!image || (!a.pb.colors && !a.pb.face_colors))) return PERT_E_NULL;
+    if (((uintptr_t)image & 15) || ((uintptr_t)counts & 1) || ((uintptr_t)hist & 3) || ((uintptr_t)a.pb.colors & 3))
+        return PERT_E_ALIGN;
+    if (f & PERT_F_PHILOX7) return PERT_E_UNSUPPORTED;
+    if (cauchy_flags_bad(f) || no_vr_flags_bad(f)) return PERT_E_UNSUPPORTED;
+    if (f & PERT_F_NO_VR) a.pb.flags |= PERT_F_PER_SAMPLE_NOISE;  // as in pert_shade_render
+    a.image = image;
+    a.counts = counts;
+    a.hist = hist;
+    FwdArgs fb;
+    rc = fwd_launch_records(a, fb, false);  // the tiles of pert_shade_fwd's phase calls
+    if (rc < 0) return rc;
+    return cuda_rc(launch_shade_render(a, nullptr, (cudaStream_t)stream));
+}
+
 extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image, const uint16_t* counts,
                               const float* rsum, const void* winners, const uint16_t* pixstate, float* grad_dists,
                               float* grad_zbuf, float* grad_colors, float* scalar_partials, float* grad_scalars,

@@ -43,7 +43,8 @@ void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes,
 // `fb` (optional): launch record of the fallback pass of the sparse-first mode (half-size tiles)
 int launch_shade_fwd(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st);
 int launch_shade_bwd(const BwdArgs& a, const BwdArgs* fb, float* grad_scalars, cudaStream_t st);
-// forward-only render: image only (a.counts = the fallback pass's workspace or NULL; no other saved state)
+// forward-only render: image only (a.counts = the fallback pass's workspace or NULL; no other saved state); with one phase
+// bit (pert_shade_render_phase) a.counts / a.hist are that phase's inputs and outputs
 int launch_shade_render(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st);
 
 void soft_smem_layout(int tp, int K, bool bwd, SmemLayout& L);

@@ -52,10 +52,11 @@ constexpr int kCmpMin = 12;
 // WOVR = true: the estimator without control variates (PERT_F_NO_VR): rsum = sum_s h psi(U), so an entry that is
 // covered by every sample still draws them all; only the side x < -sigma*Umax (h = 0 always) is skipped, and the
 // compound sampler (which produces sum_s (h - h0) U only) is compiled out.  Counts, winners and image are unchanged.
-// RENDER = true: the forward-only render (pert_shade_render): nothing is stored for backward (no rsum, winners, pixstate
-// or tile blob); coverage computes counts only, from the same counters, so counts, histogram and image are those of the
-// training forward.  Counts go to global memory only in the coverage-sample launch of a split fallback pass (a.counts is
-// then the caller's S-independent workspace), which the aggregation launch reads back.
+// RENDER = true: the forward-only render (pert_shade_render, pert_shade_render_phase): nothing is stored for backward (no
+// rsum, winners, pixstate or tile blob); coverage computes counts only, from the same counters, so counts, histogram and
+// image are those of the training forward.  Counts go to global memory only in a coverage-only call: the coverage-sample
+// launch of a split fallback pass (a.counts is then the caller's S-independent workspace), which the aggregation launch
+// reads back, or the RAST call of a phase-split render (PHASED).
 // Fallback records (common.cuh; training with a tile blob, a.blob then points at the records region): the coverage launch
 // stores the half-tile's valid list; REC = true (aggregation launch) loads it instead of re-scanning pix_to_face and stores
 // what backward would recompute, the per-pixel logit summary and zeta.
@@ -474,11 +475,14 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
 
 // CTAs (= warps) per SM of the main kernel.  Training: 32 (64 registers); the Cauchy instantiations (SCORE = 1) and those
 // without control variates (WOVR) get 24 (80 registers): at 64 the in-kernel Cauchy stream and the ungated coverage samples
-// of WOVR spill.  Render: 28 (72 registers; at 64 the Philox-10 and explicit-noise renders spill), 24 for Cauchy.
-constexpr int fwd_min_ctas(int score, bool wovr, bool render) { return (score || wovr) ? 24 : render ? 28 : 32; }
+// of WOVR spill.  Render: 28 (72 registers; at 64 the Philox-10 and explicit-noise renders spill), 24 for Cauchy and for the
+// phase-split render (its in-kernel Gaussian and explicit-rast instantiations spill at 72).
+constexpr int fwd_min_ctas(int score, bool wovr, bool render, bool phased) {
+    return (score || wovr || (render && phased)) ? 24 : render ? 28 : 32;
+}
 
 template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER, int SCORE, bool WOVR, bool RENDER>
-__global__ void __launch_bounds__(FNT, fwd_min_ctas(SCORE, WOVR, RENDER))
+__global__ void __launch_bounds__(FNT, fwd_min_ctas(SCORE, WOVR, RENDER, PHASED))
     shade_fwd_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     NoiseR nr = noise_r;
@@ -594,10 +598,10 @@ static int launch_production(const FwdArgs& a, const FwdArgs* fb, cudaStream_t s
 // Cauchy noise turns off every skip of the Gaussian path (kBounded): each valid entry draws all its coverage samples and
 // every finite logit takes part in the argmax.  The pair without control variates keeps the two skips that stay exact for
 // it, entries with x < -sigma*Umax and logits that cannot win.  In-kernel Gaussian noise runs the production kernels, or in
-// training the phase-split ones of the sample-sharded job.
-template <class PN, int SCORE, bool WOVR, bool RENDER>
+// training the phase-split ones of the sample-sharded job.  PHASED: the instantiations carry the phase-split code; always in
+// training, in the render only for the phase calls of pert_shade_render_phase.
+template <class PN, int SCORE, bool WOVR, bool RENDER, bool PHASED = !RENDER>
 static int launch_pair(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    constexpr bool PHASED = !RENDER;  // the render has no phase-split form
     const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
     PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
     ExplicitNoise xr{a.pb.noise_rast, a.L.P, a.pb.K, a.pb.S_rast}, xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
@@ -611,9 +615,9 @@ static int launch_pair(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
             const uint32_t all = PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
             if ((a.pb.flags & all) != all || a.hist != nullptr) {  // compile-time lanes per pixel for the benchmark geometries
                 switch (a.L.G) {
-                    case 4: return launch_t<PN, PN, 4, true, false, 0, false, false>(a, pr, pa, st);
-                    case 8: return launch_t<PN, PN, 8, true, false, 0, false, false>(a, pr, pa, st);
-                    default: return launch_t<PN, PN, 0, true, false, 0, false, false>(a, pr, pa, st);
+                    case 4: return launch_t<PN, PN, 4, true, false, 0, false, RENDER>(a, pr, pa, st);
+                    case 8: return launch_t<PN, PN, 8, true, false, 0, false, RENDER>(a, pr, pa, st);
+                    default: return launch_t<PN, PN, 0, true, false, 0, false, RENDER>(a, pr, pa, st);
                 }
             }
         }
@@ -628,11 +632,14 @@ int launch_shade_fwd(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
     return launch_pair<PhiloxNoise, 0, false, false>(a, fb, st);
 }
 
-// The forward with RENDER = true (shade_fwd_tile): single calls only, nothing saved for backward.  The pair without control
-// variates renders on the Gaussian per-sample path (cabi.cu), whose counts, histogram and image it shares.
+// The forward with RENDER = true (shade_fwd_tile): nothing saved for backward.  A single call runs the single-call
+// instantiations; a call with a phase bit (pert_shade_render_phase: exactly one) the phase-split ones.  The pair without
+// control variates renders on the Gaussian per-sample path (cabi.cu), whose counts, histogram and image it shares.
 int launch_shade_render(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    if (a.pb.flags & PERT_F_CAUCHY) return launch_pair<PhiloxCauchy, 1, false, true>(a, fb, st);
-    return launch_pair<PhiloxNoise, 0, false, true>(a, fb, st);
+    const bool phased = (a.pb.flags & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND)) != 0;
+    if (a.pb.flags & PERT_F_CAUCHY)
+        return phased ? launch_pair<PhiloxCauchy, 1, false, true, true>(a, fb, st) : launch_pair<PhiloxCauchy, 1, false, true>(a, fb, st);
+    return phased ? launch_pair<PhiloxNoise, 0, false, true, true>(a, fb, st) : launch_pair<PhiloxNoise, 0, false, true>(a, fb, st);
 }
 
 }  // namespace pert

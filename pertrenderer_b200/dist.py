@@ -16,6 +16,8 @@ Noise-sample sharding (BASELINE config 4: few pixels, thousands of samples)
     (NCCL over NVLink on the GPU box, gloo in the CPU tests); the phases are the PERT_PH_* phases of
     the fused kernels.  The orchestration is written against a small ``stages`` interface so that
     the CPU tests can drive it with the oracle while production drives it with the CUDA kernels.
+    Without gradients (``torch.no_grad``) the same AR1 / AR2 sequence drives the forward-only phases
+    (``pert_shade_render_phase``), which store nothing for backward: no buffer grows with the sample counts.
 """
 
 from __future__ import annotations
@@ -84,44 +86,59 @@ class CudaStages:
     (AR2), and ONE flat float buffer holds, back to back, the argmax score sums (P,K1), the two per-pixel sums (P,2) and
     the coverage score sums rsum (P,K) -- the kernels write / read its three regions through separate pointers and AR3
     reduces it in one call (rsum is only needed by the last backward phase, SURVEY.md §8e, so it rides along there
-    instead of doubling AR1)."""
+    instead of doubling AR1).
 
-    def __init__(self, pr):
+    ``render=True``: the forward-only phases (pert_shade_render_phase), for calls that need no gradient.  They keep only
+    the uint16 counts, their int32 all-reduce copy and the histogram, none of which depends on the sample counts; there
+    is no backward."""
+
+    def __init__(self, pr, render=False):
         from . import _cabi, ops
-        self.ops, self.cabi, self.pr = ops, _cabi, pr
+        self.ops, self.cabi, self.pr, self.render = ops, _cabi, pr, render
         N, H, W, K = pr.shape
         dev = pr.device
         P, K1 = N * H * W, K + 1
-        self.flat = torch.zeros((P * K1 + 2 * P + P * K,), dtype=torch.float32, device=dev)
-        self.acc = self.flat[:P * K1].view(N, H, W, K1)
-        self.pixstat = self.flat[P * K1:P * K1 + 2 * P].view(N, H, W, 2)
-        rsum = self.flat[P * K1 + 2 * P:].view(N, H, W, K)
-        sa_loc = pr.s_agg[1] - pr.s_agg[0]
-        self.saved = ops.ShadeSaved(
-            counts=torch.zeros((N, H, W, K), dtype=torch.int16, device=dev), rsum=rsum,
-            winners=torch.empty((N, H, W, sa_loc), dtype=pr.winner_dtype(), device=dev),
-            pixstate=torch.empty((N, H, W), dtype=torch.int16, device=dev),
-            hist=torch.empty((N, H, W, K1), dtype=torch.int32, device=dev))
+        if render:
+            self.saved = ops.ShadeSaved(counts=torch.zeros((N, H, W, K), dtype=torch.int16, device=dev), rsum=None,
+                                        winners=None, pixstate=None,
+                                        hist=torch.empty((N, H, W, K1), dtype=torch.int32, device=dev))
+        else:
+            self.flat = torch.zeros((P * K1 + 2 * P + P * K,), dtype=torch.float32, device=dev)
+            self.acc = self.flat[:P * K1].view(N, H, W, K1)
+            self.pixstat = self.flat[P * K1:P * K1 + 2 * P].view(N, H, W, 2)
+            rsum = self.flat[P * K1 + 2 * P:].view(N, H, W, K)
+            sa_loc = pr.s_agg[1] - pr.s_agg[0]
+            self.saved = ops.ShadeSaved(
+                counts=torch.zeros((N, H, W, K), dtype=torch.int16, device=dev), rsum=rsum,
+                winners=torch.empty((N, H, W, sa_loc), dtype=pr.winner_dtype(), device=dev),
+                pixstate=torch.empty((N, H, W), dtype=torch.int16, device=dev),
+                hist=torch.empty((N, H, W, K1), dtype=torch.int32, device=dev))
         self.counts32 = torch.empty((N, H, W, K), dtype=torch.int32, device=dev)
+
+    def _phase(self, phase):
+        if self.render:
+            return self.ops.shade_render_phase(self.pr, phase, self.saved.counts, self.saved.hist)
+        return self.ops.shade_forward(self.pr, phases=phase, saved=self.saved)[0]
 
     def rast(self):
         # entries the kernel does not touch (padding) must be defined: they are summed over ranks
         self.saved.counts.zero_()
-        self.saved.rsum.zero_()
-        self.ops.shade_forward(self.pr, phases=self.cabi.PH_RAST, saved=self.saved)
-        torch.bitwise_and(self.saved.counts.to(torch.int32), 0xFFFF, out=self.counts32)
+        if not self.render:
+            self.saved.rsum.zero_()
+        self._phase(self.cabi.PH_RAST)
+        # widened in place (no (P,K) int32 temporary): int16 -> int32 sign-extends, the mask restores the uint16 value
+        self.counts32.copy_(self.saved.counts).bitwise_and_(0xFFFF)
         return self.counts32
 
     def agg(self, counts32):
         self.saved.counts.copy_(counts32)  # int32 -> the uint16 bit pattern (S_rast <= 65535)
-        self.ops.shade_forward(self.pr, phases=self.cabi.PH_AGG, saved=self.saved)
+        self._phase(self.cabi.PH_AGG)
         return self.saved.hist
 
     def blend(self, hist):
         if hist is not self.saved.hist:
             self.saved.hist.copy_(hist)
-        image, _ = self.ops.shade_forward(self.pr, phases=self.cabi.PH_BLEND, saved=self.saved)
-        return image
+        return self._phase(self.cabi.PH_BLEND)
 
     def bwd_sample(self, grad_image):
         self.ops.shade_backward(self.pr, self.saved, grad_image, phases=self.cabi.PH_BWD_SAMPLE, acc=self.acc,
@@ -151,46 +168,53 @@ def sharded_backward(stages, grad_image, group=None, need_colors=True):
     return stages.bwd_finish(grad_image, packed, need_colors=need_colors)
 
 
+def _sharded_problem(colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg):
+    """This rank's ShadeProblem of a sample-sharded call: its two seeds (broadcast from rank 0 with ``sync_seeds``) and
+    its sample shards.  Shared by the training and the forward-only path, so that the same ``torch.manual_seed`` gives
+    the same image with and without gradients."""
+    from . import ops
+    group = cfg.get("group")
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    dev = pix_to_face.device
+    if cfg.get("sync_seeds", False):
+        # reproduce the single-GPU sample path: rank 0 draws the two seeds, everyone receives them
+        # (one broadcast and one host read per forward)
+        seeds = torch.zeros(2, dtype=torch.int64)
+        if rank == 0:
+            seeds[0] = ops.draw_seed()
+            if cfg["fixed_noise"]:
+                torch.manual_seed(1)
+            seeds[1] = ops.draw_seed()
+        seeds = seeds.to(dev)
+        dist.broadcast(seeds, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
+        seed_r, seed_a = (int(v) for v in seeds.cpu())
+    else:
+        # every rank draws its own seeds from its own torch generator: the shards own disjoint sample
+        # indices, so whatever the seeds are the union is S independent samples (no communication)
+        seed_r = ops.draw_seed()
+        if cfg["fixed_noise"]:
+            torch.manual_seed(1)
+        seed_a = ops.draw_seed()
+    S_r, S_a = int(cfg["S_rast"]), int(cfg["S_agg"])
+    # decided on data every rank has, so that either all ranks raise or none does (a rank that raised alone would
+    # leave the others blocked in the first all-reduce)
+    check_sample_sharding(S_r, S_a, world)
+    sr, sa = sample_range(S_r, world, rank), sample_range(S_a, world, rank)
+    return ops.ShadeProblem(
+        pix_to_face=pix_to_face, zbuf=zbuf, dists=dists, colors=colors, znear=znear, zfar=zfar,
+        background=cfg["background"], sigma=float(sigma), gamma=float(gamma), alpha=float(alpha),
+        eps=float(cfg["eps"]), S_rast=S_r, S_agg=S_a, seed_rast=seed_r, seed_agg=seed_a,
+        flags=ops.current_flags() | int(cfg.get("flags", 0)), s_rast=sr, s_agg=sa)
+
+
 class _SampleShardedShade(Function):
     """Autograd wrapper of the sample-sharded shader; same differentiable inputs as the fused
     single-GPU Function (random_rasterizer._PerturbedShade)."""
 
     @staticmethod
     def forward(ctx, colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg):
-        from . import ops
         group = cfg.get("group")
-        world, rank = dist.get_world_size(group), dist.get_rank(group)
-        dev = pix_to_face.device
-        if cfg.get("sync_seeds", False):
-            # reproduce the single-GPU sample path: rank 0 draws the two seeds, everyone receives them
-            # (one broadcast and one host read per forward)
-            seeds = torch.zeros(2, dtype=torch.int64)
-            if rank == 0:
-                seeds[0] = ops.draw_seed()
-                if cfg["fixed_noise"]:
-                    torch.manual_seed(1)
-                seeds[1] = ops.draw_seed()
-            seeds = seeds.to(dev)
-            dist.broadcast(seeds, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
-            seed_r, seed_a = (int(v) for v in seeds.cpu())
-        else:
-            # every rank draws its own seeds from its own torch generator: the shards own disjoint sample
-            # indices, so whatever the seeds are the union is S independent samples (no communication)
-            seed_r = ops.draw_seed()
-            if cfg["fixed_noise"]:
-                torch.manual_seed(1)
-            seed_a = ops.draw_seed()
-        S_r, S_a = int(cfg["S_rast"]), int(cfg["S_agg"])
-        # decided on data every rank has, so that either all ranks raise or none does (a rank that raised alone would
-        # leave the others blocked in the first all-reduce)
-        check_sample_sharding(S_r, S_a, world)
-        sr, sa = sample_range(S_r, world, rank), sample_range(S_a, world, rank)
-        pr = ops.ShadeProblem(
-            pix_to_face=pix_to_face, zbuf=zbuf, dists=dists, colors=colors, znear=znear, zfar=zfar,
-            background=cfg["background"], sigma=float(sigma), gamma=float(gamma), alpha=float(alpha),
-            eps=float(cfg["eps"]), S_rast=S_r, S_agg=S_a, seed_rast=seed_r, seed_agg=seed_a,
-            flags=ops.current_flags() | int(cfg.get("flags", 0)), s_rast=sr, s_agg=sa)
-        stages = CudaStages(pr)
+        stages = CudaStages(_sharded_problem(colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg))
         image = sharded_forward(stages, group)
         ctx.stages, ctx.group, ctx.scalars = stages, group, (sigma, gamma, alpha)
         return image
@@ -224,8 +248,13 @@ def smooth_rgb_blend_sample_sharded(colors, fragments, smoothrast, smoothagg, bl
     cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps, S_rast=smoothrast.nb_samples,
                S_agg=smoothagg.nb_samples, fixed_noise=bool(smoothagg.fixed_noise), group=group, sync_seeds=sync_seeds,
                flags=flags)
-    return _SampleShardedShade.apply(colors, fragments.dists, fragments.zbuf, smoothrast.sigma, smoothagg.gamma,
-                                     smoothagg.alpha, fragments.pix_to_face, znear, zfar, cfg)
+    args = (colors, fragments.dists, fragments.zbuf, smoothrast.sigma, smoothagg.gamma, smoothagg.alpha,
+            fragments.pix_to_face, znear, zfar, cfg)
+    # no gradient wanted: the forward-only phases, whose buffers do not grow with the sample counts.  Decided here:
+    # inside Function.forward grad mode is always off
+    if not torch.is_grad_enabled():
+        return sharded_forward(CudaStages(_sharded_problem(*args), render=True), group)
+    return _SampleShardedShade.apply(*args)
 
 
 class GraphedSampleShardedStep:

@@ -316,6 +316,23 @@ def shade_render(pr: ShadeProblem, return_worklist: bool = False):
     return (image, worklist) if return_worklist else image
 
 
+def shade_render_phase(pr: ShadeProblem, phase: int, counts: torch.Tensor, hist: Optional[torch.Tensor] = None):
+    """Launch pert_shade_render_phase: one phase (PH_RAST, PH_AGG or PH_BLEND) of the sample-sharded forward on the shards
+    ``pr.s_rast`` / ``pr.s_agg``, without the state backward would need.  ``counts`` int16 storage of uint16 (N,H,W,K): the
+    shard's hit counts (PH_RAST writes the valid entries only), then the all-shard counts (PH_AGG, PH_BLEND read them).
+    ``hist`` int32 (N,H,W,K+1): PH_AGG writes the shard's winner histogram, PH_BLEND reads the all-shard one.  Returns the
+    image (N,H,W,4) for PH_BLEND, else None."""
+    fn = _cabi.shade_render_phase_fn()
+    require_cuda(counts, hist)
+    N, H, W, K = pr.shape
+    dev = pr.device
+    with torch.cuda.device(dev):
+        image = torch.empty((N, H, W, 4), dtype=torch.float32, device=dev) if phase & PH_BLEND else None
+        rc = fn(pr.c_struct(flags=pr.flags | phase), ptr(image), ptr(counts), ptr(hist), stream_ptr(dev))
+    check(rc, "pert_shade_render_phase")
+    return image
+
+
 def shade_backward(pr: ShadeProblem, saved: ShadeSaved, grad_image: torch.Tensor, need_colors: bool = True,
                    phases: int = 0, acc=None, pixstat=None, use_hist: bool = False):
     """Launch pert_shade_bwd.  Returns (grad_dists, grad_zbuf, grad_colors | None, grad_scalars(3))."""
