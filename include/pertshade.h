@@ -339,6 +339,32 @@ int pert_phong_bwd(const pert_phong* ph, const float* grad_colors, float* grad_t
                    float* grad_face_verts, float* grad_face_normals, float* grad_lighting, void* stream);
 
 /*
+ * Phong with a per-face texture atlas as the texel source (pytorch3d TexturesAtlas, the ShapeNet models of
+ * experiments/eval.py:216-238): atlas float (ph->num_faces, R, R, 3), R = atlas_size, indexed by the packed face id.  The
+ * texel of a valid entry is the atlas cell that its first two barycentric coordinates w0, w1 pick, in float32:
+ *   w   = torch.nan_to_num(w, nan=0): NaN -> 0, +-inf -> +-FLT_MAX (both coordinates)
+ *   wxy = trunc(clamp(w * R, -1, R)), then at most R - 1
+ *   below = (w0 + w1) * R - (wx + wy) <= 1     (each operation rounded once, no fused multiply-add)
+ *   (wx, wy) = below ? (wx, wy) : (R - 1 - wx, R - 1 - wy), then clamped to [0, R - 1]
+ *   texel = atlas[face, wy, wx]
+ * which is AtlasTexels.materialize (pertrenderer_b200/structures.py).  Padded entries get texel 0.  Everything else
+ * (flags, lighting, sparse / unlit modes, validation) is pert_phong_fwd / pert_phong_bwd's, except the texel source:
+ * ph->texels, face_colors, face_vert_colors and uv_map must all be NULL (else PERT_E_UNSUPPORTED); a NULL atlas returns
+ * PERT_E_NULL, atlas_size <= 0 PERT_E_SHAPE, and num_faces * R^2 * 3 > 2^31 - 1 (32-bit atlas offsets) PERT_E_UNSUPPORTED.
+ * Neither call synchronises: both can be captured in a CUDA graph.
+ */
+int pert_phong_atlas_fwd(const pert_phong* ph, const float* atlas, int32_t atlas_size, float* colors, void* stream);
+/*
+ * Backward of pert_phong_atlas_fwd.  Outputs as pert_phong_bwd's, each optional (NULL: not computed), with grad_atlas in
+ * the place of grad_texels: the atlas's shape, ZEROED BY THE CALLER, the texel gradient atomically added into the cell of
+ * every entry (summation order is not fixed).  The atlas texel is piecewise constant in the barycentric coordinates, so
+ * it adds nothing to grad_bary: lit entries get the gradient of their position and normal only, unlit entries zero.
+ */
+int pert_phong_atlas_bwd(const pert_phong* ph, const float* atlas, int32_t atlas_size, const float* grad_colors,
+                         float* grad_atlas, float* grad_bary, float* grad_face_verts, float* grad_face_normals,
+                         float* grad_lighting, void* stream);
+
+/*
  * Fragment producer: K-deep rasterisation of packed triangle meshes with a blur radius, the Fragments
  * (pix_to_face, zbuf, bary_coords, dists) of pytorch3d's MeshRasterizer as the reference configures it
  * (experiments/eval.py:135-141: blur_radius = log(1/1e-4 - 1) * sigma, faces_per_pixel = 50,

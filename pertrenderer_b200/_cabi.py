@@ -32,7 +32,8 @@ PH_BWD_SAMPLE, PH_BWD_FINISH = 0x100, 0x200
 EXPORTS = [
     "pert_version", "pert_shade_fused_flags", "pert_strerror", "pert_last_cuda_error", "pert_num_tiles", "pert_winner_bytes", "pert_blob_bytes",
     "pert_shade_fwd", "pert_shade_render", "pert_shade_render_phase", "pert_shade_bwd", "pert_soft_shade_fwd", "pert_soft_shade_bwd", "pert_rast_fwd", "pert_rast_bwd", "pert_argmax_fwd",
-    "pert_argmax_bwd", "pert_noise_fill", "pert_seed_advance", "pert_phong_fwd", "pert_phong_bwd", "pert_rasterize_fwd", "pert_rasterize_bwd", "pert_rasterize_num_bins", "pert_rasterize_bin",
+    "pert_argmax_bwd", "pert_noise_fill", "pert_seed_advance", "pert_phong_fwd", "pert_phong_bwd", "pert_phong_atlas_fwd", "pert_phong_atlas_bwd",
+    "pert_rasterize_fwd", "pert_rasterize_bwd", "pert_rasterize_num_bins", "pert_rasterize_bin",
 ]
 
 RAST_CULL_BACKFACES = 1  # PERT_RAST_CULL_BACKFACES
@@ -222,6 +223,27 @@ def shade_render_phase_fn():
     if _render_phase is None or _render_phase[0] is not load():
         _render_phase = _bind_render("pert_shade_render_phase", "the sample-sharded forward-only render")
     return _render_phase[1]
+
+
+_phong_atlas = None  # (library, its bound pert_phong_atlas_fwd, pert_phong_atlas_bwd)
+
+
+def phong_atlas_fns():
+    """(``pert_phong_atlas_fwd``, ``pert_phong_atlas_bwd``) of the loaded library, bound on first use rather than in
+    :func:`load`, so that a library built before them keeps serving every other call; with such a library this raises
+    PertLibraryError asking for a rebuild."""
+    global _phong_atlas
+    lib = load()
+    if _phong_atlas is None or _phong_atlas[0] is not lib:
+        fwd, bwd = getattr(lib, "pert_phong_atlas_fwd", None), getattr(lib, "pert_phong_atlas_bwd", None)
+        if fwd is None or bwd is None:
+            raise PertLibraryError(f"{LIB_PATH} predates the texture-atlas Phong kernels (pert_phong_atlas_fwd / _bwd): "
+                                   "rebuild it with `python -m pertrenderer_b200.build --force`")
+        fwd.restype = bwd.restype = C.c_int
+        fwd.argtypes = [C.POINTER(PertPhong), C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+        bwd.argtypes = [C.POINTER(PertPhong), C.c_void_p, C.c_int32] + [C.c_void_p] * 7
+        _phong_atlas = (lib, fwd, bwd)
+    return _phong_atlas[1], _phong_atlas[2]
 
 
 def check(rc: int, what: str):

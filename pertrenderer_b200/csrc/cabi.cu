@@ -526,7 +526,8 @@ extern "C" int pert_noise_fill(uint64_t seed, int32_t stage, int64_t P, int32_t 
     return cuda_rc(launch_noise_fill(seed, stage, P, slots, s_begin, s_end, pixel_offset, out, (cudaStream_t)stream));
 }
 
-static int check_phong(const pert_phong* ph) {
+// atlas: the call brings its own texel source (pert_phong_atlas_*), and none of ph's may be set
+static int check_phong(const pert_phong* ph, bool atlas = false) {
     if (!ph) return PERT_E_NULL;
     if (ph->P <= 0 || ph->HW <= 0 || ph->K <= 0 || ph->num_faces <= 0 || ph->P % ph->HW != 0) return PERT_E_SHAPE;
     if (ph->num_faces > 0x7fffffff / 27 || ph->P >= ((int64_t)1 << 32) / ph->K) return PERT_E_UNSUPPORTED;  // 32-bit entry indices
@@ -534,8 +535,9 @@ static int check_phong(const pert_phong* ph) {
     if (!unlit && ph->light_rows != 1 && ph->light_rows != ph->P / ph->HW) return PERT_E_SHAPE;
     if (!ph->pix_to_face || !ph->bary) return PERT_E_NULL;
     if (!unlit && (!ph->face_verts || !ph->face_normals || !ph->lighting)) return PERT_E_NULL;
-    if ((ph->texels != nullptr) + (ph->face_colors != nullptr) + (ph->face_vert_colors != nullptr) + (ph->uv_map != nullptr) != 1)
-        return PERT_E_NULL;
+    const int sources = (ph->texels != nullptr) + (ph->face_colors != nullptr) + (ph->face_vert_colors != nullptr) + (ph->uv_map != nullptr);
+    if (atlas && sources != 0) return PERT_E_UNSUPPORTED;
+    if (!atlas && sources != 1) return PERT_E_NULL;
     if (ph->uv_map && (!ph->face_uvs || ph->map_h <= 0 || ph->map_w <= 0 || (ph->map_count != 1 && ph->map_count != ph->P / ph->HW)))
         return PERT_E_SHAPE;
     if (((uintptr_t)ph->uv_map & 3) || ((uintptr_t)ph->face_uvs & 3)) return PERT_E_ALIGN;
@@ -566,6 +568,41 @@ extern "C" int pert_phong_bwd(const pert_phong* ph, const float* grad_colors, fl
                                               (cudaStream_t)stream)))
             return rc;
     if (grad_lighting) return cuda_rc(launch_phong_light_bwd(*ph, grad_colors, grad_lighting, (cudaStream_t)stream));
+    return PERT_OK;
+}
+
+static int check_phong_atlas(const pert_phong* ph, const float* atlas, int32_t atlas_size) {
+    if (int rc = check_phong(ph, true)) return rc;
+    if (!atlas) return PERT_E_NULL;
+    if (atlas_size <= 0) return PERT_E_SHAPE;
+    // 32-bit atlas offsets: num_faces R^2 3 <= 2^31 - 1 (written so that nothing overflows)
+    if ((int64_t)atlas_size * atlas_size > 0x7fffffff / 3 / ph->num_faces) return PERT_E_UNSUPPORTED;
+    if ((uintptr_t)atlas & 3) return PERT_E_ALIGN;
+    return PERT_OK;
+}
+
+extern "C" int pert_phong_atlas_fwd(const pert_phong* ph, const float* atlas, int32_t atlas_size, float* colors, void* stream) {
+    if (int rc = check_phong_atlas(ph, atlas, atlas_size)) return rc;
+    if (!colors) return PERT_E_NULL;
+    if ((uintptr_t)colors & 3) return PERT_E_ALIGN;
+    return cuda_rc(launch_phong_fwd(*ph, colors, (cudaStream_t)stream, atlas, atlas_size));
+}
+
+extern "C" int pert_phong_atlas_bwd(const pert_phong* ph, const float* atlas, int32_t atlas_size, const float* grad_colors,
+                                    float* grad_atlas, float* grad_bary, float* grad_face_verts, float* grad_face_normals,
+                                    float* grad_lighting, void* stream) {
+    if (int rc = check_phong_atlas(ph, atlas, atlas_size)) return rc;
+    if (!grad_colors) return PERT_E_NULL;
+    if (((uintptr_t)grad_colors & 3) || ((uintptr_t)grad_atlas & 3) || ((uintptr_t)grad_bary & 3) ||
+        ((uintptr_t)grad_face_verts & 3) || ((uintptr_t)grad_face_normals & 3) || ((uintptr_t)grad_lighting & 3))
+        return PERT_E_ALIGN;
+    if (grad_lighting && (ph->flags & PERT_PHONG_UNLIT)) return PERT_E_UNSUPPORTED;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (grad_atlas || grad_bary || grad_face_verts || grad_face_normals)
+        if (int rc = cuda_rc(launch_phong_bwd(*ph, grad_colors, grad_atlas, grad_bary, grad_face_verts, grad_face_normals, st, atlas,
+                                              atlas_size)))
+            return rc;
+    if (grad_lighting) return cuda_rc(launch_phong_light_bwd(*ph, grad_colors, grad_lighting, st, atlas, atlas_size));
     return PERT_OK;
 }
 

@@ -62,10 +62,13 @@ int launch_argmax_fwd(const float* z, int64_t P, int K1, int S, int s_begin, int
 int launch_argmax_bwd(const float* grad_l, const float* z, const void* winners, int64_t P, int K1, int S, int s_begin,
                       int s_end, float gamma, uint64_t seed, int64_t pixel_offset, const float* noise, uint32_t flags,
                       float* grad_z, float* partials, float* grad_gamma, cudaStream_t st);
-int launch_phong_fwd(const pert_phong& ph, float* colors, cudaStream_t st);
+// atlas != NULL: the texel source is the (num_faces, atlas_r, atlas_r, 3) atlas (pert_phong_atlas_fwd / _bwd), and
+// grad_texels is its gradient
+int launch_phong_fwd(const pert_phong& ph, float* colors, cudaStream_t st, const float* atlas = nullptr, int atlas_r = 0);
 int launch_phong_bwd(const pert_phong& ph, const float* grad_colors, float* grad_texels, float* grad_bary, float* grad_fv,
-                     float* grad_fn, cudaStream_t st);
-int launch_phong_light_bwd(const pert_phong& ph, const float* grad_colors, float* grad_lighting, cudaStream_t st);
+                     float* grad_fn, cudaStream_t st, const float* atlas = nullptr, int atlas_r = 0);
+int launch_phong_light_bwd(const pert_phong& ph, const float* grad_colors, float* grad_lighting, cudaStream_t st,
+                           const float* atlas = nullptr, int atlas_r = 0);
 int launch_rasterize_bin(const pert_raster& rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
                          int64_t* bin_faces, cudaStream_t st);
 int launch_rasterize_fwd(const pert_raster& rs, int64_t* pix_to_face, float* zbuf, float* bary, float* dists, cudaStream_t st);

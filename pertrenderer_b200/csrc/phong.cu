@@ -190,6 +190,42 @@ __device__ __forceinline__ V3 texel_of(const pert_phong& ph, int64_t e, int64_t 
     if (ph.uv_map) return uv_texel(uv_src(ph), e, face, b);
     return texel_of_plain(ph, e, face, b);
 }
+// Per-face texture atlas (TexturesAtlas; the ShapeNet models of experiments/eval.py:216-238): atlas (F,R,R,3), an R x R
+// grid of texels per packed face.  pert_phong has no room for it, so the atlas kernels take this record as a parameter of
+// their own, BY VALUE for the reason given at UvSrc; only the ATLAS instantiations read it.
+struct AtlasSrc {
+    const float* atlas;
+    int R;
+};
+// Float offset of the cell that (w0, w1) picks: AtlasTexels.materialize's rule (structures.py), op for op in float32 --
+// torch.nan_to_num (NaN -> 0, +-inf -> +-FLT_MAX); w R rounded once, clamped to [-1, R] before the truncation, then to
+// R - 1; the point is below the diagonal when (w0 + w1) R - (wx + wy) <= 1 (each op rounded once, no FMA), else the cell
+// is reflected; finally clamped to the grid.
+// The barycentric coordinates of the rasteriser are unclipped (outside [0, 1] in the blur band): every cell stays in range.
+// num_faces R^2 3 < 2^31 (pert_phong_atlas_fwd refuses larger atlases): 32-bit offsets.
+__device__ __forceinline__ int atlas_cell(AtlasSrc a, int face, float w0, float w1) {
+    const float rf = (float)a.R;
+    w0 = isnan(w0) ? 0.0f : fminf(fmaxf(w0, -CUDART_MAX_NORMAL_F), CUDART_MAX_NORMAL_F);
+    w1 = isnan(w1) ? 0.0f : fminf(fmaxf(w1, -CUDART_MAX_NORMAL_F), CUDART_MAX_NORMAL_F);
+    int wx = min((int)fminf(fmaxf(__fmul_rn(w0, rf), -1.0f), rf), a.R - 1);
+    int wy = min((int)fminf(fmaxf(__fmul_rn(w1, rf), -1.0f), rf), a.R - 1);
+    if (!(__fsub_rn(__fmul_rn(__fadd_rn(w0, w1), rf), (float)(wx + wy)) <= 1.0f)) {
+        wx = a.R - 1 - wx;
+        wy = a.R - 1 - wy;
+    }
+    wx = min(max(wx, 0), a.R - 1);
+    wy = min(max(wy, 0), a.R - 1);
+    return ((face * a.R + wy) * a.R + wx) * 3;
+}
+__device__ __forceinline__ V3 atlas_texel(AtlasSrc a, int64_t face, V3 b) { return ld3(a.atlas + atlas_cell(a, (int)face, b.x, b.y)); }
+
+// Texel of the call's source: the atlas in the ATLAS instantiations, else texel_of
+template <bool ATLAS>
+__device__ __forceinline__ V3 texel_src(const pert_phong& ph, AtlasSrc at, int64_t e, int64_t face, V3 b) {
+    if (ATLAS) return atlas_texel(at, face, b);
+    return texel_of(ph, e, face, b);
+}
+
 // floats per face of the texel source's gradient table (0: dense (P,K,3) gradient, or the UV map's own gradient)
 __host__ __device__ __forceinline__ int tex_floats(const pert_phong& ph) {
     return ph.uv_map ? 0 : (ph.face_vert_colors ? 9 : (ph.face_colors ? 3 : 0));
@@ -232,15 +268,16 @@ struct WarpCtx {
     float* srow;      // 2 * PERT_PHONG_STRIDE
 };
 
+template <bool ATLAS>
 __global__ void __launch_bounds__(PT) phong_fwd_kernel(const pert_phong ph, float* __restrict__ colors, int64_t E,
-                                                       int64_t nchunks, int vec_ok) {
+                                                       int64_t nchunks, int vec_ok, AtlasSrc at) {
     __shared__ __align__(16) uint16_t s_vlist[PW][WCHUNK];
     __shared__ float s_row[PW][2 * PERT_PHONG_STRIDE];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     uint16_t* const vlist = s_vlist[warp];
     float* const srow = s_row[warp];
     const bool sparse = ph.flags & PERT_PHONG_SPARSE, unlit = ph.flags & PERT_PHONG_UNLIT;
-    const bool table_tex = ph.face_colors || ph.face_vert_colors || ph.uv_map;
+    const bool table_tex = ATLAS || ph.face_colors || ph.face_vert_colors || ph.uv_map;
     const int64_t HWK = ph.HW * ph.K;
     int64_t cached_b0 = -1;
     const int64_t w0 = (int64_t)blockIdx.x * PW + warp, wstride = (int64_t)gridDim.x * PW;
@@ -276,7 +313,7 @@ __global__ void __launch_bounds__(PT) phong_fwd_kernel(const pert_phong ph, floa
             const int64_t e = e_base + vlist[i];
             const int64_t face = __ldg(ph.pix_to_face + e);
             const V3 b = ld3(ph.bary + e * 3);
-            const V3 t = texel_of(ph, e, face, b);
+            const V3 t = texel_src<ATLAS>(ph, at, e, face, b);
             if (unlit) {  // texture sampling only (Meshes.sample_textures)
                 st3(colors + e * 3, t);
                 continue;
@@ -321,11 +358,11 @@ __device__ __forceinline__ void scatter9(bool in_table, float* sm, float* gl, V3
 
 // the streaming loop is latency-bound: resident warps matter more than a few spills in the rare branches
 // (measured without the cap: 80 -> 120 registers as texel sources were added, 154 -> 224 us)
-template <bool TABLE, int NT, bool UV>
+template <bool TABLE, int NT, bool UV, bool ATLAS>
 __global__ void __launch_bounds__(NT, NT <= 128 ? 6 : 1) phong_bwd_kernel(const pert_phong ph, const float* __restrict__ grad_colors,
                                                        float* __restrict__ grad_texels, float* __restrict__ grad_bary,
                                                        float* __restrict__ grad_fv, float* __restrict__ grad_fn, int64_t E,
-                                                       int64_t nchunks, int tfaces, int per_image) {
+                                                       int64_t nchunks, int tfaces, int per_image, AtlasSrc at) {
     // dynamic shared memory: [TABLE: F*9 (verts) | F*9 (normals) | F*3 (face colours) or F*9 (corner colours)] then per warp
     // vlist u16[WCHUNK] | hlist u16[WCHUNK] | lighting rows float[2 * PERT_PHONG_STRIDE]
     extern __shared__ __align__(16) float table[];
@@ -348,7 +385,8 @@ __global__ void __launch_bounds__(NT, NT <= 128 ? 6 : 1) phong_bwd_kernel(const 
     float* const t_fc = table + F * 18;
     constexpr bool uv_tex = UV;  // UV map: texel gradient scattered into the map (grad_texels = d/d uv_map); its own
                                  // instantiation, so that the common kernels carry none of its code
-    const bool face_tex = ph.face_colors || ph.face_vert_colors || uv_tex;  // texel gradient not dense
+    // ATLAS: texel gradient added into the atlas cell (grad_texels = d/d atlas), global atomics; its own instantiation too
+    const bool face_tex = ATLAS || ph.face_colors || ph.face_vert_colors || uv_tex;  // texel gradient not dense
     const bool vert_tex = ph.face_vert_colors != nullptr;
     const int TF = tex_floats(ph);
     const bool unlit = ph.flags & PERT_PHONG_UNLIT;
@@ -421,7 +459,7 @@ __global__ void __launch_bounds__(NT, NT <= 128 ? 6 : 1) phong_bwd_kernel(const 
             const bool tab = TABLE && fl >= 0 && fl < F;
             const V3 gc = ld3(grad_colors + e * 3);
             const V3 b = ld3(ph.bary + e * 3);
-            const V3 t = UV ? uv_texel(uv_src(ph), e, face, b) : texel_of_plain(ph, e, face, b);
+            const V3 t = ATLAS ? atlas_texel(at, face, b) : (UV ? uv_texel(uv_src(ph), e, face, b) : texel_of_plain(ph, e, face, b));
             Row L;
             Lit o;
             V3 v0, v1, v2, n0, n1, n2;
@@ -443,6 +481,13 @@ __global__ void __launch_bounds__(NT, NT <= 128 ? 6 : 1) phong_bwd_kernel(const 
             }
             if (uv_tex) {  // texel = bilinear(map, sum_i b_i uv_i): gradient to the four taps and, through (u, v), to bary
                 gb = uv_texel_bwd(uv_src(ph), e, face, b, gt, grad_texels);
+            } else if (ATLAS) {  // texel = atlas[face, cell(b)]: piecewise constant in b, nothing to bary
+                if (grad_texels) {
+                    float* dst = grad_texels + atlas_cell(at, face, b.x, b.y);
+                    atomicAdd(dst, gt.x);
+                    atomicAdd(dst + 1, gt.y);
+                    atomicAdd(dst + 2, gt.z);
+                }
             } else if (grad_texels) {
                 if (vert_tex) {
                     scatter9(tab, t_fc + fl * 9, grad_texels + (int64_t)face * 9, b, gt);
@@ -503,8 +548,10 @@ __global__ void __launch_bounds__(NT, NT <= 128 ? 6 : 1) phong_bwd_kernel(const 
 // camera centre): a second sparse pass launched only when the caller asks for it (lights and cameras are constants in
 // the reference's pose optimisation, eval.py:233-262, but eval.py:411-470 and :693-725 optimise them).  Every lane
 // keeps the sixteen sums of its entries in registers and adds them to grad_lighting once (per row of the table).
+template <bool ATLAS>
 __global__ void __launch_bounds__(PT) phong_light_bwd_kernel(const pert_phong ph, const float* __restrict__ grad_colors,
-                                                             float* __restrict__ grad_lighting, int64_t E, int64_t nchunks) {
+                                                             float* __restrict__ grad_lighting, int64_t E, int64_t nchunks,
+                                                             AtlasSrc at) {
     __shared__ __align__(16) uint16_t s_vlist[PW][WCHUNK];
     __shared__ float s_row[PW][2 * PERT_PHONG_STRIDE];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -545,7 +592,7 @@ __global__ void __launch_bounds__(PT) phong_light_bwd_kernel(const pert_phong ph
             if (gc.x == 0.0f && gc.y == 0.0f && gc.z == 0.0f) continue;
             const int64_t face = __ldg(ph.pix_to_face + e);
             const V3 b = ld3(ph.bary + e * 3);
-            const V3 t = texel_of(ph, e, face, b);
+            const V3 t = texel_src<ATLAS>(ph, at, e, face, b);
             const float* fv = ph.face_verts + face * 9;
             const float* fn = ph.face_normals + face * 9;
             const V3 p = b.x * ld3(fv) + b.y * ld3(fv + 3) + b.z * ld3(fv + 6);
@@ -598,19 +645,24 @@ unsigned phong_grid(int64_t nchunks, int ctas_per_sm, int warps_per_cta = PW) {
 
 static int vec_ok_of(const pert_phong& ph) { return ((uintptr_t)ph.pix_to_face & 15) == 0; }
 
-int launch_phong_fwd(const pert_phong& ph, float* colors, cudaStream_t st) {
+int launch_phong_fwd(const pert_phong& ph, float* colors, cudaStream_t st, const float* atlas, int atlas_r) {
     const int64_t E = ph.P * ph.K, nchunks = (E + WCHUNK - 1) / WCHUNK;
-    phong_fwd_kernel<<<phong_grid(nchunks, 9), PT, 0, st>>>(ph, colors, E, nchunks, vec_ok_of(ph));
+    const AtlasSrc at{atlas, atlas_r};
+    if (atlas)
+        phong_fwd_kernel<true><<<phong_grid(nchunks, 9), PT, 0, st>>>(ph, colors, E, nchunks, vec_ok_of(ph), at);
+    else
+        phong_fwd_kernel<false><<<phong_grid(nchunks, 9), PT, 0, st>>>(ph, colors, E, nchunks, vec_ok_of(ph), at);
     return (int)cudaGetLastError();
 }
 
-template <bool TABLE, int NT, bool UV = false>
+template <bool TABLE, int NT, bool UV = false, bool ATLAS = false>
 static int launch_bwd_t(const pert_phong& ph, const float* grad_colors, float* grad_texels, float* grad_bary, float* grad_fv,
-                        float* grad_fn, int64_t E, int64_t nchunks, int ctas_per_sm, int tfaces, bool per_image, cudaStream_t st) {
+                        float* grad_fn, int64_t E, int64_t nchunks, int ctas_per_sm, int tfaces, bool per_image, cudaStream_t st,
+                        AtlasSrc at = AtlasSrc{nullptr, 0}) {
     const size_t table = TABLE ? (((size_t)tfaces * (18 + tex_floats(ph)) * 4 + 15) & ~(size_t)15) : 0;
     const size_t smem = table + (size_t)(NT / 32) * (2 * WCHUNK * 2 + 2 * PERT_PHONG_STRIDE * 4);
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(phong_bwd_kernel<TABLE, NT, UV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(phong_bwd_kernel<TABLE, NT, UV, ATLAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
     dim3 grid(phong_grid(nchunks, ctas_per_sm, NT / 32));
@@ -620,20 +672,30 @@ static int launch_bwd_t(const pert_phong& ph, const float* grad_colors, float* g
         const int64_t most = (img_chunks + NT / 32 - 1) / (NT / 32);
         grid = dim3((unsigned)(ctas < most ? ctas : most), (unsigned)n_img);
     }
-    phong_bwd_kernel<TABLE, NT, UV><<<grid, NT, smem, st>>>(ph, grad_colors, grad_texels, grad_bary, grad_fv, grad_fn, E, nchunks,
-                                                       tfaces, per_image ? 1 : 0);
+    phong_bwd_kernel<TABLE, NT, UV, ATLAS><<<grid, NT, smem, st>>>(ph, grad_colors, grad_texels, grad_bary, grad_fv, grad_fn, E,
+                                                                  nchunks, tfaces, per_image ? 1 : 0, at);
     return (int)cudaGetLastError();
 }
 
-int launch_phong_light_bwd(const pert_phong& ph, const float* grad_colors, float* grad_lighting, cudaStream_t st) {
+int launch_phong_light_bwd(const pert_phong& ph, const float* grad_colors, float* grad_lighting, cudaStream_t st,
+                           const float* atlas, int atlas_r) {
     const int64_t E = ph.P * ph.K, nchunks = (E + WCHUNK - 1) / WCHUNK;
-    phong_light_bwd_kernel<<<phong_grid(nchunks, 4), PT, 0, st>>>(ph, grad_colors, grad_lighting, E, nchunks);
+    const AtlasSrc at{atlas, atlas_r};
+    if (atlas)
+        phong_light_bwd_kernel<true><<<phong_grid(nchunks, 4), PT, 0, st>>>(ph, grad_colors, grad_lighting, E, nchunks, at);
+    else
+        phong_light_bwd_kernel<false><<<phong_grid(nchunks, 4), PT, 0, st>>>(ph, grad_colors, grad_lighting, E, nchunks, at);
     return (int)cudaGetLastError();
 }
 
 int launch_phong_bwd(const pert_phong& ph, const float* grad_colors, float* grad_texels, float* grad_bary, float* grad_fv,
-                     float* grad_fn, cudaStream_t st) {
+                     float* grad_fn, cudaStream_t st, const float* atlas, int atlas_r) {
     const int64_t E = ph.P * ph.K, nchunks = (E + WCHUNK - 1) / WCHUNK;
+    // Atlas: its own instantiation, every gradient straight to global memory.  A ShapeNet atlas (tens of thousands of
+    // faces) is far beyond the shared-memory table, and so are the face-vertex and normal tables of such a mesh
+    if (atlas)
+        return launch_bwd_t<false, PT, false, true>(ph, grad_colors, grad_texels, grad_bary, grad_fv, grad_fn, E, nchunks, 6, 0,
+                                                    false, st, AtlasSrc{atlas, atlas_r});
     const bool scatter = grad_fv || grad_fn || (tex_floats(ph) && grad_texels);
     const size_t per_face = (size_t)(18 + tex_floats(ph)) * 4;
     // Small meshes: every entry's 18 atomic adds would land on the same few thousand L2 addresses (measured at

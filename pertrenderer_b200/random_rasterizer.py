@@ -20,7 +20,7 @@ from torch.autograd import Function
 from . import ops
 from .smoothagg import CauchyAgg, GaussianAgg, GaussianAgg_wovr, SoftAgg  # noqa: F401
 from .smoothrast import ArctanRast, GaussianRast, GaussianRast_wovr, SoftRast
-from .structures import BlendParams, FaceTexels, UVTexels, VertexTexels
+from .structures import AtlasTexels, BlendParams, FaceTexels, UVTexels, VertexTexels
 
 
 def _background_tuple(blend_params):
@@ -145,9 +145,9 @@ def smooth_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, zne
 
     ``colors`` (N,H,W,K,3); ``fragments`` with ``pix_to_face`` / ``zbuf`` / ``dists`` (N,H,W,K);
     ``znear`` / ``zfar`` python floats or tensors broadcastable to (N,1,1,1)."""
-    if isinstance(colors, (VertexTexels, UVTexels)):
-        # TexturesVertex / TexturesUV: interpolate the vertex colours with the texture-only mode of the Phong kernel; the fused
-        # pairs read colours of valid entries only, so the padded ones need not be written
+    if isinstance(colors, (VertexTexels, UVTexels, AtlasTexels)):
+        # TexturesVertex / TexturesUV / TexturesAtlas: sample the texels with the texture-only mode of the Phong kernel; the
+        # fused pairs read colours of valid entries only, so the padded ones need not be written
         from .shading import sample_lazy_textures
         colors = sample_lazy_textures(colors, fragments, sparse=_fused_pair(smoothrast, smoothagg))
     face = isinstance(colors, FaceTexels)
@@ -213,7 +213,7 @@ class SimpleShader(nn.Module):
     def forward(self, fragments, meshes, **kwargs) -> torch.Tensor:
         blend_params = kwargs.get("blend_params", self.blend_params)
         texels = meshes.sample_textures(fragments)
-        if isinstance(texels, (FaceTexels, VertexTexels, UVTexels)):
+        if isinstance(texels, (FaceTexels, VertexTexels, UVTexels, AtlasTexels)):
             from .shading import sample_lazy_textures
             texels = sample_lazy_textures(texels, fragments)
         covered = fragments.pix_to_face[..., 0] >= 0

@@ -26,7 +26,7 @@ from torch.autograd import Function
 
 from . import _cabi
 from ._cabi import PHONG_SPARSE, PHONG_STRIDE, PHONG_UNLIT, PertPhong, check, ptr, require_cuda, stream_ptr
-from .structures import FaceTexels, UVTexels, VertexTexels
+from .structures import AtlasTexels, FaceTexels, UVTexels, VertexTexels
 
 
 def _f32c(t):
@@ -86,7 +86,7 @@ def _pack_lighting(lights, materials, cameras, N, device, directional):
 
 
 def _phong_struct(pix_to_face, bary, face_verts, face_normals, texels, face_colors, lighting, flags, vert_colors=None,
-                  faces_per_mesh=0, uv=None):
+                  faces_per_mesh=0, uv=None, atlas=None):
     N, H, W, K = pix_to_face.shape
     ph = PertPhong()
     ph.P, ph.HW, ph.K = N * H * W, H * W, K
@@ -96,6 +96,10 @@ def _phong_struct(pix_to_face, bary, face_verts, face_normals, texels, face_colo
         ph.uv_map, ph.face_uvs = uv[0].data_ptr(), uv[1].data_ptr()
         ph.map_count, ph.map_h, ph.map_w = uv[0].shape[0], uv[0].shape[1], uv[0].shape[2]
         table = table if table is not None else uv[1]
+    if atlas is not None:  # (F,R,R,3): passed to the atlas entry points beside the struct
+        table = table if table is not None else atlas
+        if atlas.shape[0] != table.shape[0]:
+            raise ValueError(f"the atlas has {atlas.shape[0]} faces, the mesh {table.shape[0]}")
     ph.num_faces = table.shape[0]
     ph.flags = flags
     ph.faces_per_mesh = int(faces_per_mesh)
@@ -110,29 +114,32 @@ def _phong_struct(pix_to_face, bary, face_verts, face_normals, texels, face_colo
 
 
 def phong_forward(pix_to_face, bary, face_verts, face_normals, texels, face_colors, lighting, sparse=False,
-                  vert_colors=None, unlit=False, uv=None):
-    """Launch pert_phong_fwd.  Returns colors (N,H,W,K,3); with ``sparse`` the entries with
-    pix_to_face < 0 are left unwritten (the fused shader kernels never read them).  Exactly one texel
-    source: ``texels`` (N,H,W,K,3), ``face_colors`` (F,3) or ``vert_colors`` (F,3,3).  ``unlit``: colour =
-    texel (texture sampling only; the face tables and ``lighting`` may be None)."""
+                  vert_colors=None, unlit=False, uv=None, atlas=None):
+    """Launch pert_phong_fwd (pert_phong_atlas_fwd with ``atlas``).  Returns colors (N,H,W,K,3); with ``sparse`` the
+    entries with pix_to_face < 0 are left unwritten (the fused shader kernels never read them).  Exactly one texel
+    source: ``texels`` (N,H,W,K,3), ``face_colors`` (F,3), ``vert_colors`` (F,3,3), ``uv`` or ``atlas`` (F,R,R,3).
+    ``unlit``: colour = texel (texture sampling only; the face tables and ``lighting`` may be None)."""
     lib = _cabi.load()
-    require_cuda(pix_to_face, bary, face_verts, face_normals, texels, face_colors, lighting, vert_colors)
+    require_cuda(pix_to_face, bary, face_verts, face_normals, texels, face_colors, lighting, vert_colors, atlas)
     N, H, W, K = pix_to_face.shape
     dev = pix_to_face.device
     with torch.cuda.device(dev):
         colors = torch.empty((N, H, W, K, 3), dtype=torch.float32, device=dev)
         ph = _phong_struct(pix_to_face, bary, face_verts, face_normals, texels, face_colors, lighting,
-                           (PHONG_SPARSE if sparse else 0) | (PHONG_UNLIT if unlit else 0), vert_colors, uv=uv)
-        rc = lib.pert_phong_fwd(ph, ptr(colors), stream_ptr(dev))
-    check(rc, "pert_phong_fwd")
+                           (PHONG_SPARSE if sparse else 0) | (PHONG_UNLIT if unlit else 0), vert_colors, uv=uv, atlas=atlas)
+        if atlas is not None:
+            rc = _cabi.phong_atlas_fns()[0](ph, ptr(atlas), atlas.shape[1], ptr(colors), stream_ptr(dev))
+        else:
+            rc = lib.pert_phong_fwd(ph, ptr(colors), stream_ptr(dev))
+    check(rc, "pert_phong_atlas_fwd" if atlas is not None else "pert_phong_fwd")
     return colors
 
 
 def phong_backward(pix_to_face, bary, face_verts, face_normals, texels, face_colors, lighting, grad_colors,
                    need_texels=True, need_bary=True, need_verts=True, need_normals=True, sparse=False, vert_colors=None,
-                   unlit=False, faces_per_mesh=0, need_lighting=False, uv=None):
-    """Launch pert_phong_bwd.  Returns (grad_texels | grad_face_colors, grad_bary, grad_face_verts,
-    grad_face_normals), ``None`` where not requested.  Every entry of the dense outputs is defined (they
+                   unlit=False, faces_per_mesh=0, need_lighting=False, uv=None, atlas=None):
+    """Launch pert_phong_bwd (pert_phong_atlas_bwd with ``atlas``).  Returns (grad_texels | grad_face_colors |
+    grad_atlas, grad_bary, grad_face_verts, grad_face_normals), ``None`` where not requested.  Every entry of the dense outputs is defined (they
     flow on to the caller's own tensors): with ``sparse`` the kernel skips the padded entries, whose
     gradients are the zeros the buffers are created with."""
     lib = _cabi.load()
@@ -144,7 +151,7 @@ def phong_backward(pix_to_face, bary, face_verts, face_normals, texels, face_col
         alloc = torch.zeros if sparse else torch.empty
         if need_texels:
             table = face_colors if face_colors is not None else (vert_colors if vert_colors is not None else
-                                                                    (uv[0] if uv is not None else None))
+                                                                    (uv[0] if uv is not None else atlas))
             g_tex = torch.zeros_like(table) if table is not None else alloc((N, H, W, K, 3), dtype=torch.float32, device=dev)
         else:
             g_tex = None
@@ -153,9 +160,14 @@ def phong_backward(pix_to_face, bary, face_verts, face_normals, texels, face_col
         g_fn = torch.zeros_like(face_normals) if (need_normals and not unlit) else None
         g_light = torch.zeros_like(lighting) if (need_lighting and not unlit) else None
         ph = _phong_struct(pix_to_face, bary, face_verts, face_normals, texels, face_colors, lighting,
-                           (PHONG_SPARSE if sparse else 0) | (PHONG_UNLIT if unlit else 0), vert_colors, faces_per_mesh, uv=uv)
-        rc = lib.pert_phong_bwd(ph, ptr(grad_colors), ptr(g_tex), ptr(g_bary), ptr(g_fv), ptr(g_fn), ptr(g_light), stream_ptr(dev))
-    check(rc, "pert_phong_bwd")
+                           (PHONG_SPARSE if sparse else 0) | (PHONG_UNLIT if unlit else 0), vert_colors, faces_per_mesh, uv=uv,
+                           atlas=atlas)
+        if atlas is not None:
+            rc = _cabi.phong_atlas_fns()[1](ph, ptr(atlas), atlas.shape[1], ptr(grad_colors), ptr(g_tex), ptr(g_bary), ptr(g_fv),
+                                            ptr(g_fn), ptr(g_light), stream_ptr(dev))
+        else:
+            rc = lib.pert_phong_bwd(ph, ptr(grad_colors), ptr(g_tex), ptr(g_bary), ptr(g_fv), ptr(g_fn), ptr(g_light), stream_ptr(dev))
+    check(rc, "pert_phong_atlas_bwd" if atlas is not None else "pert_phong_bwd")
     if need_lighting:
         return g_tex, g_bary, g_fv, g_fn, g_light
     return g_tex, g_bary, g_fv, g_fn
@@ -163,7 +175,7 @@ def phong_backward(pix_to_face, bary, face_verts, face_normals, texels, face_col
 
 class _PhongShade(Function):
     """colors = phong(face_verts, face_normals, texel source, bary); constants: pix_to_face, lighting.
-    ``tex_mode``: "texels" (N,H,W,K,3), "face" (F,3) or "vert" (F,3,3)."""
+    ``tex_mode``: "texels" (N,H,W,K,3), "face" (F,3), "vert" (F,3,3), "uv" (the map) or "atlas" (F,R,R,3)."""
 
     @staticmethod
     def forward(ctx, face_verts, face_normals, texels, bary, pix_to_face, lighting, tex_mode, sparse, unlit, faces_per_mesh=0,
@@ -174,7 +186,7 @@ class _PhongShade(Function):
         p2f = pix_to_face.contiguous()
         src = dict(texels=tx if tex_mode == "texels" else None, face_colors=tx if tex_mode == "face" else None,
                    vert_colors=tx if tex_mode == "vert" else None,
-                   uv=(tx, _f32c(face_uvs.detach())) if tex_mode == "uv" else None)
+                   uv=(tx, _f32c(face_uvs.detach())) if tex_mode == "uv" else None, atlas=tx if tex_mode == "atlas" else None)
         ctx.uv_faces = src["uv"][1] if tex_mode == "uv" else None
         lighting = None if lighting is None else _f32c(lighting.detach())
         colors = phong_forward(p2f, bc, fv, fn, lighting=lighting, sparse=sparse, unlit=unlit, **src)
@@ -191,7 +203,8 @@ class _PhongShade(Function):
             fv, fn, tx, bc, p2f, lighting = ctx.saved_tensors
         need = ctx.needs_input_grad
         src = dict(texels=tx if ctx.tex_mode == "texels" else None, face_colors=tx if ctx.tex_mode == "face" else None,
-                   vert_colors=tx if ctx.tex_mode == "vert" else None, uv=(tx, ctx.uv_faces) if ctx.tex_mode == "uv" else None)
+                   vert_colors=tx if ctx.tex_mode == "vert" else None, uv=(tx, ctx.uv_faces) if ctx.tex_mode == "uv" else None,
+                   atlas=tx if ctx.tex_mode == "atlas" else None)
         out = phong_backward(
             p2f, bc, fv, fn, lighting=lighting, grad_colors=grad_colors, need_texels=need[2], need_bary=need[3],
             need_verts=need[0], need_normals=need[1], sparse=ctx.sparse, unlit=ctx.unlit,
@@ -209,13 +222,16 @@ def _texel_source(texels):
         return texels.face_vert_colors(), "vert"
     if isinstance(texels, UVTexels):
         return texels.maps, "uv"
+    if isinstance(texels, AtlasTexels):
+        return texels.atlas, "atlas"
     return texels, "texels"
 
 
 def sample_lazy_textures(texels, fragments, sparse: bool = False) -> torch.Tensor:
-    """Materialise lazy texels (:class:`FaceTexels`, :class:`VertexTexels`) as the (N,H,W,K,3) tensor
-    ``Meshes.sample_textures`` returns (random_rasterizer.py:101,170), with the texture-only mode of the Phong
-    kernel (PERT_PHONG_UNLIT); gradients flow to the colour table and, for vertex colours, to bary_coords."""
+    """Materialise lazy texels (:class:`FaceTexels`, :class:`VertexTexels`, :class:`UVTexels`, :class:`AtlasTexels`) as
+    the (N,H,W,K,3) tensor ``Meshes.sample_textures`` returns (random_rasterizer.py:101,170), with the texture-only mode
+    of the Phong kernel (PERT_PHONG_UNLIT); gradients flow to the colour table, map or atlas and, for vertex colours and
+    UV maps, to bary_coords (an atlas texel is piecewise constant in them)."""
     tex, mode = _texel_source(texels)
     if mode == "texels":
         return tex
@@ -224,8 +240,8 @@ def sample_lazy_textures(texels, fragments, sparse: bool = False) -> torch.Tenso
         pix_to_face = pix_to_face.to(torch.int64)
     bary = fragments.bary_coords
     if bary is None:
-        if mode in ("vert", "uv"):
-            raise ValueError("vertex colours / UV maps need fragments.bary_coords (N,H,W,K,3)")
+        if mode in ("vert", "uv", "atlas"):
+            raise ValueError("vertex colours / UV maps / atlases need fragments.bary_coords (N,H,W,K,3)")
         bary = torch.zeros(pix_to_face.shape + (3,), dtype=torch.float32, device=pix_to_face.device)
     return _PhongShade.apply(None, None, tex, bary, pix_to_face, None, mode, bool(sparse), True, 0,
                              texels.face_uvs() if mode == "uv" else None)
@@ -234,9 +250,10 @@ def sample_lazy_textures(texels, fragments, sparse: bool = False) -> torch.Tenso
 def phong_shading(meshes, fragments, lights, cameras, materials, texels, sparse: bool = False) -> torch.Tensor:
     """pytorch3d.renderer.mesh.shading.phong_shading, same arguments (random_rasterizer.py:103-110).
 
-    ``texels`` (N,H,W,K,3), or lazy :class:`FaceTexels` / :class:`VertexTexels` (per-face colours gathered
-    through pix_to_face, vertex colours interpolated with bary_coords, both inside the kernel: the texel
-    tensor of ``sample_textures`` is never materialised).  Returns colors (N,H,W,K,3)."""
+    ``texels`` (N,H,W,K,3), or lazy :class:`FaceTexels` / :class:`VertexTexels` / :class:`UVTexels` /
+    :class:`AtlasTexels` (per-face colours gathered through pix_to_face, vertex colours interpolated with bary_coords,
+    UV maps sampled, atlas cells looked up, all inside the kernel: the texel tensor of ``sample_textures`` is never
+    materialised).  Returns colors (N,H,W,K,3)."""
     pix_to_face = fragments.pix_to_face
     if fragments.bary_coords is None:
         raise ValueError("phong_shading needs fragments.bary_coords (N,H,W,K,3)")

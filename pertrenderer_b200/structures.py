@@ -131,8 +131,15 @@ class AtlasTexels:
     atlas texel at its first two barycentric coordinates, with the cell reflected when the point lies above the grid's
     diagonal.  Restates ``TexturesAtlas.sample_textures`` of pytorch3d 0.4.0 (renderer/mesh/textures.py; the package is
     not installable here: parity unpinned, anchored on the known answers of tests/test_cabi_cpu.py).  A nearest lookup:
-    gradients reach the atlas (index scatter, by autograd), not the barycentric coordinates.  One deliberate difference:
-    a barycentric coordinate of exactly 1 indexes cell R in pytorch3d (out of range); here it is clamped to R - 1."""
+    gradients reach the atlas (index scatter, by autograd), not the barycentric coordinates.  Deliberate differences:
+    a barycentric coordinate of exactly 1 indexes cell R in pytorch3d (out of range); here it is clamped to R - 1.
+    The rasteriser's barycentric coordinates are unclipped (outside [0, 1] in the blur band, far outside for sliver
+    faces), where pytorch3d's rule wraps negative cells or overflows the grid: here NaN counts as 0, w R is clamped to
+    [-1, R] before the truncation and the (possibly reflected) cell to the grid, so every cell is in range.  Wherever
+    pytorch3d's rule picks an in-range cell without wrapping, this one picks the same cell.
+
+    On a CUDA device the Phong kernels look the cells up in place (``pert_phong_atlas_fwd/bwd``, the same rule op for
+    op); :meth:`materialize` builds the (N,H,W,K,3) tensor with torch ops."""
 
     def __init__(self, atlas: torch.Tensor):
         if atlas.dim() != 4 or atlas.shape[1] != atlas.shape[2] or atlas.shape[3] != 3:
@@ -143,11 +150,13 @@ class AtlasTexels:
         R = self.atlas.shape[1]
         mask = pix_to_face >= 0
         w01 = torch.where(mask[..., None], bary[..., :2], torch.zeros_like(bary[..., :2]))
-        w_xy = (w01 * R).to(torch.int64).clamp(max=R - 1)
-        below = (w01.sum(dim=-1) * R - w_xy.to(w01.dtype).sum(dim=-1)) <= 1.0
+        w01 = torch.nan_to_num(w01, nan=0.0)
+        w_xy = (w01 * R).clamp(-1, R).to(torch.int64).clamp(max=R - 1)
+        w0, w1 = w01.unbind(-1)
         w_x, w_y = w_xy.unbind(-1)
-        w_x = torch.where(below, w_x, R - 1 - w_x)
-        w_y = torch.where(below, w_y, R - 1 - w_y)
+        below = ((w0 + w1) * R - (w_x + w_y).to(w01.dtype)) <= 1.0  # each op rounded once, as in the kernel
+        w_x = torch.where(below, w_x, R - 1 - w_x).clamp(0, R - 1)
+        w_y = torch.where(below, w_y, R - 1 - w_y).clamp(0, R - 1)
         return self.atlas[pix_to_face.clamp(min=0), w_y, w_x] * mask[..., None].to(self.atlas.dtype)
 
 
@@ -238,7 +247,7 @@ class TriMeshes:
     it, vertices (N,V,3) (``extend`` / ``update_padded`` as in eval.py:343,281-283).  The packed representation
     (``verts_packed`` (N*V,3), ``faces_packed`` (N*F,3)) is what ``pix_to_face`` indexes.  Textures: one colour per
     face (lazy :class:`FaceTexels`), one colour per vertex (lazy :class:`VertexTexels`), a UV map (lazy
-    :class:`UVTexels`) or a preset texel tensor.
+    :class:`UVTexels`), a per-face atlas (:class:`AtlasTexels`, lazy on a CUDA device) or a preset texel tensor.
     ``verts_normals_packed`` follows pytorch3d's area-weighted vertex normals (cross products of the face edges
     summed onto the corners, then normalised with eps 1e-6)."""
 
@@ -282,10 +291,13 @@ class TriMeshes:
             return self.texels
         n = len(self)
         if self.atlas is not None:
-            # a nearest-texel lookup: materialised with torch indexing (its autograd scatters the gradient into the atlas)
+            # a nearest-texel lookup: lazy on a CUDA device (the Phong kernels look the cells up in place and scatter the
+            # gradient into the atlas), materialised with torch indexing elsewhere
             if fragments.bary_coords is None:
                 raise ValueError("atlas textures need fragments.bary_coords (N,H,W,K,3)")
             atlas = self.atlas if n == 1 else self.atlas.repeat(n, 1, 1, 1)
+            if atlas.is_cuda:
+                return AtlasTexels(atlas)
             return AtlasTexels(atlas).materialize(fragments.pix_to_face, fragments.bary_coords)
         if self.uv is not None:
             maps, verts_uvs, faces_uvs = self.uv
