@@ -378,6 +378,9 @@ int pert_phong_atlas_bwd(const pert_phong* ph, const float* atlas, int32_t atlas
  * (N,H,W,K,3), dists float (N,H,W,K) signed squared NDC distance to the face (negative inside).
  */
 #define PERT_RAST_CULL_BACKFACES 1u
+/* the rs->bin_* lists are the bounded layout of pert_rasterize_bin_bounded (num_bins + N bins; the last N are the
+ * images' wide lists).  Requires rs->bin_faces (else PERT_E_NULL) */
+#define PERT_RAST_BIN_WIDE 2u
 
 typedef struct pert_raster {
     int64_t N;
@@ -393,9 +396,10 @@ typedef struct pert_raster {
                                   order.  Forward, K <= 64 only */
     /* optional coarse bins (forward, K <= 64): one list of candidate faces per 32x4 pixel tile, built by two
      * pert_rasterize_bin calls; every tile then walks its own list instead of all faces of its mesh.  For meshes of
-     * thousands of faces.  NULL: off */
-    const int32_t* bin_count;  /* (N * tiles) faces per tile, tiles = ceil(W/32) * ceil(H/4) */
-    const int64_t* bin_offset; /* (N * tiles) start of every tile's list in bin_faces: exclusive prefix sum of bin_count */
+     * thousands of faces.  NULL: off.  With PERT_RAST_BIN_WIDE, the bounded layout of pert_rasterize_bin_bounded:
+     * N * tiles + N bins, every tile walking its own list and then its image's wide list */
+    const int32_t* bin_count;  /* (N * tiles [+ N]) faces per tile, tiles = ceil(W/32) * ceil(H/4) */
+    const int64_t* bin_offset; /* (N * tiles [+ N]) start of every list in bin_faces: exclusive prefix sum of bin_count */
     const int64_t* bin_faces;  /* (sum of bin_count) packed face indices */
 } pert_raster;
 
@@ -410,6 +414,19 @@ int64_t pert_rasterize_num_bins(const pert_raster* rs);
  */
 int pert_rasterize_bin(const pert_raster* rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
                        int64_t* bin_faces, void* stream);
+/*
+ * Coarse binning whose total length is known on the host, so that nothing is read back between the two calls (a CUDA
+ * graph can capture them).  A face whose grown bounding box overlaps at most C tiles (C, a compile-time constant: 8)
+ * is listed in those tiles, as by pert_rasterize_bin; a face overlapping more (a box reaching +-inf or NaN covers the
+ * whole axis) is listed once in the WIDE list of its image, which every tile of that image walks too.  The arrays hold
+ * pert_rasterize_num_bins(rs) + N entries: the tile bins, then the wide lists of images 0..N-1.  The two calls and
+ * their rules are those of pert_rasterize_bin; bin_faces needs at most pert_rasterize_bin_capacity(rs) entries.  The
+ * forward reads the result with rs->flags |= PERT_RAST_BIN_WIDE.
+ */
+int pert_rasterize_bin_bounded(const pert_raster* rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
+                               int64_t* bin_faces, void* stream);
+/* upper bound of the total length of pert_rasterize_bin_bounded's lists: C * num_faces (0 for a NULL or empty problem) */
+int64_t pert_rasterize_bin_capacity(const pert_raster* rs);
 
 int pert_rasterize_fwd(const pert_raster* rs, int64_t* pix_to_face, float* zbuf, float* bary, float* dists, void* stream);
 /*

@@ -33,10 +33,12 @@ EXPORTS = [
     "pert_version", "pert_shade_fused_flags", "pert_strerror", "pert_last_cuda_error", "pert_num_tiles", "pert_winner_bytes", "pert_blob_bytes",
     "pert_shade_fwd", "pert_shade_render", "pert_shade_render_phase", "pert_shade_bwd", "pert_soft_shade_fwd", "pert_soft_shade_bwd", "pert_rast_fwd", "pert_rast_bwd", "pert_argmax_fwd",
     "pert_argmax_bwd", "pert_noise_fill", "pert_seed_advance", "pert_phong_fwd", "pert_phong_bwd", "pert_phong_atlas_fwd", "pert_phong_atlas_bwd",
-    "pert_rasterize_fwd", "pert_rasterize_bwd", "pert_rasterize_num_bins", "pert_rasterize_bin",
+    "pert_rasterize_fwd", "pert_rasterize_bwd", "pert_rasterize_num_bins", "pert_rasterize_bin", "pert_rasterize_bin_bounded",
+    "pert_rasterize_bin_capacity",
 ]
 
 RAST_CULL_BACKFACES = 1  # PERT_RAST_CULL_BACKFACES
+RAST_BIN_WIDE = 2  # PERT_RAST_BIN_WIDE
 
 PHONG_STRIDE = 20  # PERT_PHONG_STRIDE
 PHONG_SPARSE = 1  # PERT_PHONG_SPARSE
@@ -244,6 +246,27 @@ def phong_atlas_fns():
         bwd.argtypes = [C.POINTER(PertPhong), C.c_void_p, C.c_int32] + [C.c_void_p] * 7
         _phong_atlas = (lib, fwd, bwd)
     return _phong_atlas[1], _phong_atlas[2]
+
+
+_raster_bins = None  # (library, its bound pert_rasterize_bin_bounded, pert_rasterize_bin_capacity)
+
+
+def raster_bin_fns():
+    """(``pert_rasterize_bin_bounded``, ``pert_rasterize_bin_capacity``) of the loaded library, bound on first use rather
+    than in :func:`load`, so that a library built before them keeps serving every other call.  Such a library would
+    ignore RAST_BIN_WIDE and drop the faces of the wide lists, so this raises PertLibraryError asking for a rebuild."""
+    global _raster_bins
+    lib = load()
+    if _raster_bins is None or _raster_bins[0] is not lib:
+        fill, cap = getattr(lib, "pert_rasterize_bin_bounded", None), getattr(lib, "pert_rasterize_bin_capacity", None)
+        if fill is None or cap is None:
+            raise PertLibraryError(f"{LIB_PATH} predates the bounded coarse bins (pert_rasterize_bin_bounded / "
+                                   "pert_rasterize_bin_capacity): rebuild it with `python -m pertrenderer_b200.build --force`")
+        fill.restype, cap.restype = C.c_int, C.c_int64
+        fill.argtypes = [C.POINTER(PertRaster)] + [C.c_void_p] * 5
+        cap.argtypes = [C.POINTER(PertRaster)]
+        _raster_bins = (lib, fill, cap)
+    return _raster_bins[1], _raster_bins[2]
 
 
 def check(rc: int, what: str):

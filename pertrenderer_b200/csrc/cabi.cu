@@ -622,6 +622,7 @@ extern "C" int pert_rasterize_fwd(const pert_raster* rs, int64_t* pix_to_face, f
     if (int rc = check_raster(rs)) return rc;
     if (!pix_to_face || !zbuf || !bary || !dists) return PERT_E_NULL;
     if (rs->bin_faces && (!rs->bin_count || !rs->bin_offset)) return PERT_E_NULL;
+    if ((rs->flags & PERT_RAST_BIN_WIDE) && !rs->bin_faces) return PERT_E_NULL;
     if (((uintptr_t)rs->bin_count & 3) || ((uintptr_t)rs->bin_offset & 7) || ((uintptr_t)rs->bin_faces & 7)) return PERT_E_ALIGN;
     if (((uintptr_t)pix_to_face & 7) || ((uintptr_t)zbuf & 3) || ((uintptr_t)bary & 3) || ((uintptr_t)dists & 3)) return PERT_E_ALIGN;
     return cuda_rc(launch_rasterize_fwd(*rs, pix_to_face, zbuf, bary, dists, (cudaStream_t)stream));
@@ -642,11 +643,28 @@ extern "C" int64_t pert_rasterize_num_bins(const pert_raster* rs) {
     return rs->N * (int64_t)((rs->W + 31) / 32) * (int64_t)((rs->H + 3) / 4);  // TW x TH tiles of csrc/raster.cu
 }
 
-extern "C" int pert_rasterize_bin(const pert_raster* rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
-                                  int64_t* bin_faces, void* stream) {
+static int check_bin(const pert_raster* rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
+                     int64_t* bin_faces) {
     if (int rc = check_raster(rs)) return rc;
     if (bin_faces ? (!bin_offset || !bin_cursor) : !bin_count) return PERT_E_NULL;
     if (((uintptr_t)bin_count & 3) || ((uintptr_t)bin_offset & 7) || ((uintptr_t)bin_cursor & 3) || ((uintptr_t)bin_faces & 7))
         return PERT_E_ALIGN;
+    return PERT_OK;
+}
+
+extern "C" int pert_rasterize_bin(const pert_raster* rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
+                                  int64_t* bin_faces, void* stream) {
+    if (int rc = check_bin(rs, bin_count, bin_offset, bin_cursor, bin_faces)) return rc;
     return cuda_rc(launch_rasterize_bin(*rs, bin_count, bin_offset, bin_cursor, bin_faces, (cudaStream_t)stream));
+}
+
+extern "C" int pert_rasterize_bin_bounded(const pert_raster* rs, int32_t* bin_count, const int64_t* bin_offset,
+                                          int32_t* bin_cursor, int64_t* bin_faces, void* stream) {
+    if (int rc = check_bin(rs, bin_count, bin_offset, bin_cursor, bin_faces)) return rc;
+    return cuda_rc(launch_rasterize_bin_bounded(*rs, bin_count, bin_offset, bin_cursor, bin_faces, (cudaStream_t)stream));
+}
+
+extern "C" int64_t pert_rasterize_bin_capacity(const pert_raster* rs) {
+    if (!rs || rs->num_faces <= 0) return 0;
+    return (int64_t)RASTER_BIN_CAP * rs->num_faces;
 }

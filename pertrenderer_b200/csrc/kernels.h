@@ -69,6 +69,14 @@ int launch_phong_bwd(const pert_phong& ph, const float* grad_colors, float* grad
                      float* grad_fn, cudaStream_t st, const float* atlas = nullptr, int atlas_r = 0);
 int launch_phong_light_bwd(const pert_phong& ph, const float* grad_colors, float* grad_lighting, cudaStream_t st,
                            const float* atlas = nullptr, int atlas_r = 0);
+// most tile entries of one face in the bounded bins of pert_rasterize_bin_bounded (csrc/raster.cu); chosen by
+// measurement among 4, 8 and 16 (profiles/r10_raster_bins.txt; the others built with -DPERT_RASTER_BIN_CAP=C)
+#ifndef PERT_RASTER_BIN_CAP
+#define PERT_RASTER_BIN_CAP 8
+#endif
+constexpr int RASTER_BIN_CAP = PERT_RASTER_BIN_CAP;
+int launch_rasterize_bin_bounded(const pert_raster& rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
+                                 int64_t* bin_faces, cudaStream_t st);
 int launch_rasterize_bin(const pert_raster& rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
                          int64_t* bin_faces, cudaStream_t st);
 int launch_rasterize_fwd(const pert_raster& rs, int64_t* pix_to_face, float* zbuf, float* bary, float* dists, cudaStream_t st);

@@ -13,6 +13,12 @@
 //             output rows for larger K (stable insertion: ascending depth, ties in face order); bary / dists of the
 //             kept faces are recomputed at the end and the padding of each row is written by the warp as coalesced
 //             stores.
+//   bins      for large meshes (K <= 64), candidate lists per tile built by one thread per face in two passes (count,
+//             then fill) around the caller's prefix sum.  pert_rasterize_bin lists a face in every tile its box
+//             overlaps, so the total length is only known on the device.  pert_rasterize_bin_bounded lists a face in
+//             at most RASTER_BIN_CAP tiles and puts a face that overlaps more into one wide list per image, which every
+//             tile of the image walks after its own: the total is at most RASTER_BIN_CAP * num_faces, the caller sizes
+//             the lists from shapes alone, and the render needs no host synchronisation (CUDA-graph capturable).
 //   backward  a streaming pass over the (P,K) entries, warp-autonomous chunks with compact valid lists (the machinery
 //             of the Phong kernels): every valid entry recomputes its barycentric / distance arithmetic and scatters
 //             d(zbuf, bary, dists)/d(face_verts) with atomics.
@@ -215,7 +221,10 @@ __global__ void __launch_bounds__(RT) rasterize_fwd_rows_kernel(const pert_raste
 // the keys is the depth order with ties in face order; local memory is interleaved per thread, so the accesses of a warp
 // are coalesced (the per-pixel output rows of the generic kernel are K*4 bytes apart: every shift of its sorted
 // insertion was its own sector, 2.2 ms at config 2).
-template <int KMAX>
+//
+// WIDE: the bins are the bounded layout of pert_rasterize_bin_bounded: the tile walks its own list, then its image's wide
+// list (bin num_bins + n), as one run of positions [f_lo, f_hi) whose tail is remapped into the wide list.
+template <int KMAX, bool WIDE>
 __global__ void __launch_bounds__(RT) rasterize_fwd_keys_kernel(const pert_raster rs, int64_t* __restrict__ pix_to_face,
                                                                 float* __restrict__ zbuf, float* __restrict__ bary,
                                                                 float* __restrict__ dists) {
@@ -245,10 +254,17 @@ __global__ void __launch_bounds__(RT) rasterize_fwd_keys_kernel(const pert_raste
     // does not depend on the order: keys are unique.
     const int64_t* const fmap = rs.bin_faces ? rs.bin_faces : rs.face_order;
     int64_t f_lo = f_begin, f_hi = f_end;
+    int64_t f_split = 0, f_jump = 0;  // WIDE: positions >= f_split read bin_faces[position + f_jump]
     if (rs.bin_faces) {
         const int64_t bin = ((int64_t)n * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
         f_lo = __ldg(rs.bin_offset + bin);
         f_hi = f_lo + __ldg(rs.bin_count + bin);
+        if (WIDE) {
+            const int64_t wide = (int64_t)gridDim.z * gridDim.y * gridDim.x + n;
+            f_split = f_hi;
+            f_jump = __ldg(rs.bin_offset + wide) - f_split;
+            f_hi += __ldg(rs.bin_count + wide);
+        }
     }
 
 #pragma unroll 1
@@ -259,7 +275,7 @@ __global__ void __launch_bounds__(RT) rasterize_fwd_keys_kernel(const pert_raste
         float v[9];
         float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
         if (fpos < f_hi) {
-            if (fmap) f = __ldg(fmap + fpos);
+            if (fmap) f = __ldg(fmap + (WIDE && fpos >= f_split ? fpos + f_jump : fpos));
 #pragma unroll
             for (int i = 0; i < 9; ++i) v[i] = __ldg(rs.face_verts + f * 9 + i);
             bb = make_float4(fminf(fminf(v[0], v[3]), v[6]) - r, fmaxf(fmaxf(v[0], v[3]), v[6]) + r,
@@ -382,24 +398,18 @@ __global__ void __launch_bounds__(RT) rasterize_fwd_keys_kernel(const pert_raste
 // ---------------------------------------------------------------------------------------------------------
 // coarse binning for large meshes: which faces can touch which 32x4 pixel tile
 // ---------------------------------------------------------------------------------------------------------
-// One thread per face: the tiles overlapped by its bounding box grown by sqrt(blur_radius) (conservative by a pixel).
-// FILL = false counts (atomics into bin_count, zeroed by the caller); FILL = true appends the face to every such
-// tile's list at bin_offset[bin] + cursor++ (bin_cursor zeroed by the caller).  The order inside a list is arbitrary;
-// the packed-key K-buffer makes the fragments independent of it.
-template <bool FILL>
-__global__ void __launch_bounds__(256) rasterize_bin_kernel(const pert_raster rs, int32_t* __restrict__ bin_count,
-                                                            const int64_t* __restrict__ bin_offset, int32_t* __restrict__ bin_cursor,
-                                                            int64_t* __restrict__ bin_faces) {
-    const int64_t f = (int64_t)blockIdx.x * 256 + threadIdx.x;
-    if (f >= rs.num_faces) return;
+// The tiles of face f (one thread per face): its image n and the tile rectangle [tx0, tx1] x [ty0, ty1] overlapped by
+// its bounding box grown by sqrt(blur_radius) (conservative by a pixel).  False for a face outside the ranges of
+// face_start, culled (behind the camera, zero area, back face when culling) or whose box misses the image.
+__device__ __forceinline__ bool face_tiles(const pert_raster& rs, int64_t f, int& n, int& tx0, int& tx1, int& ty0, int& ty1) {
     // image of this face: last n with face_start[n] <= f
     int lo = 0, hi = (int)rs.N;
     while (hi - lo > 1) {
         const int mid = (lo + hi) >> 1;
         if (__ldg(rs.face_start + mid) <= f) lo = mid; else hi = mid;
     }
-    const int n = lo;
-    if (f < __ldg(rs.face_start + n) || f >= __ldg(rs.face_start + n + 1)) return;
+    n = lo;
+    if (f < __ldg(rs.face_start + n) || f >= __ldg(rs.face_start + n + 1)) return false;
     float v[9];
 #pragma unroll
     for (int i = 0; i < 9; ++i) v[i] = __ldg(rs.face_verts + f * 9 + i);
@@ -408,7 +418,7 @@ __global__ void __launch_bounds__(256) rasterize_bin_kernel(const pert_raster rs
     const float ymin = fminf(fminf(v[1], v[4]), v[7]) - r, ymax = fmaxf(fmaxf(v[1], v[4]), v[7]) + r;
     const float zmax = fmaxf(fmaxf(v[2], v[5]), v[8]);
     const float area = edge(P2{v[0], v[1]}, P2{v[3], v[4]}, P2{v[6], v[7]});
-    if (zmax < 0.0f || (area <= kEps && area >= -kEps) || ((rs.flags & PERT_RAST_CULL_BACKFACES) && area < 0.0f)) return;
+    if (zmax < 0.0f || (area <= kEps && area >= -kEps) || ((rs.flags & PERT_RAST_CULL_BACKFACES) && area < 0.0f)) return false;
     const int H = rs.H, W = rs.W;
     // pixel index i (from the -X / -Y side) whose centre is x: x = -range + (2 i + 1) range / S.  The float indices
     // are clamped to [-2, S+1] before the conversion: a box reaching |x| ~ 2^32 / S or inf would otherwise saturate
@@ -420,18 +430,61 @@ __global__ void __launch_bounds__(256) rasterize_bin_kernel(const pert_raster rs
     const float fy0 = floorf(((ymin + ry) * (float)H / ry - 1.0f) * 0.5f), fy1 = ceilf(((ymax + ry) * (float)H / ry - 1.0f) * 0.5f);
     const int ix0 = (int)fminf(fmaxf(fx0, -2.0f), (float)(W + 1)) - 1, ix1 = (int)fmaxf(fminf(fx1, (float)(W + 1)), -2.0f) + 1;
     const int iy0 = (int)fminf(fmaxf(fy0, -2.0f), (float)(H + 1)) - 1, iy1 = (int)fmaxf(fminf(fy1, (float)(H + 1)), -2.0f) + 1;
-    if (ix1 < 0 || iy1 < 0 || ix0 > W - 1 || iy0 > H - 1) return;
+    if (ix1 < 0 || iy1 < 0 || ix0 > W - 1 || iy0 > H - 1) return false;
     // image column = W-1-i, row = H-1-i
     const int cx0 = W - 1 - min(ix1, W - 1), cx1 = W - 1 - max(ix0, 0), cy0 = H - 1 - min(iy1, H - 1), cy1 = H - 1 - max(iy0, 0);
-    const int tiles_x = (W + TW - 1) / TW, tiles_y = (H + TH - 1) / TH;
-    for (int ty = cy0 / TH; ty <= cy1 / TH; ++ty)
-        for (int tx = cx0 / TW; tx <= cx1 / TW; ++tx) {
+    tx0 = cx0 / TW, tx1 = cx1 / TW, ty0 = cy0 / TH, ty1 = cy1 / TH;
+    return true;
+}
+
+// Every tile of face_tiles gets the face.  FILL = false counts (atomics into bin_count, zeroed by the caller);
+// FILL = true appends the face to every such tile's list at bin_offset[bin] + cursor++ (bin_cursor zeroed by the
+// caller).  The order inside a list is arbitrary; the packed-key K-buffer makes the fragments independent of it.
+template <bool FILL>
+__global__ void __launch_bounds__(256) rasterize_bin_kernel(const pert_raster rs, int32_t* __restrict__ bin_count,
+                                                            const int64_t* __restrict__ bin_offset, int32_t* __restrict__ bin_cursor,
+                                                            int64_t* __restrict__ bin_faces) {
+    const int64_t f = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (f >= rs.num_faces) return;
+    int n, tx0, tx1, ty0, ty1;
+    if (!face_tiles(rs, f, n, tx0, tx1, ty0, ty1)) return;
+    const int tiles_x = (rs.W + TW - 1) / TW, tiles_y = (rs.H + TH - 1) / TH;
+    for (int ty = ty0; ty <= ty1; ++ty)
+        for (int tx = tx0; tx <= tx1; ++tx) {
             const int64_t bin = ((int64_t)n * tiles_y + ty) * tiles_x + tx;
             if (FILL)
                 bin_faces[__ldg(bin_offset + bin) + atomicAdd(bin_cursor + bin, 1)] = f;
             else
                 atomicAdd(bin_count + bin, 1);
         }
+}
+
+// Bounded layout (pert_rasterize_bin_bounded): a face with at most RASTER_BIN_CAP tiles goes into those tiles' lists
+// (bins [0, num_bins)), as above; a face with more goes once into its image's wide list, bin num_bins + n, which every
+// tile of the image walks after its own.  So no face has more than RASTER_BIN_CAP entries, and the caller sizes
+// bin_faces as RASTER_BIN_CAP * num_faces without reading the counts back.  A face whose box reaches +-inf or NaN
+// covers a whole axis, so it is wide unless the image has at most RASTER_BIN_CAP tiles along that axis.
+template <bool FILL>
+__global__ void __launch_bounds__(256) rasterize_bin_bounded_kernel(const pert_raster rs, int32_t* __restrict__ bin_count,
+                                                                    const int64_t* __restrict__ bin_offset,
+                                                                    int32_t* __restrict__ bin_cursor, int64_t* __restrict__ bin_faces) {
+    const int64_t f = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (f >= rs.num_faces) return;
+    int n, tx0, tx1, ty0, ty1;
+    if (!face_tiles(rs, f, n, tx0, tx1, ty0, ty1)) return;
+    const int tiles_x = (rs.W + TW - 1) / TW, tiles_y = (rs.H + TH - 1) / TH;
+    const auto put = [&](int64_t bin) {
+        if (FILL)
+            bin_faces[__ldg(bin_offset + bin) + atomicAdd(bin_cursor + bin, 1)] = f;
+        else
+            atomicAdd(bin_count + bin, 1);
+    };
+    if ((tx1 - tx0 + 1) * (ty1 - ty0 + 1) > RASTER_BIN_CAP) {
+        put(rs.N * tiles_y * tiles_x + n);
+        return;
+    }
+    for (int ty = ty0; ty <= ty1; ++ty)
+        for (int tx = tx0; tx <= tx1; ++tx) put(((int64_t)n * tiles_y + ty) * tiles_x + tx);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -566,13 +619,33 @@ int launch_rasterize_bin(const pert_raster& rs, int32_t* bin_count, const int64_
     return (int)cudaGetLastError();
 }
 
+int launch_rasterize_bin_bounded(const pert_raster& rs, int32_t* bin_count, const int64_t* bin_offset, int32_t* bin_cursor,
+                                 int64_t* bin_faces, cudaStream_t st) {
+    const unsigned grid = (unsigned)((rs.num_faces + 255) / 256);
+    if (bin_faces)
+        rasterize_bin_bounded_kernel<true><<<grid, 256, 0, st>>>(rs, bin_count, bin_offset, bin_cursor, bin_faces);
+    else
+        rasterize_bin_bounded_kernel<false><<<grid, 256, 0, st>>>(rs, bin_count, bin_offset, bin_cursor, bin_faces);
+    return (int)cudaGetLastError();
+}
+
+template <bool WIDE>
+static cudaError_t launch_keys(const pert_raster& rs, dim3 grid, int64_t* pix_to_face, float* zbuf, float* bary, float* dists,
+                               cudaStream_t st) {
+    const size_t smem = (size_t)rs.K * RT * sizeof(unsigned long long);  // K = 50: 50 KB
+    cudaError_t e = cudaFuncSetAttribute(rasterize_fwd_keys_kernel<64, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    rasterize_fwd_keys_kernel<64, WIDE><<<grid, RT, smem, st>>>(rs, pix_to_face, zbuf, bary, dists);
+    return cudaSuccess;
+}
+
 int launch_rasterize_fwd(const pert_raster& rs, int64_t* pix_to_face, float* zbuf, float* bary, float* dists, cudaStream_t st) {
     const dim3 grid((unsigned)((rs.W + TW - 1) / TW), (unsigned)((rs.H + TH - 1) / TH), (unsigned)rs.N);
     if (rs.K <= 64) {
-        const size_t smem = (size_t)rs.K * RT * sizeof(unsigned long long);  // K = 50: 50 KB
-        cudaError_t e = cudaFuncSetAttribute(rasterize_fwd_keys_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        const cudaError_t e = rs.bin_faces && (rs.flags & PERT_RAST_BIN_WIDE)
+                                  ? launch_keys<true>(rs, grid, pix_to_face, zbuf, bary, dists, st)
+                                  : launch_keys<false>(rs, grid, pix_to_face, zbuf, bary, dists, st);
         if (e != cudaSuccess) return (int)e;
-        rasterize_fwd_keys_kernel<64><<<grid, RT, smem, st>>>(rs, pix_to_face, zbuf, bary, dists);
     } else  // K-buffer in the pixel's own output rows
         rasterize_fwd_rows_kernel<<<grid, RT, 0, st>>>(rs, pix_to_face, zbuf, bary, dists);
     return (int)cudaGetLastError();

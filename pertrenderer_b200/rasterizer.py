@@ -52,6 +52,38 @@ def _raster_struct(face_verts, face_start, N, H, W, K, blur_radius, cull_backfac
     return rs
 
 
+def _bounded_bins_pay(rs, bin_capacity, H, W, blur_radius):
+    """Whether the bounded bins are no slower than the synchronising ones.  Every face's box is grown by sqrt(blur_radius)
+    on each side; where that margin alone spans more than C tiles, every face goes to its image's wide list and each tile
+    walks all faces of its mesh: at 8 x 256^2 and 16 x 1024^2 with eval.py's blur the bounded bins are 1.15x and 1.7x
+    slower, at 1 x 128^2 they are faster and keep the host free (profiles/r10_raster_bins.txt)."""
+    margin = 2.0 * math.sqrt(blur_radius) * min(H, W) / 2.0  # pixels: the box's least width and height
+    return (margin / 4 + 1) * (margin / 32 + 1) <= bin_capacity(rs) // rs.num_faces  # 32x4 tiles
+
+
+def _build_bins(lib, rs, N, H, W, blur_radius, dev):
+    """Coarse bins of a large mesh in rs.bin_*, two kernel passes around a prefix sum; returns the tensors that hold them.
+    Inside a CUDA-graph capture, or where _bounded_bins_pay, the bounded bins (one candidate list per 32x4 pixel tile and
+    one wide list per image, sized from the face count: nothing is read back to the host).  Elsewhere one list per tile
+    holding every face whose box overlaps it, sized from a total read back from the device: a host sync."""
+    bin_bounded, bin_capacity = _cabi.raster_bin_fns()
+    st = stream_ptr(dev)
+    bounded = torch.cuda.is_current_stream_capturing() or _bounded_bins_pay(rs, bin_capacity, H, W, blur_radius)
+    fill, name = (bin_bounded, "pert_rasterize_bin_bounded") if bounded else (lib.pert_rasterize_bin, "pert_rasterize_bin")
+    nb = int(lib.pert_rasterize_num_bins(rs)) + (N if bounded else 0)
+    count = torch.zeros((nb,), dtype=torch.int32, device=dev)
+    check(fill(rs, ptr(count), None, None, None, st), name)
+    ends = torch.cumsum(count, 0, dtype=torch.int64)
+    offset = (ends - count).contiguous()
+    lists = torch.empty((max(int(bin_capacity(rs) if bounded else ends[-1].item()), 1),), dtype=torch.int64, device=dev)
+    cursor = torch.zeros((nb,), dtype=torch.int32, device=dev)
+    check(fill(rs, ptr(count), ptr(offset), ptr(cursor), ptr(lists), st), name)
+    rs.bin_count, rs.bin_offset, rs.bin_faces = count.data_ptr(), offset.data_ptr(), lists.data_ptr()
+    if bounded:
+        rs.flags |= _cabi.RAST_BIN_WIDE
+    return [count, offset, lists]
+
+
 class _Rasterize(Function):
     @staticmethod
     def forward(ctx, face_verts, face_start, H, W, K, blur_radius, cull_backfaces):
@@ -70,18 +102,7 @@ class _Rasterize(Function):
             rs = _raster_struct(fv, fs, N, H, W, K, blur_radius, cull_backfaces)
             keep = []
             if K <= 64 and fv.shape[0] >= BIN_MIN_FACES * N:
-                # large meshes: coarse bins, one candidate list per 32x4 pixel tile (two kernel passes around a prefix
-                # sum; the total length of the lists is read back to size the buffer: the one host sync of this path)
-                nb = int(lib.pert_rasterize_num_bins(rs))
-                count = torch.zeros((nb,), dtype=torch.int32, device=dev)
-                check(lib.pert_rasterize_bin(rs, ptr(count), None, None, None, stream_ptr(dev)), "pert_rasterize_bin")
-                ends = torch.cumsum(count, 0, dtype=torch.int64)
-                offset = (ends - count).contiguous()
-                lists = torch.empty((max(int(ends[-1].item()), 1),), dtype=torch.int64, device=dev)
-                cursor = torch.zeros((nb,), dtype=torch.int32, device=dev)
-                check(lib.pert_rasterize_bin(rs, ptr(count), ptr(offset), ptr(cursor), ptr(lists), stream_ptr(dev)), "pert_rasterize_bin")
-                rs.bin_count, rs.bin_offset, rs.bin_faces = count.data_ptr(), offset.data_ptr(), lists.data_ptr()
-                keep = [count, offset, lists]
+                keep = _build_bins(lib, rs, N, H, W, blur_radius, dev)
             rc = lib.pert_rasterize_fwd(rs, ptr(p2f), ptr(zbuf), ptr(bary), ptr(dists), stream_ptr(dev))
             del keep
         check(rc, "pert_rasterize_fwd")
