@@ -243,6 +243,57 @@ int pert_shade_bwd(const pert_problem* pb, const float* grad_image, const uint16
                    void* stream);
 
 /*
+ * Texture sampled inside the fused kernels: the texel of a valid entry (p,k) is computed from bary[p,k] and a per-face
+ * table at the moment the kernels blend it, so that the (P,K,3) colour tensor of Meshes.sample_textures
+ * (random_rasterizer.py:170) and its gradient are never materialised.  The texel is the same float expression as the
+ * texture-only Phong kernel's (pert_phong_fwd / pert_phong_atlas_fwd with PERT_PHONG_UNLIT):
+ *   PERT_TEX_VERTEX  table (num_faces,3,3) colours at the face corners, texel = sum_i bary_i table[f,i]   (TexturesVertex)
+ *   PERT_TEX_UV      table (map_count,map_h,map_w,3) maps, map_count 1 or N, face_uvs (num_faces,3,2): the bilinear tap
+ *                    of pert_phong's uv_map at sum_i bary_i face_uvs[f,i]                   (TexturesUV, legacy Textures)
+ *   PERT_TEX_ATLAS   table (num_faces,R,R,3), R = atlas_size: the cell rule of pert_phong_atlas_fwd      (TexturesAtlas)
+ * with f = pix_to_face[p,k] (a packed face index below num_faces).  bary float (P,K,3) is fragments.bary_coords.
+ */
+#define PERT_TEX_VERTEX 1
+#define PERT_TEX_UV 2
+#define PERT_TEX_ATLAS 3
+
+typedef struct pert_texture {
+    int32_t kind;       /* PERT_TEX_* */
+    int32_t atlas_size; /* R (PERT_TEX_ATLAS) */
+    const float* bary;  /* (P,K,3) */
+    const float* table; /* (F,3,3) vertex colours, (M,Hm,Wm,3) maps or (F,R,R,3) atlas */
+    const float* face_uvs; /* (F,3,2) (PERT_TEX_UV) */
+    int32_t map_h, map_w, map_count; /* (PERT_TEX_UV) */
+    int64_t num_faces;
+} pert_texture;
+
+/*
+ * pert_shade_fwd / pert_shade_bwd / pert_shade_render with the colour of every entry sampled from `tex` inside the kernels.
+ * Arguments, flags and flag rules are those of the counterpart (PERT_F_CAUCHY, PERT_F_NO_VR, PERT_F_PHILOX7, explicit
+ * noise, seed_device, pixel_offset, worklist, tile blob); for the same problem and noise the image, grad_dists, grad_zbuf
+ * and grad_scalars equal the counterpart's fed with the materialised colours, bit for bit.  Nothing depends on the sample
+ * counts and nothing synchronises: the calls can be captured in a CUDA graph.  Backward outputs, each optional (NULL: not
+ * computed):
+ *   grad_table  the table's shape, ZEROED BY THE CALLER, atomic adds (summation order is not fixed): w_k * dL/drgb of every
+ *               entry, scattered as the texel was gathered (vertex: b_i w G into corner i; UV: the four bilinear taps;
+ *               atlas: the cell).  face_uvs gets no gradient
+ *   grad_bary   float (P,K,3), ZEROED BY THE CALLER, written at entries with pix_to_face >= 0 that some sample picked:
+ *               vertex <table[f,i], w G>; UV the chain through (u, v) of pert_phong_bwd; atlas nothing (piecewise constant)
+ * Refusals: any PERT_PH_* bit, or pb->colors / pb->face_colors set as well, PERT_E_UNSUPPORTED (a sample-sharded call
+ * materialises the colours); a NULL tex, tex->bary or tex->table PERT_E_NULL (and face_uvs for PERT_TEX_UV); an unknown kind,
+ * num_faces <= 0, non-positive map sizes, map_count other than 1 or N, or atlas_size <= 0 PERT_E_SHAPE; num_faces * R^2 * 3
+ * > 2^31 - 1 PERT_E_UNSUPPORTED; a pointer not aligned to its element type PERT_E_ALIGN.
+ */
+int pert_shade_tex_fwd(const pert_problem* pb, const pert_texture* tex, float* image, uint16_t* counts, float* rsum,
+                       void* winners, uint16_t* pixstate, int32_t* hist, int32_t* worklist, void* tile_blob, void* stream);
+int pert_shade_tex_render(const pert_problem* pb, const pert_texture* tex, float* image, uint16_t* counts_ws,
+                          int32_t* worklist, void* stream);
+int pert_shade_tex_bwd(const pert_problem* pb, const pert_texture* tex, const float* grad_image, const uint16_t* counts,
+                       const float* rsum, const void* winners, const uint16_t* pixstate, float* grad_dists, float* grad_zbuf,
+                       float* grad_table, float* grad_bary, float* scalar_partials, float* grad_scalars, float* acc,
+                       float* pixstat, const int32_t* hist, int32_t* worklist, const void* tile_blob, void* stream);
+
+/*
  * SoftRas pair: SoftRast + SoftAgg, the DEFAULT operators of RandomSimpleShader
  * (randomras/random_rasterizer.py:139-140; smoothrast.py:126-134; smoothagg.py:165-182), fused and
  * deterministic: P = sigmoid(-dists/sigma)*mask, w = softmax(logits/gamma), same logits, alpha channel and

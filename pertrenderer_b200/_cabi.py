@@ -31,7 +31,7 @@ PH_BWD_SAMPLE, PH_BWD_FINISH = 0x100, 0x200
 
 EXPORTS = [
     "pert_version", "pert_shade_fused_flags", "pert_strerror", "pert_last_cuda_error", "pert_num_tiles", "pert_winner_bytes", "pert_blob_bytes",
-    "pert_shade_fwd", "pert_shade_render", "pert_shade_render_phase", "pert_shade_bwd", "pert_soft_shade_fwd", "pert_soft_shade_bwd", "pert_rast_fwd", "pert_rast_bwd", "pert_argmax_fwd",
+    "pert_shade_fwd", "pert_shade_render", "pert_shade_render_phase", "pert_shade_bwd", "pert_shade_tex_fwd", "pert_shade_tex_bwd", "pert_shade_tex_render", "pert_soft_shade_fwd", "pert_soft_shade_bwd", "pert_rast_fwd", "pert_rast_bwd", "pert_argmax_fwd",
     "pert_argmax_bwd", "pert_noise_fill", "pert_seed_advance", "pert_phong_fwd", "pert_phong_bwd", "pert_phong_atlas_fwd", "pert_phong_atlas_bwd",
     "pert_rasterize_fwd", "pert_rasterize_bwd", "pert_rasterize_num_bins", "pert_rasterize_bin", "pert_rasterize_bin_bounded",
     "pert_rasterize_bin_capacity",
@@ -39,6 +39,8 @@ EXPORTS = [
 
 RAST_CULL_BACKFACES = 1  # PERT_RAST_CULL_BACKFACES
 RAST_BIN_WIDE = 2  # PERT_RAST_BIN_WIDE
+
+TEX_VERTEX, TEX_UV, TEX_ATLAS = 1, 2, 3  # PERT_TEX_* (pert_texture.kind)
 
 PHONG_STRIDE = 20  # PERT_PHONG_STRIDE
 PHONG_SPARSE = 1  # PERT_PHONG_SPARSE
@@ -64,6 +66,16 @@ class PertProblem(C.Structure):
         ("noise_rast", C.c_void_p), ("noise_agg", C.c_void_p),
         ("face_colors", C.c_void_p), ("num_faces", C.c_int64),
         ("seed_device", C.c_void_p),
+    ]
+
+
+class PertTexture(C.Structure):
+    """Mirror of ``struct pert_texture``."""
+    _fields_ = [
+        ("kind", C.c_int32), ("atlas_size", C.c_int32),
+        ("bary", C.c_void_p), ("table", C.c_void_p), ("face_uvs", C.c_void_p),
+        ("map_h", C.c_int32), ("map_w", C.c_int32), ("map_count", C.c_int32),
+        ("num_faces", C.c_int64),
     ]
 
 
@@ -246,6 +258,32 @@ def phong_atlas_fns():
         bwd.argtypes = [C.POINTER(PertPhong), C.c_void_p, C.c_int32] + [C.c_void_p] * 7
         _phong_atlas = (lib, fwd, bwd)
     return _phong_atlas[1], _phong_atlas[2]
+
+
+_shade_tex = None  # (library, its bound pert_shade_tex_fwd, pert_shade_tex_bwd, pert_shade_tex_render)
+
+
+def shade_tex_fns():
+    """(``pert_shade_tex_fwd``, ``pert_shade_tex_bwd``, ``pert_shade_tex_render``) of the loaded library, bound on first use
+    rather than in :func:`load`, so that a library built before them keeps serving every other call; with such a library
+    this raises PertLibraryError asking for a rebuild (the texture is never materialised behind the caller's back)."""
+    global _shade_tex
+    lib = load()
+    if _shade_tex is None or _shade_tex[0] is not lib:
+        names = ("pert_shade_tex_fwd", "pert_shade_tex_bwd", "pert_shade_tex_render")
+        fns = [getattr(lib, n, None) for n in names]
+        if any(f is None for f in fns):
+            raise PertLibraryError(f"{LIB_PATH} predates the textures sampled inside the fused shading kernels "
+                                   "(pert_shade_tex_fwd / _bwd / _render): rebuild it with "
+                                   "`python -m pertrenderer_b200.build --force`")
+        fwd, bwd, render = fns
+        pp, pt, vp = C.POINTER(PertProblem), C.POINTER(PertTexture), C.c_void_p
+        fwd.restype = bwd.restype = render.restype = C.c_int
+        fwd.argtypes = [pp, pt] + [vp] * 9
+        bwd.argtypes = [pp, pt] + [vp] * 17
+        render.argtypes = [pp, pt] + [vp] * 4
+        _shade_tex = (lib, fwd, bwd, render)
+    return _shade_tex[1], _shade_tex[2], _shade_tex[3]
 
 
 _raster_bins = None  # (library, its bound pert_rasterize_bin_bounded, pert_rasterize_bin_capacity)

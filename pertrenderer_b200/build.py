@@ -16,7 +16,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC_DIR = os.path.join(HERE, "csrc")
 SOURCES = [os.path.join(SRC_DIR, f) for f in ("cabi.cu", "shade_fwd.cu", "shade_bwd.cu", "shade_soft.cu", "ops_standalone.cu", "phong.cu", "raster.cu")]
-HEADERS = [os.path.join(SRC_DIR, f) for f in ("philox.cuh", "common.cuh", "tile.cuh", "kernels.h")] + \
+HEADERS = [os.path.join(SRC_DIR, f) for f in ("philox.cuh", "common.cuh", "tile.cuh", "texel.cuh", "kernels.h")] + \
     [os.path.join(os.path.dirname(HERE), "include", "pertshade.h")]
 LIB_PATH = os.path.join(HERE, "libpertshade.so")
 

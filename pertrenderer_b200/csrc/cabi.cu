@@ -219,7 +219,7 @@ static bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
 
 // Launch records of a single forward call: `a` (pointers set) gets the main pass's tile geometry and, in sparse-first mode,
 // `fb` the fallback pass's (half-size tiles, full capacity).  Returns 1 in sparse-first mode, 0 without it, or a PERT_E_*.
-static int fwd_launch_records(FwdArgs& a, FwdArgs& fb, bool sparse) {
+static int fwd_launch_records(FwdLaunch& a, FwdLaunch& fb, bool sparse) {
     const int64_t P = a.pb.N * a.pb.H * a.pb.W;
     if (sparse) {  // the fallback pass runs FBT/32 warps per CTA: its tiles must fit that many times
         SmemLayout t;
@@ -244,18 +244,40 @@ static int fwd_launch_records(FwdArgs& a, FwdArgs& fb, bool sparse) {
     return 1;
 }
 
-extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t* counts, float* rsum, void* winners,
-                              uint16_t* pixstate, int32_t* hist, int32_t* worklist, void* tile_blob, void* stream) {
+// The texture of a pert_shade_tex_* call as the kernels' TexArgs, or a PERT_E_* code (pertshade.h)
+static int check_texture(const pert_problem* pb, const pert_texture* tex, TexArgs& t) {
+    if (!tex) return PERT_E_NULL;
+    if (pb->flags & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND | PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH)) return PERT_E_UNSUPPORTED;
+    if (pb->colors || pb->face_colors) return PERT_E_UNSUPPORTED;
+    if (!tex->bary || !tex->table || (tex->kind == PERT_TEX_UV && !tex->face_uvs)) return PERT_E_NULL;
+    if (tex->kind < PERT_TEX_VERTEX || tex->kind > PERT_TEX_ATLAS || tex->num_faces <= 0) return PERT_E_SHAPE;
+    if (tex->kind == PERT_TEX_UV && (tex->map_h <= 0 || tex->map_w <= 0 || (tex->map_count != 1 && tex->map_count != pb->N)))
+        return PERT_E_SHAPE;
+    if (tex->kind == PERT_TEX_ATLAS) {
+        if (tex->atlas_size <= 0) return PERT_E_SHAPE;
+        // 32-bit atlas offsets (texel.cuh atlas_cell): num_faces R^2 3 <= 2^31 - 1, written so that nothing overflows
+        if ((int64_t)tex->atlas_size * tex->atlas_size > 0x7fffffff / 3 / tex->num_faces) return PERT_E_UNSUPPORTED;
+    }
+    if (((uintptr_t)tex->bary & 3) || ((uintptr_t)tex->table & 3) || ((uintptr_t)tex->face_uvs & 3)) return PERT_E_ALIGN;
+    t = TexArgs{tex->kind + (TX_VERT - PERT_TEX_VERTEX), tex->atlas_size, tex->bary, tex->table, tex->face_uvs,
+                tex->map_h, tex->map_w, tex->map_count, nullptr};
+    return PERT_OK;
+}
+
+// pert_shade_fwd, and pert_shade_tex_fwd with tx.kind != TX_DENSE (a validated texture)
+static int shade_fwd_call(const pert_problem* pb_in, const TexArgs& tx, float* image, uint16_t* counts, float* rsum,
+                          void* winners, uint16_t* pixstate, int32_t* hist, int32_t* worklist, void* tile_blob, void* stream) {
     int rc = check_problem(pb_in);
     if (rc) return rc;
-    FwdArgs a;
+    FwdLaunch a;
     a.pb = *pb_in;
+    a.tex = tx;
     if (!(a.pb.flags & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND))) a.pb.flags |= PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
     const uint32_t f = a.pb.flags;
     if (!counts) return PERT_E_NULL;
     if ((f & PERT_PH_RAST) && !rsum) return PERT_E_NULL;
     if ((f & PERT_PH_AGG) && (!winners || !pixstate)) return PERT_E_NULL;
-    if ((f & PERT_PH_BLEND) && (!image || (!a.pb.colors && !a.pb.face_colors))) return PERT_E_NULL;
+    if ((f & PERT_PH_BLEND) && (!image || (!a.pb.colors && !a.pb.face_colors && tx.kind == TX_DENSE))) return PERT_E_NULL;
     if (((f & PERT_PH_AGG) != 0) != ((f & PERT_PH_BLEND) != 0) && !hist) return PERT_E_NULL;
     if (((uintptr_t)image & 15) || ((uintptr_t)counts & 1) || ((uintptr_t)rsum & 3) || ((uintptr_t)hist & 3) ||
         ((uintptr_t)a.pb.colors & 3) || ((uintptr_t)pixstate & 1) || ((uintptr_t)winners & 3))
@@ -272,7 +294,7 @@ extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t*
     a.hist = hist;
     a.worklist = worklist;
     a.blob = (int32_t*)tile_blob;  // the fallback pass's records follow the tile blobs (fwd_launch_records)
-    FwdArgs fb;
+    FwdLaunch fb;
     rc = fwd_launch_records(a, fb, sparse_first_ok(&a.pb, worklist, (f & all) == all && !hist));
     if (rc < 0) return rc;
     const bool sparse = rc == 1;
@@ -285,18 +307,34 @@ extern "C" int pert_shade_fwd(const pert_problem* pb_in, float* image, uint16_t*
     return cuda_rc(launch_shade_fwd(a, &fb, st));
 }
 
-extern "C" int pert_shade_render(const pert_problem* pb_in, float* image, uint16_t* counts_ws, int32_t* worklist,
-                                 void* stream) {
+extern "C" int pert_shade_fwd(const pert_problem* pb, float* image, uint16_t* counts, float* rsum, void* winners,
+                              uint16_t* pixstate, int32_t* hist, int32_t* worklist, void* tile_blob, void* stream) {
+    return shade_fwd_call(pb, TexArgs{}, image, counts, rsum, winners, pixstate, hist, worklist, tile_blob, stream);
+}
+
+extern "C" int pert_shade_tex_fwd(const pert_problem* pb, const pert_texture* tex, float* image, uint16_t* counts, float* rsum,
+                                  void* winners, uint16_t* pixstate, int32_t* hist, int32_t* worklist, void* tile_blob,
+                                  void* stream) {
+    TexArgs t;
+    if (int rc = check_problem(pb)) return rc;
+    if (int rc = check_texture(pb, tex, t)) return rc;
+    return shade_fwd_call(pb, t, image, counts, rsum, winners, pixstate, hist, worklist, tile_blob, stream);
+}
+
+// pert_shade_render, and pert_shade_tex_render with tx.kind != TX_DENSE
+static int shade_render_call(const pert_problem* pb_in, const TexArgs& tx, float* image, uint16_t* counts_ws, int32_t* worklist,
+                             void* stream) {
     int rc = check_problem(pb_in);
     if (rc) return rc;
-    FwdArgs a = {};
+    FwdLaunch a = {};
     a.pb = *pb_in;
+    a.tex = tx;
     const uint32_t f = a.pb.flags;
     // one call renders every sample: the phase-split (sample-sharded) forward has no forward-only form
     if (f & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND | PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH)) return PERT_E_UNSUPPORTED;
     if (a.pb.s_rast_begin != 0 || a.pb.s_rast_end != a.pb.S_rast || a.pb.s_agg_begin != 0 || a.pb.s_agg_end != a.pb.S_agg)
         return PERT_E_UNSUPPORTED;
-    if (!image || (!a.pb.colors && !a.pb.face_colors)) return PERT_E_NULL;
+    if (!image || (!a.pb.colors && !a.pb.face_colors && tx.kind == TX_DENSE)) return PERT_E_NULL;
     if (((uintptr_t)image & 15) || ((uintptr_t)counts_ws & 1) || ((uintptr_t)a.pb.colors & 3) || ((uintptr_t)worklist & 15))
         return PERT_E_ALIGN;
     if ((f & PERT_F_PHILOX7) && (a.pb.noise_rast || a.pb.noise_agg)) return PERT_E_UNSUPPORTED;
@@ -310,7 +348,7 @@ extern "C" int pert_shade_render(const pert_problem* pb_in, float* image, uint16
     a.image = image;
     a.counts = counts_ws;
     a.worklist = worklist;
-    FwdArgs fb;
+    FwdLaunch fb;
     rc = fwd_launch_records(a, fb, sparse_ok);
     if (rc < 0) return rc;
     cudaStream_t st = (cudaStream_t)stream;
@@ -320,11 +358,23 @@ extern "C" int pert_shade_render(const pert_problem* pb_in, float* image, uint16
     return cuda_rc(launch_shade_render(a, &fb, st));
 }
 
+extern "C" int pert_shade_render(const pert_problem* pb, float* image, uint16_t* counts_ws, int32_t* worklist, void* stream) {
+    return shade_render_call(pb, TexArgs{}, image, counts_ws, worklist, stream);
+}
+
+extern "C" int pert_shade_tex_render(const pert_problem* pb, const pert_texture* tex, float* image, uint16_t* counts_ws,
+                                     int32_t* worklist, void* stream) {
+    TexArgs t;
+    if (int rc = check_problem(pb)) return rc;
+    if (int rc = check_texture(pb, tex, t)) return rc;
+    return shade_render_call(pb, t, image, counts_ws, worklist, stream);
+}
+
 extern "C" int pert_shade_render_phase(const pert_problem* pb_in, float* image, uint16_t* counts, int32_t* hist,
                                        void* stream) {
     int rc = check_problem(pb_in);
     if (rc) return rc;
-    FwdArgs a = {};
+    FwdLaunch a = {};
     a.pb = *pb_in;
     const uint32_t f = a.pb.flags;
     const uint32_t ph = f & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND);
@@ -341,32 +391,37 @@ extern "C" int pert_shade_render_phase(const pert_problem* pb_in, float* image, 
     a.image = image;
     a.counts = counts;
     a.hist = hist;
-    FwdArgs fb;
+    FwdLaunch fb;
     rc = fwd_launch_records(a, fb, false);  // the tiles of pert_shade_fwd's phase calls
     if (rc < 0) return rc;
     return cuda_rc(launch_shade_render(a, nullptr, (cudaStream_t)stream));
 }
 
-extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image, const uint16_t* counts,
-                              const float* rsum, const void* winners, const uint16_t* pixstate, float* grad_dists,
-                              float* grad_zbuf, float* grad_colors, float* scalar_partials, float* grad_scalars,
-                              float* acc, float* pixstat, const int32_t* hist, int32_t* worklist,
-                              const void* tile_blob, void* stream) {
+// pert_shade_bwd, and pert_shade_tex_bwd with tx.kind != TX_DENSE (grad_colors = the table's gradient)
+static int shade_bwd_call(const pert_problem* pb_in, const TexArgs& tx, const float* grad_image, const uint16_t* counts,
+                          const float* rsum, const void* winners, const uint16_t* pixstate, float* grad_dists,
+                          float* grad_zbuf, float* grad_colors, float* grad_bary, float* scalar_partials, float* grad_scalars,
+                          float* acc, float* pixstat, const int32_t* hist, int32_t* worklist,
+                          const void* tile_blob, void* stream) {
     int rc = check_problem(pb_in);
     if (rc) return rc;
-    BwdArgs a;
+    BwdLaunch a;
     a.pb = *pb_in;
+    a.tex = tx;
+    a.tex.grad_bary = grad_bary;
+    const bool tex = tx.kind != TX_DENSE;
     if (!(a.pb.flags & (PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH))) a.pb.flags |= PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH;
     const uint32_t f = a.pb.flags;
     const bool smp = f & PERT_PH_BWD_SAMPLE, fin = f & PERT_PH_BWD_FINISH;
-    if (!grad_image || !counts || !rsum || !pixstate || (!a.pb.colors && !a.pb.face_colors)) return PERT_E_NULL;
+    if (!grad_image || !counts || !rsum || !pixstate || (!a.pb.colors && !a.pb.face_colors && !tex)) return PERT_E_NULL;
     if (smp && !winners) return PERT_E_NULL;
     if (fin && (!grad_dists || !grad_zbuf || !scalar_partials || !grad_scalars)) return PERT_E_NULL;
     if (smp != fin && (!acc || !pixstat)) return PERT_E_NULL;
     if (fin && !smp && grad_colors && !hist) return PERT_E_NULL;
     if (((uintptr_t)grad_image & 15) || ((uintptr_t)grad_colors & 3) || ((uintptr_t)grad_dists & 3) ||
         ((uintptr_t)grad_zbuf & 3) || ((uintptr_t)counts & 1) || ((uintptr_t)rsum & 3) || ((uintptr_t)pixstate & 1) ||
-        ((uintptr_t)scalar_partials & 15) || ((uintptr_t)acc & 3) || ((uintptr_t)pixstat & 3) || ((uintptr_t)hist & 3))
+        ((uintptr_t)scalar_partials & 15) || ((uintptr_t)acc & 3) || ((uintptr_t)pixstat & 3) || ((uintptr_t)hist & 3) ||
+        ((uintptr_t)grad_bary & 3))
         return PERT_E_ALIGN;
     if ((uintptr_t)worklist & 15) return PERT_E_ALIGN;
     if ((f & PERT_F_PHILOX7) && (!(smp && fin) || hist || a.pb.noise_agg)) return PERT_E_UNSUPPORTED;
@@ -380,7 +435,7 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
         if ((size_t)sl.bytes * (FBT / 32) > 200 * 1024) sparse = false;
     }
     const bool ptr_ok = aligned16(a.pb.pix_to_face) && aligned16(grad_dists) && aligned16(grad_zbuf) &&
-                        (a.pb.face_colors || aligned16(grad_colors));
+                        (a.pb.face_colors || tex || aligned16(grad_colors));
     a.L = make_launch(&a.pb, sparse ? sparse_tp(a.pb.K, a.pb.N * a.pb.H * a.pb.W) : dense_tp(a.pb.K, a.pb.N * a.pb.H * a.pb.W));
     a.L.vec_ok = a.L.vec_ok && ptr_ok;
     if (sparse) a.L.cap = sparse_cap(a.pb.K, a.L.tp);
@@ -406,7 +461,7 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
     a.blob = sparse ? (const int32_t*)tile_blob : nullptr;
     cudaStream_t st = (cudaStream_t)stream;
     if (!sparse) return cuda_rc(launch_shade_bwd(a, nullptr, grad_scalars, st));
-    BwdArgs fb = a;  // fallback pass: half-size tiles, full capacity, dense per-logit arrays
+    BwdLaunch fb = a;  // fallback pass: half-size tiles, full capacity, dense per-logit arrays
     fb.blob = a.blob ? a.blob + blob_records_off(a.pb.K, a.L.P) : nullptr;
     fb.L = make_launch(&a.pb, a.L.tp / 2);
     fb.L.vec_ok = fb.L.vec_ok && ptr_ok;
@@ -416,6 +471,26 @@ extern "C" int pert_shade_bwd(const pert_problem* pb_in, const float* grad_image
     cudaError_t e = cudaMemsetAsync(worklist, 0, 16, st);
     if (e != cudaSuccess) return cuda_fail((int)e);
     return cuda_rc(launch_shade_bwd(a, &fb, grad_scalars, st));
+}
+
+extern "C" int pert_shade_bwd(const pert_problem* pb, const float* grad_image, const uint16_t* counts, const float* rsum,
+                              const void* winners, const uint16_t* pixstate, float* grad_dists, float* grad_zbuf,
+                              float* grad_colors, float* scalar_partials, float* grad_scalars, float* acc, float* pixstat,
+                              const int32_t* hist, int32_t* worklist, const void* tile_blob, void* stream) {
+    return shade_bwd_call(pb, TexArgs{}, grad_image, counts, rsum, winners, pixstate, grad_dists, grad_zbuf, grad_colors,
+                          nullptr, scalar_partials, grad_scalars, acc, pixstat, hist, worklist, tile_blob, stream);
+}
+
+extern "C" int pert_shade_tex_bwd(const pert_problem* pb, const pert_texture* tex, const float* grad_image,
+                                  const uint16_t* counts, const float* rsum, const void* winners, const uint16_t* pixstate,
+                                  float* grad_dists, float* grad_zbuf, float* grad_table, float* grad_bary,
+                                  float* scalar_partials, float* grad_scalars, float* acc, float* pixstat, const int32_t* hist,
+                                  int32_t* worklist, const void* tile_blob, void* stream) {
+    TexArgs t;
+    if (int rc = check_problem(pb)) return rc;
+    if (int rc = check_texture(pb, tex, t)) return rc;
+    return shade_bwd_call(pb, t, grad_image, counts, rsum, winners, pixstate, grad_dists, grad_zbuf, grad_table, grad_bary,
+                          scalar_partials, grad_scalars, acc, pixstat, hist, worklist, tile_blob, stream);
 }
 
 // ---- SoftRas pair (SoftRast + SoftAgg), deterministic -----------------------------------------------

@@ -4,6 +4,19 @@
 
 namespace pert {
 
+// Texel source of the fused kernels (template parameter TEX): TX_DENSE / TX_FACE are the pert_problem's colors / face_colors,
+// the others a pert_texture record (pert_shade_tex_*), sampled from bary and the table where the kernels blend
+enum { TX_DENSE = 0, TX_FACE = 1, TX_VERT = 2, TX_UV = 3, TX_ATLAS = 4 };
+struct TexArgs {
+    int kind;  // TX_*; TX_DENSE (0) for the calls without a pert_texture, whatever their pert_problem carries
+    int R;     // atlas_size
+    const float* bary;
+    const float* table;
+    const float* face_uvs;
+    int map_h, map_w, map_count;
+    float* grad_bary;  // backward: (P,K,3) or NULL (BwdArgs::grad_colors is then the table's gradient, or NULL)
+};
+
 struct FwdArgs {
     pert_problem pb;
     Launch L;
@@ -36,16 +49,25 @@ struct BwdArgs {
     const int32_t* blob;  // tile blobs of forward, or NULL: backward then rescans and recomputes
 };
 
+// What the launchers get: the kernels' argument record and the texel source, which travels as a kernel parameter of its
+// own, after the others (the instantiations without a pert_texture keep the parameter layout they had without it)
+struct FwdLaunch : FwdArgs {
+    TexArgs tex;
+};
+struct BwdLaunch : BwdArgs {
+    TexArgs tex;
+};
+
 int fwd_smem_layout(int tp, int cap, SmemLayout& L);  // returns the bytes the coverage-sample phase needs
 void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes, bool compact, bool lean, SmemLayout& L);
 
 // return a cudaError_t as int (0 = success)
 // `fb` (optional): launch record of the fallback pass of the sparse-first mode (half-size tiles)
-int launch_shade_fwd(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st);
-int launch_shade_bwd(const BwdArgs& a, const BwdArgs* fb, float* grad_scalars, cudaStream_t st);
+int launch_shade_fwd(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st);
+int launch_shade_bwd(const BwdLaunch& a, const BwdLaunch* fb, float* grad_scalars, cudaStream_t st);
 // forward-only render: image only (a.counts = the fallback pass's workspace or NULL; no other saved state); with one phase
 // bit (pert_shade_render_phase) a.counts / a.hist are that phase's inputs and outputs
-int launch_shade_render(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st);
+int launch_shade_render(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st);
 
 void soft_smem_layout(int tp, int K, bool bwd, SmemLayout& L);
 int launch_soft_fwd(const pert_problem& pb, const Launch& L, float* image, cudaStream_t st);

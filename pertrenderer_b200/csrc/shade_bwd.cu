@@ -17,6 +17,7 @@
 //   4  chain rule per valid entry -> scattered stores over the zero-filled rows; scalar partials
 #include <climits>
 #include "kernels.h"
+#include "texel.cuh"
 #include "tile.cuh"
 
 namespace pert {
@@ -51,7 +52,9 @@ void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes,
 // GT = lanes per pixel as a compile-time constant (1, 2, 4, 8), or 0 to read it from the launch record.
 // PHASED = false is the production instantiation: both phases in one launch, histogram rebuilt from the
 // saved winners (the phase-split code of the sample-sharded job is compiled out to keep the hot code small).
-// FACE = true: colours gathered through pix_to_face from pb.face_colors, grad scattered by atomics
+// TEX = the texel source (kernels.h): TX_DENSE pb.colors; TX_FACE colours gathered through pix_to_face from pb.face_colors,
+// grad scattered by atomics; TX_VERT / TX_UV / TX_ATLAS texels sampled from a.tex (texel.cuh), their gradient scattered into
+// the table (a.grad_colors) and, for vertex colours and UV maps, written to tx.grad_bary
 // COMPACT = true (sparse-first mode): the per-logit arrays are indexed by the position of the logit
 // among the pixel's valid entries (plus a background and a masked-logits slot) instead of densely by j,
 // and every array holds a.L.cap valid entries; tiles with more go to the fallback pass.
@@ -65,10 +68,10 @@ void bwd_smem_layout(int tp, int K, int cap, int sc, int nchunks, int win_bytes,
 // (forward wrote no winners row for them when a0 was their only live logit: a_s = a0 is known) and the pixels
 // without any valid entry (the background wins every sample; their only output is the gamma term, whose norm runs
 // over all K + 1 logits).  Every V_sj of every logit is regenerated (per-sample noise, dense per-logit arrays).
-template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0, bool WOVR = false>
+template <class NoiseA, int GT, bool PHASED, int TEX, bool COMPACT, bool BLOB, int SCORE = 0, bool WOVR = false>
 __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& noise_a, const int64_t tile,
                                                const int64_t prow /* row of the scalar partials */,
-                                               unsigned char* smem_raw, const int lane) {
+                                               unsigned char* smem_raw, const int lane, const TexArgs& tx) {
     const pert_problem& pb = a.pb;
     const int G = GT ? GT : a.L.G;
     const int gshift = GT ? (GT == 16 ? 4 : GT == 8 ? 3 : GT == 4 ? 2 : GT == 2 ? 1 : 0) : a.L.gshift;
@@ -152,7 +155,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
         if (do_finish) {
             zero_fill(a.grad_dists + g0, E, a.L.vec_ok);
             zero_fill(a.grad_zbuf + g0, E, a.L.vec_ok);
-            if (a.grad_colors && !FACE) zero_fill(a.grad_colors + g0 * 3, E * 3, a.L.vec_ok);
+            if (a.grad_colors && TEX == TX_DENSE) zero_fill(a.grad_colors + g0 * 3, E * 3, a.L.vec_ok);
         } else {
             zero_fill(a.acc + pix0 * K1, npx * K1, false);
             if (lane < npx) {
@@ -182,10 +185,12 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                 if constexpr (COMPACT) cn32[i] = (uint32_t)__ldg(bl + blob_cnt_off(tp, cap) + i);
                 // needed a few round trips later (g_j of the logits that can win; chain rule): start them now
                 const int e0 = v2 & 0xffff, e1 = v2 >> 16;
-                if (!FACE) prefetch_l1(colors_t + e0 * 3);
+                if (TEX == TX_DENSE) prefetch_l1(colors_t + e0 * 3);
+                if (TEX >= TX_VERT) prefetch_l1(tx.bary + (g0 + e0) * 3);
                 prefetch_l1(rsum_t + e0);
                 if (2 * i + 1 < nv) {
-                    if (!FACE) prefetch_l1(colors_t + e1 * 3);
+                    if (TEX == TX_DENSE) prefetch_l1(colors_t + e1 * 3);
+                    if (TEX >= TX_VERT) prefetch_l1(tx.bary + (g0 + e1) * 3);
                     prefetch_l1(rsum_t + e1);
                 }
             }
@@ -226,7 +231,8 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                     zs[n] = __ldg(zbuf_t + e);
                     cnt[n] = counts_t[e];
                     // needed a few round trips later (g_j of the logits that can win; chain rule): start them now
-                    if (!FACE) prefetch_l1(colors_t + e * 3);
+                    if (TEX == TX_DENSE) prefetch_l1(colors_t + e * 3);
+                    if (TEX >= TX_VERT) prefetch_l1(tx.bary + (g0 + e) * 3);
                     prefetch_l1(rsum_t + e);
                 }
             }
@@ -257,7 +263,7 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
         float t2sum = 0.f, csum = 0.f;
         const float* gacc = a.acc + gp * K1;  // FINISH-only: sums over all sample shards
         const float* const colors_p = pb.colors + gp * K * 3;
-        const float* const fcol = FACE ? pb.face_colors : nullptr;  // per-face colours gathered through pix_to_face
+        const float* const fcol = TEX == TX_FACE ? pb.face_colors : nullptr;  // per-face colours gathered through pix_to_face
         const int64_t* const p2f_p = pb.pix_to_face + gp * K;
         __syncwarp();
 
@@ -290,7 +296,11 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                     const int sl = COMPACT ? sb + idx : sb + j;
                     if (z > -CUDART_INF_F && z >= floor_v) {
                         float gj;
-                        if (j < K) {
+                        if (TEX >= TX_VERT && j < K) {
+                            const int64_t ge = gp * K + j;
+                            const V3 c = tex_texel<TEX>(tx, a.L.HW * K, ge, __ldg(p2f_p + j), ld3(tx.bary + ge * 3));
+                            gj = Gi.x * c.x + Gi.y * c.y + Gi.z * c.z;
+                        } else if (j < K) {
                             const float* c = fcol ? fcol + 3 * (int)__ldg(p2f_p + j) : colors_p + j * 3;
                             gj = Gi.x * __ldg(c) + Gi.y * __ldg(c + 1) + Gi.z * __ldg(c + 2);
                         } else {
@@ -568,8 +578,9 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
             const float* const rsum_t = a.rsum + g0;
             float* const gd_t = a.grad_dists + g0;
             float* const gz_t = a.grad_zbuf + g0;
-            float* const gc_t = (a.grad_colors && !fcol) ? a.grad_colors + g0 * 3 : nullptr;
+            float* const gc_t = (TEX < TX_VERT && a.grad_colors && !fcol) ? a.grad_colors + g0 * 3 : nullptr;
             float* const gfc = fcol ? a.grad_colors : nullptr;  // (num_faces,3), atomic scatter
+            const bool gtex = TEX >= TX_VERT && (a.grad_colors || tx.grad_bary);  // the sampled texture's table and bary
 #pragma unroll 1
             for (int n = vs + lig; n < ve; n += G) {
                 const int e = vlist[n];
@@ -598,14 +609,19 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
                 gd_t[e] = -gx;
                 p_sigma += gx;
                 // grad_colors = w_k * G_rgb
-                if (gc_t || gfc) {
+                if (gc_t || gfc || gtex) {
                     int h;
                     if (ghist) h = ghist[gp * K1 + k];  // all-shard histogram when sample-sharded
                     else if (act) h = hj[sl];
                     else h = (k == a0) ? sa_loc : 0;
                     if (h > 0) {
                         const float w = (float)h * invS;
-                        if (gfc) {
+                        if (TEX >= TX_VERT) {
+                            const int64_t ge = gp * K + k;
+                            const V3 gb = tex_texel_bwd<TEX>(tx, a.L.HW * K, ge, __ldg(p2f_p + k), ld3(tx.bary + ge * 3),
+                                                             mk(w * Gi.x, w * Gi.y, w * Gi.z), a.grad_colors);
+                            if (TEX != TX_ATLAS && tx.grad_bary) st3(tx.grad_bary + ge * 3, gb);
+                        } else if (gfc) {
                             float* gc = gfc + 3 * (int)__ldg(p2f_p + k);
                             atomicAdd(gc, w * Gi.x);
                             atomicAdd(gc + 1, w * Gi.y);
@@ -634,18 +650,23 @@ __device__ __forceinline__ void shade_bwd_tile(const BwdArgs& a, const NoiseA& n
 // CTAs (= warps) per SM the main pass is compiled for: 64 registers, no spills; the shared-memory layout allows 30
 // (25 / 28 / 32 measured on the sparse set: 0.326 / 0.311 / 0.323 ms)
 constexpr int BWD_MAIN_CTAS = 28;
-template <class NoiseA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB, int SCORE = 0, bool WOVR = false>
-__global__ void __launch_bounds__(FNT, BWD_MAIN_CTAS) shade_bwd_kernel(const BwdArgs a, const NoiseA noise_a) {
+// A UV texture (TX_UV) calls two out-of-line functions (uv_texel, uv_texel_bwd), across which more values stay live: the
+// compiler takes 72 registers, which allows 28 warps per SM where the other sources (64 registers) keep the 30 the
+// shared-memory layout allows.  Bounded to 64 registers (32 CTAs) it spills 8 bytes and measured the same, 0.53 ms at
+// BASELINE config 2 (profiles/r11_tex_shade.txt): the UV backward is bound by its four taps and atomics, not residency.
+template <class NoiseA, int GT, bool PHASED, int TEX, bool COMPACT, bool BLOB, int SCORE = 0, bool WOVR = false>
+__global__ void __launch_bounds__(FNT, BWD_MAIN_CTAS) shade_bwd_kernel(const BwdArgs a, const NoiseA noise_a, const TexArgs tex) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     NoiseA na = noise_a;
     if (a.pb.seed_device) na.mix(__ldg(a.pb.seed_device + 1));  // device-side seed, see shade_fwd.cu
-    shade_bwd_tile<NoiseA, GT, PHASED, FACE, COMPACT, BLOB, SCORE, WOVR>(a, na, blockIdx.x, blockIdx.x, smem_raw, threadIdx.x);
+    shade_bwd_tile<NoiseA, GT, PHASED, TEX, COMPACT, BLOB, SCORE, WOVR>(a, na, blockIdx.x, blockIdx.x, smem_raw, threadIdx.x, tex);
 }
 
 // Fallback pass of the sparse-first mode (see shade_fwd.cu): work-list tiles as half-size tiles with dense
 // per-logit arrays; their scalar partials go to the rows after the main pass's.  BLOB: from forward's fallback records.
-template <class NoiseA, int GT, bool FACE, bool BLOB>
-__global__ void __launch_bounds__(FBT, 12) shade_bwd_fallback_kernel(const BwdArgs a, const NoiseA noise_a, int64_t prow0) {
+template <class NoiseA, int GT, int TEX, bool BLOB>
+__global__ void __launch_bounds__(FBT, 12) shade_bwd_fallback_kernel(const BwdArgs a, const NoiseA noise_a, int64_t prow0,
+                                                                                 const TexArgs tex) {
     extern __shared__ __align__(16) unsigned char smem_all[];
     unsigned char* smem_raw = smem_all + (threadIdx.x >> 5) * a.L.warp_smem;  // FBT/32 independent warps per CTA
     const int n = 2 * a.worklist[0];
@@ -659,7 +680,7 @@ __global__ void __launch_bounds__(FBT, 12) shade_bwd_fallback_kernel(const BwdAr
         if (i >= n) break;
         const int64_t tile = (int64_t)a.worklist[4 + (i >> 1)] * 2 + (i & 1);
         if (tile < a.L.ntiles) {
-            shade_bwd_tile<NoiseA, GT, false, FACE, false, BLOB>(a, na, tile, prow0 + i, smem_raw, threadIdx.x & 31);
+            shade_bwd_tile<NoiseA, GT, false, TEX, false, BLOB>(a, na, tile, prow0 + i, smem_raw, threadIdx.x & 31, tex);
         } else if ((threadIdx.x & 31) == 0) {
             reinterpret_cast<float4*>(a.partials)[prow0 + i] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
@@ -728,46 +749,63 @@ static int set_smem(K kern, size_t smem) {
     return 0;
 }
 
-template <class NA, int GT, bool PHASED, bool FACE, bool COMPACT, bool BLOB = false, int SCORE = 0, bool WOVR = false>
-static int launch_bwd_f(const BwdArgs& a, const NA& na, cudaStream_t st) {
+template <class NA, int GT, bool PHASED, int TEX, bool COMPACT, bool BLOB = false, int SCORE = 0, bool WOVR = false>
+static int launch_bwd_f(const BwdLaunch& a, const NA& na, cudaStream_t st) {
     const size_t smem = (size_t)a.L.warp_smem;
-    if (int rc = set_smem(shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE, WOVR>, smem)) return rc;
-    shade_bwd_kernel<NA, GT, PHASED, FACE, COMPACT, BLOB, SCORE, WOVR><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, na);
+    if (int rc = set_smem(shade_bwd_kernel<NA, GT, PHASED, TEX, COMPACT, BLOB, SCORE, WOVR>, smem)) return rc;
+    shade_bwd_kernel<NA, GT, PHASED, TEX, COMPACT, BLOB, SCORE, WOVR><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, na, a.tex);
     return (int)cudaGetLastError();
 }
+// dense per-logit arrays.  A sampled texture runs with lanes per pixel read at run time (GT = 0): these launches serve the
+// explicit-noise, Cauchy and no-control-variate calls and calls without a work list
 template <class NA, int GT, bool PHASED, int SCORE = 0, bool WOVR = false>
-static int launch_bwd_t(const BwdArgs& a, const NA& na, cudaStream_t st) {
-    return a.pb.face_colors ? launch_bwd_f<NA, GT, PHASED, true, false, false, SCORE, WOVR>(a, na, st)
-                            : launch_bwd_f<NA, GT, PHASED, false, false, false, SCORE, WOVR>(a, na, st);
+static int launch_bwd_t(const BwdLaunch& a, const NA& na, cudaStream_t st) {
+    if constexpr (GT == 0) {
+        switch (a.tex.kind) {
+            case TX_VERT: return launch_bwd_f<NA, 0, PHASED, TX_VERT, false, false, SCORE, WOVR>(a, na, st);
+            case TX_UV: return launch_bwd_f<NA, 0, PHASED, TX_UV, false, false, SCORE, WOVR>(a, na, st);
+            case TX_ATLAS: return launch_bwd_f<NA, 0, PHASED, TX_ATLAS, false, false, SCORE, WOVR>(a, na, st);
+            default: break;
+        }
+    } else {
+        if (a.tex.kind != TX_DENSE) return launch_bwd_t<NA, 0, PHASED, SCORE, WOVR>(a, na, st);
+    }
+    return a.pb.face_colors ? launch_bwd_f<NA, GT, PHASED, TX_FACE, false, false, SCORE, WOVR>(a, na, st)
+                            : launch_bwd_f<NA, GT, PHASED, TX_DENSE, false, false, SCORE, WOVR>(a, na, st);
 }
 // sparse-first main pass (compact per-logit arrays); PN = the Philox variant
-template <class PN, int GT>
-static int launch_bwd_c(const BwdArgs& a, const PN& na, cudaStream_t st) {
+template <class PN, int GT, int TEX>
+static int launch_bwd_c_t(const BwdLaunch& a, const PN& na, cudaStream_t st) {
     if (a.blob) {  // forward left tile blobs: no re-scan, no logit recomputation (the common geometries only)
-        if constexpr (GT == 2 || GT == 4) {
-            return a.pb.face_colors ? launch_bwd_f<PN, GT, false, true, true, true>(a, na, st)
-                                    : launch_bwd_f<PN, GT, false, false, true, true>(a, na, st);
-        }
+        if constexpr (GT == 2 || GT == 4) return launch_bwd_f<PN, GT, false, TEX, true, true>(a, na, st);
     }
-    return a.pb.face_colors ? launch_bwd_f<PN, GT, false, true, true>(a, na, st)
-                            : launch_bwd_f<PN, GT, false, false, true>(a, na, st);
+    return launch_bwd_f<PN, GT, false, TEX, true>(a, na, st);
 }
-template <class PN, int GT, bool FACE, bool BLOB>
-static int launch_bwd_fb_b(const BwdArgs& a, const PN& na, int64_t prow0, cudaStream_t st) {
+template <class PN, int GT>
+static int launch_bwd_c(const BwdLaunch& a, const PN& na, cudaStream_t st) {
+    switch (a.tex.kind) {
+        case TX_VERT: return launch_bwd_c_t<PN, GT, TX_VERT>(a, na, st);
+        case TX_UV: return launch_bwd_c_t<PN, GT, TX_UV>(a, na, st);
+        case TX_ATLAS: return launch_bwd_c_t<PN, GT, TX_ATLAS>(a, na, st);
+        default: return a.pb.face_colors ? launch_bwd_c_t<PN, GT, TX_FACE>(a, na, st) : launch_bwd_c_t<PN, GT, TX_DENSE>(a, na, st);
+    }
+}
+template <class PN, int GT, int TEX, bool BLOB>
+static int launch_bwd_fb_b(const BwdLaunch& a, const PN& na, int64_t prow0, cudaStream_t st) {
     const size_t smem = (size_t)a.L.warp_smem * (FBT / 32);
-    if (int rc = set_smem(shade_bwd_fallback_kernel<PN, GT, FACE, BLOB>, smem)) return rc;
-    shade_bwd_fallback_kernel<PN, GT, FACE, BLOB>
-        <<<resident_grid(shade_bwd_fallback_kernel<PN, GT, FACE, BLOB>, FBT, smem), FBT, smem, st>>>(a, na, prow0);
+    if (int rc = set_smem(shade_bwd_fallback_kernel<PN, GT, TEX, BLOB>, smem)) return rc;
+    shade_bwd_fallback_kernel<PN, GT, TEX, BLOB>
+        <<<resident_grid(shade_bwd_fallback_kernel<PN, GT, TEX, BLOB>, FBT, smem), FBT, smem, st>>>(a, na, prow0, a.tex);
     return (int)cudaGetLastError();
 }
-template <class PN, int GT, bool FACE>
-static int launch_bwd_fb(const BwdArgs& a, const PN& na, int64_t prow0, cudaStream_t st) {
-    return a.blob ? launch_bwd_fb_b<PN, GT, FACE, true>(a, na, prow0, st) : launch_bwd_fb_b<PN, GT, FACE, false>(a, na, prow0, st);
+template <class PN, int GT, int TEX>
+static int launch_bwd_fb(const BwdLaunch& a, const PN& na, int64_t prow0, cudaStream_t st) {
+    return a.blob ? launch_bwd_fb_b<PN, GT, TEX, true>(a, na, prow0, st) : launch_bwd_fb_b<PN, GT, TEX, false>(a, na, prow0, st);
 }
 
 // both phases in one launch, in-kernel noise
 template <class PN>
-static int launch_bwd_production(const BwdArgs& a, const BwdArgs* fb, cudaStream_t st) {
+static int launch_bwd_production(const BwdLaunch& a, const BwdLaunch* fb, cudaStream_t st) {
     const PN pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
     int rc;
     if (fb) {  // sparse-first: compact main pass, then half-size tiles for whatever did not fit
@@ -778,12 +816,19 @@ static int launch_bwd_production(const BwdArgs& a, const BwdArgs* fb, cudaStream
             default: rc = launch_bwd_c<PN, 8>(a, pa, st); break;
         }
         if (rc) return rc;
+        // a sampled texture's fallback pass reads the lanes per pixel at run time (it is empty on real, sparse fragments)
+        switch (a.tex.kind) {
+            case TX_VERT: return launch_bwd_fb<PN, 0, TX_VERT>(*fb, pa, a.L.ntiles, st);
+            case TX_UV: return launch_bwd_fb<PN, 0, TX_UV>(*fb, pa, a.L.ntiles, st);
+            case TX_ATLAS: return launch_bwd_fb<PN, 0, TX_ATLAS>(*fb, pa, a.L.ntiles, st);
+            default: break;
+        }
         const bool face = a.pb.face_colors != nullptr;
         switch (fb->L.G) {
-            case 2: return face ? launch_bwd_fb<PN, 2, true>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 2, false>(*fb, pa, a.L.ntiles, st);
-            case 4: return face ? launch_bwd_fb<PN, 4, true>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 4, false>(*fb, pa, a.L.ntiles, st);
-            case 8: return face ? launch_bwd_fb<PN, 8, true>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 8, false>(*fb, pa, a.L.ntiles, st);
-            default: return face ? launch_bwd_fb<PN, 16, true>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 16, false>(*fb, pa, a.L.ntiles, st);
+            case 2: return face ? launch_bwd_fb<PN, 2, TX_FACE>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 2, TX_DENSE>(*fb, pa, a.L.ntiles, st);
+            case 4: return face ? launch_bwd_fb<PN, 4, TX_FACE>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 4, TX_DENSE>(*fb, pa, a.L.ntiles, st);
+            case 8: return face ? launch_bwd_fb<PN, 8, TX_FACE>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 8, TX_DENSE>(*fb, pa, a.L.ntiles, st);
+            default: return face ? launch_bwd_fb<PN, 16, TX_FACE>(*fb, pa, a.L.ntiles, st) : launch_bwd_fb<PN, 16, TX_DENSE>(*fb, pa, a.L.ntiles, st);
         }
     }
     switch (a.L.G) {  // lanes per pixel known at compile time
@@ -794,7 +839,7 @@ static int launch_bwd_production(const BwdArgs& a, const BwdArgs* fb, cudaStream
     }
 }
 
-int launch_shade_bwd(const BwdArgs& a, const BwdArgs* fb, float* grad_scalars, cudaStream_t st) {
+int launch_shade_bwd(const BwdLaunch& a, const BwdLaunch* fb, float* grad_scalars, cudaStream_t st) {
     int rc;
     const uint32_t both = PERT_PH_BWD_SAMPLE | PERT_PH_BWD_FINISH;
     const bool phased = (a.pb.flags & both) != both || a.hist != nullptr;

@@ -11,6 +11,7 @@
 //   3  perturbed argmax samples over (pixel, sample-quad) items -> winners, histogram
 //   4  blend -> image; per-pixel state (a0, active) for backward
 #include "kernels.h"
+#include "texel.cuh"
 #include "tile.cuh"
 
 namespace pert {
@@ -60,10 +61,13 @@ constexpr int kCmpMin = 12;
 // Fallback records (common.cuh; training with a tile blob, a.blob then points at the records region): the coverage launch
 // stores the half-tile's valid list; REC = true (aggregation launch) loads it instead of re-scanning pix_to_face and stores
 // what backward would recompute, the per-pixel logit summary and zeta.
+// TEX = the texel source (kernels.h): TX_DENSE reads pb.colors or, when set, pb.face_colors (a run-time choice); TX_VERT,
+// TX_UV and TX_ATLAS sample a.tex at the entries the blend weighs (texel.cuh), so no colour tensor exists.
 template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER = false, int CPH = 0x70, int SCORE = 0,
-          bool WOVR = false, bool RENDER = false, bool REC = false>
+          bool WOVR = false, bool RENDER = false, bool REC = false, int TEX = TX_DENSE>
 __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& noise_r, const NoiseA& noise_a,
-                                               const int64_t tile, unsigned char* smem_raw, const int lane) {
+                                               const int64_t tile, unsigned char* smem_raw, const int lane,
+                                               const TexArgs& tx) {
     const pert_problem& pb = a.pb;
     const int G = GT ? GT : a.L.G;
     const int gshift = GT ? (GT == 16 ? 4 : GT == 8 ? 3 : GT == 4 ? 2 : GT == 2 ? 1 : 0) : a.L.gshift;
@@ -167,7 +171,8 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
             const int e = vlist[n];
             if (do_agg || do_blend) {
                 zs[n] = __ldg(zbuf_t + e);
-                if (!pb.face_colors) prefetch_l1(pb.colors + (g0 + e) * 3);  // blended at the very end of the tile
+                if constexpr (TEX != TX_DENSE) prefetch_l1(tx.bary + (g0 + e) * 3);  // sampled at the very end of the tile
+                else if (!pb.face_colors) prefetch_l1(pb.colors + (g0 + e) * 3);  // blended at the very end of the tile
             }
             if (do_rast) {
                 const float x = -__ldg(dists_t + e);
@@ -434,10 +439,18 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
                 const float w = (float)hcount / fS;
                 const int j = lj[lb + l];
                 if (j < K) {
-                    const float* c = fcol ? fcol + 3 * (int)__ldg(p2f_p + j) : colors_p + j * 3;
-                    r += w * __ldg(c);
-                    g += w * __ldg(c + 1);
-                    bl += w * __ldg(c + 2);
+                    if constexpr (TEX != TX_DENSE) {  // the texel of entry j, sampled here
+                        const int64_t e = gp * K + j;
+                        const V3 c = tex_texel<TEX>(tx, a.L.HW * K, e, __ldg(p2f_p + j), ld3(tx.bary + e * 3));
+                        r += w * c.x;
+                        g += w * c.y;
+                        bl += w * c.z;
+                    } else {
+                        const float* c = fcol ? fcol + 3 * (int)__ldg(p2f_p + j) : colors_p + j * 3;
+                        r += w * __ldg(c);
+                        g += w * __ldg(c + 1);
+                        bl += w * __ldg(c + 2);
+                    }
                 } else {
                     r += w * pb.background[0];
                     g += w * pb.background[1];
@@ -455,10 +468,18 @@ __device__ __forceinline__ void shade_fwd_tile(const FwdArgs& a, const NoiseR& n
             if (hcount > 0) {
                 const float w = (float)hcount / fS;
                 if (j < K) {
-                    const float* c = fcol ? fcol + 3 * (int)__ldg(p2f_p + j) : colors_p + j * 3;
-                    r += w * __ldg(c);
-                    g += w * __ldg(c + 1);
-                    bl += w * __ldg(c + 2);
+                    if constexpr (TEX != TX_DENSE) {  // the texel of entry j, sampled here
+                        const int64_t e = gp * K + j;
+                        const V3 c = tex_texel<TEX>(tx, a.L.HW * K, e, __ldg(p2f_p + j), ld3(tx.bary + e * 3));
+                        r += w * c.x;
+                        g += w * c.y;
+                        bl += w * c.z;
+                    } else {
+                        const float* c = fcol ? fcol + 3 * (int)__ldg(p2f_p + j) : colors_p + j * 3;
+                        r += w * __ldg(c);
+                        g += w * __ldg(c + 1);
+                        bl += w * __ldg(c + 2);
+                    }
                 } else {
                     r += w * pb.background[0];
                     g += w * pb.background[1];
@@ -481,9 +502,9 @@ constexpr int fwd_min_ctas(int score, bool wovr, bool render, bool phased) {
     return (score || wovr || (render && phased)) ? 24 : render ? 28 : 32;
 }
 
-template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER, int SCORE, bool WOVR, bool RENDER>
+template <class NoiseR, class NoiseA, int GT, bool PHASED, bool DEFER, int SCORE, bool WOVR, bool RENDER, int TEX = TX_DENSE>
 __global__ void __launch_bounds__(FNT, fwd_min_ctas(SCORE, WOVR, RENDER, PHASED))
-    shade_fwd_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a) {
+    shade_fwd_kernel(const FwdArgs a, const NoiseR noise_r, const NoiseA noise_a, const TexArgs tex) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     NoiseR nr = noise_r;
     NoiseA na = noise_a;
@@ -491,7 +512,7 @@ __global__ void __launch_bounds__(FNT, fwd_min_ctas(SCORE, WOVR, RENDER, PHASED)
         nr.mix(__ldg(a.pb.seed_device));
         na.mix(__ldg(a.pb.seed_device + 1));
     }
-    shade_fwd_tile<NoiseR, NoiseA, GT, PHASED, DEFER, 0x70, SCORE, WOVR, RENDER>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x);
+    shade_fwd_tile<NoiseR, NoiseA, GT, PHASED, DEFER, 0x70, SCORE, WOVR, RENDER, false, TEX>(a, nr, na, blockIdx.x, smem_raw, threadIdx.x, tex);
 }
 
 // Fallback pass of the sparse-first mode: the tiles whose valid entries did not fit the compact arrays,
@@ -502,8 +523,9 @@ __global__ void __launch_bounds__(FNT, fwd_min_ctas(SCORE, WOVR, RENDER, PHASED)
 // the coverage-sample launch makes room for them -- were measured at -1 % / 0 %: the passes are bound by the FMA and ALU
 // pipes, not by latency; profiles/r2_notes.md)
 constexpr int FB_MIN_CTAS = 12;
-template <class PN, int GT, int CPH, bool RENDER, bool REC>
-__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(const FwdArgs a, const PN noise_r, const PN noise_a) {
+template <class PN, int GT, int CPH, bool RENDER, bool REC, int TEX = TX_DENSE>
+__global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(const FwdArgs a, const PN noise_r, const PN noise_a,
+                                                                               const TexArgs tex) {
     extern __shared__ __align__(16) unsigned char smem_all[];
     // FBT/32 independent warps per CTA; the coverage-sample launch carries the front of the layout only
     unsigned char* smem_raw = smem_all + (threadIdx.x >> 5) * (CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem);
@@ -523,71 +545,77 @@ __global__ void __launch_bounds__(FBT, FB_MIN_CTAS) shade_fwd_fallback_kernel(co
         if (i >= n) break;
         const int64_t tile = (int64_t)a.worklist[4 + (i >> 1)] * 2 + (i & 1);
         if (tile < a.L.ntiles)
-            shade_fwd_tile<PN, PN, GT, false, false, CPH, 0, false, RENDER, REC>(a, nr, na, tile, smem_raw, threadIdx.x & 31);
+            shade_fwd_tile<PN, PN, GT, false, false, CPH, 0, false, RENDER, REC, TEX>(a, nr, na, tile, smem_raw, threadIdx.x & 31, tex);
         __syncwarp();
     }
 }
 
-template <class NR, class NA, int GT, bool PHASED, bool DEFER, int SCORE, bool WOVR, bool RENDER>
-static int launch_t(const FwdArgs& a, const NR& nr, const NA& na, cudaStream_t st) {
+template <class NR, class NA, int GT, bool PHASED, bool DEFER, int SCORE, bool WOVR, bool RENDER, int TEX>
+static int launch_t(const FwdLaunch& a, const NR& nr, const NA& na, cudaStream_t st) {
     const size_t smem = (size_t)a.L.warp_smem;
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR, RENDER>,
+        cudaError_t e = cudaFuncSetAttribute(shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR, RENDER, TEX>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
-    shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR, RENDER><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na);
+    shade_fwd_kernel<NR, NA, GT, PHASED, DEFER, SCORE, WOVR, RENDER, TEX><<<(unsigned)a.L.ntiles, FNT, smem, st>>>(a, nr, na, a.tex);
     return (int)cudaGetLastError();
 }
 
-template <class PN, int GT, int CPH, bool RENDER, bool REC = false>
-static int launch_fallback_ph(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
+template <class PN, int GT, int CPH, bool RENDER, int TEX, bool REC = false>
+static int launch_fallback_ph(const FwdLaunch& a, const PN& nr, const PN& na, cudaStream_t st) {
     const size_t smem = (size_t)(CPH == (int)PERT_PH_RAST ? a.L.warp_smem_rast : a.L.warp_smem) * (FBT / 32);
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC>,
+        cudaError_t e = cudaFuncSetAttribute(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC, TEX>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
-    shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC>
-        <<<resident_grid(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC>, FBT, smem), FBT, smem, st>>>(a, nr, na);
+    shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC, TEX>
+        <<<resident_grid(shade_fwd_fallback_kernel<PN, GT, CPH, RENDER, REC, TEX>, FBT, smem), FBT, smem, st>>>(a, nr, na, a.tex);
     return (int)cudaGetLastError();
 }
 
 // with a tile blob (training) the aggregation launch takes the valid lists from the fallback records
-template <class PN, int GT, bool RENDER>
-static int launch_fallback(const FwdArgs& a, const PN& nr, const PN& na, cudaStream_t st) {
-    const int rc = launch_fallback_ph<PN, GT, PERT_PH_RAST, RENDER>(a, nr, na, st);
+template <class PN, int GT, bool RENDER, int TEX>
+static int launch_fallback(const FwdLaunch& a, const PN& nr, const PN& na, cudaStream_t st) {
+    const int rc = launch_fallback_ph<PN, GT, PERT_PH_RAST, RENDER, TEX>(a, nr, na, st);
     if (rc) return rc;
     if constexpr (!RENDER) {
-        if (a.blob) return launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, false, true>(a, nr, na, st);
+        if (a.blob) return launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, false, TEX, true>(a, nr, na, st);
     }
-    return launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, RENDER>(a, nr, na, st);
+    return launch_fallback_ph<PN, GT, PERT_PH_AGG | PERT_PH_BLEND, RENDER, TEX>(a, nr, na, st);
 }
 
 // all phases in one launch, lanes per pixel known at compile time
-template <class PN, bool DEFER, bool RENDER>
-static int launch_main(const FwdArgs& a, const PN& pr, const PN& pa, cudaStream_t st) {
+template <class PN, bool DEFER, bool RENDER, int TEX>
+static int launch_main(const FwdLaunch& a, const PN& pr, const PN& pa, cudaStream_t st) {
     switch (a.L.G) {
-        case 1: return launch_t<PN, PN, 1, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
-        case 2: return launch_t<PN, PN, 2, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
-        case 4: return launch_t<PN, PN, 4, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
-        default: return launch_t<PN, PN, 8, false, DEFER, 0, false, RENDER>(a, pr, pa, st);
+        case 1: return launch_t<PN, PN, 1, false, DEFER, 0, false, RENDER, TEX>(a, pr, pa, st);
+        case 2: return launch_t<PN, PN, 2, false, DEFER, 0, false, RENDER, TEX>(a, pr, pa, st);
+        case 4: return launch_t<PN, PN, 4, false, DEFER, 0, false, RENDER, TEX>(a, pr, pa, st);
+        default: return launch_t<PN, PN, 8, false, DEFER, 0, false, RENDER, TEX>(a, pr, pa, st);
     }
 }
 
 // production path (in-kernel Gaussian noise in both stages, all phases in one launch); PN = the Philox variant
-template <class PN, bool RENDER>
-static int launch_production(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
+template <class PN, bool RENDER, int TEX>
+static int launch_production(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st) {
     const PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
-    if (!fb) return launch_main<PN, false, RENDER>(a, pr, pa, st);
+    if (!fb) return launch_main<PN, false, RENDER, TEX>(a, pr, pa, st);
     // sparse-first main pass: defers the tiles the compound sampler is worth running on
-    const int rc = launch_main<PN, true, RENDER>(a, pr, pa, st);
+    const int rc = launch_main<PN, true, RENDER, TEX>(a, pr, pa, st);
     if (rc) return rc;
-    switch (fb->L.G) {  // sparse-first mode: half-size tiles for whatever did not fit
-        case 2: return launch_fallback<PN, 2, RENDER>(*fb, pr, pa, st);
-        case 4: return launch_fallback<PN, 4, RENDER>(*fb, pr, pa, st);
-        case 8: return launch_fallback<PN, 8, RENDER>(*fb, pr, pa, st);
-        default: return launch_fallback<PN, 16, RENDER>(*fb, pr, pa, st);
+    // the fallback pass of a sampled texture runs with lanes per pixel read at run time (one instantiation per launch
+    // instead of four: it is empty on real, sparse fragments)
+    if constexpr (TEX != TX_DENSE) {
+        return launch_fallback<PN, 0, RENDER, TEX>(*fb, pr, pa, st);
+    } else {
+        switch (fb->L.G) {  // sparse-first mode: half-size tiles for whatever did not fit
+            case 2: return launch_fallback<PN, 2, RENDER, TEX>(*fb, pr, pa, st);
+            case 4: return launch_fallback<PN, 4, RENDER, TEX>(*fb, pr, pa, st);
+            case 8: return launch_fallback<PN, 8, RENDER, TEX>(*fb, pr, pa, st);
+            default: return launch_fallback<PN, 16, RENDER, TEX>(*fb, pr, pa, st);
+        }
     }
 }
 
@@ -600,46 +628,76 @@ static int launch_production(const FwdArgs& a, const FwdArgs* fb, cudaStream_t s
 // it, entries with x < -sigma*Umax and logits that cannot win.  In-kernel Gaussian noise runs the production kernels, or in
 // training the phase-split ones of the sample-sharded job.  PHASED: the instantiations carry the phase-split code; always in
 // training, in the render only for the phase calls of pert_shade_render_phase.
-template <class PN, int SCORE, bool WOVR, bool RENDER, bool PHASED = !RENDER>
-static int launch_pair(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
+template <class PN, int SCORE, bool WOVR, bool RENDER, int TEX, bool PHASED = !RENDER>
+static int launch_pair(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st) {
     const bool er = a.pb.noise_rast != nullptr, ea = a.pb.noise_agg != nullptr;
     PN pr(a.pb.seed_rast, 0, a.pb.pixel_offset), pa(a.pb.seed_agg, 1, a.pb.pixel_offset);
     ExplicitNoise xr{a.pb.noise_rast, a.L.P, a.pb.K, a.pb.S_rast}, xa{a.pb.noise_agg, a.L.P, a.pb.K + 1, a.pb.S_agg};
-    if (er && ea) return launch_t<ExplicitNoise, ExplicitNoise, 0, PHASED, false, SCORE, WOVR, RENDER>(a, xr, xa, st);
-    if (er) return launch_t<ExplicitNoise, PN, 0, PHASED, false, SCORE, WOVR, RENDER>(a, xr, pa, st);
-    if (ea) return launch_t<PN, ExplicitNoise, 0, PHASED, false, SCORE, WOVR, RENDER>(a, pr, xa, st);
+    if (er && ea) return launch_t<ExplicitNoise, ExplicitNoise, 0, PHASED, false, SCORE, WOVR, RENDER, TEX>(a, xr, xa, st);
+    if (er) return launch_t<ExplicitNoise, PN, 0, PHASED, false, SCORE, WOVR, RENDER, TEX>(a, xr, pa, st);
+    if (ea) return launch_t<PN, ExplicitNoise, 0, PHASED, false, SCORE, WOVR, RENDER, TEX>(a, pr, xa, st);
     if constexpr (SCORE || WOVR) {
-        return launch_t<PN, PN, 0, PHASED, false, SCORE, WOVR, RENDER>(a, pr, pa, st);
+        return launch_t<PN, PN, 0, PHASED, false, SCORE, WOVR, RENDER, TEX>(a, pr, pa, st);
     } else {
         if constexpr (PHASED) {
             const uint32_t all = PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND;
             if ((a.pb.flags & all) != all || a.hist != nullptr) {  // compile-time lanes per pixel for the benchmark geometries
-                switch (a.L.G) {
-                    case 4: return launch_t<PN, PN, 4, true, false, 0, false, RENDER>(a, pr, pa, st);
-                    case 8: return launch_t<PN, PN, 8, true, false, 0, false, RENDER>(a, pr, pa, st);
-                    default: return launch_t<PN, PN, 0, true, false, 0, false, RENDER>(a, pr, pa, st);
+                if constexpr (TEX != TX_DENSE) {  // a sampled texture: lanes per pixel read at run time
+                    return launch_t<PN, PN, 0, true, false, 0, false, RENDER, TEX>(a, pr, pa, st);
+                } else {
+                    switch (a.L.G) {
+                        case 4: return launch_t<PN, PN, 4, true, false, 0, false, RENDER, TEX>(a, pr, pa, st);
+                        case 8: return launch_t<PN, PN, 8, true, false, 0, false, RENDER, TEX>(a, pr, pa, st);
+                        default: return launch_t<PN, PN, 0, true, false, 0, false, RENDER, TEX>(a, pr, pa, st);
+                    }
                 }
             }
         }
-        return (a.pb.flags & PERT_F_PHILOX7) ? launch_production<PhiloxNoise7, RENDER>(a, fb, st)
-                                             : launch_production<PhiloxNoise, RENDER>(a, fb, st);
+        return (a.pb.flags & PERT_F_PHILOX7) ? launch_production<PhiloxNoise7, RENDER, TEX>(a, fb, st)
+                                             : launch_production<PhiloxNoise, RENDER, TEX>(a, fb, st);
     }
 }
 
-int launch_shade_fwd(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    if (a.pb.flags & PERT_F_CAUCHY) return launch_pair<PhiloxCauchy, 1, false, false>(a, fb, st);
-    if (a.pb.flags & PERT_F_NO_VR) return launch_pair<PhiloxNoise, 0, true, false>(a, fb, st);
-    return launch_pair<PhiloxNoise, 0, false, false>(a, fb, st);
+template <int TEX>
+static int launch_shade_fwd_t(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st) {
+    if (a.pb.flags & PERT_F_CAUCHY) return launch_pair<PhiloxCauchy, 1, false, false, TEX>(a, fb, st);
+    if (a.pb.flags & PERT_F_NO_VR) return launch_pair<PhiloxNoise, 0, true, false, TEX>(a, fb, st);
+    return launch_pair<PhiloxNoise, 0, false, false, TEX>(a, fb, st);
+}
+
+int launch_shade_fwd(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st) {
+    switch (a.tex.kind) {
+        case TX_VERT: return launch_shade_fwd_t<TX_VERT>(a, fb, st);
+        case TX_UV: return launch_shade_fwd_t<TX_UV>(a, fb, st);
+        case TX_ATLAS: return launch_shade_fwd_t<TX_ATLAS>(a, fb, st);
+        default: return launch_shade_fwd_t<TX_DENSE>(a, fb, st);
+    }
 }
 
 // The forward with RENDER = true (shade_fwd_tile): nothing saved for backward.  A single call runs the single-call
 // instantiations; a call with a phase bit (pert_shade_render_phase: exactly one) the phase-split ones.  The pair without
 // control variates renders on the Gaussian per-sample path (cabi.cu), whose counts, histogram and image it shares.
-int launch_shade_render(const FwdArgs& a, const FwdArgs* fb, cudaStream_t st) {
-    const bool phased = (a.pb.flags & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND)) != 0;
-    if (a.pb.flags & PERT_F_CAUCHY)
-        return phased ? launch_pair<PhiloxCauchy, 1, false, true, true>(a, fb, st) : launch_pair<PhiloxCauchy, 1, false, true>(a, fb, st);
-    return phased ? launch_pair<PhiloxNoise, 0, false, true, true>(a, fb, st) : launch_pair<PhiloxNoise, 0, false, true>(a, fb, st);
+// A sampled texture (TEX != TX_DENSE) renders single calls only (pert_shade_tex_render).
+template <int TEX>
+static int launch_shade_render_t(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st) {
+    if constexpr (TEX == TX_DENSE) {
+        const bool phased = (a.pb.flags & (PERT_PH_RAST | PERT_PH_AGG | PERT_PH_BLEND)) != 0;
+        if (a.pb.flags & PERT_F_CAUCHY)
+            return phased ? launch_pair<PhiloxCauchy, 1, false, true, TEX, true>(a, fb, st) : launch_pair<PhiloxCauchy, 1, false, true, TEX>(a, fb, st);
+        return phased ? launch_pair<PhiloxNoise, 0, false, true, TEX, true>(a, fb, st) : launch_pair<PhiloxNoise, 0, false, true, TEX>(a, fb, st);
+    } else {
+        if (a.pb.flags & PERT_F_CAUCHY) return launch_pair<PhiloxCauchy, 1, false, true, TEX>(a, fb, st);
+        return launch_pair<PhiloxNoise, 0, false, true, TEX>(a, fb, st);
+    }
+}
+
+int launch_shade_render(const FwdLaunch& a, const FwdLaunch* fb, cudaStream_t st) {
+    switch (a.tex.kind) {
+        case TX_VERT: return launch_shade_render_t<TX_VERT>(a, fb, st);
+        case TX_UV: return launch_shade_render_t<TX_UV>(a, fb, st);
+        case TX_ATLAS: return launch_shade_render_t<TX_ATLAS>(a, fb, st);
+        default: return launch_shade_render_t<TX_DENSE>(a, fb, st);
+    }
 }
 
 }  // namespace pert

@@ -16,7 +16,7 @@ import torch
 
 from . import _cabi
 from ._cabi import (F_CAUCHY, F_GUMBEL, F_NO_SKIP, F_NO_VR, F_PHILOX7, F_UNIFORM, F_PER_SAMPLE_NOISE, F_SKIP_DEAD_NOISE, PH_AGG, PH_BLEND, PH_BWD_FINISH, PH_BWD_SAMPLE, PH_RAST,
-                    PertProblem, check, ptr, require_cuda, stream_ptr)
+                    TEX_ATLAS, TEX_UV, TEX_VERTEX, PertProblem, PertTexture, check, ptr, require_cuda, stream_ptr)
 
 _tls = threading.local()
 
@@ -107,6 +107,52 @@ def depth_plane(v, N, device):
 
 
 @dataclass
+class ShadeTexture:
+    """A texture the fused kernels sample themselves (``pert_texture``): the colour of entry (n,h,w,k) is computed from
+    ``bary[n,h,w,k]`` and a per-face table where the kernels blend it, and no (N,H,W,K,3) colour tensor exists.
+    ``kind``: "vert" (``table`` (F,3,3) corner colours), "uv" (``table`` (M,Hm,Wm,3) maps, M = 1 or N, ``face_uvs``
+    (F,3,2)) or "atlas" (``table`` (F,R,R,3)).  ``bary`` (N,H,W,K,3) is ``fragments.bary_coords``."""
+    kind: str
+    bary: torch.Tensor
+    table: torch.Tensor
+    face_uvs: Optional[torch.Tensor] = None
+
+    _KINDS = {"vert": TEX_VERTEX, "uv": TEX_UV, "atlas": TEX_ATLAS}
+
+    def __post_init__(self):
+        if self.kind not in self._KINDS:
+            raise ValueError(f"texture kind must be one of {sorted(self._KINDS)}, got {self.kind!r}")
+        require_cuda(self.bary, self.table, self.face_uvs)
+        self.bary, self.table = _f32c(self.bary.detach()), _f32c(self.table.detach())
+        if self.face_uvs is not None:
+            self.face_uvs = _f32c(self.face_uvs.detach())
+        t = self.table
+        if self.kind == "vert" and (t.dim() != 3 or tuple(t.shape[1:]) != (3, 3)):
+            raise ValueError("vertex colours must be (F,3,3)")
+        if self.kind == "uv" and (t.dim() != 4 or t.shape[3] != 3 or self.face_uvs is None or self.face_uvs.dim() != 3
+                                  or tuple(self.face_uvs.shape[1:]) != (3, 2)):
+            raise ValueError("a UV texture needs maps (M,Hm,Wm,3) and face_uvs (F,3,2)")
+        if self.kind == "atlas" and (t.dim() != 4 or t.shape[1] != t.shape[2] or t.shape[3] != 3):
+            raise ValueError("an atlas must be (F,R,R,3)")
+
+    @property
+    def num_faces(self) -> int:
+        return self.face_uvs.shape[0] if self.kind == "uv" else self.table.shape[0]
+
+    def c_struct(self) -> PertTexture:
+        tx = PertTexture()
+        tx.kind = self._KINDS[self.kind]
+        tx.bary, tx.table = self.bary.data_ptr(), self.table.data_ptr()
+        tx.num_faces = self.num_faces
+        if self.kind == "uv":
+            tx.face_uvs = self.face_uvs.data_ptr()
+            tx.map_count, tx.map_h, tx.map_w = self.table.shape[0], self.table.shape[1], self.table.shape[2]
+        if self.kind == "atlas":
+            tx.atlas_size = self.table.shape[1]
+        return tx
+
+
+@dataclass
 class ShadeProblem:
     """Everything a forward/backward pair shares.  Built once per forward call."""
     pix_to_face: torch.Tensor
@@ -132,6 +178,7 @@ class ShadeProblem:
     noise_agg: Optional[torch.Tensor] = None
     face_colors: Optional[torch.Tensor] = None  # (F,3): colours gathered through pix_to_face inside the kernels
     seed_device: Optional[torch.Tensor] = None  # int64 (2,) on the device: effective seeds = seed_* ^ seed_device (graphs)
+    texture: Optional[ShadeTexture] = None  # sampled inside the kernels (pert_shade_tex_*); colors / face_colors are then None
     _keep: list = field(default_factory=list)
 
     def __post_init__(self):
@@ -153,8 +200,13 @@ class ShadeProblem:
             self.face_colors = _f32c(self.face_colors.detach())
             if self.face_colors.dim() != 2 or self.face_colors.shape[1] != 3:
                 raise ValueError("face_colors must be (F,3)")
-        elif self.colors is None:
-            raise ValueError("either colors (N,H,W,K,3) or face_colors (F,3) is required")
+        elif self.colors is None and self.texture is None:
+            raise ValueError("one of colors (N,H,W,K,3), face_colors (F,3) or texture is required")
+        if self.texture is not None:
+            if self.colors is not None or self.face_colors is not None:
+                raise ValueError("a texture is the only colour source of its problem: colors and face_colors must be None")
+            if tuple(self.texture.bary.shape) != (N, H, W, K, 3):
+                raise ValueError("the texture's bary must be (N,H,W,K,3)")
         dev = self.pix_to_face.device
         self.znear = depth_plane(self.znear, N, dev)
         self.zfar = depth_plane(self.zfar, N, dev)
@@ -288,9 +340,13 @@ def shade_forward(pr: ShadeProblem, want_hist: bool = False, phases: int = 0, sa
         do_blend = (phases == 0) or bool(phases & PH_BLEND)
         image = torch.empty((N, H, W, 4), dtype=torch.float32, device=dev) if do_blend else None
         pb = pr.c_struct(flags=pr.flags | phases)
-        rc = lib.pert_shade_fwd(pb, ptr(image), ptr(saved.counts), ptr(saved.rsum), ptr(saved.winners),
-                                ptr(saved.pixstate), ptr(saved.hist), ptr(saved.worklist), ptr(saved.blob), stream_ptr(dev))
-    check(rc, "pert_shade_fwd")
+        args = (ptr(image), ptr(saved.counts), ptr(saved.rsum), ptr(saved.winners), ptr(saved.pixstate), ptr(saved.hist),
+                ptr(saved.worklist), ptr(saved.blob), stream_ptr(dev))
+        if pr.texture is not None:
+            rc = _cabi.shade_tex_fns()[0](pb, pr.texture.c_struct(), *args)
+        else:
+            rc = lib.pert_shade_fwd(pb, *args)
+    check(rc, "pert_shade_tex_fwd" if pr.texture is not None else "pert_shade_fwd")
     return image, saved
 
 
@@ -301,6 +357,7 @@ def shade_render(pr: ShadeProblem, return_worklist: bool = False):
     ``return_worklist``: return ``(image, worklist)``; word 0 of the work list is the number of tiles the fallback pass
     redid (None where the sparse-first mode does not run)."""
     fn = _cabi.shade_render_fn()
+    tex_fn = _cabi.shade_tex_fns()[2] if pr.texture is not None else None
     _cabi.require_fused_flags(pr.flags)
     if pr.s_rast != (0, pr.S_rast) or pr.s_agg != (0, pr.S_agg):
         raise ValueError("shade_render renders all samples in one call: the sample-sharded forward needs shade_forward")
@@ -311,8 +368,9 @@ def shade_render(pr: ShadeProblem, return_worklist: bool = False):
         worklist = torch.empty((4 + pr.num_tiles(),), dtype=torch.int32, device=dev) if sparse else None
         counts_ws = torch.empty((N, H, W, K), dtype=torch.int16, device=dev) if sparse else None
         image = torch.empty((N, H, W, 4), dtype=torch.float32, device=dev)
-        rc = fn(pr.c_struct(), ptr(image), ptr(counts_ws), ptr(worklist), stream_ptr(dev))
-    check(rc, "pert_shade_render")
+        args = (ptr(image), ptr(counts_ws), ptr(worklist), stream_ptr(dev))
+        rc = tex_fn(pr.c_struct(), pr.texture.c_struct(), *args) if tex_fn else fn(pr.c_struct(), *args)
+    check(rc, "pert_shade_tex_render" if tex_fn else "pert_shade_render")
     return (image, worklist) if return_worklist else image
 
 
@@ -334,8 +392,10 @@ def shade_render_phase(pr: ShadeProblem, phase: int, counts: torch.Tensor, hist:
 
 
 def shade_backward(pr: ShadeProblem, saved: ShadeSaved, grad_image: torch.Tensor, need_colors: bool = True,
-                   phases: int = 0, acc=None, pixstat=None, use_hist: bool = False):
-    """Launch pert_shade_bwd.  Returns (grad_dists, grad_zbuf, grad_colors | None, grad_scalars(3))."""
+                   phases: int = 0, acc=None, pixstat=None, use_hist: bool = False, need_bary: bool = False):
+    """Launch pert_shade_bwd.  Returns (grad_dists, grad_zbuf, grad_colors | None, grad_scalars(3)).  With ``pr.texture``
+    (pert_shade_tex_bwd) the third element is the pair (grad_table | None, grad_bary | None): the gradient of the texture's
+    table (``need_colors``) and of its ``bary`` (N,H,W,K,3) (``need_bary``; zero at the entries no sample picked)."""
     lib = _cabi.load()
     _cabi.require_fused_flags(pr.flags)
     N, H, W, K = pr.shape
@@ -346,19 +406,26 @@ def shade_backward(pr: ShadeProblem, saved: ShadeSaved, grad_image: torch.Tensor
         finish = (phases == 0) or bool(phases & PH_BWD_FINISH)
         gd = torch.empty((N, H, W, K), dtype=torch.float32, device=dev) if finish else None
         gz = torch.empty((N, H, W, K), dtype=torch.float32, device=dev) if finish else None
-        if pr.face_colors is not None:  # scatter target of the in-kernel gather: atomics into zeros
+        gb = None
+        if pr.texture is not None:  # scatter targets of the in-kernel sampling: atomics into zeros
+            gc = torch.zeros_like(pr.texture.table) if (finish and need_colors) else None
+            gb = torch.zeros_like(pr.texture.bary) if (finish and need_bary) else None
+        elif pr.face_colors is not None:  # scatter target of the in-kernel gather: atomics into zeros
             gc = torch.zeros_like(pr.face_colors) if (finish and need_colors) else None
         else:
             gc = torch.empty((N, H, W, K, 3), dtype=torch.float32, device=dev) if (finish and need_colors) else None
         partials = torch.empty((3 * pr.num_tiles(), 4), dtype=torch.float32, device=dev) if finish else None
         scal = torch.empty((3,), dtype=torch.float32, device=dev) if finish else None
         pb = pr.c_struct(flags=pr.flags | phases)
-        rc = lib.pert_shade_bwd(pb, ptr(grad_image), ptr(saved.counts), ptr(saved.rsum), ptr(saved.winners),
-                                ptr(saved.pixstate), ptr(gd), ptr(gz), ptr(gc), ptr(partials), ptr(scal), ptr(acc), ptr(pixstat),
-                                ptr(saved.hist) if use_hist else None, None if phases else ptr(saved.worklist),
-                                None if phases else ptr(saved.blob), stream_ptr(dev))
-    check(rc, "pert_shade_bwd")
-    return gd, gz, gc, scal
+        saved_in = (ptr(grad_image), ptr(saved.counts), ptr(saved.rsum), ptr(saved.winners), ptr(saved.pixstate), ptr(gd), ptr(gz))
+        rest = (ptr(partials), ptr(scal), ptr(acc), ptr(pixstat), ptr(saved.hist) if use_hist else None,
+                None if phases else ptr(saved.worklist), None if phases else ptr(saved.blob), stream_ptr(dev))
+        if pr.texture is not None:
+            rc = _cabi.shade_tex_fns()[1](pb, pr.texture.c_struct(), *saved_in, ptr(gc), ptr(gb), *rest)
+        else:
+            rc = lib.pert_shade_bwd(pb, *saved_in, ptr(gc), *rest)
+    check(rc, "pert_shade_tex_bwd" if pr.texture is not None else "pert_shade_bwd")
+    return gd, gz, (gc, gb) if pr.texture is not None else gc, scal
 
 
 # ---------------------------------------------------------------------------------------------

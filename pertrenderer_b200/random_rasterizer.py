@@ -6,7 +6,8 @@ unchanged.  With the (GaussianRast, GaussianAgg) pair, the Cauchy pair (ArctanRa
 without control variates (GaussianRast_wovr, GaussianAgg_wovr) the whole chain — coverage sampling, mask, alpha, logits, perturbed argmax, blend, and the score-function
 backward — is ONE forward and ONE backward sm_100a kernel (``pert_shade_fwd`` / ``pert_shade_bwd``).  A call made
 without gradients (``torch.no_grad`` / ``torch.inference_mode``) renders with ``pert_shade_render`` instead: the same
-image, nothing saved for backward, no buffer that grows with the sample counts.
+image, nothing saved for backward, no buffer that grows with the sample counts.  A CUDA ``VertexTexels`` / ``UVTexels`` /
+``AtlasTexels`` texture is sampled inside those kernels (``pert_shade_tex_*``): no (N,H,W,K,3) colour tensor is built.
 Any other operator pair falls through to the operator-by-operator composition of the reference, where
 the perturbed operators still run on their own CUDA kernels.
 """
@@ -33,11 +34,12 @@ def _background_tuple(blend_params):
     return bg
 
 
-def _perturbed_problem(colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg) -> ops.ShadeProblem:
+def _perturbed_problem(colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg, texture=None) -> ops.ShadeProblem:
     """The fused kernels' problem for one call of a perturbed pair, with its noise seeds drawn from torch's generator in
     the reference's order: coverage draw first (smoothrast.py:21), then the optional global reseed (smoothagg.py:18-19),
     then the aggregation draw (smoothagg.py:21).  The training forward and the forward-only render both build it here,
-    so that the same ``torch.manual_seed`` gives both the same noise."""
+    so that the same ``torch.manual_seed`` gives both the same noise.  ``texture`` (an ``ops.ShadeTexture``): the colour
+    source the kernels sample themselves; ``colors`` is then None."""
     noise_r, noise_a = ops.current_explicit_noise()
     seed_r = 0 if noise_r is not None else ops.draw_seed()
     if cfg["fixed_noise"]:
@@ -51,7 +53,7 @@ def _perturbed_problem(colors, dists, zbuf, sigma, gamma, alpha, pix_to_face, zn
         eps=float(cfg["eps"]), S_rast=int(cfg["S_rast"]), S_agg=int(cfg["S_agg"]),
         seed_rast=seed_r, seed_agg=seed_a, pixel_offset=int(cfg.get("pixel_offset", 0)),
         flags=ops.current_flags() | int(cfg.get("flags", 0)), noise_rast=noise_r, noise_agg=noise_a,
-        seed_device=None if (noise_r is not None or noise_a is not None) else ops.current_seed_device())
+        seed_device=None if (noise_r is not None or noise_a is not None) else ops.current_seed_device(), texture=texture)
 
 
 class _PerturbedShade(Function):
@@ -87,6 +89,56 @@ class _PerturbedShade(Function):
                     out_scal[i] = host[i].to(dtype=t.dtype).reshape(t.shape).to(t.device)
         return (gc if need[0] else None, gd if need[1] else None, gz if need[2] else None,
                 out_scal[0], out_scal[1], out_scal[2], None, None, None, None)
+
+
+class _PerturbedTexShade(Function):
+    """:class:`_PerturbedShade` with a texture the fused kernels sample themselves (``pert_shade_tex_fwd`` / ``_bwd``): the
+    (N,H,W,K,3) colour tensor and its gradient are never materialised.  Differentiable inputs: the texture's table
+    ((F,3,3) vertex colours, (M,Hm,Wm,3) maps or (F,R,R,3) atlas), ``bary`` (fragments.bary_coords), dists, zbuf and the
+    three scalars; ``face_uvs`` and ``kind`` are constants."""
+
+    @staticmethod
+    def forward(ctx, table, bary, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, face_uvs, kind, cfg):
+        tex = ops.ShadeTexture(kind=kind, bary=bary, table=table, face_uvs=face_uvs)
+        pr = _perturbed_problem(None, dists, zbuf, sigma, gamma, alpha, pix_to_face, znear, zfar, cfg, texture=tex)
+        image, saved = ops.shade_forward(pr)
+        ctx.pr, ctx.saved = pr, saved
+        ctx.scalars = (sigma, gamma, alpha)
+        ctx.save_for_backward(table, bary, dists, zbuf, pix_to_face)  # in-place edits before backward raise (see _PerturbedShade)
+        return image
+
+    @staticmethod
+    def backward(ctx, grad_image):
+        need = ctx.needs_input_grad
+        ctx.saved_tensors  # noqa: B018
+        # an atlas texel is piecewise constant in bary: its gradient is None (zero), nothing is allocated for it
+        gd, gz, (gt, gb), scal = ops.shade_backward(ctx.pr, ctx.saved, grad_image, need_colors=need[0],
+                                                    need_bary=need[1] and ctx.pr.texture.kind != "atlas")
+        out_scal = [None, None, None]
+        if any(need[4:7]):
+            host = scal.cpu()
+            for i, t in enumerate(ctx.scalars):
+                if need[4 + i] and torch.is_tensor(t):
+                    out_scal[i] = host[i].to(dtype=t.dtype).reshape(t.shape).to(t.device)
+        return (gt if need[0] else None, gb if need[1] else None, gd if need[2] else None, gz if need[3] else None,
+                out_scal[0], out_scal[1], out_scal[2], None, None, None, None, None, None)
+
+
+def _fused_texture(colors, fragments):
+    """(kind, table, face_uvs) of a lazy texture the fused perturbed kernels can sample themselves, or None (today's
+    materialising path): a CUDA VertexTexels / UVTexels / AtlasTexels with fragments.bary_coords."""
+    bary = fragments.bary_coords
+    if bary is None:
+        return None
+    if isinstance(colors, VertexTexels):
+        kind, table, face_uvs = "vert", colors.face_vert_colors(), None
+    elif isinstance(colors, UVTexels):
+        kind, table, face_uvs = "uv", colors.maps, colors.face_uvs()
+    else:
+        kind, table, face_uvs = "atlas", colors.atlas, None
+    if not all(t is None or t.is_cuda for t in (table, face_uvs, bary, fragments.pix_to_face)):
+        return None
+    return kind, table, face_uvs
 
 
 class _SoftShade(Function):
@@ -145,14 +197,29 @@ def smooth_rgb_blend(colors, fragments, smoothrast, smoothagg, blend_params, zne
 
     ``colors`` (N,H,W,K,3); ``fragments`` with ``pix_to_face`` / ``zbuf`` / ``dists`` (N,H,W,K);
     ``znear`` / ``zfar`` python floats or tensors broadcastable to (N,1,1,1)."""
+    flags = _perturbed_pair_flags(smoothrast, smoothagg)
     if isinstance(colors, (VertexTexels, UVTexels, AtlasTexels)):
-        # TexturesVertex / TexturesUV / TexturesAtlas: sample the texels with the texture-only mode of the Phong kernel; the
-        # fused pairs read colours of valid entries only, so the padded ones need not be written
+        tex = _fused_texture(colors, fragments) if flags is not None else None
+        if tex is not None:
+            # TexturesVertex / TexturesUV / TexturesAtlas with a perturbed pair: the fused kernels sample the texels where
+            # they blend them, and scatter the gradient into the table and bary_coords
+            ops.require_cuda(fragments.zbuf, fragments.dists)
+            kind, table, face_uvs = tex
+            cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps,
+                       S_rast=smoothrast.nb_samples, S_agg=smoothagg.nb_samples,
+                       fixed_noise=bool(smoothagg.fixed_noise), flags=flags)
+            args = (table, fragments.bary_coords, fragments.dists, fragments.zbuf, smoothrast.sigma, smoothagg.gamma,
+                    smoothagg.alpha, fragments.pix_to_face, znear, zfar, face_uvs, kind, cfg)
+            if not torch.is_grad_enabled():
+                return ops.shade_render(_perturbed_problem(None, *args[2:10], cfg, texture=ops.ShadeTexture(
+                    kind=kind, bary=fragments.bary_coords, table=table, face_uvs=face_uvs)))
+            return _PerturbedTexShade.apply(*args)
+        # otherwise sample the texels with the texture-only mode of the Phong kernel; the fused pairs read colours of
+        # valid entries only, so the padded ones need not be written
         from .shading import sample_lazy_textures
         colors = sample_lazy_textures(colors, fragments, sparse=_fused_pair(smoothrast, smoothagg))
     face = isinstance(colors, FaceTexels)
     ops.require_cuda(colors.face_colors if face else colors, fragments.pix_to_face, fragments.zbuf, fragments.dists)
-    flags = _perturbed_pair_flags(smoothrast, smoothagg)
     if flags is not None:
         cfg = dict(background=_background_tuple(blend_params), eps=smoothagg.eps,
                    S_rast=smoothrast.nb_samples, S_agg=smoothagg.nb_samples,
